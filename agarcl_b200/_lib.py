@@ -15,6 +15,7 @@ SYMBOLS = [
     "agarcl_make_layout", "agarcl_batch_create", "agarcl_batch_destroy", "agarcl_batch_get_layout",
     "agarcl_batch_seed", "agarcl_batch_reset", "agarcl_batch_set_actions", "agarcl_batch_step",
     "agarcl_batch_obs", "agarcl_batch_rewards", "agarcl_batch_dones", "agarcl_batch_step_host",
+    "agarcl_batch_reset_device", "agarcl_batch_set_autoreset", "agarcl_batch_step_autoreset", "agarcl_batch_episode",
     "agarcl_batch_mirror", "agarcl_batch_sync_mirror", "agarcl_batch_step_mirror", "agarcl_batch_mirror_stats", "agarcl_batch_mirror_timing", "agarcl_batch_step_lists", "agarcl_batch_lists_expand",
     "agarcl_batch_download_state", "agarcl_batch_upload_state", "agarcl_batch_save_env_state", "agarcl_batch_load_env_state",
     "agarcl_snapshot_write", "agarcl_snapshot_read", "agarcl_batch_set_replay",
@@ -48,6 +49,10 @@ def lib():
         L.agarcl_batch_rewards.argtypes = [_vp, C.POINTER(_vp)]
         L.agarcl_batch_dones.argtypes = [_vp, C.POINTER(_vp)]
         L.agarcl_batch_step_host.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp]
+        L.agarcl_batch_reset_device.argtypes = [_vp, _vp, _vp]
+        L.agarcl_batch_set_autoreset.argtypes = [_vp, C.c_int32, C.c_int32, C.c_int32]
+        L.agarcl_batch_step_autoreset.argtypes = [_vp, _vp]
+        L.agarcl_batch_episode.argtypes = [_vp, _vp]
         L.agarcl_batch_mirror.argtypes = [_vp, C.POINTER(_vp), C.POINTER(C.c_int64 * 4), C.POINTER(C.c_int32)]
         L.agarcl_batch_sync_mirror.argtypes = [_vp, _vp]
         L.agarcl_batch_step_mirror.argtypes = [_vp, _vp, _vp, _vp, _vp]

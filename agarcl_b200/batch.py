@@ -28,6 +28,11 @@ class _ObsListsStruct(C.Structure):
                [(n, C.c_uint32) for n in ("off_rec", "off_entries", "chunk_words")] + [("chunks", _vp), ("slot_of", _vp)]
 
 
+class _EpisodeStruct(C.Structure):
+    """struct agarcl_episode"""
+    _fields_ = [(n, _vp) for n in ("done_out", "reset_mask", "steps", "final_return", "final_length", "final_obs", "final_ram")]
+
+
 class ObsLists:
     """numpy view of the lists of the last Batch.step_lists (layout: include/agarcl_b200.h, agarcl_obs_lists)"""
 
@@ -145,6 +150,64 @@ class Batch:
         _lib.check(_lib.lib().agarcl_batch_reset(self._h, m.ctypes.data_as(_vp) if m is not None else None, _vp(stream)))
         if m is None:  # strict_reference: the player order of the new episode (quirk Q3)
             _lib.check(_lib.lib().agarcl_batch_get_layout(self._h, C.byref(self.layout)))
+
+    def reset_device(self, mask, stream=0):
+        """masked reset with a CUDA uint8 / bool tensor of N entries: read by the device, the host does not wait"""
+        import torch
+        dev = torch.device("cuda", self.cfg.device)
+        if not (isinstance(mask, torch.Tensor) and mask.is_cuda and mask.device == dev):
+            raise _lib.AgarclError(f"the reset mask must be a tensor on {dev}")
+        if mask.dtype not in (torch.uint8, torch.bool):
+            raise _lib.AgarclError(f"the reset mask must be uint8 or bool, got {mask.dtype}")
+        if not mask.is_contiguous() or mask.numel() != self.N:
+            raise _lib.AgarclError(f"the reset mask must be contiguous with {self.N} entries (one per instance)")
+        _lib.check(_lib.lib().agarcl_batch_reset_device(self._h, _vp(mask.data_ptr()), _vp(stream)))
+
+    def set_autoreset(self, max_steps=0, keep_final_obs=False, reset=True):
+        """enables the episode bookkeeping of step_autoreset (include/agarcl_b200.h, agarcl_batch_set_autoreset)"""
+        _lib.check(_lib.lib().agarcl_batch_set_autoreset(self._h, int(max_steps), int(bool(keep_final_obs)), int(bool(reset))))
+        self._episode = None
+
+    def step_autoreset(self, stream=0):
+        """step, then on the device: done flags with the step limit, the reset mask, episode statistics, the final observation
+        (when kept) and the reset of the finished instances"""
+        _lib.check(_lib.lib().agarcl_batch_step_autoreset(self._h, _vp(stream)))
+
+    def _episode_struct(self):
+        if getattr(self, "_episode", None) is None:
+            e = _EpisodeStruct()
+            _lib.check(_lib.lib().agarcl_batch_episode(self._h, C.byref(e)))
+            self._episode = e
+        return self._episode
+
+    def episode(self):
+        """zero-copy device views of the episode buffers, overwritten by every step_autoreset: done (u8 [N*A]), reset_mask
+        (u8 [N]), steps (i64 [N]), episode_return (f64 [N*A]) and episode_length (i64 [N]); the last two hold each instance's
+        last finished episode, to be read where reset_mask is set"""
+        import torch
+        e, N, NA, dev = self._episode_struct(), self.N, self.N * self.A, f"cuda:{self.cfg.device}"
+        view = lambda p, n, t: torch.as_tensor(_CudaView(p, (n,), t, self), device=dev)  # noqa: E731
+        return {"done": view(e.done_out, NA, "|u1"), "reset_mask": view(e.reset_mask, N, "|u1"), "steps": view(e.steps, N, "<i8"),
+                "episode_return": view(e.final_return, NA, "<f8"), "episode_length": view(e.final_length, N, "<i8")}
+
+    def final_obs(self):
+        """observation images [N*A, frames*C, G, G] the reset instances of the last step_autoreset ended their episode on"""
+        import torch
+        e = self._episode_struct()
+        if not e.final_obs:
+            raise _lib.AgarclError("no final observation images: set_autoreset(keep_final_obs=True) with a grid observation")
+        return torch.as_tensor(_CudaView(e.final_obs, self.obs_shape, "<i2" if self.obs_dtype == np.int16 else "<i4", self),
+                               device=f"cuda:{self.cfg.device}")
+
+    def final_ram(self):
+        """ram records [N, P, RAM_RECORD] float32 the reset instances of the last step_autoreset ended their episode on"""
+        import torch
+        from ._abi import RAM_RECORD
+        e = self._episode_struct()
+        if not e.final_ram:
+            raise _lib.AgarclError("no final ram records: set_autoreset(keep_final_obs=True) with cfg.ram_obs")
+        return torch.as_tensor(_CudaView(e.final_ram, (self.N, self.layout.P, RAM_RECORD), "<f4", self),
+                               device=f"cuda:{self.cfg.device}")
 
     def set_actions(self, dxdy, act, stream=0):
         dxdy = np.ascontiguousarray(dxdy, dtype=np.float32)

@@ -29,6 +29,8 @@ cudaError_t launch_obs(const ObsParams& P, cudaStream_t stream);
 cudaError_t launch_reset(const ResetParams& P, cudaStream_t stream);
 cudaError_t launch_ram(const RamParams& P, cudaStream_t stream);
 cudaError_t launch_flags(const uint8_t* state, const agarcl_layout& L, int N, uint32_t* out33, cudaStream_t stream);
+cudaError_t launch_episode(const EpisodeParams& P, cudaStream_t stream);
+cudaError_t launch_masked_bytes(void* dst, const void* src, size_t per, const uint8_t* mask, int N, cudaStream_t stream);
 }  // namespace ag
 
 struct agarcl_batch {
@@ -80,6 +82,14 @@ struct agarcl_batch {
   int fuse_clear = 2;  // 0: k_obs writes everything; 1: the engine-tick kernel clears channels 1..C-1 while ticking;
                        // 2: it also writes channel 0 and scatters the entities (one kernel per step).  AGARCL_FUSE_CLEAR overrides (A/B timing)
   int launches_last_step = 0;
+  // vector-env episode bookkeeping (agarcl_batch_set_autoreset); buffers allocated on first use
+  bool autoreset = false, autoreset_reset = true, keep_final = false;
+  int32_t max_steps = 0;
+  uint8_t *d_done_out = nullptr, *d_reset_mask = nullptr;
+  int64_t *d_steps = nullptr, *d_final_len = nullptr;
+  double *d_ret = nullptr, *d_final_ret = nullptr;
+  void* d_final_obs = nullptr;       // [N*A, frames*C, G, G], only with keep_final_obs and a grid observation
+  float* d_final_ram = nullptr;      // [N, P, AGARCL_RAM_RECORD], only with keep_final_obs and cfg.ram_obs
   ag::HostMirror* mirror = nullptr;  // host-resident observation mirror (mirror.cu), created on first use
   ag::HostMirror* lists = nullptr;   // the lists-only twin behind agarcl_batch_step_lists (no dense tensor, no worker threads)
   uint64_t mirror_launch_us = 0, mirror_call_us = 0;  // last agarcl_batch_step_mirror: staging + launch, whole call
@@ -276,6 +286,8 @@ extern "C" int agarcl_batch_destroy(agarcl_batch* b) {
   cudaFree(b->d_dxdy); cudaFree(b->d_act); cudaFree(b->d_replay); cudaFree(b->d_seeds); cudaFree(b->d_mask); cudaFree(b->d_tickets); cudaFree(b->d_cost); cudaFree(b->d_perm);
   cudaFree(b->d_fresh); cudaFree(b->d_flagbuf); cudaFree(b->d_sched);
   cudaFree(b->d_lut_radius); cudaFree(b->d_lut_speed); cudaFree(b->d_lut_split);
+  cudaFree(b->d_done_out); cudaFree(b->d_reset_mask); cudaFree(b->d_steps); cudaFree(b->d_final_len); cudaFree(b->d_ret);
+  cudaFree(b->d_final_ret); cudaFree(b->d_final_obs); cudaFree(b->d_final_ram);
   for (cudaEvent_t e : b->ev) cudaEventDestroy(e);
   delete b;
   return AGARCL_OK;
@@ -497,19 +509,28 @@ extern "C" int agarcl_batch_render(agarcl_batch* b, void* stream) {
   return render_frame(b, b->frames - 1, (cudaStream_t)stream, 0);
 }
 
-extern "C" int agarcl_batch_reset(agarcl_batch* b, const uint8_t* mask, void* stream) {
-  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+static ag::EpisodeParams episode_params(const agarcl_batch* b) {
+  ag::EpisodeParams E;
+  E.dones = b->d_dones; E.rewards = b->d_rewards;
+  E.done_out = b->d_done_out; E.reset_mask = b->d_reset_mask; E.steps = b->d_steps;
+  E.ret = b->d_ret; E.final_ret = b->d_final_ret; E.final_len = b->d_final_len;
+  E.clear_mask = nullptr;
+  E.N = b->N; E.A = b->A; E.max_steps = b->max_steps;
+  E.reset = b->autoreset_reset ? 1 : 0;
+  E.clear = 0;
+  return E;
+}
+
+// The masked reset: instances with d_mask[i] != 0 (device memory; nullptr = all).  Everything is enqueued on `s`; the
+// host neither reads the mask nor waits, except for refill_replay's draw cursor read-back under AGARCL_RNG_MT19937.
+// clear_episode: restart the episode counters of the reset instances (agarcl_batch_step_autoreset has done so already).
+static int reset_impl(agarcl_batch* b, const uint8_t* dm, cudaStream_t s, bool clear_episode) {
   CK(cudaSetDevice(b->cfg.device));
-  cudaStream_t s = (cudaStream_t)stream;
   ag::ResetParams P;
   P.L = b->L;
   P.T = b->T;
   P.state = b->d_state;
-  P.mask = nullptr;
-  if (mask) {
-    CK(cudaMemcpyAsync(b->d_mask, mask, b->N, cudaMemcpyHostToDevice, s));
-    P.mask = b->d_mask;
-  }
+  P.mask = dm;
   P.seeds = b->d_seeds;
   P.replay = b->d_replay;
   P.fresh = b->d_fresh;
@@ -520,7 +541,7 @@ extern "C" int agarcl_batch_reset(agarcl_batch* b, const uint8_t* mask, void* st
   P.num_pellets = b->cfg.num_pellets;
   P.num_viruses = b->cfg.num_viruses;
   P.W = (float)b->cfg.arena_size;
-  if (b->cfg.strict_reference && !mask) {
+  if (b->cfg.strict_reference && !dm) {
     // BaseEnvironment::reset of every instance (BaseEnvironment.hpp:179-197): players.clear(), then add_player for the agents and
     // the bots with the pids that follow the last episode's; a masked reset (one instance of a vector env) keeps the batch's order
     b->pmap.clear();
@@ -532,36 +553,43 @@ extern "C" int agarcl_batch_reset(agarcl_batch* b, const uint8_t* mask, void* st
   }
   CK(ag::launch_reset(P, s));
   b->was_reset = true;
-  { int rc = refill_replay(b, s); if (rc) return rc; }
-  if (b->d_ram) {  // GoBiggerEnvironment::reset ends with observation.clear() (GoBiggerEnvironment.hpp:698-702)
-    const size_t per = (size_t)b->L.P * AGARCL_RAM_RECORD * sizeof(float);
-    if (!mask) CK(cudaMemsetAsync(b->d_ram, 0, per * b->N, s));
-    else
-      for (int i = 0; i < b->N; i++)
-        if (mask[i]) CK(cudaMemsetAsync((uint8_t*)b->d_ram + per * i, 0, per, s));
+  if (clear_episode && b->autoreset) {
+    ag::EpisodeParams E = episode_params(b);
+    E.clear = 1;
+    E.clear_mask = dm;
+    CK(ag::launch_episode(E, s));
   }
-  // the reference ends reset() with _partial_observation (BaseEnvironment.hpp:202-203)
-  // (a masked reset touches only the observations of the instances it resets)
-  if (b->cfg.ram_obs == 2) return AGARCL_OK;  // no grid observation in this mode
-  const uint8_t* dm = mask ? b->d_mask : nullptr;
-  auto clear_obs = [&]() -> cudaError_t {
-    if (!mask) return cudaMemsetAsync(b->d_obs, 0, b->obs_bytes, s);
-    const size_t per = b->obs_bytes / (size_t)b->N;
-    for (int i = 0; i < b->N; i++)
-      if (mask[i]) {
-        cudaError_t e = cudaMemsetAsync((uint8_t*)b->d_obs + per * i, 0, per, s);
-        if (e != cudaSuccess) return e;
-      }
-    return cudaSuccess;
+  { int rc = refill_replay(b, s); if (rc) return rc; }
+  // (a masked reset touches only the records and observations of the instances it resets)
+  auto clear = [&](void* buf, size_t bytes) -> cudaError_t {
+    if (!dm) return cudaMemsetAsync(buf, 0, bytes, s);
+    return ag::launch_masked_bytes(buf, nullptr, bytes / (size_t)b->N, dm, b->N, s);
   };
+  if (b->d_ram)  // GoBiggerEnvironment::reset ends with observation.clear() (GoBiggerEnvironment.hpp:698-702)
+    CK(clear(b->d_ram, (size_t)b->N * b->L.P * AGARCL_RAM_RECORD * sizeof(float)));
+  // the reference ends reset() with _partial_observation (BaseEnvironment.hpp:202-203)
+  if (b->cfg.ram_obs == 2) return AGARCL_OK;  // no grid observation in this mode
   if (b->cfg.strict_reference) {
-    CK(clear_obs());
+    CK(clear(b->d_obs, b->obs_bytes));
     int frame = 0 - (b->cfg.ticks_per_step - b->frames);
     if (frame >= 0) return render_frame(b, frame, s, 0, 0, dm);
     return AGARCL_OK;
   }
-  if (b->frames > 1) CK(clear_obs());
+  if (b->frames > 1) CK(clear(b->d_obs, b->obs_bytes));
   return render_frame(b, b->frames - 1, s, 0, 0, dm);
+}
+
+extern "C" int agarcl_batch_reset(agarcl_batch* b, const uint8_t* mask, void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  CK(cudaSetDevice(b->cfg.device));
+  cudaStream_t s = (cudaStream_t)stream;
+  if (mask) CK(cudaMemcpyAsync(b->d_mask, mask, b->N, cudaMemcpyHostToDevice, s));
+  return reset_impl(b, mask ? b->d_mask : nullptr, s, true);
+}
+
+extern "C" int agarcl_batch_reset_device(agarcl_batch* b, const uint8_t* d_mask, void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  return reset_impl(b, d_mask, (cudaStream_t)stream, true);
 }
 
 extern "C" int agarcl_batch_set_actions(agarcl_batch* b, const float* dxdy, const int32_t* act, int on_device, void* stream) {
@@ -647,6 +675,72 @@ static int step_impl(agarcl_batch* b, cudaStream_t s, bool want_lists, bool* lis
 extern "C" int agarcl_batch_step(agarcl_batch* b, void* stream) {
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
   return step_impl(b, (cudaStream_t)stream, false, nullptr);
+}
+
+extern "C" int agarcl_batch_set_autoreset(agarcl_batch* b, int32_t max_steps, int32_t keep_final_obs, int32_t reset) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (max_steps < 0) return agarcl_set_error(AGARCL_ERR_INVALID, "max_steps must be >= 0 (0: no step limit)");
+  if (keep_final_obs && !reset) return agarcl_set_error(AGARCL_ERR_INVALID, "keep_final_obs needs reset: nothing is overwritten without one");
+  CK(cudaSetDevice(b->cfg.device));
+  const size_t NA = (size_t)b->N * b->A;
+#define ALLOC0(ptr, bytes)                                                                                            \
+  do {                                                                                                                \
+    if (!(ptr)) {                                                                                                     \
+      cudaError_t e__ = cudaMalloc((void**)&(ptr), (bytes));                                                          \
+      if (e__ != cudaSuccess)                                                                                         \
+        return agarcl_set_error(AGARCL_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", (size_t)(bytes), cudaGetErrorString(e__)); \
+      CK(cudaMemset((ptr), 0, (bytes)));                                                                              \
+    }                                                                                                                 \
+  } while (0)
+  ALLOC0(b->d_done_out, NA);
+  ALLOC0(b->d_reset_mask, (size_t)b->N);
+  ALLOC0(b->d_steps, (size_t)b->N * sizeof(int64_t));
+  ALLOC0(b->d_final_len, (size_t)b->N * sizeof(int64_t));
+  ALLOC0(b->d_ret, NA * sizeof(double));
+  ALLOC0(b->d_final_ret, NA * sizeof(double));
+  if (keep_final_obs) {
+    if (b->cfg.ram_obs != 2) ALLOC0(b->d_final_obs, b->obs_bytes);
+    if (b->d_ram) ALLOC0(b->d_final_ram, (size_t)b->N * b->L.P * AGARCL_RAM_RECORD * sizeof(float));
+  }
+#undef ALLOC0
+  // every instance starts counting here
+  CK(cudaMemset(b->d_steps, 0, (size_t)b->N * sizeof(int64_t)));
+  CK(cudaMemset(b->d_ret, 0, NA * sizeof(double)));
+  CK(cudaDeviceSynchronize());  // (the zeroing is done before a step on any stream can read the counters)
+  b->autoreset = true;
+  b->autoreset_reset = reset != 0;
+  b->keep_final = keep_final_obs != 0;
+  b->max_steps = max_steps;
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_step_autoreset(agarcl_batch* b, void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (!b->autoreset) return agarcl_set_error(AGARCL_ERR_STATE, "agarcl_batch_step_autoreset before agarcl_batch_set_autoreset");
+  cudaStream_t s = (cudaStream_t)stream;
+  int rc = step_impl(b, s, false, nullptr);
+  if (rc) return rc;
+  CK(ag::launch_episode(episode_params(b), s));
+  if (!b->autoreset_reset) return AGARCL_OK;
+  if (b->keep_final) {  // the observation the finished episode ended on, before the reset overwrites it
+    if (b->d_final_obs) CK(ag::launch_masked_bytes(b->d_final_obs, b->d_obs, b->obs_bytes / (size_t)b->N, b->d_reset_mask, b->N, s));
+    if (b->d_final_ram)
+      CK(ag::launch_masked_bytes(b->d_final_ram, b->d_ram, (size_t)b->L.P * AGARCL_RAM_RECORD * sizeof(float), b->d_reset_mask, b->N, s));
+  }
+  return reset_impl(b, b->d_reset_mask, s, false);
+}
+
+extern "C" int agarcl_batch_episode(agarcl_batch* b, agarcl_episode* out) {
+  if (!b || !out) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
+  if (!b->autoreset) return agarcl_set_error(AGARCL_ERR_STATE, "no episode bookkeeping: call agarcl_batch_set_autoreset first");
+  out->done_out = b->d_done_out;
+  out->reset_mask = b->d_reset_mask;
+  out->steps = b->d_steps;
+  out->final_return = b->d_final_ret;
+  out->final_length = b->d_final_len;
+  out->final_obs = b->keep_final ? b->d_final_obs : nullptr;
+  out->final_ram = b->keep_final ? b->d_final_ram : nullptr;
+  return AGARCL_OK;
 }
 
 extern "C" int agarcl_batch_set_timing(agarcl_batch* b, int enable) {

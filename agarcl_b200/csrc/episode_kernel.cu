@@ -1,0 +1,88 @@
+// episode_kernel.cu — what a vector environment with auto-reset does around the step, on the device: the episode
+// bookkeeping of agarcl_batch_step_autoreset (done flags with the step limit folded in, the reset mask, step counters,
+// returns) and the masked per-instance byte copy / clear used by a masked reset and by the final-observation copy.
+// Neither needs the host to look at the step's dones, so the step, the bookkeeping and the reset queue back to back.
+#include <cuda_runtime.h>
+
+#include "sim_params.h"
+
+namespace ag {
+
+// One thread per instance.
+//   clear == 0, after a step: done_out = dones | (max_steps > 0 && steps >= max_steps), checked before the increment like
+//     gym_agario's AgarioEnv.step; steps += 1; ret += rewards.  With `reset`, an instance with any done agent gets
+//     reset_mask = 1, its return and length go to final_ret / final_len, and its steps and ret restart at 0.  Must run
+//     before k_reset, which zeroes the dones of the instances it resets.
+//   clear == 1, a reset of the instances in clear_mask (nullptr: all): their steps and ret restart at 0.
+__global__ void __launch_bounds__(256) k_episode(const __grid_constant__ EpisodeParams P) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.N) return;
+  const int A = P.A;
+  if (P.clear) {
+    if (P.clear_mask && !P.clear_mask[i]) return;
+    P.steps[i] = 0;
+    for (int a = 0; a < A; a++) P.ret[(size_t)i * A + a] = 0.0;
+    return;
+  }
+  int64_t s = P.steps[i];
+  const bool limit = P.max_steps > 0 && s >= (int64_t)P.max_steps;
+  bool any = false;
+  for (int a = 0; a < A; a++) {
+    const size_t k = (size_t)i * A + a;
+    const bool d = P.dones[k] != 0 || limit;
+    P.done_out[k] = d ? 1 : 0;
+    any |= d;
+  }
+  s += 1;
+  const bool reset = P.reset && any;
+  for (int a = 0; a < A; a++) {
+    const size_t k = (size_t)i * A + a;
+    const double r = P.ret[k] + P.rewards[k];
+    if (reset) P.final_ret[k] = r;
+    P.ret[k] = reset ? 0.0 : r;
+  }
+  if (reset) P.final_len[i] = s;
+  P.steps[i] = reset ? 0 : s;
+  P.reset_mask[i] = reset ? 1 : 0;
+}
+
+// One CTA per instance: bytes [i * per, (i + 1) * per) of dst get those of src (kCopy) or zeros, for the instances with
+// mask[i] != 0; the CTAs of the others exit at once.  dst and src are allocations of the same alignment, so both share
+// the head that precedes the first 16-byte boundary; the body moves in 16-byte vectors, four in flight per thread.
+template <bool kCopy>
+__global__ void __launch_bounds__(kMaskedThreads) k_masked_bytes(uint8_t* __restrict__ dst, const uint8_t* __restrict__ src,
+                                                                 size_t per, const uint8_t* __restrict__ mask) {
+  const int inst = blockIdx.x;
+  if (!mask[inst]) return;
+  uint8_t* d = dst + (size_t)inst * per;
+  const uint8_t* s = kCopy ? src + (size_t)inst * per : nullptr;
+  size_t head = (16u - ((uintptr_t)d & 15u)) & 15u;
+  if (head > per) head = per;
+  const size_t nvec = (per - head) / 16, tail = head + nvec * 16;
+  const int t = threadIdx.x, nt = blockDim.x;
+  for (size_t k = t; k < head; k += nt) d[k] = kCopy ? s[k] : 0;
+  for (size_t k = tail + t; k < per; k += nt) d[k] = kCopy ? s[k] : 0;
+  uint4* dv = reinterpret_cast<uint4*>(d + head);
+  const uint4* sv = kCopy ? reinterpret_cast<const uint4*>(s + head) : nullptr;
+  const uint4 z = make_uint4(0u, 0u, 0u, 0u);
+  size_t k = t;
+  for (; k + 3 * (size_t)nt < nvec; k += 4 * (size_t)nt) {
+    uint4 v0 = z, v1 = z, v2 = z, v3 = z;
+    if (kCopy) { v0 = sv[k]; v1 = sv[k + nt]; v2 = sv[k + 2 * nt]; v3 = sv[k + 3 * nt]; }
+    dv[k] = v0; dv[k + nt] = v1; dv[k + 2 * nt] = v2; dv[k + 3 * nt] = v3;
+  }
+  for (; k < nvec; k += nt) dv[k] = kCopy ? sv[k] : z;
+}
+
+cudaError_t launch_episode(const EpisodeParams& P, cudaStream_t stream) {
+  k_episode<<<(P.N + 255) / 256, 256, 0, stream>>>(P);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_masked_bytes(void* dst, const void* src, size_t per, const uint8_t* mask, int N, cudaStream_t stream) {
+  if (src) k_masked_bytes<true><<<N, kMaskedThreads, 0, stream>>>((uint8_t*)dst, (const uint8_t*)src, per, mask);
+  else k_masked_bytes<false><<<N, kMaskedThreads, 0, stream>>>((uint8_t*)dst, nullptr, per, mask);
+  return cudaGetLastError();
+}
+
+}  // namespace ag

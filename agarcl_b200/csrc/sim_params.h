@@ -156,4 +156,22 @@ struct RamParams {
   int32_t pid_base;        // CloneInfo::owner is the player's pid: index + pid of player 0 (non-zero only in later episodes of strict_reference, Q3)
 };
 
+constexpr int kMaskedThreads = 512;  // threads of k_masked_bytes, one CTA per instance
+
+// Episode bookkeeping of agarcl_batch_step_autoreset (episode_kernel.cu, k_episode)
+struct EpisodeParams {
+  const uint8_t* dones;      // [N*A] of the step that just ran
+  const double* rewards;     // [N*A]
+  uint8_t* done_out;         // [N*A] dones with the step limit folded in
+  uint8_t* reset_mask;       // [N]
+  int64_t* steps;            // [N] steps since the instance's last reset
+  double* ret;               // [N*A] rewards summed since the instance's last reset
+  double* final_ret;         // [N*A] ret of the episode that finished last
+  int64_t* final_len;        // [N] steps of the episode that finished last
+  const uint8_t* clear_mask; // clear mode: the instances being reset, nullptr = all
+  int32_t N, A, max_steps;
+  int32_t reset;             // 1: finished instances are reset by this step (auto-reset); 0: bookkeeping only
+  int32_t clear;             // 1: a reset restarts the counters of clear_mask's instances (no step)
+};
+
 }  // namespace ag

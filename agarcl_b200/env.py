@@ -333,13 +333,17 @@ class BatchedGridEnvironment(_Base):
         if self._batch is not None:
             self._batch.seed(self._seeds)
 
-    def reset(self, mask=None):
-        self._ensure().reset(mask)
-        return self._batch.obs_tensor()
-
-    def step(self, dxdy, act, stream=0):
-        """dxdy: [N*A, 2] float32, act: [N*A] int32 — numpy (copied) or CUDA torch tensors (zero-copy)"""
+    def reset(self, mask=None, stream=0):
+        """all instances, or those with mask != 0: a host array (copied to the device) or a CUDA uint8 / bool tensor of
+        n_instances entries (read by the device, no host wait)"""
         b = self._ensure()
+        if getattr(mask, "is_cuda", False):
+            b.reset_device(mask, stream)
+        else:
+            b.reset(mask, stream)
+        return b.obs_tensor()
+
+    def _set_actions(self, b, dxdy, act, stream):
         if hasattr(dxdy, "data_ptr"):
             import torch
             # the C ABI reads the raw device buffers as float32 / int32: anything else would be silently reinterpreted
@@ -356,8 +360,30 @@ class BatchedGridEnvironment(_Base):
             b.set_actions_device(dxdy.data_ptr(), act.data_ptr(), stream)
         else:
             b.set_actions(dxdy, act, stream)
+
+    def step(self, dxdy, act, stream=0):
+        """dxdy: [N*A, 2] float32, act: [N*A] int32 — numpy (copied) or CUDA torch tensors (zero-copy)"""
+        b = self._ensure()
+        self._set_actions(b, dxdy, act, stream)
         b.step(stream)
         return b.obs_tensor(), b.rewards_tensor(), b.dones_tensor()
+
+    def set_autoreset(self, max_steps=0, final_obs=False, reset=True):
+        """enables step_autoreset: max_steps > 0 ends an episode after that many steps (0: continuing), final_obs keeps the
+        observation a finished episode ended on, reset=False keeps the bookkeeping (done with the step limit, step counters)
+        without resetting anything"""
+        self._ensure().set_autoreset(max_steps, final_obs, reset)
+
+    def step_autoreset(self, dxdy, act, stream=0):
+        """step() followed, on the device, by the episode bookkeeping and the reset of every instance with a done agent;
+        returns obs, rewards and the done flags with the step limit folded in (u8 [N*A]); episode() has the rest"""
+        b = self._ensure()
+        self._set_actions(b, dxdy, act, stream)
+        b.step_autoreset(stream)
+        return b.obs_tensor(), b.rewards_tensor(), b.episode()["done"]
+
+    def episode(self):
+        return self._ensure().episode()
 
     def ram(self):
         return self._ensure().ram_tensor()

@@ -183,26 +183,41 @@ class AgarioEnv(_EnvBase):
 
 
 class BatchedAgarioEnv:
-    """Vector environment: N lockstep instances on one GPU, device tensors in and out, auto-reset.
+    """Vector environment: N lockstep instances on one GPU, device tensors in and out, auto-reset on the device.
 
     step(dxdy [N*A, 2] float32, act [N*A] int32) -> obs, rewards (float32), dones, truncations (bool tensors), info.
-    An instance whose agent 0 is done, or that reached `number_steps` (episodic), is reset before the next step and
-    its observation is the first of the new episode (the final one is in info["final_obs_mask"] semantics of vector
-    envs is not reproduced: rewards/dones of the finished step are returned as they were)."""
+    An instance with a done agent, or that reached `number_steps` (episodic, env_type 0), is reset within the same step: its
+    observation is the first of the new episode, while the rewards and dones returned are those of the finished step.  The
+    host never waits for the device, so step t+1 can be queued while step t runs.  info (device tensors):
+      steps           i64 [N]    steps since the instance's last reset
+      reset_mask      bool [N]   instances reset by this step
+      episode_return  f64 [N*A]  return of the episode an instance just finished (read where reset_mask is set)
+      episode_length  i64 [N]    its length in steps (likewise)
+      final_obs       the observation that episode ended on (grid: [N*A, C*frames, G, G]; ram: [N, A, RAM_RECORD]); only
+                      with final_obs=True, which allocates as much device memory again as the observation
+    obs, dones and every info tensor are views of library-owned buffers that the next step() overwrites: copy what must
+    outlive it.  With auto_reset=False nothing is reset: the step limit is folded into dones, steps keeps counting, and
+    info has "steps" only."""
 
-    def __init__(self, n_envs, obs_type="grid", auto_reset=True, **kwargs):
+    def __init__(self, n_envs, obs_type="grid", auto_reset=True, final_obs=False, **kwargs):
         if obs_type not in ("grid", "ram"):
             raise ValueError(obs_type)
         a = _env_args(kwargs)
         self.n_envs, self.num_agents, self.obs_type, self.auto_reset = n_envs, a["num_agents"], obs_type, auto_reset
+        self.final_obs = bool(final_obs)
+        if self.final_obs and not auto_reset:
+            raise ValueError("final_obs needs auto_reset: without a reset no observation is overwritten")
         self.number_of_steps = kwargs.get("number_steps", 500)
         self.env_type = kwargs.get("env_type", 0)
+        if self.env_type == 0 and self.number_of_steps < 1:
+            raise ValueError("number_steps must be >= 1 for an episodic environment (env_type 0)")
         extra = {k: kwargs[k] for k in ("device", "rng_mode", "obs_dtype", "instance_base") if k in kwargs}
         self._env = BatchedGridEnvironment(n_envs, a["num_agents"], a["ticks_per_step"], a["arena_size"], a["pellet_regen"],
                                            a["num_pellets"], a["num_viruses"], a["num_bots"], a["reward_type"], a["c_death"],
                                            a["mode"], ram_obs=(2 if obs_type == "ram" else 0), **extra)
         self._env.configure_observation({k: kwargs[k] for k in _OBS_KEYS if k in kwargs})
-        self._steps = None
+        self._ep_batch = None
+        self._ep = None
 
     def seed(self, seed):
         self._env.seed(seed)
@@ -214,28 +229,28 @@ class BatchedAgarioEnv:
         return ram[:, :self.num_agents, :]
 
     def reset(self):
-        import torch
-        self._env.reset()
-        self._steps = torch.zeros(self.n_envs, dtype=torch.int64, device=self._env.batch.obs_tensor().device)
+        b = self._env.batch
+        if self._ep_batch is not b:
+            b.set_autoreset(self.number_of_steps if self.env_type == 0 else 0, self.final_obs, self.auto_reset)
+            self._ep_batch = b
+            self._ep = b.episode()
+            self._final = (b.final_obs() if self.obs_type == "grid" else b.final_ram()[:, :self.num_agents, :]) if self.final_obs else None
+        self._env.reset()  # (restarts every instance's step counter and return)
         return self._obs(), {}
 
     def step(self, dxdy, act):
         import torch
-        assert self._steps is not None, "Cannot call step() before calling reset()"
-        _, rew, done = self._env.step(dxdy, act)
-        A = self.num_agents
-        done = done.view(self.n_envs, A).bool()
-        trunc = torch.zeros_like(done)
-        if self.env_type == 0:
-            done = done | (self._steps >= self.number_of_steps).unsqueeze(1)
-        self._steps += 1
-        rewards = rew.float()
+        assert self._ep is not None, "Cannot call step() before calling reset()"
+        _, rew, _ = self._env.step_autoreset(dxdy, act)
+        ep = self._ep
+        done = ep["done"].view(torch.bool)
+        info = {"steps": ep["steps"]}
         if self.auto_reset:
-            mask = done.any(dim=1)
-            if bool(mask.any()):
-                self._env.reset(mask.to(torch.uint8).cpu().numpy())
-                self._steps[mask] = 0
-        return self._obs(), rewards, done.view(-1), trunc.view(-1), {"steps": self._steps}
+            info.update(reset_mask=ep["reset_mask"].view(torch.bool), episode_return=ep["episode_return"],
+                        episode_length=ep["episode_length"])
+            if self.final_obs:
+                info["final_obs"] = self._final
+        return self._obs(), rew.float(), done, torch.zeros_like(done), info
 
     def flags(self):
         """(OR over all instances, {AGARCL_FLAG name: instances}) -- fixed capacities hit since the instances' last reset"""

@@ -196,6 +196,42 @@ int agarcl_batch_dones(agarcl_batch* b, uint8_t** dev_ptr);  /* dones(), u8[N*A]
 int agarcl_batch_step_host(agarcl_batch* b, const float* dxdy, const int32_t* act,
                            void* obs_out, double* rewards_out, uint8_t* dones_out);
 
+/* ---------------------------------------------------- vector environment: auto-reset on the device
+ * What gym_agario's AgarioEnv.step (AgarioEnv.py:77-112) adds around the step, for every instance, without the host reading
+ * anything back, so the host can queue step t+1 while step t runs:
+ *   done_out[i*A+a] = dones[i*A+a] | (max_steps > 0 && steps[i] >= max_steps)   (checked before the increment)
+ *   reset_mask[i]   = any agent of i done;  steps[i] += 1;  then the instances in reset_mask are reset (same step: the
+ *                     observation of a reset instance is the first of its new episode; rewards and done_out are the finished step's)
+ * Episode statistics: per agent the f64 sum of the rewards since the instance's last reset, per instance its steps; where
+ * reset_mask is set they are written to final_return / final_length and restart at 0.  Every reset, agarcl_batch_reset
+ * included, restarts the counters of the instances it resets.
+ *   agarcl_batch_reset_device   agarcl_batch_reset with mask[N] in DEVICE memory (NULL = all): no copy, no host loop, no wait.
+ *   agarcl_batch_set_autoreset  enables the bookkeeping and allocates its buffers (synchronises the device; every instance's
+ *                               counters start at 0).  max_steps 0: no step limit (continuing task).  keep_final_obs != 0: before
+ *                               the reset, the observation images of the reset instances are copied to final_obs
+ *                               [N*A, frames*C, G, G] (not with ram_obs = 2) and their ram records to final_ram [N, P,
+ *                               AGARCL_RAM_RECORD] (cfg.ram_obs) -- as much memory again as the observation.  reset = 0:
+ *                               bookkeeping only -- done_out and steps as above, nothing is reset, reset_mask stays 0 (requires
+ *                               keep_final_obs = 0).  May be called again to change the settings.
+ *   agarcl_batch_step_autoreset step, bookkeeping, final copy, masked reset, all enqueued on `stream`; AGARCL_ERR_STATE before
+ *                               agarcl_batch_set_autoreset.  Under AGARCL_RNG_MT19937 the host reads the draw cursors back
+ *                               now and then to refill the draw ring, as after any step or reset: the one wait that remains.
+ *   agarcl_batch_episode        device pointers of the buffers below; each step_autoreset overwrites them.  The final_* entries
+ *                               hold the last finished episode of each instance: read them where reset_mask is set.   */
+typedef struct agarcl_episode {
+  uint8_t* done_out;       /* u8 [N*A] */
+  uint8_t* reset_mask;     /* u8 [N] */
+  int64_t* steps;          /* [N] steps since the instance's last reset */
+  double* final_return;    /* f64 [N*A] */
+  int64_t* final_length;   /* [N] */
+  void* final_obs;         /* observation dtype [N*A, frames*C, G, G]; NULL unless keep_final_obs and a grid observation */
+  float* final_ram;        /* [N, P, AGARCL_RAM_RECORD]; NULL unless keep_final_obs and cfg.ram_obs */
+} agarcl_episode;
+int agarcl_batch_reset_device(agarcl_batch* b, const uint8_t* d_mask, void* stream);
+int agarcl_batch_set_autoreset(agarcl_batch* b, int32_t max_steps, int32_t keep_final_obs, int32_t reset);
+int agarcl_batch_step_autoreset(agarcl_batch* b, void* stream);
+int agarcl_batch_episode(agarcl_batch* b, agarcl_episode* out);
+
 /* ---------------------------------------------------- host-resident observation mirror
  * get_state (bindings.cpp:67-91) hands every agent's frame to HOST memory; for a batch that is 512 KB per agent
  * per step, and the dense copy above is bound by PCIe.  The mirror is a library-owned, pinned host tensor

@@ -51,21 +51,21 @@ def main():
         env.reset()
         gen = torch.Generator(device="cuda")
         gen.manual_seed(k)
-        ret = torch.zeros(N, device="cuda")
-        finished, ret_sum = 0, 0.0
+        # finished episodes and their returns come from info, summed on the device: the loop never waits for it
+        finished = torch.zeros((), dtype=torch.int64, device="cuda")
+        ret_sum = torch.zeros((), dtype=torch.float64, device="cuda")
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         for t in range(args.steps):
             dxdy = (torch.rand((N, 2), device="cuda", generator=gen) * 2 - 1).float()
             act = torch.randint(0, 3, (N,), device="cuda", generator=gen, dtype=torch.int32)
-            _, rew, done, _, _ = env.step(dxdy, act)
-            ret += rew
-            if bool(done.any()):
-                finished += int(done.sum())
-                ret_sum += float(ret[done].sum())
-                ret[done] = 0
+            _, _, _, _, info = env.step(dxdy, act)
+            m = info["reset_mask"]
+            finished += m.sum()
+            ret_sum += torch.where(m, info["episode_return"], 0.0).sum()
         torch.cuda.synchronize()
         sec = time.perf_counter() - t0
+        finished, ret_sum = int(finished), float(ret_sum)
         f, names = env.flags()
         print(json.dumps({"task": f"mode_{k}", "envs": N, "steps": args.steps, "env_steps_per_s": N * args.steps / sec,
                           "episode_steps": kw["number_steps"], "episodes_finished": finished,
