@@ -42,11 +42,16 @@ def build_pybind(force=False):
     return out
 
 
+def nvcc_command(out, extra=(), verbose=False):
+    """The nvcc command that compiles SOURCES into the shared library `out`: the product library, and the variants of
+    tools/build_variant.sh (`extra`: more nvcc flags)."""
+    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+    return [nvcc] + NVCC_FLAGS + list(extra) + (["-Xptxas", "-v"] if verbose else []) + ["-o", out] + [os.path.join(CSRC, f) for f in SOURCES]
+
+
 def build(force=False, verbose=False):
     if force or needs_build():
-        nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-        cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB] + [os.path.join(CSRC, f) for f in SOURCES]
-        subprocess.check_call(cmd)
+        subprocess.check_call(nvcc_command(LIB, verbose=verbose))
     build_pybind(force)
     return LIB
 

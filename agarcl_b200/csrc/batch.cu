@@ -11,6 +11,7 @@
 #include <cstdlib>
 #include <chrono>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <random>
 #include <unordered_map>
@@ -21,17 +22,42 @@
 #include "sim_params.h"
 #include "sim_shared.cuh"
 
-namespace ag {
-cudaError_t launch_step(const SimParams& P, cudaStream_t stream);
-cudaError_t selftest_std_sort(const float* ys, int n, uint16_t* order_out);
-cudaError_t launch_order(const uint32_t* cost, uint32_t* perm, int N, uint32_t* sched, cudaStream_t stream);
-cudaError_t launch_obs(const ObsParams& P, cudaStream_t stream);
-cudaError_t launch_reset(const ResetParams& P, cudaStream_t stream);
-cudaError_t launch_ram(const RamParams& P, cudaStream_t stream);
-cudaError_t launch_flags(const uint8_t* state, const agarcl_layout& L, int N, uint32_t* out33, cudaStream_t stream);
-cudaError_t launch_episode(const EpisodeParams& P, cudaStream_t stream);
-cudaError_t launch_masked_bytes(void* dst, const void* src, size_t per, const uint8_t* mask, int N, cudaStream_t stream);
-}  // namespace ag
+// Device memory owned by a batch: freed with it.
+template <typename T>
+class DevBuf {
+ public:
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { cudaFree(p_); }
+  cudaError_t alloc(size_t bytes) { return cudaMalloc((void**)&p_, bytes); }
+  T* get() const { return p_; }
+  operator T*() const { return p_; }
+
+ private:
+  T* p_ = nullptr;
+};
+
+// The A/B knobs of the step (names, defaults and effects: DESIGN.md section 8), read from the environment when a batch is created
+struct Knobs {
+  int fuse_clear = 2, sort_schedule = 1, auto_schedule = 1, tick_barrier = 6, dyn_stripes = 1, zero_chunks = 0;
+  int warps = 0;  // > 0: at most this many warps per k_step CTA
+  double hash_per_cell = 3.0;
+};
+
+static Knobs read_knobs() {
+  Knobs k;
+  auto env_int = [](const char* name, int& v) { if (const char* e = std::getenv(name)) v = std::atoi(e); };
+  env_int("AGARCL_FUSE_CLEAR", k.fuse_clear);
+  env_int("AGARCL_SORT_SCHEDULE", k.sort_schedule);
+  env_int("AGARCL_AUTO_SCHEDULE", k.auto_schedule);
+  env_int("AGARCL_TICK_BARRIER", k.tick_barrier);
+  env_int("AGARCL_DYNAMIC_STRIPES", k.dyn_stripes);
+  env_int("AGARCL_ZERO_CHUNKS", k.zero_chunks);
+  env_int("AGARCL_WARPS", k.warps);
+  if (const char* e = std::getenv("AGARCL_HASH_PER_CELL")) k.hash_per_cell = std::atof(e);
+  return k;
+}
 
 struct agarcl_batch {
   agarcl_cfg cfg;
@@ -44,26 +70,26 @@ struct agarcl_batch {
   int32_t pid_base = 0;  // pid of player index 0 in the current episode
   int N, A, G, C, frames;
   size_t obs_elems, obs_bytes;
-  uint8_t* d_state = nullptr;
-  void* d_obs = nullptr;
-  float* d_ram = nullptr;  // structured observation records [N][P][AGARCL_RAM_RECORD], only with cfg.ram_obs
-  double* d_rewards = nullptr;
-  uint8_t* d_dones = nullptr;
-  float* d_before = nullptr;
-  float* d_dxdy = nullptr;
-  int32_t* d_act = nullptr;
+  Knobs knobs;
+  ag::StepLaunch step_launch;
+  DevBuf<uint8_t> d_state;
+  DevBuf<void> d_obs;
+  DevBuf<float> d_ram;  // structured observation records [N][P][AGARCL_RAM_RECORD], only with cfg.ram_obs
+  DevBuf<double> d_rewards;
+  DevBuf<uint8_t> d_dones;
+  DevBuf<float> d_before;
+  DevBuf<float> d_dxdy;
+  DevBuf<int32_t> d_act;
   const float* cur_dxdy = nullptr;  // what the next step reads (own buffers or caller's device pointers)
   const int32_t* cur_act = nullptr;
-  float* d_replay = nullptr;
-  uint64_t* d_seeds = nullptr;
-  uint8_t* d_mask = nullptr;
-  uint32_t* d_tickets = nullptr;  // k_step's ticket counter pair (self-rewinding)
-  uint32_t* d_sched = nullptr;   // [2] schedule selector of k_step (SimParams::sched); AGARCL_AUTO_SCHEDULE=0 turns it off
-  int auto_schedule = 1;
-  uint32_t *d_cost = nullptr, *d_perm = nullptr;  // per-instance cost of the last step and the cost-sorted schedule made from it (k_order)
+  DevBuf<float> d_replay;
+  DevBuf<uint64_t> d_seeds;
+  DevBuf<uint8_t> d_mask;
+  DevBuf<uint32_t> d_tickets;  // k_step's ticket counter pair (self-rewinding)
+  DevBuf<uint32_t> d_sched;    // [2] schedule selector of k_step (SimParams::sched)
+  DevBuf<uint32_t> d_cost, d_perm;  // per-instance cost of the last step and the cost-sorted schedule made from it (k_order)
   bool perm_valid = false;
-  int sort_schedule = 1;  // AGARCL_SORT_SCHEDULE=0 turns the cost-sorted schedule off (A/B timing)
-  float *d_lut_radius = nullptr, *d_lut_speed = nullptr, *d_lut_split = nullptr;
+  DevBuf<float> d_lut_radius, d_lut_speed, d_lut_split;
   std::vector<uint64_t> seeds;
   // AGARCL_RNG_MT19937: the reference's generator per instance (GameState::rng, GameState.hpp:51), kept on the host; its
   // uniform_real_distribution<float> draws are fed to the device through d_replay used as a RING that refill_replay keeps
@@ -72,24 +98,22 @@ struct agarcl_batch {
   std::vector<uint64_t> filled;
   int64_t draw_budget = 0;      // draws every instance is known to have ahead of its cursor
   int64_t max_draws_per_step = 0;
-  uint8_t* d_fresh = nullptr;   // [N] instance (re)seeded since its last reset (ResetParams::fresh)
-  uint32_t* d_flagbuf = nullptr;  // [33] agarcl_batch_flags scratch
+  DevBuf<uint8_t> d_fresh;      // [N] instance (re)seeded since its last reset (ResetParams::fresh)
+  DevBuf<uint32_t> d_flagbuf;   // [33] agarcl_batch_flags scratch
   ag::Luts T;
   int HG;
   uint32_t smem_per_warp;
   ag::SmemOff so;
   bool was_reset = false;
-  int fuse_clear = 2;  // 0: k_obs writes everything; 1: the engine-tick kernel clears channels 1..C-1 while ticking;
-                       // 2: it also writes channel 0 and scatters the entities (one kernel per step).  AGARCL_FUSE_CLEAR overrides (A/B timing)
   int launches_last_step = 0;
   // vector-env episode bookkeeping (agarcl_batch_set_autoreset); buffers allocated on first use
   bool autoreset = false, autoreset_reset = true, keep_final = false;
   int32_t max_steps = 0;
-  uint8_t *d_done_out = nullptr, *d_reset_mask = nullptr;
-  int64_t *d_steps = nullptr, *d_final_len = nullptr;
-  double *d_ret = nullptr, *d_final_ret = nullptr;
-  void* d_final_obs = nullptr;       // [N*A, frames*C, G, G], only with keep_final_obs and a grid observation
-  float* d_final_ram = nullptr;      // [N, P, AGARCL_RAM_RECORD], only with keep_final_obs and cfg.ram_obs
+  DevBuf<uint8_t> d_done_out, d_reset_mask;
+  DevBuf<int64_t> d_steps, d_final_len;
+  DevBuf<double> d_ret, d_final_ret;
+  DevBuf<void> d_final_obs;          // [N*A, frames*C, G, G], only with keep_final_obs and a grid observation
+  DevBuf<float> d_final_ram;         // [N, P, AGARCL_RAM_RECORD], only with keep_final_obs and cfg.ram_obs
   ag::HostMirror* mirror = nullptr;  // host-resident observation mirror (mirror.cu), created on first use
   ag::HostMirror* lists = nullptr;   // the lists-only twin behind agarcl_batch_step_lists (no dense tensor, no worker threads)
   uint64_t mirror_launch_us = 0, mirror_call_us = 0;  // last agarcl_batch_step_mirror: staging + launch, whole call
@@ -99,6 +123,12 @@ struct agarcl_batch {
   size_t ev_used = 0;
   double acc_sim_ms = 0.0, acc_obs_ms = 0.0;
   int acc_steps = 0;
+
+  ~agarcl_batch() {
+    ag::mirror_destroy(mirror);
+    ag::mirror_destroy(lists);
+    for (cudaEvent_t e : ev) cudaEventDestroy(e);
+  }
 };
 
 static cudaEvent_t next_event(agarcl_batch* b) {
@@ -129,6 +159,16 @@ static void collect_timing(agarcl_batch* b) {
     if (e__ != cudaSuccess)                                                                        \
       return agarcl_set_error(AGARCL_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e__));   \
   } while (0)
+
+// Allocates `bytes` of device memory for `buf` unless it holds some already, and fills them with the byte `fill` (-1: left as is).
+template <typename T>
+static int alloc(DevBuf<T>& buf, size_t bytes, int fill = -1) {
+  if (buf) return AGARCL_OK;
+  const cudaError_t e = buf.alloc(bytes);
+  if (e != cudaSuccess) return agarcl_set_error(AGARCL_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
+  if (fill >= 0) CK(cudaMemset(buf, fill, bytes));
+  return AGARCL_OK;
+}
 
 static void fill_sim_params(const agarcl_batch* b, ag::SimParams& P) {
   P.L = b->L;
@@ -164,12 +204,9 @@ static void fill_sim_params(const agarcl_batch* b, ag::SimParams& P) {
   P.obs = nullptr;
   P.zero_vec_per_agent = 0; P.zero_skip_vec = 0; P.agent_stride_vec = 0;
   P.obs_finish = 0; P.obs_G = b->G; P.obs_C = b->C;
-  P.zero_chunks = 0;
-  if (const char* e = std::getenv("AGARCL_ZERO_CHUNKS")) P.zero_chunks = std::atoi(e);
-  P.dyn_stripes = 1;
-  if (const char* e = std::getenv("AGARCL_DYNAMIC_STRIPES")) P.dyn_stripes = std::atoi(e);  // (A/B timing)
-  P.tick_barrier = 6;  // bit mask of the alignment barriers of a tick (sim_kernel.cu, step_instance)
-  if (const char* e = std::getenv("AGARCL_TICK_BARRIER")) P.tick_barrier = std::atoi(e);  // (A/B timing)
+  P.zero_chunks = b->knobs.zero_chunks;
+  P.dyn_stripes = b->knobs.dyn_stripes;
+  P.tick_barrier = b->knobs.tick_barrier;
   P.align_group = ag::kMaxWarpsPerCta;  // the whole CTA (groups of 8 / 4 / 2 warps were slower: 1.78 / 1.97 / 2.16 vs 1.70 ms)
   P.observe_cells = b->cfg.observe_cells; P.observe_others = b->cfg.observe_others;
   P.observe_viruses = b->cfg.observe_viruses; P.observe_pellets = b->cfg.observe_pellets;
@@ -182,13 +219,13 @@ static void fill_sim_params(const agarcl_batch* b, ag::SimParams& P) {
 static bool fuse_obs_clear(const agarcl_batch* b, ag::SimParams& P, int frame) {
   const size_t esz = b->cfg.obs_dtype == AGARCL_OBS_I16 ? 2 : 4;
   const size_t plane = (size_t)b->G * b->G * esz;
-  if (plane % 16 != 0 || b->C < 2 || b->fuse_clear == 0) return false;
-  P.obs = (uint8_t*)b->d_obs + (size_t)frame * b->C * plane;
+  if (plane % 16 != 0 || b->C < 2 || b->knobs.fuse_clear == 0) return false;
+  P.obs = (uint8_t*)b->d_obs.get() + (size_t)frame * b->C * plane;
   P.zero_skip_vec = (uint32_t)(plane / 16);
   P.zero_vec_per_agent = (uint32_t)((size_t)(b->C - 1) * plane / 16);
   P.agent_stride_vec = (uint32_t)((size_t)b->frames * b->C * plane / 16);
   // the whole observation in the engine-tick kernel: rows of whole 16-byte vectors, masks fit the scratch (1: int32, 2: int16)
-  P.obs_finish = (b->fuse_clear >= 2 && ((size_t)b->G * esz) % 16 == 0 &&
+  P.obs_finish = (b->knobs.fuse_clear >= 2 && ((size_t)b->G * esz) % 16 == 0 &&
                   (size_t)b->G * esz <= (size_t)ag::kZeroTileBytes &&  // one row of channel 0 = one bulk store from the ones tile
                   (size_t)b->G * esz <= (size_t)(b->so.vcache - b->so.cellref)) ? (esz == 2 ? 2 : 1) : 0;
   if (P.obs_finish) P.tiles_bytes = ag::kZeroTileBytes + (((uint32_t)b->G * (uint32_t)esz + 127u) & ~127u);
@@ -278,17 +315,6 @@ static int refill_replay(agarcl_batch* b, cudaStream_t s) {
 }
 
 extern "C" int agarcl_batch_destroy(agarcl_batch* b) {
-  if (!b) return AGARCL_OK;
-  ag::mirror_destroy(b->mirror);
-  ag::mirror_destroy(b->lists);
-  cudaFree(b->d_ram);
-  cudaFree(b->d_state); cudaFree(b->d_obs); cudaFree(b->d_rewards); cudaFree(b->d_dones); cudaFree(b->d_before);
-  cudaFree(b->d_dxdy); cudaFree(b->d_act); cudaFree(b->d_replay); cudaFree(b->d_seeds); cudaFree(b->d_mask); cudaFree(b->d_tickets); cudaFree(b->d_cost); cudaFree(b->d_perm);
-  cudaFree(b->d_fresh); cudaFree(b->d_flagbuf); cudaFree(b->d_sched);
-  cudaFree(b->d_lut_radius); cudaFree(b->d_lut_speed); cudaFree(b->d_lut_split);
-  cudaFree(b->d_done_out); cudaFree(b->d_reset_mask); cudaFree(b->d_steps); cudaFree(b->d_final_len); cudaFree(b->d_ret);
-  cudaFree(b->d_final_ret); cudaFree(b->d_final_obs); cudaFree(b->d_final_ram);
-  for (cudaEvent_t e : b->ev) cudaEventDestroy(e);
   delete b;
   return AGARCL_OK;
 }
@@ -306,7 +332,7 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
     return agarcl_set_error(AGARCL_ERR_CUDA, "no CUDA device: agarcl_b200 has no CPU path (%s)", cudaGetErrorString(e));
   if (cfg->device < 0 || cfg->device >= ndev) return agarcl_set_error(AGARCL_ERR_INVALID, "device %d out of range", cfg->device);
   CK(cudaSetDevice(cfg->device));
-  agarcl_batch* b = new (std::nothrow) agarcl_batch();
+  std::unique_ptr<agarcl_batch> b(new (std::nothrow) agarcl_batch());  // (frees whatever was made when a step below fails)
   if (!b) return agarcl_set_error(AGARCL_ERR_NOMEM, "out of host memory");
   b->cfg = *cfg;
   b->L = L;
@@ -315,64 +341,30 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
   b->G = cfg->grid_size;
   b->C = L.obs_channels;
   b->frames = cfg->num_frames;
-  if (const char* e = std::getenv("AGARCL_FUSE_CLEAR")) b->fuse_clear = std::atoi(e);
-  if (const char* e = std::getenv("AGARCL_SORT_SCHEDULE")) b->sort_schedule = std::atoi(e);
+  b->knobs = read_knobs();
+  CK(ag::setup_step(b->knobs.warps, b->step_launch));
+  if (cfg->ram_obs) CK(ag::setup_ram(L, b->step_launch.smem_optin));
   b->obs_elems = (size_t)b->N * b->A * b->frames * b->C * b->G * b->G;
   b->obs_bytes = b->obs_elems * (cfg->obs_dtype == AGARCL_OBS_I16 ? 2 : 4);
   // spatial hash resolution: about 3 pellets per hash cell, 4..64 cells per side
-  double per_cell = 3.0;
-  if (const char* e = std::getenv("AGARCL_HASH_PER_CELL")) per_cell = std::atof(e);  // (A/B timing)
-  int hg = (int)std::floor(std::sqrt((double)L.cap_pellets / per_cell));
+  int hg = (int)std::floor(std::sqrt((double)L.cap_pellets / b->knobs.hash_per_cell));
   b->HG = hg < 4 ? 4 : (hg > 64 ? 64 : hg);
   b->smem_per_warp = ag::make_smem_offsets(L, b->HG, b->so);
-  if ((size_t)b->smem_per_warp + 2 * ag::kZeroTileBytes > 227 * 1024) {  // (room for one warp with both tiles at full size)
-    delete b;
+  if ((size_t)b->smem_per_warp + 2 * ag::kZeroTileBytes > (size_t)b->step_launch.smem_optin)  // (room for one warp with both tiles at full size)
     return agarcl_set_error(AGARCL_ERR_INVALID, "configuration needs %u B of shared memory per instance (too many pellets/viruses)", b->smem_per_warp);
-  }
-#define ALLOC(ptr, bytes)                                                                           \
-  do {                                                                                              \
-    cudaError_t e__ = cudaMalloc((void**)&(ptr), (bytes));                                          \
-    if (e__ != cudaSuccess) {                                                                       \
-      agarcl_batch_destroy(b);                                                                      \
-      return agarcl_set_error(AGARCL_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", (size_t)(bytes), cudaGetErrorString(e__)); \
-    }                                                                                               \
-  } while (0)
-  const size_t NA = (size_t)b->N * b->A;
-  ALLOC(b->d_state, (size_t)b->N * L.stride);
-  ALLOC(b->d_obs, b->obs_bytes);
-  ALLOC(b->d_rewards, NA * sizeof(double));
-  ALLOC(b->d_dones, NA);
-  ALLOC(b->d_before, NA * sizeof(float));
-  ALLOC(b->d_dxdy, NA * 2 * sizeof(float));
-  ALLOC(b->d_act, NA * sizeof(int32_t));
-  ALLOC(b->d_seeds, (size_t)b->N * sizeof(uint64_t));
-  ALLOC(b->d_mask, (size_t)b->N);
-  ALLOC(b->d_tickets, 2 * sizeof(uint32_t));
-  ALLOC(b->d_cost, (size_t)b->N * sizeof(uint32_t));
-  ALLOC(b->d_perm, (size_t)b->N * sizeof(uint32_t));
-  cudaMemset(b->d_tickets, 0, 2 * sizeof(uint32_t));
-  ALLOC(b->d_sched, 2 * sizeof(uint32_t));
-  { const uint32_t init[2] = {1u, 0u}; cudaMemcpy(b->d_sched, init, sizeof(init), cudaMemcpyHostToDevice); }
-  if (const char* e = std::getenv("AGARCL_AUTO_SCHEDULE")) b->auto_schedule = std::atoi(e);
-  ALLOC(b->d_fresh, (size_t)b->N);
-  cudaMemset(b->d_fresh, 1, (size_t)b->N);
-  ALLOC(b->d_flagbuf, 33 * sizeof(uint32_t));
-  if (L.cap_replay > 0) ALLOC(b->d_replay, (size_t)b->N * L.cap_replay * sizeof(float));
-  if (cfg->ram_obs) {
-    ALLOC(b->d_ram, (size_t)b->N * L.P * AGARCL_RAM_RECORD * sizeof(float));
-    cudaMemset(b->d_ram, 0, (size_t)b->N * L.P * AGARCL_RAM_RECORD * sizeof(float));
-  }
-  ALLOC(b->d_lut_radius, AGARCL_LUT_SIZE * sizeof(float));
-  ALLOC(b->d_lut_speed, AGARCL_LUT_SIZE * sizeof(float));
-  ALLOC(b->d_lut_split, AGARCL_LUT_SIZE * sizeof(float));
-#undef ALLOC
-  cudaMemset(b->d_state, 0, (size_t)b->N * L.stride);
-  cudaMemset(b->d_obs, 0, b->obs_bytes);
-  cudaMemset(b->d_rewards, 0, NA * sizeof(double));
-  cudaMemset(b->d_dones, 0, NA);
-  cudaMemset(b->d_dxdy, 0, NA * 2 * sizeof(float));
-  cudaMemset(b->d_act, 0, NA * sizeof(int32_t));
-  if (b->d_replay) cudaMemset(b->d_replay, 0, (size_t)b->N * L.cap_replay * sizeof(float));
+  const size_t NA = (size_t)b->N * b->A, lut_bytes = AGARCL_LUT_SIZE * sizeof(float);
+  if ((rc = alloc(b->d_state, (size_t)b->N * L.stride, 0)) || (rc = alloc(b->d_obs, b->obs_bytes, 0)) ||
+      (rc = alloc(b->d_rewards, NA * sizeof(double), 0)) || (rc = alloc(b->d_dones, NA, 0)) || (rc = alloc(b->d_before, NA * sizeof(float))) ||
+      (rc = alloc(b->d_dxdy, NA * 2 * sizeof(float), 0)) || (rc = alloc(b->d_act, NA * sizeof(int32_t), 0)) ||
+      (rc = alloc(b->d_seeds, (size_t)b->N * sizeof(uint64_t))) || (rc = alloc(b->d_mask, (size_t)b->N)) ||
+      (rc = alloc(b->d_tickets, 2 * sizeof(uint32_t), 0)) || (rc = alloc(b->d_cost, (size_t)b->N * sizeof(uint32_t))) ||
+      (rc = alloc(b->d_perm, (size_t)b->N * sizeof(uint32_t))) || (rc = alloc(b->d_sched, 2 * sizeof(uint32_t))) ||
+      (rc = alloc(b->d_fresh, (size_t)b->N, 1)) || (rc = alloc(b->d_flagbuf, 33 * sizeof(uint32_t))) ||
+      (L.cap_replay > 0 && (rc = alloc(b->d_replay, (size_t)b->N * L.cap_replay * sizeof(float), 0))) ||
+      (cfg->ram_obs && (rc = alloc(b->d_ram, (size_t)b->N * L.P * AGARCL_RAM_RECORD * sizeof(float), 0))) ||
+      (rc = alloc(b->d_lut_radius, lut_bytes)) || (rc = alloc(b->d_lut_speed, lut_bytes)) || (rc = alloc(b->d_lut_split, lut_bytes)))
+    return rc;
+  { const uint32_t init[2] = {1u, 0u}; CK(cudaMemcpy(b->d_sched, init, sizeof(init), cudaMemcpyHostToDevice)); }
   b->cur_dxdy = b->d_dxdy;
   b->cur_act = b->d_act;
   // lookup tables of functions of an integer mass, computed with the host libm the reference uses
@@ -386,9 +378,9 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
       v = (v < 20.0) ? 20.0 : v;
       spl[m] = (float)v;
     }
-    cudaMemcpy(b->d_lut_radius, rad.data(), rad.size() * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(b->d_lut_speed, spd.data(), spd.size() * 4, cudaMemcpyHostToDevice);
-    cudaMemcpy(b->d_lut_split, spl.data(), spl.size() * 4, cudaMemcpyHostToDevice);
+    CK(cudaMemcpy(b->d_lut_radius, rad.data(), lut_bytes, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(b->d_lut_speed, spd.data(), lut_bytes, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(b->d_lut_split, spl.data(), lut_bytes, cudaMemcpyHostToDevice));
     b->T.radius = b->d_lut_radius;
     b->T.max_speed = b->d_lut_speed;
     b->T.split_speed = b->d_lut_split;
@@ -400,11 +392,9 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
   b->max_draws_per_step = 2 * ((int64_t)L.cap_pellets + L.cap_viruses + L.P);  // regen deficits + respawns of one step; a whole reset
   if (cfg->rng_mode == AGARCL_RNG_MT19937) {
     // an UNSEEDED reference environment draws from std::random_device (GameState.hpp:59): so does an unseeded batch
-    if ((int64_t)L.cap_replay <= b->max_draws_per_step) {
-      agarcl_batch_destroy(b);
+    if ((int64_t)L.cap_replay <= b->max_draws_per_step)
       return agarcl_set_error(AGARCL_ERR_INVALID, "cap_replay %d cannot hold the draws of one step (%lld): raise cfg.cap_replay", L.cap_replay,
                               (long long)b->max_draws_per_step);
-    }
     b->gens.resize(b->N);
     b->filled.assign(b->N, 0);
     std::random_device rd;
@@ -412,14 +402,13 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
       uint64_t s0;
       try { s0 = rd(); } catch (...) { s0 = (uint64_t)(cfg->instance_base + i) * 0x9E3779B97F4A7C15ull + 1u; }
       b->seeds[i] = s0 & 0xffffffffull;
-      int rc2 = mt_restart(b, i, b->seeds[i], 0);
-      if (rc2) { agarcl_batch_destroy(b); return rc2; }
+      if ((rc = mt_restart(b.get(), i, b->seeds[i], 0))) return rc;
     }
     b->draw_budget = L.cap_replay;
   }
-  cudaMemcpy(b->d_seeds, b->seeds.data(), b->N * sizeof(uint64_t), cudaMemcpyHostToDevice);
+  CK(cudaMemcpy(b->d_seeds, b->seeds.data(), b->N * sizeof(uint64_t), cudaMemcpyHostToDevice));
   CK(cudaDeviceSynchronize());
-  *out = b;
+  *out = b.release();
   return AGARCL_OK;
 }
 
@@ -584,7 +573,7 @@ extern "C" int agarcl_batch_reset(agarcl_batch* b, const uint8_t* mask, void* st
   CK(cudaSetDevice(b->cfg.device));
   cudaStream_t s = (cudaStream_t)stream;
   if (mask) CK(cudaMemcpyAsync(b->d_mask, mask, b->N, cudaMemcpyHostToDevice, s));
-  return reset_impl(b, mask ? b->d_mask : nullptr, s, true);
+  return reset_impl(b, mask ? b->d_mask.get() : nullptr, s, true);
 }
 
 extern "C" int agarcl_batch_reset_device(agarcl_batch* b, const uint8_t* d_mask, void* stream) {
@@ -624,45 +613,41 @@ static int step_impl(agarcl_batch* b, cudaStream_t s, bool want_lists, bool* lis
     // quirk Q11: one _partial_observation(agent, 0) after all ticks, frame_index = -(tps - num_frames)
     P.n_ticks = tps; P.do_begin = 1; P.do_end = 1;
     CK(cudaMemsetAsync(b->d_obs, 0, b->obs_bytes, s));  // _step_hook: clear_data
-    CK(ag::launch_step(P, s)); launches++;
+    CK(ag::launch_step(P, b->step_launch, s)); launches++;
     int frame = 0 - (tps - b->frames);
     if (frame >= 0) { int rc = render_frame(b, frame, s, 1); if (rc) return rc; launches++; }
-  } else if (b->cfg.ram_obs == 2) {
-    // structured observation only (agario-ram-v0): no grid frame is rendered at all
+  } else if (b->cfg.ram_obs == 2 || b->frames == 1) {
+    // one k_step runs every tick of the step; a grid frame (none with the structured observation only, agario-ram-v0) is
+    // finished by k_step itself or by k_obs behind it
+    const bool grid = b->cfg.ram_obs != 2;
     P.n_ticks = tps; P.do_begin = 1; P.do_end = 1;
-    const bool sorted = P.tick_barrier && b->sort_schedule;
-    if (sorted) { P.cost = b->d_cost; P.perm = b->perm_valid ? b->d_perm : nullptr; P.sched = b->auto_schedule ? b->d_sched : nullptr; }
-    if (b->timing) { if (b->ev_used >= 3 * 2048) collect_timing(b); CK(cudaEventRecord(next_event(b), s)); }
-    CK(ag::launch_step(P, s)); launches++;
-    if (b->timing) CK(cudaEventRecord(next_event(b), s));
-    if (sorted) { CK(ag::launch_order(b->d_cost, b->d_perm, b->N, P.sched, s)); b->perm_valid = true; launches++; }
-  } else if (b->frames == 1) {
-    P.n_ticks = tps; P.do_begin = 1; P.do_end = 1;
-    const int fused = fuse_obs_clear(b, P, 0) ? 1 : 0;
+    const int fused = grid && fuse_obs_clear(b, P, 0) ? 1 : 0;
     if (want_lists && P.obs_finish && target && 6 + 2 * ((b->G + 31) / 32) <= 32) {  // (the image's record is one warp store)
       P.pk = ag::mirror_pack_out(target);
       *lists_made = true;
     }
-    const bool sorted = P.tick_barrier && b->sort_schedule;
-    if (sorted) { P.cost = b->d_cost; P.perm = b->perm_valid ? b->d_perm : nullptr; P.sched = b->auto_schedule ? b->d_sched : nullptr; }
+    const bool sorted = P.tick_barrier && b->knobs.sort_schedule;
+    if (sorted) { P.cost = b->d_cost; P.perm = b->perm_valid ? b->d_perm.get() : nullptr; P.sched = b->knobs.auto_schedule ? b->d_sched.get() : nullptr; }
     if (b->timing) { if (b->ev_used >= 3 * 2048) collect_timing(b); CK(cudaEventRecord(next_event(b), s)); }
-    CK(ag::launch_step(P, s)); launches++;
+    CK(ag::launch_step(P, b->step_launch, s)); launches++;
     if (b->timing) CK(cudaEventRecord(next_event(b), s));
     if (sorted) { CK(ag::launch_order(b->d_cost, b->d_perm, b->N, P.sched, s)); b->perm_valid = true; launches++; }
-    if (!P.obs_finish) { int rc = render_frame(b, 0, s, 1, fused); if (rc) return rc; launches++; }
-    if (b->timing) CK(cudaEventRecord(next_event(b), s));
+    if (grid) {
+      if (!P.obs_finish) { int rc = render_frame(b, 0, s, 1, fused); if (rc) return rc; launches++; }
+      if (b->timing) CK(cudaEventRecord(next_event(b), s));
+    }
   } else {
     // the last num_frames ticks of the step each contribute one frame (the documented intent of
     // GridEnvironment::_partial_observation, GridEnvironment.hpp:413-433)
     if (b->frames > tps) CK(cudaMemsetAsync(b->d_obs, 0, b->obs_bytes, s));
     for (int t = 0; t < tps; t++) {
       P.n_ticks = 1; P.do_begin = (t == 0); P.do_end = 0;
-      CK(ag::launch_step(P, s)); launches++;
+      CK(ag::launch_step(P, b->step_launch, s)); launches++;
       int frame = t - (tps - b->frames);
       if (frame >= 0) { int rc = render_frame(b, frame, s, 1); if (rc) return rc; launches++; }
     }
     P.n_ticks = 0; P.do_begin = 0; P.do_end = 1;
-    CK(ag::launch_step(P, s)); launches++;
+    CK(ag::launch_step(P, b->step_launch, s)); launches++;
   }
   if (b->d_ram) {
     int rc = render_ram(b, s, 1); if (rc) return rc; launches++;
@@ -683,26 +668,15 @@ extern "C" int agarcl_batch_set_autoreset(agarcl_batch* b, int32_t max_steps, in
   if (keep_final_obs && !reset) return agarcl_set_error(AGARCL_ERR_INVALID, "keep_final_obs needs reset: nothing is overwritten without one");
   CK(cudaSetDevice(b->cfg.device));
   const size_t NA = (size_t)b->N * b->A;
-#define ALLOC0(ptr, bytes)                                                                                            \
-  do {                                                                                                                \
-    if (!(ptr)) {                                                                                                     \
-      cudaError_t e__ = cudaMalloc((void**)&(ptr), (bytes));                                                          \
-      if (e__ != cudaSuccess)                                                                                         \
-        return agarcl_set_error(AGARCL_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", (size_t)(bytes), cudaGetErrorString(e__)); \
-      CK(cudaMemset((ptr), 0, (bytes)));                                                                              \
-    }                                                                                                                 \
-  } while (0)
-  ALLOC0(b->d_done_out, NA);
-  ALLOC0(b->d_reset_mask, (size_t)b->N);
-  ALLOC0(b->d_steps, (size_t)b->N * sizeof(int64_t));
-  ALLOC0(b->d_final_len, (size_t)b->N * sizeof(int64_t));
-  ALLOC0(b->d_ret, NA * sizeof(double));
-  ALLOC0(b->d_final_ret, NA * sizeof(double));
+  int rc;
+  if ((rc = alloc(b->d_done_out, NA, 0)) || (rc = alloc(b->d_reset_mask, (size_t)b->N, 0)) ||
+      (rc = alloc(b->d_steps, (size_t)b->N * sizeof(int64_t), 0)) || (rc = alloc(b->d_final_len, (size_t)b->N * sizeof(int64_t), 0)) ||
+      (rc = alloc(b->d_ret, NA * sizeof(double), 0)) || (rc = alloc(b->d_final_ret, NA * sizeof(double), 0)))
+    return rc;
   if (keep_final_obs) {
-    if (b->cfg.ram_obs != 2) ALLOC0(b->d_final_obs, b->obs_bytes);
-    if (b->d_ram) ALLOC0(b->d_final_ram, (size_t)b->N * b->L.P * AGARCL_RAM_RECORD * sizeof(float));
+    if (b->cfg.ram_obs != 2 && (rc = alloc(b->d_final_obs, b->obs_bytes, 0))) return rc;
+    if (b->d_ram && (rc = alloc(b->d_final_ram, (size_t)b->N * b->L.P * AGARCL_RAM_RECORD * sizeof(float), 0))) return rc;
   }
-#undef ALLOC0
   // every instance starts counting here
   CK(cudaMemset(b->d_steps, 0, (size_t)b->N * sizeof(int64_t)));
   CK(cudaMemset(b->d_ret, 0, NA * sizeof(double)));
@@ -738,8 +712,8 @@ extern "C" int agarcl_batch_episode(agarcl_batch* b, agarcl_episode* out) {
   out->steps = b->d_steps;
   out->final_return = b->d_final_ret;
   out->final_length = b->d_final_len;
-  out->final_obs = b->keep_final ? b->d_final_obs : nullptr;
-  out->final_ram = b->keep_final ? b->d_final_ram : nullptr;
+  out->final_obs = b->keep_final ? b->d_final_obs.get() : nullptr;
+  out->final_ram = b->keep_final ? b->d_final_ram.get() : nullptr;
   return AGARCL_OK;
 }
 
@@ -914,7 +888,7 @@ extern "C" int agarcl_batch_lists_expand(agarcl_batch* b, int32_t image, void* d
   if (ag::mirror_lists_expand(b->lists, image, dense_out) == 1) {  // overflowed its slot: the dense frame is on the device
     CK(cudaSetDevice(b->cfg.device));
     const size_t bytes = b->obs_bytes / ((size_t)b->N * b->A);
-    CK(cudaMemcpy(dense_out, (const uint8_t*)b->d_obs + bytes * (size_t)image, bytes, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(dense_out, (const uint8_t*)b->d_obs.get() + bytes * (size_t)image, bytes, cudaMemcpyDeviceToHost));
   }
   return AGARCL_OK;
 }

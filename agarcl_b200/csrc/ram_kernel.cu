@@ -173,16 +173,22 @@ __global__ void __launch_bounds__(kRamWarps * 32) k_ram(const __grid_constant__ 
   }
 }
 
+// pellets + one candidate list per warp
+static size_t ram_smem(const agarcl_layout& L) {
+  const size_t cand_cap = ((size_t)L.cap_pellets + 7) & ~(size_t)7;
+  return cand_cap * sizeof(float2) + (size_t)kRamWarps * cand_cap * sizeof(uint16_t);
+}
+
+cudaError_t setup_ram(const agarcl_layout& L, int smem_optin) {
+  const size_t smem = ram_smem(L);
+  if (smem > (size_t)smem_optin) return cudaErrorInvalidValue;
+  // (the device's whole opt-in, so that the batches of other layouts on this device keep what they were set up with)
+  if (smem > 48 * 1024) return cudaFuncSetAttribute(k_ram, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin);
+  return cudaSuccess;
+}
+
 cudaError_t launch_ram(const RamParams& P, cudaStream_t stream) {
-  const size_t cand_cap = ((size_t)P.L.cap_pellets + 7) & ~(size_t)7;
-  size_t smem = cand_cap * sizeof(float2) + (size_t)kRamWarps * cand_cap * sizeof(uint16_t);  // pellets + one candidate list per warp
-  static size_t configured = 0;
-  if (smem > 48 * 1024 && smem > configured) {
-    cudaError_t e = cudaFuncSetAttribute(k_ram, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    configured = smem;
-  }
-  k_ram<<<P.N, kRamWarps * 32, smem, stream>>>(P);
+  k_ram<<<P.N, kRamWarps * 32, ram_smem(P.L), stream>>>(P);
   return cudaGetLastError();
 }
 

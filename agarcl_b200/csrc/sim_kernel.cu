@@ -3244,25 +3244,23 @@ cudaError_t selftest_std_sort(const float* ys, int n, uint16_t* order_out) {
   return e;
 }
 
-// One CTA per SM, as many warps (= concurrent instances) as the shared memory holds, at most kMaxWarpsPerCta.
-cudaError_t launch_step(const SimParams& P, cudaStream_t stream) {
-  static int sms = 0, smem_max = 0;
+cudaError_t setup_step(int warps_cap, StepLaunch& S) {
+  int dev = 0;
   cudaError_t e;
-  if (sms == 0) {
-    int dev = 0;
-    if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
-    if ((e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    if ((e = cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
-    if ((e = cudaFuncSetAttribute(k_step, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max)) != cudaSuccess) return e;
-  }
-  int warps = (int)(((size_t)smem_max - P.tiles_bytes) / P.smem_per_warp);
-  if (warps > kMaxWarpsPerCta) warps = kMaxWarpsPerCta;
-  static const int cap = [] { const char* e = std::getenv("AGARCL_WARPS"); return e ? std::atoi(e) : 0; }();  // (A/B timing)
-  if (cap > 0 && warps > cap) warps = cap;
+  if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+  if ((e = cudaDeviceGetAttribute(&S.sms, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
+  if ((e = cudaDeviceGetAttribute(&S.smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
+  S.max_warps = warps_cap > 0 && warps_cap < kMaxWarpsPerCta ? warps_cap : kMaxWarpsPerCta;
+  return cudaFuncSetAttribute(k_step, cudaFuncAttributeMaxDynamicSharedMemorySize, S.smem_optin);
+}
+
+cudaError_t launch_step(const SimParams& P, const StepLaunch& S, cudaStream_t stream) {
+  int warps = (int)(((size_t)S.smem_optin - P.tiles_bytes) / P.smem_per_warp);
+  if (warps > S.max_warps) warps = S.max_warps;
   if (warps < 1) return cudaErrorInvalidConfiguration;
   const size_t smem = (size_t)P.tiles_bytes + (size_t)P.smem_per_warp * warps;
   int ctas = (P.N + warps - 1) / warps;
-  if (ctas > sms) ctas = sms;
+  if (ctas > S.sms) ctas = S.sms;
   k_step<<<ctas, warps * 32, smem, stream>>>(P);
   return cudaGetLastError();
 }

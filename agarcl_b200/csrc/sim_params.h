@@ -1,5 +1,7 @@
 // sim_params.h — kernel parameter blocks shared by the host API (batch.cu) and the kernels.
 #pragma once
+#include <cuda_runtime.h>
+
 #include <cstdint>
 
 #include "../../include/agarcl_b200.h"
@@ -118,6 +120,20 @@ struct SimParams {
   int32_t inst_first;           // this launch steps instances [inst_first, inst_first + N) of the batch
 };
 
+// How k_step is launched on one device: found by setup_step when a batch is created there and kept by the batch, because
+// function attributes belong to the device's context and a process may hold batches on several devices
+struct StepLaunch {
+  int sms;         // k_step's persistent grid has at most one CTA per SM
+  int smem_optin;  // opt-in shared memory per block: the dynamic shared memory k_step (and k_ram) may use on this device
+  int max_warps;   // warps per CTA at most: kMaxWarpsPerCta, or fewer when capped (AGARCL_WARPS)
+};
+// On the current device: fills S and opts k_step in to S.smem_optin bytes of dynamic shared memory.  warps_cap > 0 caps S.max_warps.
+cudaError_t setup_step(int warps_cap, StepLaunch& S);
+// One CTA per SM, as many warps (= concurrent instances) as the shared memory holds, at most S.max_warps.
+cudaError_t launch_step(const SimParams& P, const StepLaunch& S, cudaStream_t stream);
+cudaError_t launch_order(const uint32_t* cost, uint32_t* perm, int N, uint32_t* sched, cudaStream_t stream);
+cudaError_t selftest_std_sort(const float* ys, int n, uint16_t* order_out);
+
 struct ResetParams {
   agarcl_layout L;
   Luts T;
@@ -132,6 +148,8 @@ struct ResetParams {
   int32_t N, instance_base, rng_mode, num_pellets, num_viruses;
   float W;
 };
+cudaError_t launch_reset(const ResetParams& P, cudaStream_t stream);
+cudaError_t launch_flags(const uint8_t* state, const agarcl_layout& L, int N, uint32_t* out33, cudaStream_t stream);
 
 struct ObsParams {
   agarcl_layout L;
@@ -145,6 +163,7 @@ struct ObsParams {
   const uint8_t* mask;     // [N] or nullptr: render only the instances with mask != 0 (masked reset)
   float W;
 };
+cudaError_t launch_obs(const ObsParams& P, cudaStream_t stream);
 
 struct RamParams {
   agarcl_layout L;
@@ -155,6 +174,9 @@ struct RamParams {
   int32_t pre_respawn;     // 1: players respawned at the end of the step are still dead (BaseEnvironment.hpp:96-101)
   int32_t pid_base;        // CloneInfo::owner is the player's pid: index + pid of player 0 (non-zero only in later episodes of strict_reference, Q3)
 };
+// On the current device: opts k_ram in to the dynamic shared memory it needs for layout L (up to smem_optin bytes)
+cudaError_t setup_ram(const agarcl_layout& L, int smem_optin);
+cudaError_t launch_ram(const RamParams& P, cudaStream_t stream);
 
 constexpr int kMaskedThreads = 512;  // threads of k_masked_bytes, one CTA per instance
 
@@ -173,5 +195,8 @@ struct EpisodeParams {
   int32_t reset;             // 1: finished instances are reset by this step (auto-reset); 0: bookkeeping only
   int32_t clear;             // 1: a reset restarts the counters of clear_mask's instances (no step)
 };
+cudaError_t launch_episode(const EpisodeParams& P, cudaStream_t stream);
+// dst = src (nullptr: zeros) in the `per`-byte slices of the instances with mask != 0
+cudaError_t launch_masked_bytes(void* dst, const void* src, size_t per, const uint8_t* mask, int N, cudaStream_t stream);
 
 }  // namespace ag
