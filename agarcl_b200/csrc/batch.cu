@@ -214,6 +214,17 @@ static void fill_sim_params(const agarcl_batch* b, ag::SimParams& P) {
   P.inst_first = 0;
 }
 
+// Whether the engine-tick kernel writes the whole observation frame itself (SimParams::obs_finish): 0 no (k_obs renders
+// it), 1 int32, 2 int16.  Needs the fused clear, rows of whole 16-byte vectors, one row of channel 0 = one bulk store from
+// the ones tile, and the row of y masks in the collision scratch.
+static int obs_finish_kind(const agarcl_batch* b) {
+  const size_t esz = b->cfg.obs_dtype == AGARCL_OBS_I16 ? 2 : 4;
+  const size_t row = (size_t)b->G * esz;
+  if ((row * b->G) % 16 != 0 || b->C < 2 || b->knobs.fuse_clear < 2) return 0;
+  if (row % 16 != 0 || row > (size_t)ag::kZeroTileBytes || row > (size_t)(b->so.vcache - b->so.cellref)) return 0;
+  return esz == 2 ? 2 : 1;
+}
+
 // Lets the engine-tick kernel clear channels 1..C-1 of frame slot `frame` (see SimParams); false when
 // the planes are not 16-byte multiples.
 static bool fuse_obs_clear(const agarcl_batch* b, ag::SimParams& P, int frame) {
@@ -224,12 +235,17 @@ static bool fuse_obs_clear(const agarcl_batch* b, ag::SimParams& P, int frame) {
   P.zero_skip_vec = (uint32_t)(plane / 16);
   P.zero_vec_per_agent = (uint32_t)((size_t)(b->C - 1) * plane / 16);
   P.agent_stride_vec = (uint32_t)((size_t)b->frames * b->C * plane / 16);
-  // the whole observation in the engine-tick kernel: rows of whole 16-byte vectors, masks fit the scratch (1: int32, 2: int16)
-  P.obs_finish = (b->knobs.fuse_clear >= 2 && ((size_t)b->G * esz) % 16 == 0 &&
-                  (size_t)b->G * esz <= (size_t)ag::kZeroTileBytes &&  // one row of channel 0 = one bulk store from the ones tile
-                  (size_t)b->G * esz <= (size_t)(b->so.vcache - b->so.cellref)) ? (esz == 2 ? 2 : 1) : 0;
+  P.obs_finish = obs_finish_kind(b);
   if (P.obs_finish) P.tiles_bytes = ag::kZeroTileBytes + (((uint32_t)b->G * (uint32_t)esz + 127u) & ~127u);
   return true;
+}
+
+// Whether the one-frame step's k_step also writes the host lists of every image (agarcl_batch_step_mirror / _step_lists):
+// it finishes the observation itself, and an image's record (count, base, image, row and column masks, reward, done) is
+// one store of a warp's 32 lanes.
+static bool kernel_writes_lists(const agarcl_batch* b) {
+  return b->frames == 1 && !b->cfg.strict_reference && b->cfg.ram_obs != 2 && obs_finish_kind(b) != 0 &&
+         6 + 2 * ((b->G + 31) / 32) <= 32;
 }
 
 static void fill_obs_params(const agarcl_batch* b, ag::ObsParams& P, int frame, int pre_respawn, int skip_zero = 0) {
@@ -622,7 +638,7 @@ static int step_impl(agarcl_batch* b, cudaStream_t s, bool want_lists, bool* lis
     const bool grid = b->cfg.ram_obs != 2;
     P.n_ticks = tps; P.do_begin = 1; P.do_end = 1;
     const int fused = grid && fuse_obs_clear(b, P, 0) ? 1 : 0;
-    if (want_lists && P.obs_finish && target && 6 + 2 * ((b->G + 31) / 32) <= 32) {  // (the image's record is one warp store)
+    if (want_lists && target && kernel_writes_lists(b)) {
       P.pk = ag::mirror_pack_out(target);
       *lists_made = true;
     }
@@ -862,6 +878,8 @@ extern "C" int agarcl_batch_step_lists(agarcl_batch* b, const float* dxdy, const
   if (!b || !dxdy || !act || !out) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
   if (b->frames != 1 || b->cfg.strict_reference || b->cfg.ram_obs == 2)
     return agarcl_set_error(AGARCL_ERR_STATE, "observation lists need the single fused step kernel (one frame, strict_reference = 0, a grid observation)");
+  if (!kernel_writes_lists(b))  // (refused before anything is enqueued: the games do not move)
+    return agarcl_set_error(AGARCL_ERR_STATE, "this observation configuration is not finished by the step kernel: no lists");
   CK(cudaSetDevice(b->cfg.device));
   if (!b->lists) {
     b->lists = ag::mirror_create(b->N * b->A, b->A, b->frames * b->C, b->C, b->G, b->cfg.obs_dtype, true);
@@ -871,9 +889,9 @@ extern "C" int agarcl_batch_step_lists(agarcl_batch* b, const float* dxdy, const
   bool lists_made = false;
   int rc = step_impl(b, nullptr, true, &lists_made, b->lists);
   if (rc) return rc;
-  if (!lists_made) {
+  if (!lists_made) {  // (kernel_writes_lists said it would)
     CK(cudaStreamSynchronize(nullptr));
-    return agarcl_set_error(AGARCL_ERR_STATE, "this observation configuration is not finished by the step kernel: no lists");
+    return agarcl_set_error(AGARCL_ERR_STATE, "the step kernel did not write the observation lists");
   }
   rc = ag::mirror_collect_lists(b->lists, nullptr, rewards_out, dones_out);
   if (rc) return rc;

@@ -42,12 +42,25 @@ def philox_uniform_np(seed, instance, k):
     return ((w >> np.uint64(8)).astype(np.float32) * np.float32(1.0 / 16777216.0)).astype(np.float32)
 
 
+def _obs_diff(what, g, o):
+    bad = [(a, c, int((g[a][c] != o[a][c]).sum())) for a in range(o.shape[0]) for c in range(o.shape[1])
+           if not np.array_equal(g[a][c], o[a][c])]
+    return f"{what}: obs differs (agent, channel, #cells): {bad[:8]}"
+
+
 def run_parity(cfg_kwargs, seeds, steps, p_feed=1 / 3, p_split=1 / 3, boost=None, obs_every=5, replay_len=1 << 16,
-               with_obs_in_step=True, ram=False, philox=False, state_every=1, instance_base=0):
+               with_obs_in_step=True, ram=False, philox=False, state_every=1, instance_base=0, obs_ref=None, edit=None,
+               via="step"):
     """Runs len(seeds) instances on the GPU in one batch and each one through the oracle.
     philox: the GPU draws from its own counter-based Philox stream (AGARCL_RNG_PHILOX, what bench.py runs) and the oracle is
     fed the same stream computed by philox_uniform_np; otherwise both replay the mt19937_64 stream of the seed.
-    state_every: the full state is compared every that many steps (rewards and dones every step)."""
+    state_every: the full state is compared every that many steps (rewards and dones every step).
+    obs_ref: applied to the oracle's int32 frames before they are compared (int16: np.clip to the int16 range, which is
+    exact because every scatter operation is monotone).
+    edit(i, state_view): applied to the oracle's and the device's state of instance i after the reset, before the first step.
+    via: "step" (Batch.step), "mirror" (Batch.step_mirror; the host mirror is compared with the oracle as well) or "lists"
+    (Batch.step_lists; every image of ObsLists.expand and the numpy decoder on a sample are compared with the oracle).
+    The returned stats hold the launch counts seen (`launches`, sorted)."""
     oracle_lib().oracle_set_trig_mode(1)
     n = len(seeds)
     if philox:
@@ -72,6 +85,9 @@ def run_parity(cfg_kwargs, seeds, steps, p_feed=1 / 3, p_split=1 / 3, boost=None
         oras.append(o)
     b.seed(np.asarray(seeds, dtype=np.uint64))
     b.reset()
+    if ocfg.strict_reference:  # the player order the batch's reset made (quirk Q3)
+        for k in range(L.P):
+            Lo.order[k] = b.layout.order[k]
     for o in oras:
         o.reset()
     if boost:
@@ -81,6 +97,12 @@ def run_parity(cfg_kwargs, seeds, steps, p_feed=1 / 3, p_split=1 / 3, boost=None
             sv = b.download_state(i)
             for a in range(L.A):
                 sv.cells[a][0]["mass"] = boost
+            b.upload_state(i, sv)
+    if edit:
+        for i, o in enumerate(oras):
+            edit(i, o.state)
+            sv = b.download_state(i)
+            edit(i, sv)
             b.upload_state(i, sv)
     for i, o in enumerate(oras):
         d = compare_states(o.state, b.download_state(i))
@@ -95,16 +117,28 @@ def run_parity(cfg_kwargs, seeds, steps, p_feed=1 / 3, p_split=1 / 3, boost=None
             o.ram_clear()
     rngs = [np.random.default_rng(s) for s in seeds]
     A = L.A
+    launches = set()
+    h_rew, h_done = np.zeros(n * A, np.float64), np.zeros(n * A, np.uint8)
     for st in range(steps):
         dxdy = np.zeros((n, A, 2), np.float32)
         act = np.zeros((n, A), np.int32)
         for i in range(n):
             dxdy[i], act[i] = random_actions(rngs[i], A, p_feed, p_split)
-        b.set_actions(dxdy, act)
-        b.step()
+        if via == "step":
+            b.set_actions(dxdy, act)
+            b.step()
+        elif via == "mirror":
+            h_obs = b.step_mirror(dxdy, act, h_rew, h_done).reshape(n, A, *b.obs_shape[1:])
+        elif via == "lists":
+            lists = b.step_lists(dxdy, act, h_rew, h_done)
+        else:
+            raise ValueError(f"via={via!r}")
+        launches.add(b.launches_per_step())
         torch.cuda.synchronize()
         g_rew = rew_t.cpu().numpy().reshape(n, A)
         g_done = done_t.cpu().numpy().reshape(n, A)
+        if via != "step":  # what the host copy of the step handed out
+            assert np.array_equal(h_rew.reshape(n, A), g_rew) and np.array_equal(h_done.reshape(n, A), g_done), f"step {st}: {via} rewards / dones"
         want_obs = (st % obs_every == 0)
         g_obs = obs_t.cpu().numpy().reshape(n, A, *b.obs_shape[1:]) if want_obs else None
         g_ram = ram_t.cpu().numpy() if ram else None
@@ -129,15 +163,26 @@ def run_parity(cfg_kwargs, seeds, steps, p_feed=1 / 3, p_split=1 / 3, boost=None
             if want_obs:
                 if o_obs is None:
                     o_obs = np.stack([o.obs(a) for a in range(A)])
+                if obs_ref is not None:
+                    o_obs = obs_ref(o_obs)
                 if not np.array_equal(g_obs[i], o_obs):
                     bad = [(a, c, int((g_obs[i][a][c] != o_obs[a][c]).sum())) for a in range(A) for c in range(o_obs.shape[1])
                            if not np.array_equal(g_obs[i][a][c], o_obs[a][c])]
                     raise AssertionError(f"step {st} inst {i}: obs differs (agent, channel, #cells): {bad[:8]}")
+                if via == "mirror" and not np.array_equal(h_obs[i], o_obs):
+                    raise AssertionError(_obs_diff(f"step {st} inst {i}: host mirror", h_obs[i], o_obs))
+                if via == "lists":
+                    ex = np.stack([lists.expand(i * A + a) for a in range(A)])
+                    if not np.array_equal(ex, o_obs):
+                        raise AssertionError(_obs_diff(f"step {st} inst {i}: lists (C decoder)", ex, o_obs))
+                    dec = lists.decode(i * A + st % A)  # (slow: one image per instance and step; None: it took the dense copy)
+                    assert dec is None or np.array_equal(dec, o_obs[st % A]), f"step {st} inst {i}: lists (numpy decoder)"
     stats = dict(cells_eaten=sum(int(o.state.players["cells_eaten"].sum()) for o in oras),
                  viruses_eaten=sum(int(o.state.players["viruses_eaten"].sum()) for o in oras),
                  food_eaten=sum(int(o.state.players["food_eaten"].sum()) for o in oras),
                  max_cells=max(int(o.state.players["n_cells"].max()) for o in oras),
                  foods=sum(int(o.state.hdr["n_foods"]) for o in oras),
-                 flags=sorted({f for o in oras for f in o.state.flag_names()}))
+                 flags=sorted({f for o in oras for f in o.state.flag_names()}),
+                 launches=sorted(launches))
     b.close()
     return stats
