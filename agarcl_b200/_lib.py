@@ -16,6 +16,7 @@ SYMBOLS = [
     "agarcl_batch_seed", "agarcl_batch_reset", "agarcl_batch_set_actions", "agarcl_batch_step",
     "agarcl_batch_obs", "agarcl_batch_rewards", "agarcl_batch_dones", "agarcl_batch_step_host",
     "agarcl_batch_reset_device", "agarcl_batch_set_autoreset", "agarcl_batch_step_autoreset", "agarcl_batch_episode",
+    "agarcl_snapshot_slot_bytes", "agarcl_batch_save_states", "agarcl_batch_restore_states",
     "agarcl_batch_mirror", "agarcl_batch_sync_mirror", "agarcl_batch_step_mirror", "agarcl_batch_mirror_stats", "agarcl_batch_mirror_timing", "agarcl_batch_step_lists", "agarcl_batch_lists_expand",
     "agarcl_batch_download_state", "agarcl_batch_upload_state", "agarcl_batch_save_env_state", "agarcl_batch_load_env_state",
     "agarcl_snapshot_write", "agarcl_snapshot_read", "agarcl_batch_set_replay",
@@ -53,6 +54,9 @@ def lib():
         L.agarcl_batch_set_autoreset.argtypes = [_vp, C.c_int32, C.c_int32, C.c_int32]
         L.agarcl_batch_step_autoreset.argtypes = [_vp, _vp]
         L.agarcl_batch_episode.argtypes = [_vp, _vp]
+        L.agarcl_snapshot_slot_bytes.argtypes = [C.POINTER(Cfg), C.POINTER(C.c_int64)]
+        L.agarcl_batch_save_states.argtypes = [_vp, _vp, C.c_int64, _vp, _vp, C.c_int32, _vp]
+        L.agarcl_batch_restore_states.argtypes = [_vp, _vp, C.c_int64, _vp, C.POINTER(_vp), _vp]
         L.agarcl_batch_mirror.argtypes = [_vp, C.POINTER(_vp), C.POINTER(C.c_int64 * 4), C.POINTER(C.c_int32)]
         L.agarcl_batch_sync_mirror.argtypes = [_vp, _vp]
         L.agarcl_batch_step_mirror.argtypes = [_vp, _vp, _vp, _vp, _vp]
@@ -91,3 +95,10 @@ def make_layout(cfg):
     L = Layout()
     check(lib().agarcl_make_layout(C.byref(cfg), C.byref(L)))
     return L
+
+
+def snapshot_slot_bytes(cfg):
+    """bytes of one snapshot slot of configuration `cfg` (a multiple of 128; slot layout: include/agarcl_b200.h)"""
+    n = C.c_int64()
+    check(lib().agarcl_snapshot_slot_bytes(C.byref(cfg), C.byref(n)))
+    return int(n.value)

@@ -325,6 +325,65 @@ class Batch:
         _lib.check(_lib.lib().agarcl_batch_flags(self._h, _vp(stream), C.byref(o), C.byref(counts)))
         return int(o.value), {FLAG_NAMES.get(1 << i, f"bit{i}"): int(counts[i]) for i in range(32) if counts[i]}
 
+    # ---- snapshot pools (include/agarcl_b200.h, agarcl_batch_save_states / agarcl_batch_restore_states)
+    @property
+    def slot_bytes(self):
+        """bytes of one snapshot slot of this batch's configuration"""
+        if getattr(self, "_slot_bytes", None) is None:
+            self._slot_bytes = _lib.snapshot_slot_bytes(self.cfg)
+        return self._slot_bytes
+
+    def snapshot_pool(self, slots):
+        """a zeroed pool of `slots` slots: torch.uint8 [slots, slot_bytes] on the batch's device"""
+        import torch
+        if int(slots) < 1:
+            raise _lib.AgarclError("a pool needs at least one slot")
+        return torch.zeros((int(slots), self.slot_bytes), dtype=torch.uint8, device=f"cuda:{self.cfg.device}")
+
+    def _check_device_tensor(self, t, dtype, what, numel=None):
+        import torch
+        dev = torch.device("cuda", self.cfg.device)
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.device == dev):
+            raise _lib.AgarclError(f"{what} must be a tensor on {dev}")
+        if t.dtype != dtype:
+            raise _lib.AgarclError(f"{what} must be {dtype}, got {t.dtype}")
+        if not t.is_contiguous():
+            raise _lib.AgarclError(f"{what} must be contiguous")
+        if numel is not None and t.numel() != numel:
+            raise _lib.AgarclError(f"{what} must have {numel} entries, got {t.numel()}")
+
+    def _check_pool(self, pool):
+        import torch
+        self._check_device_tensor(pool, torch.uint8, "the pool")
+        if pool.dim() != 2 or pool.shape[1] != self.slot_bytes or pool.shape[0] < 1:
+            raise _lib.AgarclError(f"the pool must be [slots >= 1, {self.slot_bytes}] (slot bytes of this configuration), "
+                                   f"got {list(pool.shape)}")
+        return int(pool.shape[0])
+
+    def save_states(self, pool, src, slots=None, stream=0):
+        """pool slot slots[k] (None: slot k) <- instance src[k], for every k; int32 CUDA tensors; enqueued on `stream`, no host
+        wait.  A slot index out of range is skipped; a source out of range leaves a slot that restores reject."""
+        import torch
+        n_slots = self._check_pool(pool)
+        self._check_device_tensor(src, torch.int32, "src")
+        n = src.numel()
+        if slots is not None:
+            self._check_device_tensor(slots, torch.int32, "slots", n)
+        _lib.check(_lib.lib().agarcl_batch_save_states(self._h, _vp(pool.data_ptr()), n_slots, _vp(src.data_ptr() if n else None),
+                                                       _vp(slots.data_ptr()) if slots is not None and n else None, n, _vp(stream)))
+
+    def restore_states(self, pool, slot_of, stream=0):
+        """instance i <- pool slot slot_of[i] wherever slot_of[i] >= 0 (int32 CUDA tensor of N entries); enqueued on `stream`,
+        no host wait.  Returns a view of the library-owned result u8 [N] (0 not requested, 1 restored, 2 rejected: the slot
+        index is out of range or the slot was not saved from this configuration), which the next restore overwrites."""
+        import torch
+        n_slots = self._check_pool(pool)
+        self._check_device_tensor(slot_of, torch.int32, "slot_of", self.N)
+        r = _vp()
+        _lib.check(_lib.lib().agarcl_batch_restore_states(self._h, _vp(pool.data_ptr()), n_slots, _vp(slot_of.data_ptr()),
+                                                          C.byref(r), _vp(stream)))
+        return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
+
     # ---- parity / snapshot transport
     def download_state(self, i):
         sv = StateView(self.layout)

@@ -114,6 +114,11 @@ struct agarcl_batch {
   DevBuf<double> d_ret, d_final_ret;
   DevBuf<void> d_final_obs;          // [N*A, frames*C, G, G], only with keep_final_obs and a grid observation
   DevBuf<float> d_final_ram;         // [N, P, AGARCL_RAM_RECORD], only with keep_final_obs and cfg.ram_obs
+  // snapshot pools (agarcl_batch_save_states / _restore_states): the slot layout, the configuration's fingerprint, the
+  // library-owned result of the last restore and the mask of the instances it restored
+  ag::SnapLayout snap;
+  uint64_t fingerprint = 0;
+  DevBuf<uint8_t> d_snap_result, d_snap_restored;
   ag::HostMirror* mirror = nullptr;  // host-resident observation mirror (mirror.cu), created on first use
   ag::HostMirror* lists = nullptr;   // the lists-only twin behind agarcl_batch_step_lists (no dense tensor, no worker threads)
   uint64_t mirror_launch_us = 0, mirror_call_us = 0;  // last agarcl_batch_step_mirror: staging + launch, whole call
@@ -330,6 +335,50 @@ static int refill_replay(agarcl_batch* b, cudaStream_t s) {
   return AGARCL_OK;
 }
 
+// ---- snapshot pools: the slot layout of include/agarcl_b200.h (agarcl_snapshot_hdr) and the configuration fingerprint
+static uint64_t align_to(uint64_t v, uint64_t a) { return (v + a - 1) / a * a; }
+
+static void snapshot_layout(const agarcl_cfg& c, const agarcl_layout& L, ag::SnapLayout& S) {
+  const uint64_t esz = c.obs_dtype == AGARCL_OBS_I16 ? 2 : 4;
+  S.off_blob = sizeof(agarcl_snapshot_hdr);
+  S.off_ep = S.off_blob + L.stride;
+  S.ep_bytes = align_to(8 + 8 * (uint64_t)L.A, 16);
+  S.off_ram = S.off_ep + S.ep_bytes;
+  S.ram_bytes = c.ram_obs ? (uint64_t)L.P * AGARCL_RAM_RECORD * sizeof(float) : 0;
+  S.off_obs = S.off_ram + S.ram_bytes;
+  S.obs_bytes = (c.num_frames > 1 && c.ram_obs != 2)
+                    ? (uint64_t)L.A * c.num_frames * L.obs_channels * c.grid_size * c.grid_size * esz : 0;
+  S.slot_bytes = align_to(S.off_obs + align_to(S.obs_bytes, 16), 128);
+}
+
+// FNV-1a 64 over the layout without cap_replay and the configuration fields that shape a game state (not n_instances, the caps
+// of the layout, device or instance_base: a pool moves between batch sizes, shards and devices)
+static uint64_t config_fingerprint(const agarcl_cfg& c, const agarcl_layout& L) {
+  uint64_t h = 0xcbf29ce484222325ull;
+  auto mix = [&h](const void* p, size_t n) {
+    for (size_t k = 0; k < n; k++) { h ^= ((const uint8_t*)p)[k]; h *= 0x100000001b3ull; }
+  };
+  agarcl_layout l = L;
+  l.cap_replay = 0;
+  mix(&l, sizeof(l));
+  const int32_t f[] = {c.num_agents, c.ticks_per_step, c.arena_size, c.pellet_regen, c.num_pellets, c.num_viruses, c.num_bots,
+                       c.reward_type, c.c_death, c.mode_number, c.num_frames, c.grid_size, c.observe_cells, c.observe_others,
+                       c.observe_viruses, c.observe_pellets, c.obs_dtype, c.strict_reference, c.rng_mode, c.ram_obs};
+  mix(f, sizeof(f));
+  return h;
+}
+
+extern "C" int agarcl_snapshot_slot_bytes(const agarcl_cfg* c, int64_t* out) {
+  if (!c || !out) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
+  agarcl_layout L;
+  int rc = agarcl_make_layout(c, &L);
+  if (rc != AGARCL_OK) return rc;
+  ag::SnapLayout S;
+  snapshot_layout(*c, L, S);
+  *out = (int64_t)S.slot_bytes;
+  return AGARCL_OK;
+}
+
 extern "C" int agarcl_batch_destroy(agarcl_batch* b) {
   delete b;
   return AGARCL_OK;
@@ -358,6 +407,8 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
   b->C = L.obs_channels;
   b->frames = cfg->num_frames;
   b->knobs = read_knobs();
+  snapshot_layout(*cfg, L, b->snap);
+  b->fingerprint = config_fingerprint(*cfg, L);
   CK(ag::setup_step(b->knobs.warps, b->step_launch));
   if (cfg->ram_obs) CK(ag::setup_ram(L, b->step_launch.smem_optin));
   b->obs_elems = (size_t)b->N * b->A * b->frames * b->C * b->G * b->G;
@@ -376,6 +427,7 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
       (rc = alloc(b->d_tickets, 2 * sizeof(uint32_t), 0)) || (rc = alloc(b->d_cost, (size_t)b->N * sizeof(uint32_t))) ||
       (rc = alloc(b->d_perm, (size_t)b->N * sizeof(uint32_t))) || (rc = alloc(b->d_sched, 2 * sizeof(uint32_t))) ||
       (rc = alloc(b->d_fresh, (size_t)b->N, 1)) || (rc = alloc(b->d_flagbuf, 33 * sizeof(uint32_t))) ||
+      (rc = alloc(b->d_snap_result, (size_t)b->N, 0)) || (rc = alloc(b->d_snap_restored, (size_t)b->N, 0)) ||
       (L.cap_replay > 0 && (rc = alloc(b->d_replay, (size_t)b->N * L.cap_replay * sizeof(float), 0))) ||
       (cfg->ram_obs && (rc = alloc(b->d_ram, (size_t)b->N * L.P * AGARCL_RAM_RECORD * sizeof(float), 0))) ||
       (rc = alloc(b->d_lut_radius, lut_bytes)) || (rc = alloc(b->d_lut_speed, lut_bytes)) || (rc = alloc(b->d_lut_split, lut_bytes)))
@@ -975,5 +1027,83 @@ extern "C" int agarcl_batch_upload_state(agarcl_batch* b, int32_t instance, cons
   CK(cudaDeviceSynchronize());
   CK(cudaMemcpy(b->d_state + (size_t)instance * b->L.stride, blob, b->L.stride, cudaMemcpyHostToDevice));
   b->was_reset = true;
+  return AGARCL_OK;
+}
+
+// ---- snapshot pools (include/agarcl_b200.h): refusals are decided here, before anything is enqueued
+static int snapshot_check(agarcl_batch* b, const void* pool, int64_t pool_slots) {
+  if (b->cfg.strict_reference)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot pools are refused under strict_reference: the player order belongs to the batch");
+  if (b->cfg.rng_mode == AGARCL_RNG_MT19937)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot pools are refused under AGARCL_RNG_MT19937: its generators live on the host");
+  if (!b->was_reset) return agarcl_set_error(AGARCL_ERR_STATE, "save / restore of states before reset()");
+  if (!pool) return agarcl_set_error(AGARCL_ERR_INVALID, "null pool");
+  if ((uintptr_t)pool & 15u) return agarcl_set_error(AGARCL_ERR_INVALID, "the pool must be 16-byte aligned");
+  if (pool_slots < 1) return agarcl_set_error(AGARCL_ERR_INVALID, "pool_slots must be >= 1");
+  CK(cudaSetDevice(b->cfg.device));
+  cudaPointerAttributes a;
+  const cudaError_t e = cudaPointerGetAttributes(&a, pool);  // (does not synchronise)
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return agarcl_set_error(AGARCL_ERR_INVALID, "the pool is not device memory: %s", cudaGetErrorString(e));
+  }
+  if (a.type != cudaMemoryTypeDevice || a.device != b->cfg.device)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "the pool must be device memory of device %d", b->cfg.device);
+  return AGARCL_OK;
+}
+
+static ag::SnapParams snapshot_params(const agarcl_batch* b, const void* pool, int64_t pool_slots) {
+  ag::SnapParams P = {};
+  P.pool = (uint8_t*)pool;
+  P.pool_slots = pool_slots;
+  P.S = b->snap;
+  P.fingerprint = b->fingerprint;
+  P.state = b->d_state;
+  P.stride = b->L.stride;
+  P.off_hdr = b->L.off_hdr;
+  P.steps = b->autoreset ? b->d_steps.get() : nullptr;
+  P.ret = b->autoreset ? b->d_ret.get() : nullptr;
+  P.ram = (uint8_t*)b->d_ram.get();
+  P.obs = (uint8_t*)b->d_obs.get();
+  P.seeds = b->d_seeds;
+  P.fresh = b->d_fresh;
+  P.rewards = b->d_rewards;
+  P.dones = b->d_dones;
+  P.result = b->d_snap_result;
+  P.restored = b->d_snap_restored;
+  P.N = b->N;
+  P.A = b->A;
+  P.instance_base = b->cfg.instance_base;
+  return P;
+}
+
+extern "C" int agarcl_batch_save_states(agarcl_batch* b, void* pool, int64_t pool_slots, const int32_t* d_src, const int32_t* d_slot,
+                                        int32_t n, void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (n < 0) return agarcl_set_error(AGARCL_ERR_INVALID, "n must be >= 0");
+  if (n > 0 && !d_src) return agarcl_set_error(AGARCL_ERR_INVALID, "null source index array");
+  int rc = snapshot_check(b, pool, pool_slots);
+  if (rc) return rc;
+  if (n == 0) return AGARCL_OK;
+  ag::SnapParams P = snapshot_params(b, pool, pool_slots);
+  P.src = d_src;
+  P.slot = d_slot;
+  CK(ag::launch_snapshot_save(P, n, (cudaStream_t)stream));
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, int64_t pool_slots, const int32_t* d_slot_of,
+                                           uint8_t** d_result, void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (!d_slot_of) return agarcl_set_error(AGARCL_ERR_INVALID, "null slot index array");
+  int rc = snapshot_check(b, pool, pool_slots);
+  if (rc) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  ag::SnapParams P = snapshot_params(b, pool, pool_slots);
+  P.slot_of = d_slot_of;
+  CK(ag::launch_snapshot_restore(P, s));
+  // a one-frame grid observation is re-rendered, as the step that produced the state showed it (respawned players still dead)
+  if (b->cfg.ram_obs != 2 && b->frames == 1 && (rc = render_frame(b, 0, s, 1, 0, b->d_snap_restored))) return rc;
+  if (d_result) *d_result = b->d_snap_result;
   return AGARCL_OK;
 }

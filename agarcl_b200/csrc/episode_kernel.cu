@@ -4,6 +4,7 @@
 // Neither needs the host to look at the step's dones, so the step, the bookkeeping and the reset queue back to back.
 #include <cuda_runtime.h>
 
+#include "block_copy.cuh"
 #include "sim_params.h"
 
 namespace ag {
@@ -47,31 +48,14 @@ __global__ void __launch_bounds__(256) k_episode(const __grid_constant__ Episode
 }
 
 // One CTA per instance: bytes [i * per, (i + 1) * per) of dst get those of src (kCopy) or zeros, for the instances with
-// mask[i] != 0; the CTAs of the others exit at once.  dst and src are allocations of the same alignment, so both share
-// the head that precedes the first 16-byte boundary; the body moves in 16-byte vectors, four in flight per thread.
+// mask[i] != 0; the CTAs of the others exit at once.  dst and src are allocations of the same alignment, so the slices
+// of one instance share their alignment modulo 16 (block_copy).
 template <bool kCopy>
 __global__ void __launch_bounds__(kMaskedThreads) k_masked_bytes(uint8_t* __restrict__ dst, const uint8_t* __restrict__ src,
                                                                  size_t per, const uint8_t* __restrict__ mask) {
   const int inst = blockIdx.x;
   if (!mask[inst]) return;
-  uint8_t* d = dst + (size_t)inst * per;
-  const uint8_t* s = kCopy ? src + (size_t)inst * per : nullptr;
-  size_t head = (16u - ((uintptr_t)d & 15u)) & 15u;
-  if (head > per) head = per;
-  const size_t nvec = (per - head) / 16, tail = head + nvec * 16;
-  const int t = threadIdx.x, nt = blockDim.x;
-  for (size_t k = t; k < head; k += nt) d[k] = kCopy ? s[k] : 0;
-  for (size_t k = tail + t; k < per; k += nt) d[k] = kCopy ? s[k] : 0;
-  uint4* dv = reinterpret_cast<uint4*>(d + head);
-  const uint4* sv = kCopy ? reinterpret_cast<const uint4*>(s + head) : nullptr;
-  const uint4 z = make_uint4(0u, 0u, 0u, 0u);
-  size_t k = t;
-  for (; k + 3 * (size_t)nt < nvec; k += 4 * (size_t)nt) {
-    uint4 v0 = z, v1 = z, v2 = z, v3 = z;
-    if (kCopy) { v0 = sv[k]; v1 = sv[k + nt]; v2 = sv[k + 2 * nt]; v3 = sv[k + 3 * nt]; }
-    dv[k] = v0; dv[k + nt] = v1; dv[k + 2 * nt] = v2; dv[k + 3 * nt] = v3;
-  }
-  for (; k < nvec; k += nt) dv[k] = kCopy ? sv[k] : z;
+  block_copy<kCopy>(dst + (size_t)inst * per, kCopy ? src + (size_t)inst * per : nullptr, per);
 }
 
 cudaError_t launch_episode(const EpisodeParams& P, cudaStream_t stream) {

@@ -199,4 +199,38 @@ cudaError_t launch_episode(const EpisodeParams& P, cudaStream_t stream);
 // dst = src (nullptr: zeros) in the `per`-byte slices of the instances with mask != 0
 cudaError_t launch_masked_bytes(void* dst, const void* src, size_t per, const uint8_t* mask, int N, cudaStream_t stream);
 
+// Snapshot pools (snapshot_kernel.cu, k_snapshot): the slot layout of include/agarcl_b200.h, agarcl_snapshot_hdr
+struct SnapLayout {
+  uint64_t off_blob, off_ep, off_ram, off_obs;  // segment offsets inside a slot (16-byte aligned)
+  uint64_t ep_bytes, ram_bytes, obs_bytes;      // segment sizes; ram_bytes / obs_bytes 0 when the segment is not stored
+  uint64_t slot_bytes;                          // a multiple of 128
+};
+constexpr int kSnapThreads = 512;  // threads of k_snapshot, one CTA per saved entry / restored instance
+struct SnapParams {
+  uint8_t* pool;             // pool_slots slots of slot_bytes
+  int64_t pool_slots;
+  SnapLayout S;
+  uint64_t fingerprint;
+  uint8_t* state;            // the batch's N blobs, L.stride apart
+  uint32_t stride, off_hdr;  // L.stride, L.off_hdr
+  int64_t* steps;            // [N] episode bookkeeping, nullptr when it is off
+  double* ret;               // [N*A]
+  uint8_t* ram;              // [N] records of S.ram_bytes (when stored)
+  uint8_t* obs;              // [N] observation images of S.obs_bytes (when stored)
+  // save: pool slot (slot ? slot[k] : k) <- instance src[k], k < n
+  const int32_t* src;
+  const int32_t* slot;
+  // restore: instance i <- pool slot slot_of[i] where >= 0
+  const int32_t* slot_of;
+  uint64_t* seeds;           // [N] the reset kernel's per-instance seed
+  uint8_t* fresh;            // [N] ResetParams::fresh
+  double* rewards;           // [N*A]
+  uint8_t* dones;            // [N*A]
+  uint8_t* result;           // [N] 0 not requested, 1 restored, 2 rejected
+  uint8_t* restored;         // [N] 1 where restored: the mask of the k_obs launch behind
+  int32_t N, A, instance_base;
+};
+cudaError_t launch_snapshot_save(const SnapParams& P, int n, cudaStream_t stream);
+cudaError_t launch_snapshot_restore(const SnapParams& P, cudaStream_t stream);
+
 }  // namespace ag

@@ -1,0 +1,109 @@
+// snapshot_kernel.cu — batched save / restore of game states into a caller-owned pool of slots
+// (agarcl_batch_save_states / agarcl_batch_restore_states; slot layout: include/agarcl_b200.h, agarcl_snapshot_hdr).
+// A slot is the instance's state blob plus what the blob does not hold: the episode record of the vector environment,
+// the ram records (a player with nothing in view keeps its previous one) and, with several frames, the observation
+// history.  One CTA per entry; nothing is read back by the host.
+#include <cuda_runtime.h>
+
+#include "block_copy.cuh"
+#include "sim_params.h"
+
+namespace ag {
+
+// Copies n bytes with every thread of the CTA.  Segments of the state, the ram records and the slot share their alignment
+// modulo 16; an observation image of an odd grid may not (its instance offset is not a multiple of 16 while its slot
+// offset is), and is then copied byte by byte.
+__device__ __forceinline__ void copy_segment(uint8_t* __restrict__ d, const uint8_t* __restrict__ s, size_t n) {
+  if ((((uintptr_t)d ^ (uintptr_t)s) & 15u) == 0) {
+    block_copy<true>(d, s, n);
+    return;
+  }
+  for (size_t k = threadIdx.x; k < n; k += blockDim.x) d[k] = s[k];
+}
+
+template <bool kSave>
+__global__ void __launch_bounds__(kSnapThreads) k_snapshot(const __grid_constant__ SnapParams P) {
+  const int t = threadIdx.x, nt = blockDim.x, A = P.A;
+  if (kSave) {
+    const int k = blockIdx.x;
+    const int64_t slot = P.slot ? (int64_t)P.slot[k] : (int64_t)k;
+    if (slot < 0 || slot >= P.pool_slots) return;  // skipped
+    uint8_t* sl = P.pool + (uint64_t)slot * P.S.slot_bytes;
+    const int src = P.src[k];
+    const bool ok = src >= 0 && src < P.N;
+    if (ok) {
+      copy_segment(sl + P.S.off_blob, P.state + (size_t)src * P.stride, P.stride);
+      // episode record: steps, then the per-agent return (zeros without bookkeeping), then zero padding
+      uint64_t* ep = reinterpret_cast<uint64_t*>(sl + P.S.off_ep);
+      for (int w = t; w < (int)(P.S.ep_bytes / 8); w += nt) {
+        uint64_t v = 0;
+        if (P.steps && w == 0) v = (uint64_t)P.steps[src];
+        else if (P.steps && w <= A) v = (uint64_t)__double_as_longlong(P.ret[(size_t)src * A + (w - 1)]);
+        ep[w] = v;
+      }
+      if (P.S.ram_bytes) copy_segment(sl + P.S.off_ram, P.ram + (size_t)src * P.S.ram_bytes, P.S.ram_bytes);
+      if (P.S.obs_bytes) copy_segment(sl + P.S.off_obs, P.obs + (size_t)src * P.S.obs_bytes, P.S.obs_bytes);
+    }
+    __syncthreads();  // the header goes last; a source out of range leaves magic 0, which a restore rejects
+    if (t == 0) {  // agarcl_snapshot_hdr: magic, version, fingerprint, slot_bytes, source, zero padding
+      const uint4 z = make_uint4(0u, 0u, 0u, 0u);
+      uint4* hv = reinterpret_cast<uint4*>(sl);
+      hv[0] = ok ? make_uint4(AGARCL_SNAPSHOT_MAGIC, AGARCL_SNAPSHOT_VERSION, (uint32_t)P.fingerprint, (uint32_t)(P.fingerprint >> 32)) : z;
+      hv[1] = ok ? make_uint4((uint32_t)P.S.slot_bytes, (uint32_t)(P.S.slot_bytes >> 32), (uint32_t)(P.instance_base + src), 0u) : z;
+      hv[2] = z;
+      hv[3] = z;
+    }
+    return;
+  }
+  const int i = blockIdx.x;
+  const int32_t slot = P.slot_of[i];
+  if (slot < 0) {  // not requested: the instance is not touched
+    if (t == 0) { P.result[i] = 0; P.restored[i] = 0; }
+    return;
+  }
+  const uint8_t* sl = P.pool + (uint64_t)slot * P.S.slot_bytes;
+  bool valid = slot < P.pool_slots;
+  if (valid) {
+    const agarcl_snapshot_hdr* h = reinterpret_cast<const agarcl_snapshot_hdr*>(sl);
+    valid = h->magic == AGARCL_SNAPSHOT_MAGIC && h->version == AGARCL_SNAPSHOT_VERSION && h->fingerprint == P.fingerprint &&
+            h->slot_bytes == P.S.slot_bytes;
+  }
+  if (!valid) {  // rejected: the instance is not touched
+    if (t == 0) { P.result[i] = 2; P.restored[i] = 0; }
+    return;
+  }
+  copy_segment(P.state + (size_t)i * P.stride, sl + P.S.off_blob, P.stride);
+  if (P.steps) {
+    const uint64_t* ep = reinterpret_cast<const uint64_t*>(sl + P.S.off_ep);
+    for (int w = t; w <= A; w += nt) {
+      if (w == 0) P.steps[i] = (int64_t)ep[0];
+      else P.ret[(size_t)i * A + (w - 1)] = __longlong_as_double((long long)ep[w]);
+    }
+  }
+  if (P.S.ram_bytes) copy_segment(P.ram + (size_t)i * P.S.ram_bytes, sl + P.S.off_ram, P.S.ram_bytes);
+  if (P.S.obs_bytes) copy_segment(P.obs + (size_t)i * P.S.obs_bytes, sl + P.S.off_obs, P.S.obs_bytes);
+  for (int a = t; a < A; a += nt) {  // like after a reset
+    P.rewards[(size_t)i * A + a] = 0.0;
+    P.dones[(size_t)i * A + a] = 0;
+  }
+  if (t == 0) {
+    // the next reset of the instance continues the restored draw stream (ResetParams::fresh == 0 -> from hdr.rng_cursor)
+    const agarcl_inst_hdr* ih = reinterpret_cast<const agarcl_inst_hdr*>(sl + P.S.off_blob + P.off_hdr);
+    P.seeds[i] = (uint64_t)ih->seed_lo | ((uint64_t)ih->seed_hi << 32);
+    P.fresh[i] = 0;
+    P.result[i] = 1;
+    P.restored[i] = 1;
+  }
+}
+
+cudaError_t launch_snapshot_save(const SnapParams& P, int n, cudaStream_t stream) {
+  k_snapshot<true><<<n, kSnapThreads, 0, stream>>>(P);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_snapshot_restore(const SnapParams& P, cudaStream_t stream) {
+  k_snapshot<false><<<P.N, kSnapThreads, 0, stream>>>(P);
+  return cudaGetLastError();
+}
+
+}  // namespace ag

@@ -385,6 +385,18 @@ class BatchedGridEnvironment(_Base):
     def episode(self):
         return self._ensure().episode()
 
+    def snapshot_pool(self, slots):
+        """a zeroed snapshot pool of `slots` slots on the device (Batch.snapshot_pool)"""
+        return self._ensure().snapshot_pool(slots)
+
+    def save_states(self, pool, src, slots=None, stream=0):
+        """pool slot slots[k] (None: k) <- instance src[k] (Batch.save_states)"""
+        self._ensure().save_states(pool, src, slots, stream)
+
+    def restore_states(self, pool, slot_of, stream=0):
+        """instance i <- pool slot slot_of[i] where >= 0; returns the result u8 [N] (Batch.restore_states)"""
+        return self._ensure().restore_states(pool, slot_of, stream)
+
     def ram(self):
         return self._ensure().ram_tensor()
 

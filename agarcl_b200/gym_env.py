@@ -252,6 +252,27 @@ class BatchedAgarioEnv:
                 info["final_obs"] = self._final
         return self._obs(), rew.float(), done, torch.zeros_like(done), info
 
+    # ---- snapshot pools (Batch.save_states / restore_states): save and restore whole games, episode counters included
+    def snapshot_pool(self, slots):
+        return self._env.snapshot_pool(slots)
+
+    def save_states(self, pool, src, slots=None):
+        """pool slot slots[k] (None: k) <- environment src[k] (int32 CUDA tensors), on the current stream"""
+        assert self._ep is not None, "Cannot call save_states() before calling reset()"
+        self._env.save_states(pool, src, slots)
+
+    def restore_states(self, pool, slot_of):
+        """environment i <- pool slot slot_of[i] where >= 0 (int32 CUDA tensor of n_envs entries); returns the observation.  A
+        restored episode goes on counting towards number_steps from the step count it was saved with; restore_result() has the
+        per-environment outcome (1 restored, 2 rejected)"""
+        assert self._ep is not None, "Cannot call restore_states() before calling reset()"
+        self._restore_result = self._env.restore_states(pool, slot_of)
+        return self._obs()
+
+    def restore_result(self):
+        """u8 [n_envs] of the last restore_states: 0 not requested, 1 restored, 2 rejected"""
+        return self._restore_result
+
     def flags(self):
         """(OR over all instances, {AGARCL_FLAG name: instances}) -- fixed capacities hit since the instances' last reset"""
         return self._env.flags()

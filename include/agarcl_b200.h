@@ -232,6 +232,66 @@ int agarcl_batch_set_autoreset(agarcl_batch* b, int32_t max_steps, int32_t keep_
 int agarcl_batch_step_autoreset(agarcl_batch* b, void* stream);
 int agarcl_batch_episode(agarcl_batch* b, agarcl_episode* out);
 
+/* ---------------------------------------------------- snapshot pools: save and restore game states on the device
+ * The batched counterpart of agarcl_batch_save_env_state / load_env_state: chosen instances are copied into slots of a
+ * caller-owned POOL in device memory and slots back into chosen instances, stream-ordered, driven by index arrays in device
+ * memory, without the host waiting.  A pool is pool_slots slots of agarcl_snapshot_slot_bytes bytes (16-byte aligned device
+ * memory of cfg.device).  A slot holds no pointer: a pool may be copied to the host, stored, moved to another device and
+ * restored into any batch of the same configuration -- n_instances, device, instance_base and cap_replay may differ.
+ * Slot layout, every segment 16-byte aligned (S = layout.stride, A agents, P players, esz 4 for int32 and 2 for int16):
+ *   [0, 64)               agarcl_snapshot_hdr below
+ *   [64, 64 + S)          the state blob: it includes hdr.rng_cursor, the seed, the tick, done_sticky and the respawn mask
+ *   off_ep  = 64 + S      episode record, E = align16(8 + 8 A) bytes: int64 steps, then f64 return[A] since the instance's last
+ *                         reset (agarcl_batch_set_autoreset); zeros when the bookkeeping was off at the save, and written on a
+ *                         restore only when it is on
+ *   off_ram = off_ep + E  cfg.ram_obs: the ram records [P][AGARCL_RAM_RECORD] f32, R = P * 4 * AGARCL_RAM_RECORD bytes (copied, not
+ *                         re-rendered: a player with nothing in view keeps its previous record), else R = 0
+ *   off_obs = off_ram + R num_frames > 1 and a grid observation: the instance's images [A][frames*C][G][G], O = align16(A * frames *
+ *                         C * G * G * esz) bytes (the earlier frames are history the blob does not hold), else O = 0
+ *   slot bytes            align128(off_obs + O)
+ * A one-frame grid observation is not stored: the restore ends with k_obs on the restored instances, showing players respawned at
+ * the end of the last step as still dead -- the frame the step that produced the state showed (after a reset: the reset's).  A
+ * state saved right after agarcl_batch_render therefore comes back with the step's frame, not render()'s.
+ *   agarcl_batch_save_states     for k < n: slot d_slot[k] (d_slot NULL: slot k) <- instance d_src[k].  Slots out of
+ *                                [0, pool_slots) are skipped; a source out of [0, N) writes a header with magic 0, which a restore
+ *                                rejects.  The slots of one call must be distinct.
+ *   agarcl_batch_restore_states  for every instance i with d_slot_of[i] >= 0 (N entries): instance i <- that slot.  *d_result (may
+ *                                be NULL) receives the library-owned u8 [N] result, overwritten by the next restore:
+ *                                0 not requested, 1 restored, 2 rejected (slot out of [0, pool_slots), or magic, version,
+ *                                fingerprint or slot bytes differ): a rejected or unrequested instance is not touched, bit for bit.
+ *                                A restored instance's rewards and dones are zeroed, like after a reset; the reset_mask and done_out
+ *                                of the last agarcl_batch_step_autoreset are left as they are.  As after a reset, call
+ *                                agarcl_batch_sync_mirror before the next agarcl_batch_step_mirror.
+ * Fork = save once, then restore with several instances naming the same slot.
+ * Draw stream: the restore writes the instance's seed from the restored blob and marks the stream as not fresh, so its next reset
+ * continues the restored stream.  Under AGARCL_RNG_PHILOX the stream is keyed by (seed, global instance index, cursor): a state
+ * restored into an instance whose instance_base + i equals the source's global index reproduces the source's future exactly;
+ * restored anywhere else it continues on the destination's key and diverges from the source at its first draw (pellet regen,
+ * respawn) -- forked children that receive identical actions still differ where the game draws.
+ * Refused with an error before anything is enqueued (the games do not move): strict_reference (the player order belongs to the
+ * batch and changes with every unmasked reset), AGARCL_RNG_MT19937 (its generators live on the host), a call before the first
+ * reset, a NULL / misaligned pool or one that is not device memory of cfg.device, pool_slots < 1, n < 0, a NULL index array.
+ * The fingerprint is FNV-1a 64 over agarcl_layout without cap_replay and the agarcl_cfg fields num_agents .. ram_obs except
+ * cap_viruses, cap_foods, cap_replay, device and instance_base (those two caps are part of the layout). */
+#define AGARCL_SNAPSHOT_MAGIC 0x4E534741u /* "AGSN" */
+#define AGARCL_SNAPSHOT_VERSION 1u
+typedef struct agarcl_snapshot_hdr { /* 64 B */
+  uint32_t magic;          /* AGARCL_SNAPSHOT_MAGIC; 0: the slot holds no state */
+  uint32_t version;        /* AGARCL_SNAPSHOT_VERSION */
+  uint64_t fingerprint;    /* of the configuration the slot was saved from */
+  uint64_t slot_bytes;
+  int32_t source;          /* global index (instance_base + i) of the instance saved */
+  uint32_t pad[9];
+} agarcl_snapshot_hdr;
+/* bytes of one snapshot slot of configuration c: a multiple of 128; no device needed */
+int agarcl_snapshot_slot_bytes(const agarcl_cfg* c, int64_t* out);
+/* pool slot d_slot[k] <- instance d_src[k], k < n (device int32 arrays; d_slot NULL = slots 0..n-1); enqueued on stream */
+int agarcl_batch_save_states(agarcl_batch* b, void* pool, int64_t pool_slots, const int32_t* d_src, const int32_t* d_slot,
+                             int32_t n, void* stream);
+/* instance i <- pool slot d_slot_of[i] where >= 0; *d_result = the library-owned u8 [N] result above; enqueued on stream */
+int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, int64_t pool_slots, const int32_t* d_slot_of,
+                                uint8_t** d_result, void* stream);
+
 /* ---------------------------------------------------- host-resident observation mirror
  * get_state (bindings.cpp:67-91) hands every agent's frame to HOST memory; for a batch that is 512 KB per agent
  * per step, and the dense copy above is bound by PCIe.  The mirror is a library-owned, pinned host tensor
