@@ -5,9 +5,10 @@ Public surface:
   GridEnvironment            drop-in for agarcl.GridEnvironment (environment/bindings.cpp:99-135), N = 1
   BatchedGridEnvironment     the same interface over N instances, device tensors out
   make_cfg / Cfg / Layout    configuration records of include/agarcl_b200.h
+  task_bits                  cfg.task_modes of a list of modes (mixed-task batches: Batch.set_tasks / tasks)
   snapshot_slot_bytes        bytes of one slot of a snapshot pool (Batch.snapshot_pool / save_states / restore_states)
 """
-from ._abi import Cfg, Layout, StateView, make_cfg, OBS_I16, OBS_I32, RNG_MT19937, RNG_PHILOX, RNG_REPLAY  # noqa: F401
+from ._abi import Cfg, Layout, StateView, make_cfg, task_bits, OBS_I16, OBS_I32, RNG_MT19937, RNG_PHILOX, RNG_REPLAY  # noqa: F401
 from ._lib import snapshot_slot_bytes  # noqa: F401
 
 

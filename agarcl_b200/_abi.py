@@ -37,7 +37,7 @@ class Cfg(C.Structure):
         "reward_type", "c_death", "mode_number",
         "num_frames", "grid_size", "observe_cells", "observe_others", "observe_viruses", "observe_pellets",
         "obs_dtype", "strict_reference", "rng_mode",
-        "cap_viruses", "cap_foods", "cap_replay", "device", "instance_base", "ram_obs")] + [("reserved", C.c_int32 * 2)]
+        "cap_viruses", "cap_foods", "cap_replay", "device", "instance_base", "ram_obs", "task_modes")] + [("reserved", C.c_int32 * 1)]
 
 
 class Layout(C.Structure):
@@ -73,13 +73,26 @@ def make_cfg(n_instances=1, num_agents=1, ticks_per_step=4, arena_size=1000, pel
              num_pellets=1000, num_viruses=25, num_bots=25, reward_type=1, c_death=0, mode_number=0,
              num_frames=1, grid_size=128, observe_cells=True, observe_others=True, observe_viruses=True,
              observe_pellets=True, obs_dtype=OBS_I32, strict_reference=False, rng_mode=RNG_PHILOX,
-             cap_viruses=0, cap_foods=0, cap_replay=0, device=0, instance_base=0, ram_obs=False):
+             cap_viruses=0, cap_foods=0, cap_replay=0, device=0, instance_base=0, ram_obs=False, task_modes=0):
+    """task_modes: 0, or the bit mask of the modes a mixed-task batch may run (include/agarcl_b200.h); task_bits() makes one
+    from a list of modes"""
     c = Cfg()
     for k, v in list(locals().items()):
         if k in ("c",):
             continue
         setattr(c, k, int(v))
     return c
+
+
+def task_bits(modes):
+    """bit mask (cfg.task_modes) of an iterable of mode numbers"""
+    bits = 0
+    for m in modes:
+        m = int(m)
+        if not 0 <= m <= 10:
+            raise ValueError(f"mode {m} is outside 0..10")
+        bits |= 1 << m
+    return bits
 
 
 class StateView:

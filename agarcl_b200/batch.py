@@ -33,6 +33,11 @@ class _EpisodeStruct(C.Structure):
     _fields_ = [(n, _vp) for n in ("done_out", "reset_mask", "steps", "final_return", "final_length", "final_obs", "final_ram")]
 
 
+class _TasksStruct(C.Structure):
+    """struct agarcl_tasks"""
+    _fields_ = [(n, _vp) for n in ("mode", "max_steps", "next_mode", "next_max_steps")]
+
+
 class ObsLists:
     """numpy view of the lists of the last Batch.step_lists (layout: include/agarcl_b200.h, agarcl_obs_lists)"""
 
@@ -383,6 +388,30 @@ class Batch:
         _lib.check(_lib.lib().agarcl_batch_restore_states(self._h, _vp(pool.data_ptr()), n_slots, _vp(slot_of.data_ptr()),
                                                           C.byref(r), _vp(stream)))
         return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
+
+    # ---- mixed-task batches (include/agarcl_b200.h, cfg.task_modes)
+    def set_tasks(self, mode, max_steps=None, stream=0):
+        """the task each instance's NEXT reset plays: mode (int32 CUDA tensor of N entries, -1 keeps the pending mode) and
+        max_steps (int32 CUDA tensor of N entries or None: every pending limit kept; -1 the set_autoreset limit, 0 none).
+        Checked on the device, enqueued on `stream`, no host wait.  Returns a view of the library-owned result u8 [N] (0 nothing
+        set, 1 set, 2 rejected: mode not in task_modes or limit < -1), which the next call overwrites."""
+        import torch
+        self._check_device_tensor(mode, torch.int32, "mode", self.N)
+        if max_steps is not None:
+            self._check_device_tensor(max_steps, torch.int32, "max_steps", self.N)
+        r = _vp()
+        _lib.check(_lib.lib().agarcl_batch_set_tasks(self._h, _vp(mode.data_ptr()), _vp(max_steps.data_ptr()) if max_steps is not None else None,
+                                                     C.byref(r), _vp(stream)))
+        return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
+
+    def tasks(self):
+        """zero-copy int32 device views [N] of the task state: mode and max_steps of the current episode, next_mode and
+        next_max_steps of the next"""
+        import torch
+        t = _TasksStruct()
+        _lib.check(_lib.lib().agarcl_batch_tasks(self._h, C.byref(t)))
+        return {k: torch.as_tensor(_CudaView(getattr(t, k), (self.N,), "<i4", self), device=f"cuda:{self.cfg.device}")
+                for k in ("mode", "max_steps", "next_mode", "next_max_steps")}
 
     # ---- parity / snapshot transport
     def download_state(self, i):

@@ -119,6 +119,9 @@ struct agarcl_batch {
   ag::SnapLayout snap;
   uint64_t fingerprint = 0;
   DevBuf<uint8_t> d_snap_result, d_snap_restored;
+  // mixed-task batch (cfg.task_modes != 0, include/agarcl_b200.h): current and pending task per instance, result of the last set_tasks
+  DevBuf<int32_t> d_task_mode, d_task_max_steps, d_next_mode, d_next_max_steps;
+  DevBuf<uint8_t> d_task_result;
   ag::HostMirror* mirror = nullptr;  // host-resident observation mirror (mirror.cu), created on first use
   ag::HostMirror* lists = nullptr;   // the lists-only twin behind agarcl_batch_step_lists (no dense tensor, no worker threads)
   uint64_t mirror_launch_us = 0, mirror_call_us = 0;  // last agarcl_batch_step_mirror: staging + launch, whole call
@@ -192,6 +195,8 @@ static void fill_sim_params(const agarcl_batch* b, ag::SimParams& P) {
   P.N = b->N;
   P.instance_base = b->cfg.instance_base;
   P.mode = b->cfg.mode_number;
+  P.task_mode = b->d_task_mode;
+  P.num_bots = b->cfg.num_bots;
   P.reward_type = b->cfg.reward_type;
   P.rng_mode = b->cfg.rng_mode;
   P.target_pellets = b->cfg.num_pellets;
@@ -365,6 +370,7 @@ static uint64_t config_fingerprint(const agarcl_cfg& c, const agarcl_layout& L) 
                        c.reward_type, c.c_death, c.mode_number, c.num_frames, c.grid_size, c.observe_cells, c.observe_others,
                        c.observe_viruses, c.observe_pellets, c.obs_dtype, c.strict_reference, c.rng_mode, c.ram_obs};
   mix(f, sizeof(f));
+  if (c.task_modes) mix(&c.task_modes, sizeof(c.task_modes));  // (pools of batches without tasks keep their fingerprint)
   return h;
 }
 
@@ -433,6 +439,17 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
       (rc = alloc(b->d_lut_radius, lut_bytes)) || (rc = alloc(b->d_lut_speed, lut_bytes)) || (rc = alloc(b->d_lut_split, lut_bytes)))
     return rc;
   { const uint32_t init[2] = {1u, 0u}; CK(cudaMemcpy(b->d_sched, init, sizeof(init), cudaMemcpyHostToDevice)); }
+  if (cfg->task_modes) {  // every instance starts on mode_number with the batch's step limit
+    const size_t bytes = (size_t)b->N * sizeof(int32_t);
+    if ((rc = alloc(b->d_task_mode, bytes)) || (rc = alloc(b->d_task_max_steps, bytes)) || (rc = alloc(b->d_next_mode, bytes)) ||
+        (rc = alloc(b->d_next_max_steps, bytes)) || (rc = alloc(b->d_task_result, (size_t)b->N, 0)))
+      return rc;
+    const std::vector<int32_t> modes((size_t)b->N, cfg->mode_number), limits((size_t)b->N, -1);
+    CK(cudaMemcpy(b->d_task_mode, modes.data(), bytes, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(b->d_next_mode, modes.data(), bytes, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(b->d_task_max_steps, limits.data(), bytes, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(b->d_next_max_steps, limits.data(), bytes, cudaMemcpyHostToDevice));
+  }
   b->cur_dxdy = b->d_dxdy;
   b->cur_act = b->d_act;
   // lookup tables of functions of an integer mass, computed with the host libm the reference uses
@@ -572,6 +589,7 @@ static ag::EpisodeParams episode_params(const agarcl_batch* b) {
   E.done_out = b->d_done_out; E.reset_mask = b->d_reset_mask; E.steps = b->d_steps;
   E.ret = b->d_ret; E.final_ret = b->d_final_ret; E.final_len = b->d_final_len;
   E.clear_mask = nullptr;
+  E.task_max_steps = b->d_task_max_steps;
   E.N = b->N; E.A = b->A; E.max_steps = b->max_steps;
   E.reset = b->autoreset_reset ? 1 : 0;
   E.clear = 0;
@@ -597,6 +615,11 @@ static int reset_impl(agarcl_batch* b, const uint8_t* dm, cudaStream_t s, bool c
   P.rng_mode = b->cfg.rng_mode;
   P.num_pellets = b->cfg.num_pellets;
   P.num_viruses = b->cfg.num_viruses;
+  P.num_bots = b->cfg.num_bots;
+  P.task_mode = b->d_task_mode;
+  P.task_max_steps = b->d_task_max_steps;
+  P.next_mode = b->d_next_mode;
+  P.next_max_steps = b->d_next_max_steps;
   P.W = (float)b->cfg.arena_size;
   if (b->cfg.strict_reference && !dm) {
     // BaseEnvironment::reset of every instance (BaseEnvironment.hpp:179-197): players.clear(), then add_player for the agents and
@@ -988,7 +1011,13 @@ extern "C" int agarcl_batch_save_env_state(agarcl_batch* b, int32_t instance, co
   CK(cudaDeviceSynchronize());
   std::vector<uint8_t> blob(b->L.stride);
   CK(cudaMemcpy(blob.data(), b->d_state + (size_t)instance * b->L.stride, b->L.stride, cudaMemcpyDeviceToHost));
-  return agarcl_snapshot_write(&b->cfg, &b->L, blob.data(), path);
+  if (!b->cfg.task_modes) return agarcl_snapshot_write(&b->cfg, &b->L, blob.data(), path);
+  // mixed-task batch: the instance as a batch of its current mode sees it (its players, its mode_number)
+  agarcl_cfg c = b->cfg;
+  CK(cudaMemcpy(&c.mode_number, b->d_task_mode + instance, sizeof(int32_t), cudaMemcpyDeviceToHost));
+  agarcl_layout L;
+  task_layout(&b->cfg, &b->L, c.mode_number, &L);
+  return agarcl_snapshot_write(&c, &L, blob.data(), path);
 }
 
 extern "C" int agarcl_batch_load_env_state(agarcl_batch* b, int32_t instance, const char* path, int lossless) {
@@ -999,8 +1028,25 @@ extern "C" int agarcl_batch_load_env_state(agarcl_batch* b, int32_t instance, co
   CK(cudaDeviceSynchronize());
   std::vector<uint8_t> blob(b->L.stride);
   CK(cudaMemcpy(blob.data(), b->d_state + (size_t)instance * b->L.stride, b->L.stride, cudaMemcpyDeviceToHost));
-  int rc = agarcl_snapshot_read(&b->cfg, &b->L, blob.data(), path, lossless);
+  agarcl_cfg c = b->cfg;
+  agarcl_layout L = b->L;
+  if (b->cfg.task_modes) {  // mixed-task batch: any mode of the set, which becomes the instance's current task
+    int rc = snapshot_file_mode(path, &c.mode_number);
+    if (rc) return rc;
+    if (c.mode_number < 0 || c.mode_number > 10 || !((b->cfg.task_modes >> c.mode_number) & 1))
+      return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot mode_number %d is not in the batch's task_modes 0x%x", c.mode_number, b->cfg.task_modes);
+    task_layout(&b->cfg, &b->L, c.mode_number, &L);
+  }
+  int rc = agarcl_snapshot_read(&c, &L, blob.data(), path, lossless);
   if (rc) return rc;
+  if (b->cfg.task_modes) {
+    agarcl_player* pls = reinterpret_cast<agarcl_player*>(blob.data() + b->L.off_players);
+    for (int p = L.P; p < b->L.P; p++) {  // the mode's absent players, as a reset leaves them
+      std::memset(&pls[p], 0, sizeof(agarcl_player));
+      pls[p].bot_type = ag::mode_bot_type(c.mode_number, p, b->L.A);
+    }
+    CK(cudaMemcpy(b->d_task_mode + instance, &c.mode_number, sizeof(int32_t), cudaMemcpyHostToDevice));  // (its step limit stays)
+  }
   const agarcl_inst_hdr* hdr = reinterpret_cast<const agarcl_inst_hdr*>(blob.data() + b->L.off_hdr);
   b->seeds[instance] = (uint64_t)hdr->seed_lo | ((uint64_t)hdr->seed_hi << 32);
   CK(cudaMemcpy(b->d_seeds + instance, &b->seeds[instance], sizeof(uint64_t), cudaMemcpyHostToDevice));
@@ -1071,6 +1117,9 @@ static ag::SnapParams snapshot_params(const agarcl_batch* b, const void* pool, i
   P.dones = b->d_dones;
   P.result = b->d_snap_result;
   P.restored = b->d_snap_restored;
+  P.task_mode = b->d_task_mode;
+  P.task_max_steps = b->d_task_max_steps;
+  P.task_modes = b->cfg.task_modes;
   P.N = b->N;
   P.A = b->A;
   P.instance_base = b->cfg.instance_base;
@@ -1105,5 +1154,34 @@ extern "C" int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, in
   // a one-frame grid observation is re-rendered, as the step that produced the state showed it (respawned players still dead)
   if (b->cfg.ram_obs != 2 && b->frames == 1 && (rc = render_frame(b, 0, s, 1, 0, b->d_snap_restored))) return rc;
   if (d_result) *d_result = b->d_snap_result;
+  return AGARCL_OK;
+}
+
+// ---- mixed-task batches (include/agarcl_b200.h)
+extern "C" int agarcl_batch_set_tasks(agarcl_batch* b, const int32_t* d_mode, const int32_t* d_max_steps, uint8_t** d_result, void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (!b->cfg.task_modes) return agarcl_set_error(AGARCL_ERR_STATE, "the batch was created without task_modes");
+  if (!d_mode) return agarcl_set_error(AGARCL_ERR_INVALID, "null mode array");
+  CK(cudaSetDevice(b->cfg.device));
+  ag::SetTasksParams P;
+  P.mode = d_mode;
+  P.max_steps = d_max_steps;
+  P.next_mode = b->d_next_mode;
+  P.next_max_steps = b->d_next_max_steps;
+  P.result = b->d_task_result;
+  P.N = b->N;
+  P.task_modes = b->cfg.task_modes;
+  CK(ag::launch_set_tasks(P, (cudaStream_t)stream));
+  if (d_result) *d_result = b->d_task_result;
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_tasks(agarcl_batch* b, agarcl_tasks* out) {
+  if (!b || !out) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
+  if (!b->cfg.task_modes) return agarcl_set_error(AGARCL_ERR_STATE, "the batch was created without task_modes");
+  out->mode = b->d_task_mode;
+  out->max_steps = b->d_task_max_steps;
+  out->next_mode = b->d_next_mode;
+  out->next_max_steps = b->d_next_max_steps;
   return AGARCL_OK;
 }

@@ -1,6 +1,6 @@
 // episode_kernel.cu — what a vector environment with auto-reset does around the step, on the device: the episode
 // bookkeeping of agarcl_batch_step_autoreset (done flags with the step limit folded in, the reset mask, step counters,
-// returns) and the masked per-instance byte copy / clear used by a masked reset and by the final-observation copy.
+// returns), the pending tasks of a mixed-task batch (agarcl_batch_set_tasks) and the masked per-instance byte copy / clear used by a masked reset and by the final-observation copy.
 // Neither needs the host to look at the step's dones, so the step, the bookkeeping and the reset queue back to back.
 #include <cuda_runtime.h>
 
@@ -26,7 +26,9 @@ __global__ void __launch_bounds__(256) k_episode(const __grid_constant__ Episode
     return;
   }
   int64_t s = P.steps[i];
-  const bool limit = P.max_steps > 0 && s >= (int64_t)P.max_steps;
+  int32_t max_steps = P.max_steps;
+  if (P.task_max_steps && P.task_max_steps[i] >= 0) max_steps = P.task_max_steps[i];  // (-1: the batch's limit)
+  const bool limit = max_steps > 0 && s >= (int64_t)max_steps;
   bool any = false;
   for (int a = 0; a < A; a++) {
     const size_t k = (size_t)i * A + a;
@@ -47,6 +49,20 @@ __global__ void __launch_bounds__(256) k_episode(const __grid_constant__ Episode
   P.reset_mask[i] = reset ? 1 : 0;
 }
 
+// One thread per instance: agarcl_batch_set_tasks.  A rejected entry leaves the instance's pending task as it is.
+__global__ void __launch_bounds__(256) k_set_tasks(const __grid_constant__ SetTasksParams P) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.N) return;
+  const int32_t m = P.mode[i];
+  const bool set_mode = m != -1, set_limit = P.max_steps != nullptr;
+  const int32_t ms = set_limit ? P.max_steps[i] : -1;
+  const bool bad_mode = set_mode && (m < 0 || m > 10 || !((P.task_modes >> m) & 1));
+  if (bad_mode || ms < -1) { P.result[i] = 2; return; }
+  if (set_mode) P.next_mode[i] = m;
+  if (set_limit) P.next_max_steps[i] = ms;
+  P.result[i] = (set_mode || set_limit) ? 1 : 0;
+}
+
 // One CTA per instance: bytes [i * per, (i + 1) * per) of dst get those of src (kCopy) or zeros, for the instances with
 // mask[i] != 0; the CTAs of the others exit at once.  dst and src are allocations of the same alignment, so the slices
 // of one instance share their alignment modulo 16 (block_copy).
@@ -60,6 +76,11 @@ __global__ void __launch_bounds__(kMaskedThreads) k_masked_bytes(uint8_t* __rest
 
 cudaError_t launch_episode(const EpisodeParams& P, cudaStream_t stream) {
   k_episode<<<(P.N + 255) / 256, 256, 0, stream>>>(P);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_set_tasks(const SetTasksParams& P, cudaStream_t stream) {
+  k_set_tasks<<<(P.N + 255) / 256, 256, 0, stream>>>(P);
   return cudaGetLastError();
 }
 

@@ -9,3 +9,10 @@ int agarcl_set_error(int status, const char* fmt, ...);
 // snapshot.cpp: the reference's JSON environment snapshot to / from one instance blob (host memory)
 extern "C" int agarcl_snapshot_write(const agarcl_cfg* c, const agarcl_layout* L, const void* blob, const char* path);
 extern "C" int agarcl_snapshot_read(const agarcl_cfg* c, const agarcl_layout* L, void* blob, const char* path, int lossless);
+// snapshot.cpp: the mode_number a JSON snapshot was written in
+int snapshot_file_mode(const char* path, int* mode);
+
+// layout.cpp, mixed-task batches (cfg.task_modes): the layout of the batch as an instance of `mode` sees it -- P = A + its
+// bots, its mode flags and bot types, and the player order a batch of that mode alone uses (agarcl_make_layout checks that
+// it is the order of the batch's players < P)
+void task_layout(const agarcl_cfg* c, const agarcl_layout* L, int mode, agarcl_layout* out);

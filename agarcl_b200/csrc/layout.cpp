@@ -1,20 +1,41 @@
 // layout.cpp — host-side derivation of the per-instance state layout and of everything that is a
-// pure function of the environment configuration (mode flags, bot roster, player iteration order).
+// pure function of the environment configuration (mode flags and bot roster from mode_rules.h, player iteration order).
 //
 // Reference behaviour restated here:
-//   Engine::set_mode                     agario/engine/Engine.hpp:367-416
-//   BaseEnvironment::reset / add_bots    environment/envs/BaseEnvironment.hpp:179-204,374-425
 //   create_squared_pellets (count only)  agario/engine/Engine.hpp:426-475
 //   GridObservation::channels_per_frame  environment/envs/GridEnvironment.hpp:188-195
 //   GameState::PlayerMap iteration       agario/engine/GameState.hpp:44  (std::unordered_map<pid, ...>)
+#include <algorithm>
 #include <cstring>
 #include <random>
 #include <unordered_map>
 
 #include "../../include/agarcl_b200.h"
 #include "host_util.h"
+#include "mode_rules.h"
 
 static uint32_t align_up(uint32_t x, uint32_t a) { return (x + a - 1) / a * a; }
+
+// player iteration order: the same container the reference iterates, fed the same insert sequence
+static void player_order(int P, int32_t* order) {
+  std::unordered_map<unsigned short, int> m;
+  for (int p = 0; p < P; p++) m.insert(std::make_pair((unsigned short)p, p));
+  int k = 0;
+  for (auto& kv : m) order[k++] = kv.second;
+}
+
+void task_layout(const agarcl_cfg* c, const agarcl_layout* L, int mode, agarcl_layout* out) {
+  *out = *L;
+  const ag::ModeRules R = ag::mode_rules(mode, c->num_bots);
+  out->P = L->A + R.bots;
+  out->mass_decay = R.mass_decay;
+  out->squared_pellets = R.squared_pellets;
+  out->regen = R.regen;
+  out->agent_mass = R.agent_mass;
+  for (int p = 0; p < AGARCL_MAX_PLAYERS; p++) out->bot_type[p] = p < out->P ? ag::mode_bot_type(mode, p, L->A) : 0;
+  player_order(out->P, out->order);
+  for (int p = out->P; p < AGARCL_MAX_PLAYERS; p++) out->order[p] = 0;
+}
 
 extern "C" int agarcl_make_layout(const agarcl_cfg* c, agarcl_layout* L) {
   if (!c || !L) return agarcl_set_error(AGARCL_ERR_INVALID, "null cfg/layout");
@@ -30,45 +51,56 @@ extern "C" int agarcl_make_layout(const agarcl_cfg* c, agarcl_layout* L) {
   if (c->num_frames < 1) return agarcl_set_error(AGARCL_ERR_INVALID, "num_frames must be >= 1");
 
   const int mode = c->mode_number;
-  // Engine::set_mode
-  int base = mode;
-  if (mode == 5) base = 2;
-  if (mode == 6 || mode >= 7) base = 4;
-  L->mass_decay = (base == 0 || base == 2 || base == 4);
-  L->squared_pellets = (base == 1 || base == 2);
-  L->regen = (base == 0 || base == 3 || base == 4);
-  L->agent_mass = (mode == 5 || mode == 6) ? 1000 : 25;
+  const int task_modes = c->task_modes;
+  if (task_modes) {  // a mixed-task batch: every mode of the set can run in it (include/agarcl_b200.h, agarcl_cfg.task_modes)
+    if (task_modes & ~0x7FF) return agarcl_set_error(AGARCL_ERR_INVALID, "task_modes holds a mode outside 0..10");
+    if (!((task_modes >> mode) & 1)) return agarcl_set_error(AGARCL_ERR_INVALID, "task_modes must contain mode_number %d", mode);
+    if (c->strict_reference)
+      return agarcl_set_error(AGARCL_ERR_INVALID, "task_modes is refused under strict_reference: the player order belongs to the batch");
+  }
+  const ag::ModeRules R = ag::mode_rules(mode, c->num_bots);
+  L->mass_decay = R.mass_decay;
+  L->squared_pellets = R.squared_pellets;
+  L->regen = R.regen;
+  L->agent_mass = R.agent_mass;
 
-  // BaseEnvironment::reset: bots only in mode 0 (num_bots of them) and modes 7..10 (exactly one)
-  int bots = 0;
-  if (mode == 0) bots = c->num_bots;
-  else if (mode > 6) bots = 1;
+  // players: the agents, then the bots of the mode with the most of them
+  int bots = R.bots;
+  for (int m = 0; m <= 10; m++)
+    if ((task_modes >> m) & 1) bots = std::max(bots, ag::mode_rules(m, c->num_bots).bots);
+  if (((task_modes >> 0) & 1) && task_modes != 1) {
+    // mode 0 respawns every dead player, an absent one included: it may only share a batch with modes of its bot count
+    for (int m = 1; m <= 10; m++)
+      if (((task_modes >> m) & 1) && ag::mode_rules(m, c->num_bots).bots != c->num_bots)
+        return agarcl_set_error(AGARCL_ERR_INVALID, "task_modes: mode 0 (%d bots) cannot share a batch with mode %d (%d bots)", c->num_bots, m,
+                                ag::mode_rules(m, c->num_bots).bots);
+  }
   L->A = c->num_agents;
   L->P = c->num_agents + bots;
   if (L->P > AGARCL_MAX_PLAYERS) return agarcl_set_error(AGARCL_ERR_INVALID, "too many players per instance (agents + bots > 64)");
-  for (int p = 0; p < L->P; p++) {
-    if (p < L->A) L->bot_type[p] = -1;
-    else if (mode == 0) {
-      int i = p - L->A;  // add_bots: switch (i % num_bots_) with i < num_bots_  (quirk Q14)
-      L->bot_type[p] = (i < 4) ? i : 0;
-    } else {
-      int idx = mode - 7;  // custom_add_bot
-      L->bot_type[p] = (idx >= 0 && idx < 4) ? idx : 0;
-    }
-  }
-  // player iteration order: the same container the reference iterates, fed the same insert sequence
-  {
-    std::unordered_map<unsigned short, int> m;
-    for (int p = 0; p < L->P; p++) m.insert(std::make_pair((unsigned short)p, p));
+  for (int p = 0; p < L->P; p++) L->bot_type[p] = ag::mode_bot_type(mode, p, L->A);
+  player_order(L->P, L->order);
+  for (int m = 0; m <= 10; m++) {
+    if (!((task_modes >> m) & 1)) continue;
+    // an instance of mode m plays players 0 .. P_m - 1 in the batch's order: it must be the order of a batch of mode m alone
+    const int Pm = L->A + ag::mode_rules(m, c->num_bots).bots;
+    int alone[AGARCL_MAX_PLAYERS];
+    player_order(Pm, alone);
     int k = 0;
-    for (auto& kv : m) L->order[k++] = kv.second;
+    for (int j = 0; j < L->P; j++)
+      if (L->order[j] < Pm && L->order[j] != alone[k++])
+        return agarcl_set_error(AGARCL_ERR_INVALID, "task_modes: the player order of mode %d differs from the batch's (%d agents, %d players)", m,
+                                L->A, L->P);
   }
 
   L->cap_cells = AGARCL_MAX_CELLS;
   int cap_p = c->num_pellets;
-  if (L->squared_pellets) {
-    int sq = 4 * (c->arena_size / 2);  // 4 sides x int(min(W,H)/2 / spacing 1)
-    if (sq > cap_p) cap_p = sq;
+  for (int m = 0; m <= 10; m++) {
+    if (m != mode && !((task_modes >> m) & 1)) continue;
+    if (ag::mode_rules(m, c->num_bots).squared_pellets) {
+      int sq = 4 * (c->arena_size / 2);  // 4 sides x int(min(W,H)/2 / spacing 1)
+      if (sq > cap_p) cap_p = sq;
+    }
   }
   if (cap_p < 1) cap_p = 1;
   if (cap_p > 65000) return agarcl_set_error(AGARCL_ERR_INVALID, "pellet capacity exceeds 65000");

@@ -51,12 +51,24 @@ __global__ void __launch_bounds__(128) k_reset(const __grid_constant__ ResetPara
   agarcl_virus* vir = reinterpret_cast<agarcl_virus*>(blob + P.L.off_viruses);
   float2* pel = reinterpret_cast<float2*>(blob + P.L.off_pellets);
   const float W = P.W;
+  // the rules this episode plays: mode_number's (the layout's flags), or in a mixed-task batch the instance's pending task,
+  // which becomes its current one here
+  int squared = P.L.squared_pellets, agent_mass = P.L.agent_mass, Pm = P.L.P, mode = 0;
+  if (P.task_mode) {
+    mode = P.next_mode[inst];
+    const int32_t ms = P.next_max_steps[inst];
+    const ModeRules R = mode_rules(mode, P.num_bots);
+    squared = R.squared_pellets;
+    agent_mass = R.agent_mass;
+    Pm = P.L.A + R.bots;
+    if (lane == 0) { P.task_mode[inst] = mode; P.task_max_steps[inst] = ms; }
+  }
   // Engine::reset does not touch the RNG (Engine.hpp:98-117): a second episode goes on in the stream; only seed() restarts it
   uint32_t cursor = (P.fresh && !P.fresh[inst]) ? hdr->rng_cursor : 0u;
   __syncwarp();
   int n_pellets = 0;
 
-  if (P.L.squared_pellets) {
+  if (squared) {
     // create_squared_pellets: four sides of a centred square, one pellet per unit, kept if inside
     float square = W / 2.0f, spacing = 1.0f;
     int pps = (int)(square / spacing);
@@ -102,10 +114,15 @@ __global__ void __launch_bounds__(128) k_reset(const __grid_constant__ ResetPara
   }
   __syncwarp();
   // players: Player ctor defaults + respawn (Player.hpp:25-41; Engine.hpp:119-137)
-  const uint32_t mass = (uint32_t)(P.L.agent_mass > 25 ? P.L.agent_mass : 25);
+  const uint32_t mass = (uint32_t)(agent_mass > 25 ? agent_mass : 25);
   const float r25 = radius_of(P.T, AGARCL_CELL_MIN_SIZE);
-  const bool anchored = P.L.squared_pellets && n_pellets > 0;
-  for (int p = lane; p < P.L.P; p += 32) {
+  const bool anchored = squared && n_pellets > 0;
+  for (int p = Pm + lane; p < P.L.P; p += 32) {  // absent players (mixed-task batch): dead records, no draw
+    uint4* pr = reinterpret_cast<uint4*>(players + p);
+    for (int q = 0; q < 8; q++) pr[q] = make_uint4(0u, 0u, 0u, 0u);
+    players[p].bot_type = mode_bot_type(mode, p, P.L.A);
+  }
+  for (int p = lane; p < Pm; p += 32) {
     float x, y;
     if (anchored) {
       float2 p0 = pel[0];
@@ -119,7 +136,7 @@ __global__ void __launch_bounds__(128) k_reset(const __grid_constant__ ResetPara
     agarcl_player* pl = players + p;
     pl->n_cells = 1;
     pl->anti_team_decay = 1.0f;
-    pl->bot_type = P.L.bot_type[p];
+    pl->bot_type = P.task_mode ? mode_bot_type(mode, p, P.L.A) : P.L.bot_type[p];
     pl->min_mass_cell = AGARCL_CELL_MIN_SIZE;
     pl->highest_mass = AGARCL_CELL_MIN_SIZE;
     float4* cp = reinterpret_cast<float4*>(cells + (size_t)p * AGARCL_MAX_CELLS);
@@ -128,13 +145,13 @@ __global__ void __launch_bounds__(128) k_reset(const __grid_constant__ ResetPara
                         __uint_as_float(1u + (uint32_t)p));
     reinterpret_cast<uint4*>(cp)[2] = make_uint4(0u, 0u, 0u, 0u);  // recomb_tick = tick 0
   }
-  if (!anchored) cursor += 2u * (uint32_t)P.L.P;
+  if (!anchored) cursor += 2u * (uint32_t)Pm;
   c.flags = __reduce_or_sync(AG_FULL, c.flags);
   for (int a = lane; a < P.L.A; a += 32) P.dones[(size_t)inst * P.L.A + a] = 0;
   if (lane == 0) {
     if (P.fresh) P.fresh[inst] = 0;
     hdr->tick = 0;
-    hdr->next_cell_id = 1u + (uint32_t)P.L.P;
+    hdr->next_cell_id = 1u + (uint32_t)Pm;
     hdr->n_pellets = n_pellets;
     hdr->n_viruses = min(P.num_viruses, P.L.cap_viruses);
     hdr->n_foods = 0;

@@ -125,6 +125,7 @@ struct ColdCtx {
   int inst_local;
   int pos;              // position of the instance in this launch's schedule (the host mirror's lists are laid out by position)
   int tb;               // the alignment barriers of this launch (P.tick_barrier, or 0 when the launch runs the free-running schedule)
+  int mode;             // the instance's current mode (P.task_mode[inst] in a mixed-task batch, else P.mode)
 };
 static_assert(sizeof(ColdCtx) <= kColdCtxBytes - 16, "ColdCtx outgrew its shared-memory slot");
 
@@ -164,6 +165,13 @@ struct Ctx {
   static constexpr float dt = (float)(1.0 / 30.0);
   __device__ Ctx(const SimParams& p) : P(p) {}
   __device__ __forceinline__ agarcl_cell* pcells(int p) const { return cells_() + (size_t)p * AGARCL_MAX_CELLS; }
+  // the rules of the instance's mode: the launch parameters' unless the batch mixes tasks (mode_rules.h)
+  __device__ __forceinline__ ModeRules rules() const { return mode_rules(cold().mode, P.num_bots); }
+  __device__ __forceinline__ bool mass_decay() const { return P.task_mode ? rules().mass_decay != 0 : P.L.mass_decay != 0; }
+  __device__ __forceinline__ bool regen() const { return P.task_mode ? rules().regen != 0 : P.L.regen != 0; }
+  __device__ __forceinline__ bool squared_pellets() const { return P.task_mode ? rules().squared_pellets != 0 : P.L.squared_pellets != 0; }
+  __device__ __forceinline__ int agent_mass() const { return P.task_mode ? rules().agent_mass : P.L.agent_mass; }
+  __device__ __forceinline__ int bot_type(int p) const { return P.task_mode ? mode_bot_type(cold().mode, p, P.L.A) : P.L.bot_type[p]; }
 };
 
 // one uniform draw in [0,1): k-th draw of this instance (Engine::random<T>, Engine.hpp:1304-1311)
@@ -694,7 +702,7 @@ __device__ void premove_players(const SimParams& P, uint8_t* smem_raw, Ctx* c, i
         // to the bot's location at the START of the tick (HungryBot.hpp:19-22, Bot::nearest_pellet Bot.hpp:92-129; pellets
         // only disappear behind the loop), so the multi-cell HungryBots decide HERE, every one on its own lane, and join the
         // pool; agents keep the target of their action.  The bots that look at other players (types 1..3) stay in the loop.
-        const int bt = k < Pn ? P.L.bot_type[p] : 0;
+        const int bt = k < Pn ? c->bot_type(p) : 0;
         if (np >= 2 && np <= 16 && bt == 0 && c->n_pellets > 0 && c->hash_valid) {
           const float4 sp = c->sm.psum()[p];
           float tx = 0.0f, ty = 0.0f;
@@ -1312,7 +1320,7 @@ __device__ void tick_player(Ctx& c, int p) {
   // ---- once per 60 player-ticks: anti-team + decay
   float atd = __int_as_float(w1.z);
   int last_decay = w2.x;
-  if (c.P.L.mass_decay && elapsed % 60 == 0) {
+  if (c.mass_decay() && elapsed % 60 == 0) {
     int fall_off = elapsed - 60 * 60;
     __syncwarp();
     int t = (lane < vet_count) ? pl->vet_ticks[lane] : 0;
@@ -1568,7 +1576,7 @@ __device__ __forceinline__ void tick_players_block(Ctx& c, int base, LaneState& 
   // committed, so it is speculated LATE, alone, when the ordered commit reaches it
   enum { kIdle = 0, kPending = 1, kLate = 2, kReady = 3, kSerial = 4 };
   int st = n >= 2 ? kSerial : (n == 1 ? kPending : kIdle);  // dead players are not ticked (Engine.hpp:216)
-  if (st == kPending && c.tick % 10u == 0u && c.P.L.bot_type[p] > 0) st = kLate;
+  if (st == kPending && c.tick % 10u == 0u && c.bot_type(p) > 0) st = kLate;
   float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
   uint32_t food_mass = 0;  // mass at the time of eat_food (after pellets, before decay)
   int ne = 0;
@@ -1666,7 +1674,7 @@ __device__ __forceinline__ void tick_players_block(Ctx& c, int base, LaneState& 
     }
 
     // ---- once per 60 player-ticks: anti-team (only with remembered virus hits -> serial) + decay
-    if (c.P.L.mass_decay && elapsed % 60 == 0) {
+    if (c.mass_decay() && elapsed % 60 == 0) {
       if (vet_count > 0) break;
       if (elapsed - last_decay >= 60) {
         uint32_t nm = (uint32_t)((double)me.mass * (1 - 0.002 * (double)atd));
@@ -2746,7 +2754,7 @@ __device__ __forceinline__ void engine_tick(Ctx& c, LaneState& ls) {
   AG_PH(c, 7);
   if (c.cold().tb & 8) { c.cold().work += clock64() - c.cold().t_mark; align_barrier(c.P.align_group); c.cold().t_mark = clock64(); }
   move_foods(c);
-  if (c.P.L.regen && c.tick % 120u == 0u) regen(c);
+  if (c.regen() && c.tick % 120u == 0u) regen(c);
   c.tick++;
   AG_PH(c, 8);
 }
@@ -2754,10 +2762,11 @@ __device__ __forceinline__ void engine_tick(Ctx& c, LaneState& ls) {
 // Player::kill + Engine::respawn for a dead player, spawn point from draw pair `k` (Engine.hpp:119-137)
 __device__ void respawn_player(Ctx& c, int p, uint32_t k) {
   agarcl_player* pl = c.players_() + p;
-  uint32_t mass = (uint32_t)(c.P.L.agent_mass > 25 ? c.P.L.agent_mass : 25);
+  const int agent_mass = c.agent_mass();
+  uint32_t mass = (uint32_t)(agent_mass > 25 ? agent_mass : 25);
   float r25 = radius_of(c.P.T, AGARCL_CELL_MIN_SIZE);
   float x, y;
-  if (c.n_pellets > 0 && c.P.L.squared_pellets) {
+  if (c.n_pellets > 0 && c.squared_pellets()) {
     float2 p0 = c.sm.spel()[0];
     x = fmin_std(p0.x + 2.0f * r25, c.W - r25);
     y = fmin_std(p0.y + 2.0f * r25, c.W - r25);
@@ -2796,6 +2805,7 @@ __device__ __forceinline__ void step_instance(const SimParams& P, uint8_t* smem_
   c.cold().pos = pos;
   c.cold().work = 0; c.cold().t_mark = clock64();
   c.cold().inst_local = inst;
+  int mode = P.mode;  // (the instance's mode is requested below with the rest of the step's first round trip)
   // the pellet array comes in by one TMA bulk load (whole capacity: the count is not known yet); everything
   // below that does not touch pellets overlaps with it, build_pellet_hash is its first consumer
   const uint32_t pel_bytes = ((uint32_t)P.L.cap_pellets * 8u + 15u) & ~15u;  // pellets are the blob's last array: the pad is inside its stride
@@ -2823,6 +2833,7 @@ __device__ __forceinline__ void step_instance(const SimParams& P, uint8_t* smem_
     ls.me = cell_load(c.pcells(p0));
     ls.fresh = valid0;
   }
+  if (P.task_mode) mode = P.task_mode[inst];
   float4 vpre[2];
 #pragma unroll
   for (int j = 0; j < 2; j++) {
@@ -2850,6 +2861,7 @@ __device__ __forceinline__ void step_instance(const SimParams& P, uint8_t* smem_
     c.n_foods = h1.x; c.cold().cursor = (uint32_t)h1.y; c.flags = (uint32_t)h1.z; done_sticky = (uint32_t)h2.y;
   }
   c.nprem = 0; c.nvrem = 0;
+  c.cold().mode = mode;
   c.cold().emitted = 0; c.hash_valid = false; c.vc_valid = false; c.lanes_dirty = false; c.cold().min_vmass = 0xffffffffu;
   c.pel_dirty = false;
   c.cold().sorted_lo = 0u; c.cold().sorted_hi = 0u;
@@ -2908,7 +2920,7 @@ __device__ __forceinline__ void step_instance(const SimParams& P, uint8_t* smem_
         pl->target_y = s.y + ady * 10.0f;
         pl->action = aact;
       }
-      if (P.mode == 3 && m >= 23000u) done_sticky = 1u;
+      if (c.cold().mode == 3 && m >= 23000u) done_sticky = 1u;
     }
     // the lane that holds an agent's record in registers applies the same action to its copy
     if (valid0 && p0 < A && ls.w0.x > 0) {
@@ -2958,7 +2970,8 @@ __device__ __forceinline__ void step_instance(const SimParams& P, uint8_t* smem_
   if (P.do_end) {
     if (P.obs_finish == 1) obs_finish_warp<int32_t>(c);
     else if (P.obs_finish == 2) obs_finish_warp<int16_t>(c);
-    if (P.mode == 0) {
+    const int mode_now = c.cold().mode;
+    if (mode_now == 0) {
       // repsawn_all_players in map order: the r-th dead player takes draw pair r
       uint32_t rank_base = 0;
       uint32_t resp_lo = 0, resp_hi = 0;
@@ -2981,17 +2994,17 @@ __device__ __forceinline__ void step_instance(const SimParams& P, uint8_t* smem_
       }
       if (lane == 0) { hdr->respawned_lo = resp_lo; hdr->respawned_hi = resp_hi; }
       c.cold().next_id += rank_base;
-      if (!(P.L.squared_pellets && c.n_pellets > 0)) c.cold().cursor += 2u * rank_base;
+      if (!(c.squared_pellets() && c.n_pellets > 0)) c.cold().cursor += 2u * rank_base;
       c.flags = __reduce_or_sync(AG_FULL, c.flags);
       __syncwarp();
-    } else if (P.mode > 6) {
+    } else if (mode_now > 6) {
       bool dead = false;
       for (int p = lane; p < Pn; p += 32) dead |= __float_as_int(c.sm.psum()[p].w) == 0;
       done_sticky = __ballot_sync(AG_FULL, dead) ? 1u : 0u;  // dones_[0] rewritten every step (BaseEnvironment.hpp:103-114)
     }
     for (int a = lane; a < A; a += 32) {
       uint32_t m = __float_as_uint(c.sm.psum()[a].z);
-      if (P.mode == 3 && m >= 23000u) done_sticky = 1u;
+      if (mode_now == 3 && m >= 23000u) done_sticky = 1u;
     }
     done_sticky = __reduce_or_sync(AG_FULL, done_sticky);
     for (int a = lane; a < A; a += 32) {

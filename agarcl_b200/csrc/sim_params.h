@@ -6,6 +6,7 @@
 
 #include "../../include/agarcl_b200.h"
 #include "device_math.cuh"
+#include "mode_rules.h"
 
 namespace ag {
 
@@ -90,6 +91,9 @@ struct SimParams {
   int32_t do_begin;        // apply actions + record `before`
   int32_t do_end;          // respawn / dones / rewards
   int32_t mode, reward_type, rng_mode;
+  const int32_t* task_mode;  // [N] mixed-task batch (cfg.task_modes): each instance's current mode, read once per launch into ColdCtx;
+                             // nullptr: every instance plays `mode` with the flags of L
+  int32_t num_bots;          // cfg.num_bots (mode_rules, mixed-task batch)
   int32_t target_pellets, target_viruses;
   int32_t HG;              // spatial hash is HG x HG over the arena
   float W;                 // arena width == height
@@ -145,7 +149,11 @@ struct ResetParams {
                            // stream goes on where the last episode left it, like the reference's engine RNG across reset()
                            // (BaseEnvironment.hpp:179-204 does not reseed); cleared by the kernel
   uint8_t* dones;
-  int32_t N, instance_base, rng_mode, num_pellets, num_viruses;
+  // mixed-task batch (cfg.task_modes; nullptr otherwise): every reset instance takes its pending task (next_*) as its current one
+  // and is spawned by the rules of that mode, with players P_m .. P-1 absent
+  int32_t *task_mode, *task_max_steps;
+  const int32_t *next_mode, *next_max_steps;
+  int32_t N, instance_base, rng_mode, num_pellets, num_viruses, num_bots;
   float W;
 };
 cudaError_t launch_reset(const ResetParams& P, cudaStream_t stream);
@@ -191,11 +199,21 @@ struct EpisodeParams {
   double* final_ret;         // [N*A] ret of the episode that finished last
   int64_t* final_len;        // [N] steps of the episode that finished last
   const uint8_t* clear_mask; // clear mode: the instances being reset, nullptr = all
+  const int32_t* task_max_steps;  // [N] mixed-task batch: the instance's step limit (-1: max_steps, 0: none); nullptr: max_steps for all
   int32_t N, A, max_steps;
   int32_t reset;             // 1: finished instances are reset by this step (auto-reset); 0: bookkeeping only
   int32_t clear;             // 1: a reset restarts the counters of clear_mask's instances (no step)
 };
 cudaError_t launch_episode(const EpisodeParams& P, cudaStream_t stream);
+// agarcl_batch_set_tasks: pending task of instance i <- (mode[i], max_steps[i]) where given and valid; result[i] 0 / 1 / 2
+struct SetTasksParams {
+  const int32_t* mode;       // [N], -1 keeps the pending mode
+  const int32_t* max_steps;  // [N] or nullptr (every pending limit kept)
+  int32_t *next_mode, *next_max_steps;
+  uint8_t* result;
+  int32_t N, task_modes;
+};
+cudaError_t launch_set_tasks(const SetTasksParams& P, cudaStream_t stream);
 // dst = src (nullptr: zeros) in the `per`-byte slices of the instances with mask != 0
 cudaError_t launch_masked_bytes(void* dst, const void* src, size_t per, const uint8_t* mask, int N, cudaStream_t stream);
 
@@ -228,6 +246,9 @@ struct SnapParams {
   uint8_t* dones;            // [N*A]
   uint8_t* result;           // [N] 0 not requested, 1 restored, 2 rejected
   uint8_t* restored;         // [N] 1 where restored: the mask of the k_obs launch behind
+  int32_t* task_mode;        // [N] mixed-task batch: the current task, stored in the slot header and restored from it; else nullptr
+  int32_t* task_max_steps;   // [N]
+  int32_t task_modes;        // cfg.task_modes: a restored slot's mode must be in it
   int32_t N, A, instance_base;
 };
 cudaError_t launch_snapshot_save(const SnapParams& P, int n, cudaStream_t stream);

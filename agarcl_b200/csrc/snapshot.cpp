@@ -120,7 +120,31 @@ struct Parser {
 
 const char* kBotNames[4] = {"HungryBot", "HungryShyBot", "AggressiveBot", "AggressiveShyBot"};
 
+// the whole file parsed; AGARCL_ERR_INVALID when it cannot be read or is not a JSON object
+int parse_file(const char* path, JV& root) {
+  FILE* f = fopen(path, "r");
+  if (!f) return agarcl_set_error(AGARCL_ERR_INVALID, "Failed to open %s for reading", path);
+  std::string text;
+  char buf[1 << 16];
+  size_t n;
+  while ((n = fread(buf, 1, sizeof buf, f)) > 0) text.append(buf, n);
+  fclose(f);
+  Parser ps{text.data(), text.data() + text.size()};
+  root = ps.value();
+  if (!ps.ok || root.t != JV::OBJ) return agarcl_set_error(AGARCL_ERR_INVALID, "%s is not a JSON environment snapshot", path);
+  return AGARCL_OK;
+}
+
 }  // namespace
+
+int snapshot_file_mode(const char* path, int* mode) {
+  JV root;
+  int rc = parse_file(path, root);
+  if (rc) return rc;
+  if (!root.get("mode_number")) return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot %s has no mode_number", path);
+  *mode = (int)root.n("mode_number");
+  return AGARCL_OK;
+}
 
 // blob -> file.  `cfg` supplies what the blob does not carry (BaseEnvironment's own members).
 // Players are written in pid order: Engine::load_env_state re-adds them in file order with fresh pids
@@ -189,16 +213,9 @@ extern "C" int agarcl_snapshot_write(const agarcl_cfg* c, const agarcl_layout* L
 
 // file -> blob (Engine::load_env_state).  `blob` must be an initialised blob of this layout (its header seed/flags are kept unless the file has them).
 extern "C" int agarcl_snapshot_read(const agarcl_cfg* c, const agarcl_layout* L, void* blob_, const char* path, int lossless) {
-  FILE* f = fopen(path, "r");
-  if (!f) return agarcl_set_error(AGARCL_ERR_INVALID, "Failed to open %s for reading", path);
-  std::string text;
-  char buf[1 << 16];
-  size_t n;
-  while ((n = fread(buf, 1, sizeof buf, f)) > 0) text.append(buf, n);
-  fclose(f);
-  Parser ps{text.data(), text.data() + text.size()};
-  JV root = ps.value();
-  if (!ps.ok || root.t != JV::OBJ) return agarcl_set_error(AGARCL_ERR_INVALID, "%s is not a JSON environment snapshot", path);
+  JV root;
+  int rc = parse_file(path, root);
+  if (rc) return rc;
   if ((int)root.n("mode_number", c->mode_number) != c->mode_number)
     return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot mode_number %d does not match the environment's %d", (int)root.n("mode_number"), c->mode_number);
   const JV* players = root.get("players");

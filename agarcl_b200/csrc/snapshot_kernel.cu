@@ -45,12 +45,14 @@ __global__ void __launch_bounds__(kSnapThreads) k_snapshot(const __grid_constant
       if (P.S.obs_bytes) copy_segment(sl + P.S.off_obs, P.obs + (size_t)src * P.S.obs_bytes, P.S.obs_bytes);
     }
     __syncthreads();  // the header goes last; a source out of range leaves magic 0, which a restore rejects
-    if (t == 0) {  // agarcl_snapshot_hdr: magic, version, fingerprint, slot_bytes, source, zero padding
+    if (t == 0) {  // agarcl_snapshot_hdr: magic, version, fingerprint, slot_bytes, source, task (mixed-task batch), zero padding
       const uint4 z = make_uint4(0u, 0u, 0u, 0u);
       uint4* hv = reinterpret_cast<uint4*>(sl);
+      const bool task = ok && P.task_mode;
       hv[0] = ok ? make_uint4(AGARCL_SNAPSHOT_MAGIC, AGARCL_SNAPSHOT_VERSION, (uint32_t)P.fingerprint, (uint32_t)(P.fingerprint >> 32)) : z;
-      hv[1] = ok ? make_uint4((uint32_t)P.S.slot_bytes, (uint32_t)(P.S.slot_bytes >> 32), (uint32_t)(P.instance_base + src), 0u) : z;
-      hv[2] = z;
+      hv[1] = ok ? make_uint4((uint32_t)P.S.slot_bytes, (uint32_t)(P.S.slot_bytes >> 32), (uint32_t)(P.instance_base + src),
+                              task ? (uint32_t)P.task_mode[src] : 0u) : z;
+      hv[2] = make_uint4(task ? (uint32_t)P.task_max_steps[src] : 0u, 0u, 0u, 0u);
       hv[3] = z;
     }
     return;
@@ -67,6 +69,7 @@ __global__ void __launch_bounds__(kSnapThreads) k_snapshot(const __grid_constant
     const agarcl_snapshot_hdr* h = reinterpret_cast<const agarcl_snapshot_hdr*>(sl);
     valid = h->magic == AGARCL_SNAPSHOT_MAGIC && h->version == AGARCL_SNAPSHOT_VERSION && h->fingerprint == P.fingerprint &&
             h->slot_bytes == P.S.slot_bytes;
+    if (valid && P.task_mode) valid = h->task_mode >= 0 && h->task_mode <= 10 && ((P.task_modes >> h->task_mode) & 1);
   }
   if (!valid) {  // rejected: the instance is not touched
     if (t == 0) { P.result[i] = 2; P.restored[i] = 0; }
@@ -90,6 +93,11 @@ __global__ void __launch_bounds__(kSnapThreads) k_snapshot(const __grid_constant
     // the next reset of the instance continues the restored draw stream (ResetParams::fresh == 0 -> from hdr.rng_cursor)
     const agarcl_inst_hdr* ih = reinterpret_cast<const agarcl_inst_hdr*>(sl + P.S.off_blob + P.off_hdr);
     P.seeds[i] = (uint64_t)ih->seed_lo | ((uint64_t)ih->seed_hi << 32);
+    if (P.task_mode) {  // the slot's task becomes the current one; the pending task is left alone
+      const agarcl_snapshot_hdr* h = reinterpret_cast<const agarcl_snapshot_hdr*>(sl);
+      P.task_mode[i] = h->task_mode;
+      P.task_max_steps[i] = h->task_max_steps;
+    }
     P.fresh[i] = 0;
     P.result[i] = 1;
     P.restored[i] = 1;

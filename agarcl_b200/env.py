@@ -16,19 +16,19 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._abi import OBS_I16, OBS_I32, RNG_MT19937, RNG_PHILOX, make_cfg
+from ._abi import OBS_I16, OBS_I32, RNG_MT19937, RNG_PHILOX, make_cfg, task_bits
 from .batch import Batch
 
 
 class _Base:
     def __init__(self, n_instances, num_agents, ticks_per_step, arena_size, pellet_regen, num_pellets, num_viruses,
                  num_bots, reward_type, c_death, mode_number, rng_mode, strict_reference, device, obs_dtype, instance_base=0,
-                 ram_obs=False):
+                 ram_obs=False, task_modes=0):
         self._ctor = dict(n_instances=n_instances, num_agents=num_agents, ticks_per_step=ticks_per_step,
                           arena_size=arena_size, pellet_regen=pellet_regen, num_pellets=num_pellets, num_viruses=num_viruses,
                           num_bots=num_bots, reward_type=reward_type, c_death=c_death, mode_number=mode_number,
                           rng_mode=rng_mode, strict_reference=strict_reference, device=device, obs_dtype=obs_dtype,
-                          instance_base=instance_base, ram_obs=ram_obs)
+                          instance_base=instance_base, ram_obs=ram_obs, task_modes=task_modes)
         self._obs_cfg = dict(num_frames=1, grid_size=128, observe_cells=True, observe_others=True, observe_viruses=True,
                              observe_pellets=True)
         self._seeds = None
@@ -316,14 +316,15 @@ class GoBiggerEnvironment(GridEnvironment):
 class BatchedGridEnvironment(_Base):
     """N lockstep GridEnvironments on one GPU.  step() takes arrays/tensors and returns device tensors:
     obs [N*A, C*frames, G, G], rewards f64 [N*A], dones u8 [N*A].  With ram_obs=True the structured
-    observation records [N, P, RAM_RECORD] are produced too (ram())."""
+    observation records [N, P, RAM_RECORD] are produced too (ram()).  tasks=(1, 2, ...) makes a mixed-task batch: every
+    instance plays its own mode of that set, mode_number first, and changes it at its next reset (set_tasks)."""
 
     def __init__(self, n_instances, num_agents=1, ticks_per_step=4, arena_size=1000, pellet_regen=True, num_pellets=1000,
                  num_viruses=25, num_bots=25, reward_type=1, c_death=0, mode_number=0, *, rng_mode=RNG_PHILOX,
-                 strict_reference=False, device=0, obs_dtype=OBS_I32, instance_base=0, ram_obs=False):
+                 strict_reference=False, device=0, obs_dtype=OBS_I32, instance_base=0, ram_obs=False, tasks=None):
         super().__init__(n_instances, num_agents, ticks_per_step, arena_size, pellet_regen, num_pellets, num_viruses,
                          num_bots, reward_type, c_death, mode_number, rng_mode, strict_reference, device, obs_dtype,
-                         instance_base, ram_obs)
+                         instance_base, ram_obs, task_bits(tasks) if tasks else 0)
         self.n_instances = n_instances
         self.num_agents = num_agents
 
@@ -396,6 +397,14 @@ class BatchedGridEnvironment(_Base):
     def restore_states(self, pool, slot_of, stream=0):
         """instance i <- pool slot slot_of[i] where >= 0; returns the result u8 [N] (Batch.restore_states)"""
         return self._ensure().restore_states(pool, slot_of, stream)
+
+    def set_tasks(self, mode, max_steps=None, stream=0):
+        """the task each instance's next reset plays; returns the result u8 [N] (Batch.set_tasks)"""
+        return self._ensure().set_tasks(mode, max_steps, stream)
+
+    def tasks(self):
+        """device views of the current and pending task of every instance (Batch.tasks)"""
+        return self._ensure().tasks()
 
     def ram(self):
         return self._ensure().ram_tensor()

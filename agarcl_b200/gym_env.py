@@ -197,13 +197,20 @@ class BatchedAgarioEnv:
                       with final_obs=True, which allocates as much device memory again as the observation
     obs, dones and every info tensor are views of library-owned buffers that the next step() overwrites: copy what must
     outlive it.  With auto_reset=False nothing is reset: the step limit is folded into dones, steps keeps counting, and
-    info has "steps" only."""
+    info has "steps" only.
 
-    def __init__(self, n_envs, obs_type="grid", auto_reset=True, final_obs=False, **kwargs):
+    tasks=[1, 2, ...]: a mixed-task batch, every environment plays its own mini-game (mode) of that set -- `mode` (default:
+    the first of the list) to begin with -- and set_tasks() chooses what each one plays from its next reset on, with its own
+    step limit.  info["task"] (i32 [N]) is then every environment's current mode: after an auto-reset, the new episode's."""
+
+    def __init__(self, n_envs, obs_type="grid", auto_reset=True, final_obs=False, tasks=None, **kwargs):
         if obs_type not in ("grid", "ram"):
             raise ValueError(obs_type)
+        if tasks and "mode" not in kwargs:
+            kwargs = dict(kwargs, mode=int(list(tasks)[0]))
         a = _env_args(kwargs)
         self.n_envs, self.num_agents, self.obs_type, self.auto_reset = n_envs, a["num_agents"], obs_type, auto_reset
+        self.tasks = tuple(int(m) for m in tasks) if tasks else None
         self.final_obs = bool(final_obs)
         if self.final_obs and not auto_reset:
             raise ValueError("final_obs needs auto_reset: without a reset no observation is overwritten")
@@ -214,10 +221,11 @@ class BatchedAgarioEnv:
         extra = {k: kwargs[k] for k in ("device", "rng_mode", "obs_dtype", "instance_base") if k in kwargs}
         self._env = BatchedGridEnvironment(n_envs, a["num_agents"], a["ticks_per_step"], a["arena_size"], a["pellet_regen"],
                                            a["num_pellets"], a["num_viruses"], a["num_bots"], a["reward_type"], a["c_death"],
-                                           a["mode"], ram_obs=(2 if obs_type == "ram" else 0), **extra)
+                                           a["mode"], ram_obs=(2 if obs_type == "ram" else 0), tasks=self.tasks, **extra)
         self._env.configure_observation({k: kwargs[k] for k in _OBS_KEYS if k in kwargs})
         self._ep_batch = None
         self._ep = None
+        self._task = None
 
     def seed(self, seed):
         self._env.seed(seed)
@@ -235,6 +243,7 @@ class BatchedAgarioEnv:
             self._ep_batch = b
             self._ep = b.episode()
             self._final = (b.final_obs() if self.obs_type == "grid" else b.final_ram()[:, :self.num_agents, :]) if self.final_obs else None
+            self._task = b.tasks()["mode"] if self.tasks else None
         self._env.reset()  # (restarts every instance's step counter and return)
         return self._obs(), {}
 
@@ -250,7 +259,17 @@ class BatchedAgarioEnv:
                         episode_length=ep["episode_length"])
             if self.final_obs:
                 info["final_obs"] = self._final
+        if self._task is not None:
+            info["task"] = self._task
         return self._obs(), rew.float(), done, torch.zeros_like(done), info
+
+    def set_tasks(self, modes, number_steps=None):
+        """what every environment plays from its next reset on: modes (int32 CUDA tensor of n_envs entries, -1 keeps the pending
+        mode) and number_steps (int32 CUDA tensor or None: pending limits kept; -1 the constructor's number_steps, 0 none).
+        Returns the per-environment result u8 [n_envs]: 0 nothing set, 1 set, 2 rejected (mode not in tasks, or limit < -1)"""
+        if not self.tasks:
+            raise ValueError("set_tasks needs a mixed-task environment (tasks=[...])")
+        return self._env.set_tasks(modes, number_steps)
 
     # ---- snapshot pools (Batch.save_states / restore_states): save and restore whole games, episode counters included
     def snapshot_pool(self, slots):

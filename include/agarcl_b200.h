@@ -97,7 +97,9 @@ typedef struct agarcl_cfg {
   int32_t instance_base;    /* global index of local instance 0 (multi-GPU sharding; keys the RNG) */
   int32_t ram_obs;          /* 1: every step also produces the structured observation (agarcl_batch_ram); 2: ONLY that one
                                (agario-ram-v0: the grid frame is not rendered, agarcl_batch_obs stays zero) */
-  int32_t reserved[2];
+  int32_t task_modes;       /* 0: every instance plays mode_number.  Otherwise a MIXED-TASK batch: bit m set = mode m may run in it
+                               (see "mixed-task batches" below); mode_number's bit must be set, it is every instance's first task */
+  int32_t reserved[1];
 } agarcl_cfg;
 
 /* ------------------------------------------------------------- state records */
@@ -232,6 +234,44 @@ int agarcl_batch_set_autoreset(agarcl_batch* b, int32_t max_steps, int32_t keep_
 int agarcl_batch_step_autoreset(agarcl_batch* b, void* stream);
 int agarcl_batch_episode(agarcl_batch* b, agarcl_episode* out);
 
+/* ---------------------------------------------------- mixed-task batches: a game mode and an episode limit per instance
+ * The mini-games of AgarCL differ in mode_number only (bench/tasks_configs: modes 1..10 at the same arena, pellets, viruses).
+ * With cfg.task_modes != 0 every instance plays its own mode of that set and its own step limit, and changes them at its next
+ * reset without the host waiting -- one batch for a multi-task policy or a curriculum instead of one batch per mode.
+ * Layout: P = A + the most bots of any mode of the set (bots(0) = num_bots, bots(1..6) = 0, bots(7..10) = 1); cap_pellets the most
+ * of any mode (the squared-pellet modes 1, 2 and 5 need 4 * (arena_size / 2)).  layout.mass_decay .. agent_mass and bot_type stay
+ * those of mode_number: the kernels of a mixed batch derive the rules of each instance from its current mode.
+ * ABSENT players: an instance of mode m plays P_m = A + bots(m) players; players P_m .. P-1 are never spawned, drawn for, ticked,
+ * observed or counted -- from the reset on they are dead records (n_cells 0).  A reset draws 2 P_m spawn points and starts cell ids
+ * at 1 + P_m, so an instance of mode m is bit-identical to the same instance (seed, global index, actions) of a batch of mode m alone.
+ * Refused (AGARCL_ERR_INVALID) by agarcl_make_layout / agarcl_batch_create: strict_reference; a mode outside 0..10; mode_number not
+ * in the set; mode 0 with a mode of another bot count (mode 0 respawns every dead player, absent ones included); a set where the
+ * batch's player order, restricted to players < P_m, is not the order of a batch of mode m alone (cannot happen for one agent).
+ * Task state, library-owned device arrays of N int32 (agarcl_batch_tasks):
+ *   mode, max_steps             the current episode's task
+ *   next_mode, next_max_steps   what the instance's next reset plays
+ * Initially mode_number and -1.  A step limit of -1 means agarcl_batch_set_autoreset's max_steps, 0 no limit, > 0 that many
+ * steps.  EVERY reset (agarcl_batch_reset, _reset_device, the reset inside _step_autoreset) copies next -> current for the
+ * instances it resets before it spawns them: a running episode never changes its rules.
+ *   agarcl_batch_set_tasks  d_mode[N] (device; -1 keeps the pending mode) and d_max_steps[N] (device, may be NULL: every pending
+ *                           limit is kept) become the pending task.  Checked on the device; *d_result (may be NULL) receives the
+ *                           library-owned u8 [N] result, overwritten by the next call: 0 nothing set, 1 set, 2 rejected (the mode
+ *                           is not in task_modes or the limit is < -1: that instance's pending task is not touched).  Stream-
+ *                           ordered, no host wait.  AGARCL_ERR_STATE on a batch without task_modes.
+ *   agarcl_batch_tasks      the four device pointers; AGARCL_ERR_STATE on a batch without task_modes.
+ * Snapshot pools store the source's current mode and max_steps (agarcl_snapshot_hdr.task_mode / task_max_steps); a restore makes
+ * them the destination's current task (its pending task is untouched) and rejects a slot whose mode is not in the destination's
+ * set.  agarcl_batch_save_env_state writes the instance's current mode as "mode_number"; agarcl_batch_load_env_state accepts any
+ * mode of the set and makes it the instance's current task.                                                                    */
+typedef struct agarcl_tasks {
+  int32_t* mode;            /* [N] */
+  int32_t* max_steps;       /* [N] */
+  int32_t* next_mode;       /* [N] */
+  int32_t* next_max_steps;  /* [N] */
+} agarcl_tasks;
+int agarcl_batch_set_tasks(agarcl_batch* b, const int32_t* d_mode, const int32_t* d_max_steps, uint8_t** d_result, void* stream);
+int agarcl_batch_tasks(agarcl_batch* b, agarcl_tasks* out);
+
 /* ---------------------------------------------------- snapshot pools: save and restore game states on the device
  * The batched counterpart of agarcl_batch_save_env_state / load_env_state: chosen instances are copied into slots of a
  * caller-owned POOL in device memory and slots back into chosen instances, stream-ordered, driven by index arrays in device
@@ -272,7 +312,9 @@ int agarcl_batch_episode(agarcl_batch* b, agarcl_episode* out);
  * batch and changes with every unmasked reset), AGARCL_RNG_MT19937 (its generators live on the host), a call before the first
  * reset, a NULL / misaligned pool or one that is not device memory of cfg.device, pool_slots < 1, n < 0, a NULL index array.
  * The fingerprint is FNV-1a 64 over agarcl_layout without cap_replay and the agarcl_cfg fields num_agents .. ram_obs except
- * cap_viruses, cap_foods, cap_replay, device and instance_base (those two caps are part of the layout). */
+ * cap_viruses, cap_foods, cap_replay, device and instance_base (those two caps are part of the layout), then task_modes when it
+ * is not 0.  A mixed-task batch: the header also carries the source's task, and a slot whose task_mode is not in the
+ * destination's task_modes is rejected. */
 #define AGARCL_SNAPSHOT_MAGIC 0x4E534741u /* "AGSN" */
 #define AGARCL_SNAPSHOT_VERSION 1u
 typedef struct agarcl_snapshot_hdr { /* 64 B */
@@ -281,7 +323,9 @@ typedef struct agarcl_snapshot_hdr { /* 64 B */
   uint64_t fingerprint;    /* of the configuration the slot was saved from */
   uint64_t slot_bytes;
   int32_t source;          /* global index (instance_base + i) of the instance saved */
-  uint32_t pad[9];
+  int32_t task_mode;       /* mixed-task batch (cfg.task_modes != 0): the source's current mode; 0 otherwise */
+  int32_t task_max_steps;  /* mixed-task batch: the source's current step limit (-1 default, 0 none); 0 otherwise */
+  uint32_t pad[7];
 } agarcl_snapshot_hdr;
 /* bytes of one snapshot slot of configuration c: a multiple of 128; no device needed */
 int agarcl_snapshot_slot_bytes(const agarcl_cfg* c, int64_t* out);

@@ -4,7 +4,11 @@ viruses, mode k, 0 bots (modes 1-6) or one bot of type k-7 (modes 7-10), episode
 batched vector environment (agarcl_b200.gym_env.BatchedAgarioEnv: N lockstep instances, auto-reset) with the random-walk policy of
 bench/go_bigger_example.py:100-103, and prints one JSON line per mode: env-steps/s, episodes finished, mean return, state flags.
 
-    python tools/run_tasks_configs.py [--envs 4096] [--steps 600] [--modes 1 2 ...] [--dir /root/reference/bench/tasks_configs]
+    python tools/run_tasks_configs.py [--envs 4096] [--steps 600] [--modes 1 2 ...] [--dir DIR] [--mixed]
+
+--mixed runs the selected mini-games in ONE mixed-task batch of --envs instances instead of one batch per mode: instance i plays
+mode modes[i % len(modes)] with that mode's episode length, every auto-reset keeps it on its mode, and the finished episodes and
+returns are summed per task on the device (index_add_ on info["task"]).  It prints one JSON line per mode and one for the batch.
 
 With --dir the mode_k.json files themselves are loaded (keys the batched grid environment does not have -- screen_len, video_path,
 agent_view, render_mode, load_env_snapshot -- are ignored; obs_type "screen" is OpenGL and out of scope: the grid observation with
@@ -39,11 +43,14 @@ def main():
     ap.add_argument("--steps", type=int, default=600)
     ap.add_argument("--modes", type=int, nargs="*", default=list(range(1, 11)))
     ap.add_argument("--dir", default=None)
+    ap.add_argument("--mixed", action="store_true")
     args = ap.parse_args()
     import torch
     from agarcl_b200.gym_env import BatchedAgarioEnv
     tasks = load_dir(args.dir) if args.dir else TASKS
     N = args.envs
+    if args.mixed:
+        return run_mixed(args, tasks)
     for k in args.modes:
         kw = dict(tasks[k], observe_cells=True, observe_others=True, observe_viruses=True, observe_pellets=True)
         env = BatchedAgarioEnv(N, obs_type="grid", **kw)
@@ -71,6 +78,51 @@ def main():
                           "episode_steps": kw["number_steps"], "episodes_finished": finished,
                           "mean_return": (ret_sum / finished) if finished else None, "state_flags": names}))
         env.close()
+
+
+def run_mixed(args, tasks):
+    import torch
+    from agarcl_b200.gym_env import BatchedAgarioEnv
+    N, modes = args.envs, list(args.modes)
+    first = tasks[modes[0]]
+    for k in modes:  # one batch holds the mini-games that differ in their mode only
+        diff = {key for key in KEEP - {"mode", "number_steps", "num_bots"} if tasks[k][key] != first[key]}
+        if diff:
+            sys.exit(f"mode_{k} differs from mode_{modes[0]} in {sorted(diff)}: it cannot share a mixed-task batch")
+    kw = dict(first, observe_cells=True, observe_others=True, observe_viruses=True, observe_pellets=True, num_bots=0)
+    kw.pop("mode")
+    env = BatchedAgarioEnv(N, obs_type="grid", tasks=modes, mode=modes[0], **kw)
+    env.seed(1000)
+    mode_of = torch.tensor([modes[i % len(modes)] for i in range(N)], dtype=torch.int32, device="cuda")
+    limit_of = torch.tensor([tasks[int(m)]["number_steps"] for m in mode_of.tolist()], dtype=torch.int32, device="cuda")
+    res = env.set_tasks(mode_of, limit_of)  # (taken by the reset below)
+    env.reset()
+    assert bool((res == 1).all()), "a task was rejected"
+    gen = torch.Generator(device="cuda")
+    gen.manual_seed(1)
+    finished = torch.zeros(11, dtype=torch.int64, device="cuda")
+    ret_sum = torch.zeros(11, dtype=torch.float64, device="cuda")
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for t in range(args.steps):
+        dxdy = (torch.rand((N, 2), device="cuda", generator=gen) * 2 - 1).float()
+        act = torch.randint(0, 3, (N,), device="cuda", generator=gen, dtype=torch.int32)
+        _, _, _, _, info = env.step(dxdy, act)
+        m = info["reset_mask"]
+        task = info["task"].long()  # (after an auto-reset: the new episode's, which is the finished one's here)
+        finished.index_add_(0, task, m.long())
+        ret_sum.index_add_(0, task, torch.where(m, info["episode_return"], 0.0))
+    torch.cuda.synchronize()
+    sec = time.perf_counter() - t0
+    finished, ret_sum = finished.tolist(), ret_sum.tolist()
+    f, names = env.flags()
+    for k in modes:
+        print(json.dumps({"task": f"mode_{k}", "mixed": True, "envs": sum(1 for i in range(N) if modes[i % len(modes)] == k),
+                          "steps": args.steps, "episode_steps": tasks[k]["number_steps"], "episodes_finished": finished[k],
+                          "mean_return": (ret_sum[k] / finished[k]) if finished[k] else None}))
+    print(json.dumps({"task": "mixed", "modes": modes, "envs": N, "steps": args.steps, "env_steps_per_s": N * args.steps / sec,
+                      "ms_per_step": 1e3 * sec / args.steps, "state_flags": names}))
+    env.close()
 
 
 if __name__ == "__main__":
