@@ -27,6 +27,7 @@ RAM_OFF_SPORE = RAM_OFF_VIRUS + 4 * RAM_KV
 RAM_OFF_CLONE = RAM_OFF_SPORE + 4 * RAM_KS
 RAM_RECORD = RAM_OFF_CLONE + 8 * RAM_KC
 OBS_I32, OBS_I16 = 0, 1
+DRAW_VIEWS = {"arena": 0, "agent": 1}  # AGARCL_DRAW_ARENA, AGARCL_DRAW_AGENT
 
 
 class Cfg(C.Structure):

@@ -389,6 +389,34 @@ class Batch:
                                                           C.byref(r), _vp(stream)))
         return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
 
+    # ---- pictures of game states (include/agarcl_b200.h, agarcl_batch_draw)
+    def draw(self, src=None, size=256, view="arena", out=None, stream=0):
+        """RGB pictures uint8 [n, size, size, 3] of the current states, drawn on the device (enqueued on `stream`, no host
+        wait).  view "arena": the whole arena of instance src[k]; "agent": the observation window of image src[k] = instance * A
+        + agent.  src: int32 CUDA tensor, or None for every instance (N pictures) or every agent (N * A).  A source out of range
+        gives an all-zero picture.  out: a preallocated contiguous uint8 CUDA tensor [n, size, size, 3] to draw into."""
+        import torch
+        from ._abi import DRAW_VIEWS
+        if view not in DRAW_VIEWS:
+            raise _lib.AgarclError(f"unknown view {view!r}: 'arena' or 'agent'")
+        if src is None:
+            n = self.N * (self.A if view == "agent" else 1)
+        else:
+            self._check_device_tensor(src, torch.int32, "src")
+            n = src.numel()
+        size = int(size)
+        if out is None:
+            out = torch.empty((n, size, size, 3), dtype=torch.uint8, device=f"cuda:{self.cfg.device}")
+        else:
+            self._check_device_tensor(out, torch.uint8, "out")
+            if tuple(out.shape) != (n, size, size, 3):
+                raise _lib.AgarclError(f"out must be [{n}, {size}, {size}, 3], got {list(out.shape)}")
+        if n == 0:  # (an empty tensor has no device address to check)
+            return out
+        _lib.check(_lib.lib().agarcl_batch_draw(self._h, DRAW_VIEWS[view], size, _vp(src.data_ptr()) if src is not None else None,
+                                                n, _vp(out.data_ptr()), _vp(stream)))
+        return out
+
     # ---- mixed-task batches (include/agarcl_b200.h, cfg.task_modes)
     def set_tasks(self, mode, max_steps=None, stream=0):
         """the task each instance's NEXT reset plays: mode (int32 CUDA tensor of N entries, -1 keeps the pending mode) and

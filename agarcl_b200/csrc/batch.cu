@@ -1157,6 +1157,43 @@ extern "C" int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, in
   return AGARCL_OK;
 }
 
+// ---- pictures of game states (include/agarcl_b200.h): refusals are decided here, before anything is enqueued
+extern "C" int agarcl_batch_draw(agarcl_batch* b, int32_t view, int32_t size, const int32_t* d_src, int32_t n, uint8_t* d_out,
+                                 void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (!b->was_reset) return agarcl_set_error(AGARCL_ERR_STATE, "draw before reset()");
+  if (view != AGARCL_DRAW_ARENA && view != AGARCL_DRAW_AGENT)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "unknown view %d (AGARCL_DRAW_ARENA 0, AGARCL_DRAW_AGENT 1)", view);
+  if (size < 16 || size > 2048 || size % 16)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "picture size %d must be a multiple of 16 in [16, 2048]", size);
+  if (n < 0) return agarcl_set_error(AGARCL_ERR_INVALID, "n must be >= 0");
+  if (!d_out) return agarcl_set_error(AGARCL_ERR_INVALID, "null output");
+  if ((uintptr_t)d_out & 15u) return agarcl_set_error(AGARCL_ERR_INVALID, "the output must be 16-byte aligned");
+  CK(cudaSetDevice(b->cfg.device));
+  cudaPointerAttributes a;
+  const cudaError_t e = cudaPointerGetAttributes(&a, d_out);  // (does not synchronise)
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return agarcl_set_error(AGARCL_ERR_INVALID, "the output is not device memory: %s", cudaGetErrorString(e));
+  }
+  if (a.type != cudaMemoryTypeDevice || a.device != b->cfg.device)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "the output must be device memory of device %d", b->cfg.device);
+  if (n == 0) return AGARCL_OK;
+  ag::DrawParams P;
+  P.L = b->L;
+  P.radius = b->T.radius;
+  P.state = b->d_state;
+  P.out = d_out;
+  P.src = d_src;
+  P.n = n;
+  P.S = size;
+  P.view = view;
+  P.N = b->N;
+  P.W = (float)b->cfg.arena_size;
+  CK(ag::launch_draw(P, (cudaStream_t)stream));
+  return AGARCL_OK;
+}
+
 // ---- mixed-task batches (include/agarcl_b200.h)
 extern "C" int agarcl_batch_set_tasks(agarcl_batch* b, const int32_t* d_mode, const int32_t* d_max_steps, uint8_t** d_result, void* stream) {
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");

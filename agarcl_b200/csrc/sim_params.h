@@ -254,4 +254,16 @@ struct SnapParams {
 cudaError_t launch_snapshot_save(const SnapParams& P, int n, cudaStream_t stream);
 cudaError_t launch_snapshot_restore(const SnapParams& P, cudaStream_t stream);
 
+// Pictures of game states (draw_kernel.cu, k_draw): the spec of include/agarcl_b200.h, agarcl_batch_draw
+struct DrawParams {
+  agarcl_layout L;
+  const float* radius;     // Luts::radius
+  const uint8_t* state;    // N blobs, L.stride apart
+  uint8_t* out;            // [n][S][S][3]
+  const int32_t* src;      // [n] or nullptr (picture k shows source k)
+  int32_t n, S, view, N;
+  float W;
+};
+cudaError_t launch_draw(const DrawParams& P, cudaStream_t stream);
+
 }  // namespace ag

@@ -81,9 +81,11 @@ _OBS_KEYS = ("num_frames", "grid_size", "observe_cells", "observe_others", "obse
 class AgarioEnv(_EnvBase):
     metadata = {"render_modes": ["human", "rgb_array"], "render_fps": 60}
 
-    def __init__(self, obs_type="grid", render_mode=None, **kwargs):
+    def __init__(self, obs_type="grid", render_mode=None, render_size=512, render_view="arena", **kwargs):
         if obs_type not in ("ram", "screen", "grid", "gobigger"):
             raise ValueError(obs_type)
+        if render_view not in ("arena", "agent"):
+            raise ValueError(f"render_view must be 'arena' or 'agent', got {render_view!r}")
         if obs_type == "screen":
             raise ValueError("agarcl_b200 does not include ScreenEnvironment (OpenGL, out of scope)")
         a = _env_args(kwargs)
@@ -91,6 +93,7 @@ class AgarioEnv(_EnvBase):
         self.multi_agent = bool(kwargs.get("multi_agent", False)) or self.num_agents > 1
         self.obs_type = obs_type
         self.render_mode = render_mode
+        self.render_size, self.render_view = int(render_size), render_view
         self.number_of_steps = kwargs.get("number_steps", 500)
         self.mode = a["mode"]
         self.env_type = kwargs.get("env_type", 0)  # 0 episodic, 1 continuing
@@ -145,7 +148,13 @@ class AgarioEnv(_EnvBase):
             return [self._seed]
 
     def render(self):
-        raise RuntimeError("OpenGL rendering is out of scope of agarcl_b200")
+        """render_mode "rgb_array": an RGB picture uint8 [render_size, render_size, 3] of the game drawn on the device
+        (include/agarcl_b200.h, agarcl_batch_draw) -- the whole arena, or with render_view "agent" the agent's observation
+        window ([num_agents, S, S, 3] for a multi-agent environment).  Other render modes need OpenGL, which is out of scope."""
+        if self.render_mode != "rgb_array":
+            raise RuntimeError("OpenGL rendering is out of scope of agarcl_b200 (render_mode='rgb_array' draws pictures)")
+        pics = self._env._ensure().draw(None, self.render_size, self.render_view).cpu().numpy()
+        return pics if self.render_view == "agent" and self.multi_agent else pics[0]
 
     def close(self):
         self._env.close()
@@ -295,6 +304,19 @@ class BatchedAgarioEnv:
     def flags(self):
         """(OR over all instances, {AGARCL_FLAG name: instances}) -- fixed capacities hit since the instances' last reset"""
         return self._env.flags()
+
+    def render(self, env_ids=None, size=256, view="arena", out=None):
+        """RGB pictures uint8 [n, size, size, 3] (device tensor) of the current games, drawn on the device on the current torch
+        stream without a host wait (Batch.draw).  env_ids: int32 CUDA tensor of environments, or None for all.  view "arena": one
+        picture per environment; "agent": one per agent, environment-major (n * num_agents pictures), each the window of that
+        agent's grid observation.  out: a preallocated uint8 CUDA tensor of that shape, e.g. a slice of a video buffer."""
+        import torch
+        b = self._env.batch
+        src = env_ids.to(torch.int32) if env_ids is not None else None
+        if view == "agent" and src is not None:
+            A = self.num_agents
+            src = (src.view(-1, 1) * A + torch.arange(A, dtype=torch.int32, device=src.device)).view(-1)
+        return b.draw(src, size, view, out)  # (the stream the steps run on)
 
     def close(self):
         self._env.close()

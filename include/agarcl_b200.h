@@ -16,7 +16,8 @@
  * The same header also fixes the per-instance STATE BLOB layout that is shared by
  *   - the CUDA library (device state = N blobs, `stride` bytes apart),
  *   - oracle/oracle.c (CPU restatement, test infrastructure only),
- *   - oracle/ref_harness.cpp (the compiled reference, dumps into the same blob).
+ *   - oracle/ref_harness.cpp (the compiled reference, dumps into the same blob),
+ *   - tests/draw_oracle.c (CPU restatement of the pictures of agarcl_batch_draw, test infrastructure only).
  */
 #ifndef AGARCL_B200_H
 #define AGARCL_B200_H
@@ -335,6 +336,48 @@ int agarcl_batch_save_states(agarcl_batch* b, void* pool, int64_t pool_slots, co
 /* instance i <- pool slot d_slot_of[i] where >= 0; *d_result = the library-owned u8 [N] result above; enqueued on stream */
 int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, int64_t pool_slots, const int32_t* d_slot_of,
                                 uint8_t** d_result, void* stream);
+
+/* ---------------------------------------------------- pictures of game states, for people (render() and videos)
+ * A picture is uint8 [S][S][3], RGB, row-major (HWC): row r is world y, column c world x, row 0 the smallest y.  S is a multiple of
+ * 16 in [16, 2048].  It is drawn from the state blob as it is at the call: players respawned at the end of the last step are drawn
+ * at their new cells.  It is not a training observation and claims no likeness to the reference's OpenGL frames; this spec is
+ * what it means, and tests/draw_oracle.c (oracle_draw) restates it.
+ * Views (every operation one rounded fp32 operation, no FMA, C order of evaluation):
+ *   AGARCL_DRAW_ARENA  the arena [0, W)^2, W = (float)arena_size: pixel centre x = ((float)c + 0.5f) * W / (float)S, y the same
+ *                      with r; pixel width px = W / (float)S.
+ *   AGARCL_DRAW_AGENT  the window of the agent's grid observation: its centroid (cx, cy) as k_obs computes it (sum over its cells in
+ *                      cell order of x * (float)mass, over (float)(total mass)), view = clamp(2 * total mass, 100, 300);
+ *                      x = cx + ((float)c - (float)(S / 2.0)) * view / (float)S (GridObservation's _grid_to_world: corners), y the
+ *                      same with r; px = view / (float)S.  With S = G the out-of-arena pixels are exactly the -1 elements of
+ *                      observation channel 0, transposed.  A dead agent (no cells: NaN centroid) is all out-of-arena colour.
+ * Colour of a pixel at (x, y):
+ *   !(0 <= x < W && 0 <= y < W)  AGARCL_DRAW_RGB_OUT
+ *   otherwise                    the colour of the TOPMOST entity whose disc contains it, else AGARCL_DRAW_RGB_BACKGROUND.
+ *   disc test: dx = x - ex, dy = y - ey, dx * dx + dy * dy <= R * R; drawn radius R = max(radius(mass), px), radius(m) =
+ *   (float)sqrt((double)m / M_PI) (radius_conversion); pellets have mass AGARCL_PELLET_MASS, foods AGARCL_FOOD_MASS.  Cells and
+ *   viruses show their border colour where d2 > (0.85f * R) * (0.85f * R).
+ * Draw order, bottom to top: pellets in array order, foods in array order, then cells and viruses together by the key (mass, kind
+ * [virus 0, cell 1], cell id or virus index) ascending.  Counts are taken from the header and player records, limited to the
+ * layout's capacities (cap_pellets, cap_foods, cap_viruses, cap_cells); dead and absent players have no cells and draw nothing.
+ * Cell colours: player p < A (an agent) AGARCL_DRAW_RGB_AGENTS[p % 8]; a bot AGARCL_DRAW_RGB_BOTS[bot_type & 3] (the player
+ * record's bot_type); border = each channel * 3 / 4 (integer).  A picture whose source is out of range is all zeros.
+ *   agarcl_batch_draw  n pictures [n][size][size][3] into d_out (caller-owned, 16-byte aligned device memory of cfg.device),
+ *                      enqueued on stream, no host wait, the state only read.  d_src[k] (device int32): arena view an instance in
+ *                      [0, N); agent view an image instance * A + agent in [0, N * A), the observation's numbering.  d_src NULL:
+ *                      picture k shows source k (n = N, or N * A, draws them all).  Refused before anything is enqueued, nothing
+ *                      written: a call before the first reset (AGARCL_ERR_STATE), an unknown view, a size that is not a multiple
+ *                      of 16 in [16, 2048], n < 0, a NULL or misaligned d_out or one that is not device memory of cfg.device. */
+#define AGARCL_DRAW_ARENA 0
+#define AGARCL_DRAW_AGENT 1
+#define AGARCL_DRAW_RGB_OUT 0x2B2B33u
+#define AGARCL_DRAW_RGB_BACKGROUND 0xF4F6F8u
+#define AGARCL_DRAW_RGB_PELLET 0x8CCB5Eu
+#define AGARCL_DRAW_RGB_FOOD 0xE8A33Du
+#define AGARCL_DRAW_RGB_VIRUS 0x3DBB4Fu
+#define AGARCL_DRAW_RGB_VIRUS_BORDER 0x1E7A2Cu
+#define AGARCL_DRAW_RGB_AGENTS {0x2F6FDEu, 0xD9413Bu, 0x8E44ADu, 0x16A3A3u, 0xE67E22u, 0xC0398Eu, 0x5D6D7Eu, 0x9C7A1Eu}
+#define AGARCL_DRAW_RGB_BOTS {0x7F8C8Du, 0xA3B1C2u, 0x8B5A3Cu, 0xB86F8Fu}
+int agarcl_batch_draw(agarcl_batch* b, int32_t view, int32_t size, const int32_t* d_src, int32_t n, uint8_t* d_out, void* stream);
 
 /* ---------------------------------------------------- host-resident observation mirror
  * get_state (bindings.cpp:67-91) hands every agent's frame to HOST memory; for a batch that is 512 KB per agent
