@@ -28,6 +28,10 @@ RAM_OFF_CLONE = RAM_OFF_SPORE + 4 * RAM_KS
 RAM_RECORD = RAM_OFF_CLONE + 8 * RAM_KC
 OBS_I32, OBS_I16 = 0, 1
 DRAW_VIEWS = {"arena": 0, "agent": 1}  # AGARCL_DRAW_ARENA, AGARCL_DRAW_AGENT
+# built-in bot policies (agarcl_batch_bot_actions): AGARCL_BOT_* bot types and per-agent results
+BOT_HUNGRY, BOT_HUNGRY_SHY, BOT_AGGRESSIVE, BOT_AGGRESSIVE_SHY = 0, 1, 2, 3
+BOT_TYPES = {"hungry": BOT_HUNGRY, "hungry_shy": BOT_HUNGRY_SHY, "aggressive": BOT_AGGRESSIVE, "aggressive_shy": BOT_AGGRESSIVE_SHY}
+BOT_SKIPPED, BOT_DECIDED, BOT_NO_PELLET, BOT_DEAD, BOT_BAD_TYPE = 0, 1, 2, 3, 4
 
 
 class Cfg(C.Structure):

@@ -17,7 +17,7 @@ SYMBOLS = [
     "agarcl_batch_obs", "agarcl_batch_rewards", "agarcl_batch_dones", "agarcl_batch_step_host",
     "agarcl_batch_reset_device", "agarcl_batch_set_autoreset", "agarcl_batch_step_autoreset", "agarcl_batch_episode",
     "agarcl_snapshot_slot_bytes", "agarcl_batch_save_states", "agarcl_batch_restore_states",
-    "agarcl_batch_set_tasks", "agarcl_batch_tasks", "agarcl_batch_draw",
+    "agarcl_batch_set_tasks", "agarcl_batch_tasks", "agarcl_batch_draw", "agarcl_batch_bot_actions",
     "agarcl_batch_mirror", "agarcl_batch_sync_mirror", "agarcl_batch_step_mirror", "agarcl_batch_mirror_stats", "agarcl_batch_mirror_timing", "agarcl_batch_step_lists", "agarcl_batch_lists_expand",
     "agarcl_batch_download_state", "agarcl_batch_upload_state", "agarcl_batch_save_env_state", "agarcl_batch_load_env_state",
     "agarcl_snapshot_write", "agarcl_snapshot_read", "agarcl_batch_set_replay",
@@ -61,6 +61,7 @@ def lib():
         L.agarcl_batch_set_tasks.argtypes = [_vp, _vp, _vp, C.POINTER(_vp), _vp]
         L.agarcl_batch_tasks.argtypes = [_vp, _vp]
         L.agarcl_batch_draw.argtypes = [_vp, C.c_int32, C.c_int32, _vp, C.c_int32, _vp, _vp]
+        L.agarcl_batch_bot_actions.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp]
         L.agarcl_batch_mirror.argtypes = [_vp, C.POINTER(_vp), C.POINTER(C.c_int64 * 4), C.POINTER(C.c_int32)]
         L.agarcl_batch_sync_mirror.argtypes = [_vp, _vp]
         L.agarcl_batch_step_mirror.argtypes = [_vp, _vp, _vp, _vp, _vp]

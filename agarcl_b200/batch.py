@@ -417,6 +417,39 @@ class Batch:
                                                 n, _vp(out.data_ptr()), _vp(stream)))
         return out
 
+    # ---- built-in bot policies for agents (include/agarcl_b200.h, agarcl_batch_bot_actions)
+    def bot_actions(self, types, out=None, target=None):
+        """what a built-in bot would do for every agent on the current state, computed on the device on torch's current stream
+        (no host wait, the state is not touched).  Returns (dxdy f32 [N*A, 2], act i32 [N*A], status u8 [N*A]) device tensors
+        that go straight into set_actions_device / step.  types: a bot type (BOT_HUNGRY .. BOT_AGGRESSIVE_SHY) for every agent,
+        or an int32 CUDA tensor [N*A] with -1 for an agent to skip: its dxdy and act are not written.  dxdy = (target - location) / 10,
+        not clamped.  status: 0 skipped, 1 decided, 2 no pellet to go for (dxdy 0), 3 the agent is dead (dxdy 0), 4 not a bot
+        type.  out: preallocated (dxdy, act, status) tensors to write into (new ones start at zero).  target: an f32 CUDA tensor
+        [N*A, 2] that also receives the targets in world coordinates."""
+        import torch
+        NA, dev = self.N * self.A, torch.device("cuda", self.cfg.device)
+        if isinstance(types, torch.Tensor):
+            self._check_device_tensor(types, torch.int32, "types", NA)
+        else:
+            cache = self.__dict__.setdefault("_bot_types", {})
+            if int(types) not in cache:
+                cache[int(types)] = torch.full((NA,), int(types), dtype=torch.int32, device=dev)
+            types = cache[int(types)]
+        if out is None:
+            out = (torch.zeros((NA, 2), dtype=torch.float32, device=dev), torch.zeros(NA, dtype=torch.int32, device=dev),
+                   torch.zeros(NA, dtype=torch.uint8, device=dev))
+        dxdy, act, status = out
+        self._check_device_tensor(dxdy, torch.float32, "dxdy", 2 * NA)
+        self._check_device_tensor(act, torch.int32, "act", NA)
+        self._check_device_tensor(status, torch.uint8, "status", NA)
+        if target is not None:
+            self._check_device_tensor(target, torch.float32, "target", 2 * NA)
+        _lib.check(_lib.lib().agarcl_batch_bot_actions(
+            self._h, _vp(types.data_ptr()), _vp(dxdy.data_ptr()), _vp(act.data_ptr()),
+            _vp(target.data_ptr()) if target is not None else None, _vp(status.data_ptr()),
+            _vp(torch.cuda.current_stream(dev).cuda_stream)))
+        return dxdy, act, status
+
     # ---- mixed-task batches (include/agarcl_b200.h, cfg.task_modes)
     def set_tasks(self, mode, max_steps=None, stream=0):
         """the task each instance's NEXT reset plays: mode (int32 CUDA tensor of N entries, -1 keeps the pending mode) and

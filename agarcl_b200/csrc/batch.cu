@@ -1194,6 +1194,41 @@ extern "C" int agarcl_batch_draw(agarcl_batch* b, int32_t view, int32_t size, co
   return AGARCL_OK;
 }
 
+// ---- built-in bot policies for agents (include/agarcl_b200.h): refusals are decided here, before anything is enqueued
+extern "C" int agarcl_batch_bot_actions(agarcl_batch* b, const int32_t* d_type, float* d_dxdy, int32_t* d_act, float* d_target,
+                                        uint8_t* d_status, void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (!b->was_reset) return agarcl_set_error(AGARCL_ERR_STATE, "bot actions before reset()");
+  if (!d_type || !d_dxdy || !d_act) return agarcl_set_error(AGARCL_ERR_INVALID, "null type, dxdy or act array");
+  if (((uintptr_t)d_dxdy | (uintptr_t)d_target) & 7u)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "dxdy and target must be 8-byte aligned");
+  CK(cudaSetDevice(b->cfg.device));
+  const std::pair<const void*, const char*> arrays[] = {{d_type, "type"}, {d_dxdy, "dxdy"}, {d_act, "act"}, {d_target, "target"},
+                                                        {d_status, "status"}};
+  for (const auto& p : arrays) {
+    if (!p.first) continue;
+    cudaPointerAttributes a;
+    const cudaError_t e = cudaPointerGetAttributes(&a, p.first);  // (does not synchronise)
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return agarcl_set_error(AGARCL_ERR_INVALID, "the %s array is not device memory: %s", p.second, cudaGetErrorString(e));
+    }
+    if (a.type != cudaMemoryTypeDevice || a.device != b->cfg.device)
+      return agarcl_set_error(AGARCL_ERR_INVALID, "the %s array must be device memory of device %d", p.second, b->cfg.device);
+  }
+  ag::BotParams P;
+  P.L = b->L;
+  P.state = b->d_state;
+  P.type = d_type;
+  P.dxdy = d_dxdy;
+  P.act = d_act;
+  P.target = d_target;
+  P.status = d_status;
+  P.N = b->N;
+  CK(ag::launch_bot_actions(P, (cudaStream_t)stream));
+  return AGARCL_OK;
+}
+
 // ---- mixed-task batches (include/agarcl_b200.h)
 extern "C" int agarcl_batch_set_tasks(agarcl_batch* b, const int32_t* d_mode, const int32_t* d_max_steps, uint8_t** d_result, void* stream) {
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");

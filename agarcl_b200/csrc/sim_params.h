@@ -266,4 +266,17 @@ struct DrawParams {
 };
 cudaError_t launch_draw(const DrawParams& P, cudaStream_t stream);
 
+// Built-in bot policies for agents (bot_kernel.cu, k_bot_actions): the spec of include/agarcl_b200.h, agarcl_batch_bot_actions
+struct BotParams {
+  agarcl_layout L;         // with the batch's current player order
+  const uint8_t* state;    // N blobs, L.stride apart
+  const int32_t* type;     // [N*A] bot type per agent, -1: not requested
+  float* dxdy;             // [N*A][2]
+  int32_t* act;            // [N*A]
+  float* target;           // [N*A][2] or nullptr
+  uint8_t* status;         // [N*A] or nullptr
+  int32_t N;
+};
+cudaError_t launch_bot_actions(const BotParams& P, cudaStream_t stream);
+
 }  // namespace ag

@@ -406,6 +406,11 @@ class BatchedGridEnvironment(_Base):
         """device views of the current and pending task of every instance (Batch.tasks)"""
         return self._ensure().tasks()
 
+    def bot_actions(self, types, out=None, target=None):
+        """(dxdy, act, status) of a built-in bot policy for every agent, on the device (Batch.bot_actions); dxdy and act go
+        straight into step()"""
+        return self._ensure().bot_actions(types, out, target)
+
     def ram(self):
         return self._ensure().ram_tensor()
 

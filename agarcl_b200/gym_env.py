@@ -305,6 +305,16 @@ class BatchedAgarioEnv:
         """(OR over all instances, {AGARCL_FLAG name: instances}) -- fixed capacities hit since the instances' last reset"""
         return self._env.flags()
 
+    def bot_actions(self, types, out=None):
+        """what a built-in bot (BOT_HUNGRY .. BOT_AGGRESSIVE_SHY, agarcl_b200.BOT_TYPES) would do for every agent on the current
+        games: (dxdy f32 [n_envs * num_agents, 2], act i32, status u8) device tensors on the current stream, without a host wait.
+        dxdy and act go straight into step(): a scripted baseline, expert actions for imitation, or scripted partners and
+        opponents.  types: one type for every agent, or an int32 CUDA tensor with -1 for the agents a learner drives (their
+        entries are left as they are, so `out` can be an action buffer the policy already filled).  dxdy is not clamped to the
+        action box: the step moves towards the target the bot chose.  status: 1 decided, 2 no pellet left (dxdy 0), 3 the agent
+        is dead (dxdy 0), 0 skipped, 4 not a bot type"""
+        return self._env.bot_actions(types, out)
+
     def render(self, env_ids=None, size=256, view="arena", out=None):
         """RGB pictures uint8 [n, size, size, 3] (device tensor) of the current games, drawn on the device on the current torch
         stream without a host wait (Batch.draw).  env_ids: int32 CUDA tensor of environments, or None for all.  view "arena": one

@@ -17,7 +17,8 @@
  *   - the CUDA library (device state = N blobs, `stride` bytes apart),
  *   - oracle/oracle.c (CPU restatement, test infrastructure only),
  *   - oracle/ref_harness.cpp (the compiled reference, dumps into the same blob),
- *   - tests/draw_oracle.c (CPU restatement of the pictures of agarcl_batch_draw, test infrastructure only).
+ *   - tests/draw_oracle.c (CPU restatement of the pictures of agarcl_batch_draw, test infrastructure only),
+ *   - tests/bot_oracle.c (oracle_bot_decide: oracle.c's bot code as the spec of agarcl_batch_bot_actions, test infrastructure only).
  */
 #ifndef AGARCL_B200_H
 #define AGARCL_B200_H
@@ -378,6 +379,52 @@ int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, int64_t pool_
 #define AGARCL_DRAW_RGB_AGENTS {0x2F6FDEu, 0xD9413Bu, 0x8E44ADu, 0x16A3A3u, 0xE67E22u, 0xC0398Eu, 0x5D6D7Eu, 0x9C7A1Eu}
 #define AGARCL_DRAW_RGB_BOTS {0x7F8C8Du, 0xA3B1C2u, 0x8B5A3Cu, 0xB86F8Fu}
 int agarcl_batch_draw(agarcl_batch* b, int32_t view, int32_t size, const int32_t* d_src, int32_t n, uint8_t* d_out, void* stream);
+
+/* ---------------------------------------------------- built-in bot policies for agents: scripted actions on the device
+ * The four bots of the reference (agario/bots/HungryBot.hpp, HungryShyBot.hpp, AggressiveBot.hpp, AggressiveShyBot.hpp) as a
+ * policy for the agents: for baselines, expert actions for imitation, and scripted partners or opponents of a learner.
+ * For every agent j = i * A + a with d_type[j] in 0..3, what Bot::take_action of that bot type would leave in agent a's player
+ * record (target_x, target_y, action), on instance i's state as it is at the call: exactly oracle.c's bot_take_action run on
+ * player a with bot_type = d_type[j], and so:
+ *   - Hungry: action 0, the nearest pellet.  HungryShy: action 0; flee from the first player (other than a) in the order below
+ *     whose centre lies at distance < 25, whatever its mass (the template compares against a mass of 0, see oracle.c's bot_flee),
+ *     target = loc - (other - loc); else the nearest pellet.  Aggressive: chase the first player in the order at distance <= 20
+ *     that has a cell the agent's largest cell can eat (Cell::can_eat), target = loc + 3 * (mass-weighted centre of those cells
+ *     - loc), the action left as it is; else action 0 and the nearest pellet.  AggressiveShy: flee (action left as it is), else
+ *     chase, else action 0 and the nearest pellet.
+ *   - players are visited in the batch's current layout.order (strict_reference: the order after the latest unmasked reset).
+ *     A dead player, and an absent player of a mixed-task batch, has no cells: its location is NaN and fails every test.
+ *   - the nearest pellet is the first strict minimum in array order of sqrtf(dx * dx + dy * dy) among the pellets with
+ *     (double)d > 0.01; (0, 0) when no pellet qualifies.
+ *   - locations are Player::x / y: fp32 sums of x * (float)mass in cell order over (float)(total mass).
+ * Nothing of the state is written: no target, no action, no flag.  Outputs, caller-owned device memory of cfg.device:
+ *   d_dxdy    f32 [N*A][2]  (target - loc) / 10 in fp32, the inverse of agarcl_batch_set_actions' target = loc + 10 * dxdy.  Not
+ *                           clamped to [-1, 1] (a pellet 60 units away gives 6): the step accepts it, and clamping would change
+ *                           the speed, which is 3 * (target - cell) capped at max_speed.
+ *   d_act     i32 [N*A]
+ *   d_target  f32 [N*A][2]  the world target (may be NULL)
+ *   d_status  u8  [N*A]     (may be NULL) AGARCL_BOT_*:
+ *     SKIPPED    0  d_type[j] == -1: nothing but the status is written for j (fill only the scripted agents of an action
+ *                   buffer that a policy already wrote)
+ *     DECIDED    1
+ *     NO_PELLET  2  the nearest pellet was needed and there is none (the reference would call std::rand(), Bot.hpp:93-97):
+ *                   dxdy 0, target = loc, act 0; no state flag is raised
+ *     DEAD       3  the agent has no cells: dxdy 0, act 0, target (0, 0) (takes precedence over NO_PELLET)
+ *     BAD_TYPE   4  d_type[j] outside -1..3: nothing but the status is written for j
+ * Stream-ordered, no host wait, can be captured in a CUDA graph (the player order is taken at the call).  Refused before anything
+ * is enqueued: a call before the first reset (AGARCL_ERR_STATE); a NULL d_type, d_dxdy or d_act; an array that is not device
+ * memory of cfg.device; d_dxdy or d_target not 8-byte aligned.                                                                  */
+#define AGARCL_BOT_HUNGRY 0
+#define AGARCL_BOT_HUNGRY_SHY 1
+#define AGARCL_BOT_AGGRESSIVE 2
+#define AGARCL_BOT_AGGRESSIVE_SHY 3
+#define AGARCL_BOT_SKIPPED 0
+#define AGARCL_BOT_DECIDED 1
+#define AGARCL_BOT_NO_PELLET 2
+#define AGARCL_BOT_DEAD 3
+#define AGARCL_BOT_BAD_TYPE 4
+int agarcl_batch_bot_actions(agarcl_batch* b, const int32_t* d_type, float* d_dxdy, int32_t* d_act, float* d_target,
+                             uint8_t* d_status, void* stream);
 
 /* ---------------------------------------------------- host-resident observation mirror
  * get_state (bindings.cpp:67-91) hands every agent's frame to HOST memory; for a batch that is 512 KB per agent

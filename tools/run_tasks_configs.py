@@ -4,7 +4,12 @@ viruses, mode k, 0 bots (modes 1-6) or one bot of type k-7 (modes 7-10), episode
 batched vector environment (agarcl_b200.gym_env.BatchedAgarioEnv: N lockstep instances, auto-reset) with the random-walk policy of
 bench/go_bigger_example.py:100-103, and prints one JSON line per mode: env-steps/s, episodes finished, mean return, state flags.
 
-    python tools/run_tasks_configs.py [--envs 4096] [--steps 600] [--modes 1 2 ...] [--dir DIR] [--mixed]
+    python tools/run_tasks_configs.py [--envs 4096] [--steps 600] [--modes 1 2 ...] [--dir DIR] [--mixed] [--policy POLICY]
+
+--policy hungry | hungry_shy | aggressive | aggressive_shy drives every agent with that built-in bot instead of the random walk
+(BatchedAgarioEnv.bot_actions: the reference's bot code run for the agent on the device every step, its actions fed straight into
+step()), in both the per-mode and the --mixed runs: a scripted-baseline table for the mini-games.  Its JSON lines carry "policy";
+the default, random, prints them as before.
 
 --mixed runs the selected mini-games in ONE mixed-task batch of --envs instances instead of one batch per mode: instance i plays
 mode modes[i % len(modes)] with that mode's episode length, every auto-reset keeps it on its mode, and the finished episodes and
@@ -21,6 +26,7 @@ import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+from agarcl_b200._abi import BOT_TYPES  # noqa: E402
 
 # bench/tasks_configs/mode_k.json, the keys that reach the engine
 TASKS = {k: dict(ticks_per_step=4, num_frames=1, arena_size=350, num_pellets=500, num_viruses=0, num_bots=(1 if k >= 7 else 0),
@@ -37,6 +43,22 @@ def load_dir(d):
     return out
 
 
+def policy_actions(args, env, gen, N, bot):
+    """(dxdy, act, bot buffers) of this step: the random walk of bench/go_bigger_example.py:100-103, or the built-in bot computed
+    on the device into the buffers of the previous step"""
+    import torch
+    if args.policy == "random":
+        dxdy = (torch.rand((N, 2), device="cuda", generator=gen) * 2 - 1).float()
+        act = torch.randint(0, 3, (N,), device="cuda", generator=gen, dtype=torch.int32)
+        return dxdy, act, None
+    bot = env.bot_actions(BOT_TYPES[args.policy], out=bot)
+    return bot[0], bot[1], bot
+
+
+def with_policy(args, line):
+    return line if args.policy == "random" else dict(line, policy=args.policy)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--envs", type=int, default=4096)
@@ -44,6 +66,7 @@ def main():
     ap.add_argument("--modes", type=int, nargs="*", default=list(range(1, 11)))
     ap.add_argument("--dir", default=None)
     ap.add_argument("--mixed", action="store_true")
+    ap.add_argument("--policy", default="random", choices=["random"] + list(BOT_TYPES))
     args = ap.parse_args()
     import torch
     from agarcl_b200.gym_env import BatchedAgarioEnv
@@ -63,9 +86,9 @@ def main():
         ret_sum = torch.zeros((), dtype=torch.float64, device="cuda")
         torch.cuda.synchronize()
         t0 = time.perf_counter()
+        bot = None
         for t in range(args.steps):
-            dxdy = (torch.rand((N, 2), device="cuda", generator=gen) * 2 - 1).float()
-            act = torch.randint(0, 3, (N,), device="cuda", generator=gen, dtype=torch.int32)
+            dxdy, act, bot = policy_actions(args, env, gen, N, bot)
             _, _, _, _, info = env.step(dxdy, act)
             m = info["reset_mask"]
             finished += m.sum()
@@ -74,9 +97,9 @@ def main():
         sec = time.perf_counter() - t0
         finished, ret_sum = int(finished), float(ret_sum)
         f, names = env.flags()
-        print(json.dumps({"task": f"mode_{k}", "envs": N, "steps": args.steps, "env_steps_per_s": N * args.steps / sec,
-                          "episode_steps": kw["number_steps"], "episodes_finished": finished,
-                          "mean_return": (ret_sum / finished) if finished else None, "state_flags": names}))
+        print(json.dumps(with_policy(args, {"task": f"mode_{k}", "envs": N, "steps": args.steps, "env_steps_per_s": N * args.steps / sec,
+                                            "episode_steps": kw["number_steps"], "episodes_finished": finished,
+                                            "mean_return": (ret_sum / finished) if finished else None, "state_flags": names})))
         env.close()
 
 
@@ -104,9 +127,9 @@ def run_mixed(args, tasks):
     ret_sum = torch.zeros(11, dtype=torch.float64, device="cuda")
     torch.cuda.synchronize()
     t0 = time.perf_counter()
+    bot = None
     for t in range(args.steps):
-        dxdy = (torch.rand((N, 2), device="cuda", generator=gen) * 2 - 1).float()
-        act = torch.randint(0, 3, (N,), device="cuda", generator=gen, dtype=torch.int32)
+        dxdy, act, bot = policy_actions(args, env, gen, N, bot)
         _, _, _, _, info = env.step(dxdy, act)
         m = info["reset_mask"]
         task = info["task"].long()  # (after an auto-reset: the new episode's, which is the finished one's here)
@@ -117,11 +140,11 @@ def run_mixed(args, tasks):
     finished, ret_sum = finished.tolist(), ret_sum.tolist()
     f, names = env.flags()
     for k in modes:
-        print(json.dumps({"task": f"mode_{k}", "mixed": True, "envs": sum(1 for i in range(N) if modes[i % len(modes)] == k),
-                          "steps": args.steps, "episode_steps": tasks[k]["number_steps"], "episodes_finished": finished[k],
-                          "mean_return": (ret_sum[k] / finished[k]) if finished[k] else None}))
-    print(json.dumps({"task": "mixed", "modes": modes, "envs": N, "steps": args.steps, "env_steps_per_s": N * args.steps / sec,
-                      "ms_per_step": 1e3 * sec / args.steps, "state_flags": names}))
+        print(json.dumps(with_policy(args, {"task": f"mode_{k}", "mixed": True, "envs": sum(1 for i in range(N) if modes[i % len(modes)] == k),
+                                            "steps": args.steps, "episode_steps": tasks[k]["number_steps"], "episodes_finished": finished[k],
+                                            "mean_return": (ret_sum[k] / finished[k]) if finished[k] else None})))
+    print(json.dumps(with_policy(args, {"task": "mixed", "modes": modes, "envs": N, "steps": args.steps, "env_steps_per_s": N * args.steps / sec,
+                                        "ms_per_step": 1e3 * sec / args.steps, "state_flags": names})))
     env.close()
 
 
