@@ -1,13 +1,17 @@
-"""Shared test plumbing: loads the checkers (oracle port, compiled reference) and the product
+"""Shared test plumbing: loads the checkers (oracle port, compiled reference, picture and bot oracles) and the product
 library through ctypes and offers small wrappers.  TEST INFRASTRUCTURE ONLY."""
+import atexit
 import ctypes as C
 import hashlib
 import os
+import re
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
-from agarcl_b200._abi import (Cfg, Layout, RAM_RECORD, StateView, compare_states, make_cfg)
+from agarcl_b200._abi import (BOT_DEAD, BOT_DECIDED, BOT_NO_PELLET, Cfg, Layout, RAM_RECORD, StateView, compare_states, make_cfg)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_SO = os.path.join(ROOT, "oracle", "liboracle.so")
@@ -147,6 +151,94 @@ class Oracle:
             return self.step(with_obs=with_obs)
         finally:
             self.lib.oracle_set_ram_out(None)
+
+
+def aged_oracle(kw, seed, steps, boost=None):
+    """an oracle of make_cfg(**kw) on the mt19937 stream of `seed`, reset (the agents' first cell at mass `boost`, when given)
+    and stepped `steps` times with random actions (p_feed = p_split = 0.3)"""
+    oracle_lib().oracle_set_trig_mode(1)
+    cfg = make_cfg(rng_mode=1, cap_replay=1 << 16, **kw)
+    o = Oracle(cfg)
+    o.seed_mt(seed)
+    o.reset()
+    if boost:
+        for a in range(o.L.A):
+            o.state.cells[a][0]["mass"] = boost
+    rng = np.random.default_rng(seed)
+    for _ in range(steps):
+        o.set_actions(*random_actions(rng, o.L.A, 0.3, 0.3))
+        o.step()
+    return o
+
+
+def _compile_once(name, extra_flags=()):
+    """tests/<name>.c compiled once per session into a temporary directory (the tree may be read-only)"""
+    d = tempfile.mkdtemp(prefix=f"agarcl_{name}_")
+    atexit.register(shutil.rmtree, d, True)
+    so = os.path.join(d, f"lib{name}.so")
+    subprocess.check_call(["gcc", "-std=c11", "-O2", "-fPIC", "-shared", "-ffp-contract=off", "-Wall", *extra_flags,
+                           "-o", so, os.path.join(ROOT, "tests", f"{name}.c"), "-lm"])
+    return C.CDLL(so)
+
+
+# ---- pictures of game states: tests/draw_oracle.c
+ARENA, AGENT = 0, 1
+
+
+def _rgb_constants():
+    """AGARCL_DRAW_RGB_* of the header, as (r, g, b) tuples (the palettes as lists of them)"""
+    text = open(os.path.join(ROOT, "include", "agarcl_b200.h")).read()
+    rgb = lambda v: ((v >> 16) & 255, (v >> 8) & 255, v & 255)  # noqa: E731
+    out = {m.group(1): rgb(int(m.group(2), 16)) for m in re.finditer(r"#define AGARCL_DRAW_RGB_(\w+) (0x[0-9A-Fa-f]+)u", text)}
+    for name in ("AGENTS", "BOTS"):
+        body = re.search(r"#define AGARCL_DRAW_RGB_%s \{([^}]*)\}" % name, text).group(1)
+        out[name] = [rgb(int(v.strip().rstrip("u"), 16)) for v in body.split(",")]
+    return out
+
+
+RGB = _rgb_constants()
+_draw_lib = None
+
+
+def oracle_draw(cfg, L, blob, view, agent, size):
+    global _draw_lib
+    if _draw_lib is None:
+        _draw_lib = _compile_once("draw_oracle")
+    out = np.zeros((size, size, 3), np.uint8)
+    _draw_lib.oracle_draw(C.byref(cfg), C.byref(L), blob.ctypes.data_as(C.c_void_p), int(view), int(agent), int(size),
+                          out.ctypes.data_as(C.c_void_p))
+    return out
+
+
+# ---- built-in bot policies: tests/bot_oracle.c (which includes oracle/oracle.c, compiled with the oracle's flags)
+_bot_lib = None
+
+
+def oracle_bot_decide(cfg, L, blob, agent, bot_type):
+    """(dxdy f32 [2], target f32 [2], act, status) of oracle_bot_decide"""
+    global _bot_lib
+    if _bot_lib is None:
+        _bot_lib = _compile_once("bot_oracle", ["-Wno-unused-function"])
+    dxdy, target = np.zeros(2, np.float32), np.zeros(2, np.float32)
+    act, status = C.c_int32(0), C.c_uint8(0)
+    vp = C.c_void_p
+    _bot_lib.oracle_bot_decide(C.byref(cfg), C.byref(L), blob.ctypes.data_as(vp), int(agent), int(bot_type),
+                               dxdy.ctypes.data_as(vp), target.ctypes.data_as(vp), C.byref(act), C.byref(status))
+    return dxdy, target, int(act.value), int(status.value)
+
+
+def oracle_bot_batch(cfg, L, blobs, types):
+    """every agent of the blobs [N][stride] with types [N*A]: dxdy [N*A, 2], target [N*A, 2], act [N*A], status [N*A]; skipped
+    and bad-type agents are left at 0"""
+    NA = len(blobs) * L.A
+    dxdy, target = np.zeros((NA, 2), np.float32), np.zeros((NA, 2), np.float32)
+    act, status = np.zeros(NA, np.int32), np.zeros(NA, np.uint8)
+    for j in range(NA):
+        d, t, a, s = oracle_bot_decide(cfg, L, blobs[j // L.A], j % L.A, int(types[j]))
+        status[j] = s
+        if s in (BOT_DECIDED, BOT_NO_PELLET, BOT_DEAD):
+            dxdy[j], target[j], act[j] = d, t, a
+    return dxdy, target, act, status
 
 
 class Reference:

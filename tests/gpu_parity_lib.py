@@ -4,13 +4,117 @@ Everything discrete (counts, masses, timers, cooldowns, statistics, rewards, don
 every fp32 field must be IDENTICAL: the oracle runs with trig_mode 1 (the same restatement of
 glibc's atanf / sinf / cosf as the device, itself equal to libm: tests/test_trig_exact.py), all
 other arithmetic is IEEE-exact on both sides.
+
+Also the scaffolding the device-feature tests share: the configuration catalogue CASES, aged
+batches, the record of everything a batch holds and the no-host-wait check.
 """
 import numpy as np
 
 from _helpers import Oracle, oracle_lib, oracle_layout, random_actions
-from agarcl_b200 import RNG_REPLAY, make_cfg
-from agarcl_b200._abi import compare_states
+from agarcl_b200 import OBS_I16, RNG_MT19937, RNG_REPLAY, make_cfg
+from agarcl_b200._abi import compare_states, task_bits
 from agarcl_b200.batch import Batch
+
+SMALL = dict(num_bots=4, arena_size=300, num_pellets=300, num_viruses=4)
+# name: (make_cfg keywords, p_feed, p_split, boost); each test module selects its cases by name
+CASES = {
+    "c1": (dict(num_viruses=0, num_bots=0), 1 / 3, 1 / 3, None),
+    "c2": (dict(), 1 / 3, 1 / 3, None),
+    "c3": (dict(num_bots=8, num_viruses=10), 0.0, 0.0, None),
+    "c4_four_agents": (dict(num_agents=4, num_bots=8, cap_foods=2048), 0.3, 0.3, 1000),
+    "c5": (dict(arena_size=2000, num_pellets=4000, num_viruses=50, cap_viruses=128), 1 / 3, 1 / 3, None),
+    "configs1_two_agents": (dict(num_agents=2), 1 / 3, 1 / 3, None),
+    "mode1": (dict(mode_number=1, num_bots=0), 1 / 3, 1 / 3, None),
+    "mode7": (dict(mode_number=7), 1 / 3, 1 / 3, None),
+    "mode8": (dict(mode_number=8), 1 / 3, 1 / 3, None),
+    "mode9": (dict(mode_number=9), 1 / 3, 1 / 3, None),
+    "mode10": (dict(mode_number=10), 1 / 3, 1 / 3, None),
+    # mode 9: its one bot is the Aggressive type, which eats the random-walking agent in about one 37-step episode in ten (the
+    # Hungry-Shy bot of mode 8 never does in the oracle over 64 seeds), so an episodic run sees deaths as well as step-limit
+    # truncations
+    "mode9_deaths_and_limit": (dict(mode_number=9, num_bots=1, arena_size=200, num_pellets=300, num_viruses=0), 1 / 3, 1 / 3,
+                               None),
+    "mixed_tasks": (dict(mode_number=1, task_modes=task_bits([1, 7, 8, 10]), num_bots=0, arena_size=400, num_pellets=400), 1 / 3,
+                    1 / 3, None),
+    "int16": (dict(obs_dtype=OBS_I16, **SMALL), 1 / 3, 1 / 3, None),
+    "two_frames": (dict(num_frames=2, **SMALL), 1 / 3, 1 / 3, None),
+    "ram_obs1": (dict(ram_obs=1, **SMALL), 1 / 3, 1 / 3, None),
+    "ram_obs2": (dict(ram_obs=2, **SMALL), 1 / 3, 1 / 3, None),
+    "mt19937": (dict(rng_mode=RNG_MT19937, **SMALL), 1 / 3, 1 / 3, None),
+    # one step draws at most 2 * (150 + 2 + 4) = 312: a 1024-entry ring wraps within a few episodes
+    "mt19937_ring_wraps": (dict(rng_mode=RNG_MT19937, cap_replay=1024, num_bots=3, arena_size=60, num_pellets=150, num_viruses=2),
+                           1 / 3, 1 / 3, None),
+    # one tick per step: the step renders its frame with k_obs
+    "strict_reference": (dict(strict_reference=1, ticks_per_step=1, num_agents=2, **SMALL), 1 / 3, 1 / 3, None),
+}
+
+
+def i32(x):
+    import torch
+    return torch.as_tensor(np.asarray(x, np.int32), device="cuda")
+
+
+def aged_batch(name, N=4, seed=5, second_reset=False):
+    """a Batch of N instances of CASES[name] seeded with `seed` and reset, with the rng, p_feed and p_split for step_random.
+    A mixed-task batch plays modes 1, 7, 8, 10, then 1.  second_reset: under strict_reference, a second unmasked reset (the
+    player order of the reference's second episode).  A boost is the mass of the agents' first cell after the reset."""
+    import torch
+    kw, p_feed, p_split, boost = CASES[name]
+    b = Batch(make_cfg(n_instances=N, **kw))
+    b.seed(seed)
+    if b.cfg.task_modes:
+        b.set_tasks(i32([1, 7, 8, 10][:N] + [1] * max(0, N - 4)))
+    b.reset()
+    if second_reset and b.cfg.strict_reference:
+        b.reset()
+    if boost:
+        for i in range(N):
+            sv = b.download_state(i)
+            for a in range(b.A):
+                sv.cells[a][0]["mass"] = boost
+            b.upload_state(i, sv)
+    torch.cuda.synchronize()
+    return b, np.random.default_rng(seed), p_feed, p_split
+
+
+def step_random(b, rng, p_feed, p_split, k):
+    for _ in range(k):
+        b.set_actions(*random_actions(rng, b.N * b.A, p_feed, p_split))
+        b.step()
+
+
+def device_record(b):
+    """everything batch b holds, on the host: state blobs, observation, rewards and dones; ram records (cfg.ram_obs), the
+    episode buffers with the final observations and ram records (after set_autoreset) and the host mirror (once made)"""
+    import torch
+    torch.cuda.synchronize()
+    r = {"blobs": np.stack([b.download_state(i).blob for i in range(b.N)]), "obs": b.obs_tensor().cpu().numpy(),
+         "rewards": b.rewards_tensor().cpu().numpy(), "dones": b.dones_tensor().cpu().numpy()}
+    if b.cfg.ram_obs:
+        r["ram"] = b.ram_tensor().cpu().numpy()
+    if hasattr(b, "_episode"):
+        r.update({k: v.cpu().numpy() for k, v in b.episode().items()})
+        e = b._episode_struct()
+        if e.final_obs:
+            r["final_obs"] = b.final_obs().cpu().numpy()
+        if e.final_ram:
+            r["final_ram"] = b.final_ram().cpu().numpy()
+    if getattr(b, "_mirror", None) is not None:
+        r["mirror"] = b.mirror().copy()
+    return r
+
+
+def assert_no_host_wait(calls, stream):
+    """the host returns from calls() while `stream` is still busy with work queued before them (detects a synchronise on the
+    way; the device only sleeps).  Every kernel on the path must have been loaded before, by a warm-up."""
+    import torch
+    torch.cuda.synchronize()
+    with torch.cuda.stream(stream):
+        torch.cuda._sleep(200_000_000)  # ~0.1 s at the B200's clock
+    calls()
+    busy = not stream.query()
+    torch.cuda.synchronize()
+    assert busy, "a call waited for the device"
 
 
 def philox4x32_10_np(counter, key):

@@ -2,62 +2,20 @@
 (tests/bot_oracle.c: oracle.c's bot_take_action on a private copy of the blob) on crafted states: the nearest pellet against a
 numpy fp32 brute force, the flee and chase triggers, no pellets, a dead agent, absent players of a mixed-task layout, and the
 blob left untouched.  Also: k_bot_actions compiles for sm_100a without stack or spills.  CPU only."""
-import atexit
-import ctypes as C
 import os
 import re
-import shutil
 import subprocess
 import tempfile
 
 import numpy as np
 import pytest
 
-from _helpers import ROOT, Oracle, oracle_layout, oracle_lib, random_actions
+from _helpers import aged_oracle, oracle_bot_decide, oracle_layout
 from agarcl_b200._abi import (BOT_AGGRESSIVE, BOT_AGGRESSIVE_SHY, BOT_BAD_TYPE, BOT_DEAD, BOT_DECIDED, BOT_HUNGRY, BOT_HUNGRY_SHY,
                               BOT_NO_PELLET, BOT_SKIPPED, StateView, make_cfg, task_bits)
 
 F = np.float32
 TYPES = (BOT_HUNGRY, BOT_HUNGRY_SHY, BOT_AGGRESSIVE, BOT_AGGRESSIVE_SHY)
-_bot_lib = None
-
-
-def bot_lib():
-    """tests/bot_oracle.c (which includes oracle/oracle.c), compiled once per session into a temporary directory with the
-    oracle's flags (the tree may be read-only)"""
-    global _bot_lib
-    if _bot_lib is None:
-        d = tempfile.mkdtemp(prefix="agarcl_bot_oracle_")
-        atexit.register(shutil.rmtree, d, True)
-        so = os.path.join(d, "libbot_oracle.so")
-        subprocess.check_call(["gcc", "-std=c11", "-O2", "-fPIC", "-shared", "-ffp-contract=off", "-Wall", "-Wno-unused-function",
-                               "-o", so, os.path.join(ROOT, "tests", "bot_oracle.c"), "-lm"])
-        _bot_lib = C.CDLL(so)
-    return _bot_lib
-
-
-def oracle_bot_decide(cfg, L, blob, agent, bot_type):
-    """(dxdy f32 [2], target f32 [2], act, status) of oracle_bot_decide"""
-    dxdy, target = np.zeros(2, np.float32), np.zeros(2, np.float32)
-    act, status = C.c_int32(0), C.c_uint8(0)
-    vp = C.c_void_p
-    bot_lib().oracle_bot_decide(C.byref(cfg), C.byref(L), blob.ctypes.data_as(vp), int(agent), int(bot_type),
-                                dxdy.ctypes.data_as(vp), target.ctypes.data_as(vp), C.byref(act), C.byref(status))
-    return dxdy, target, int(act.value), int(status.value)
-
-
-def oracle_bot_batch(cfg, L, blobs, types):
-    """every agent of the blobs [N][stride] with types [N*A]: dxdy [N*A, 2], target [N*A, 2], act [N*A], status [N*A]; skipped
-    and bad-type agents are left at 0"""
-    NA = len(blobs) * L.A
-    dxdy, target = np.zeros((NA, 2), np.float32), np.zeros((NA, 2), np.float32)
-    act, status = np.zeros(NA, np.int32), np.zeros(NA, np.uint8)
-    for j in range(NA):
-        d, t, a, s = oracle_bot_decide(cfg, L, blobs[j // L.A], j % L.A, int(types[j]))
-        status[j] = s
-        if s in (BOT_DECIDED, BOT_NO_PELLET, BOT_DEAD):
-            dxdy[j], target[j], act[j] = d, t, a
-    return dxdy, target, act, status
 
 
 def _state(A=1, bots=3, pellets=64, arena=200, **kw):
@@ -278,23 +236,10 @@ def test_dead_and_absent_players_are_never_chosen():
             assert all(np.array_equal(np.asarray(x), np.asarray(y)) for x, y in zip(got, ref))
 
 
-def _aged(kw, seed, steps):
-    oracle_lib().oracle_set_trig_mode(1)
-    cfg = make_cfg(rng_mode=1, cap_replay=1 << 16, **kw)
-    o = Oracle(cfg)
-    o.seed_mt(seed)
-    o.reset()
-    rng = np.random.default_rng(seed)
-    for _ in range(steps):
-        o.set_actions(*random_actions(rng, o.L.A, 0.3, 0.3))
-        o.step()
-    return o
-
-
 def test_the_blob_is_never_modified():
     """aged multi-agent states, every agent and type, with and without pellets"""
     for seed in (1, 2):
-        o = _aged(dict(num_agents=4, num_bots=8, arena_size=300, num_pellets=300, num_viruses=4), seed, 30)
+        o = aged_oracle(dict(num_agents=4, num_bots=8, arena_size=300, num_pellets=300, num_viruses=4), seed, 30)
         before = o.state.blob.copy()
         statuses = set()
         for a in range(o.L.A):

@@ -1,58 +1,11 @@
 """Pictures of game states (include/agarcl_b200.h, agarcl_batch_draw), pinned through their CPU restatement oracle_draw
 (tests/draw_oracle.c): the disc test against a numpy fp32 evaluation, the draw order, the agent view's tie to observation
 channel 0 (of the oracle port), the one-pixel floor and the absent players of a mixed-task layout.  CPU only."""
-import atexit
-import ctypes as C
-import os
-import re
-import shutil
-import subprocess
-import tempfile
-
 import numpy as np
 import pytest
 
-from _helpers import ROOT, Oracle, oracle_layout, oracle_lib, random_actions
+from _helpers import AGENT, ARENA, RGB, aged_oracle, oracle_draw, oracle_layout
 from agarcl_b200._abi import StateView, make_cfg, task_bits
-
-ARENA, AGENT = 0, 1
-
-
-def _rgb_constants():
-    """AGARCL_DRAW_RGB_* of the header, as (r, g, b) tuples (the palettes as lists of them)"""
-    text = open(os.path.join(ROOT, "include", "agarcl_b200.h")).read()
-    rgb = lambda v: ((v >> 16) & 255, (v >> 8) & 255, v & 255)  # noqa: E731
-    out = {m.group(1): rgb(int(m.group(2), 16)) for m in re.finditer(r"#define AGARCL_DRAW_RGB_(\w+) (0x[0-9A-Fa-f]+)u", text)}
-    for name in ("AGENTS", "BOTS"):
-        body = re.search(r"#define AGARCL_DRAW_RGB_%s \{([^}]*)\}" % name, text).group(1)
-        out[name] = [rgb(int(v.strip().rstrip("u"), 16)) for v in body.split(",")]
-    return out
-
-
-RGB = _rgb_constants()
-
-
-_draw_lib = None
-
-
-def draw_lib():
-    """tests/draw_oracle.c, compiled once per session into a temporary directory (the tree may be read-only)"""
-    global _draw_lib
-    if _draw_lib is None:
-        d = tempfile.mkdtemp(prefix="agarcl_draw_oracle_")
-        atexit.register(shutil.rmtree, d, True)
-        so = os.path.join(d, "libdraw_oracle.so")
-        subprocess.check_call(["gcc", "-std=c11", "-O2", "-fPIC", "-shared", "-ffp-contract=off", "-Wall",
-                               "-o", so, os.path.join(ROOT, "tests", "draw_oracle.c"), "-lm"])
-        _draw_lib = C.CDLL(so)
-    return _draw_lib
-
-
-def oracle_draw(cfg, L, blob, view, agent, size):
-    out = np.zeros((size, size, 3), np.uint8)
-    draw_lib().oracle_draw(C.byref(cfg), C.byref(L), blob.ctypes.data_as(C.c_void_p), int(view), int(agent), int(size),
-                             out.ctypes.data_as(C.c_void_p))
-    return out
 
 
 def is_color(pic, rgb):
@@ -150,22 +103,6 @@ def test_draw_order_mass_kind_id():
         assert is_color(pic, RGB["BOTS"][t]).any()
 
 
-def _aged_oracle(kw, seed, steps, boost=None):
-    oracle_lib().oracle_set_trig_mode(1)
-    cfg = make_cfg(rng_mode=1, cap_replay=1 << 16, **kw)
-    o = Oracle(cfg)
-    o.seed_mt(seed)
-    o.reset()
-    if boost:
-        for a in range(o.L.A):
-            o.state.cells[a][0]["mass"] = boost
-    rng = np.random.default_rng(seed)
-    for _ in range(steps):
-        o.set_actions(*random_actions(rng, o.L.A, 0.3, 0.3))
-        o.step()
-    return o
-
-
 AGED = {
     "c2": (dict(), None),
     "c4": (dict(num_agents=4, num_bots=8, cap_foods=2048), 1000),
@@ -179,7 +116,7 @@ def test_agent_view_out_of_arena_is_observation_channel0(name):
     kw, boost = AGED[name]
     checked = 0
     for seed in (3, 4, 5):
-        o = _aged_oracle(kw, seed, 40, boost)
+        o = aged_oracle(kw, seed, 40, boost)
         if int(o.state.hdr["respawned_lo"]) or int(o.state.hdr["respawned_hi"]):
             continue  # (the observation of the step shows respawned players dead)
         G = o.cfg.grid_size
@@ -192,7 +129,7 @@ def test_agent_view_out_of_arena_is_observation_channel0(name):
 
 
 def test_agent_view_of_dead_agent_is_all_out_of_arena():
-    o = _aged_oracle(dict(num_agents=2, num_bots=4), 7, 5)
+    o = aged_oracle(dict(num_agents=2, num_bots=4), 7, 5)
     o.state.players["n_cells"][1] = 0
     pic = oracle_draw(o.cfg, o.L, o.state.blob, AGENT, 1, 64)
     assert is_color(pic, RGB["OUT"]).all()
@@ -201,7 +138,7 @@ def test_agent_view_of_dead_agent_is_all_out_of_arena():
 
 def test_one_pixel_floor_keeps_pellets_visible():
     """a 64-pixel picture of a 2000-unit arena: pixels are 31 units apart and a pellet's radius is 0.56, drawn at one pixel"""
-    o = _aged_oracle(dict(arena_size=2000, num_pellets=4000, num_viruses=50, cap_viruses=128), 9, 0)
+    o = aged_oracle(dict(arena_size=2000, num_pellets=4000, num_viruses=50, cap_viruses=128), 9, 0)
     pic = oracle_draw(o.cfg, o.L, o.state.blob, ARENA, 0, 64)
     assert is_color(pic, RGB["PELLET"]).sum() > 64 * 64 // 4
 

@@ -6,7 +6,8 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from agarcl_b200 import OBS_I16, RNG_MT19937, make_cfg
+from agarcl_b200 import OBS_I16, make_cfg
+from gpu_parity_lib import CASES, assert_no_host_wait, device_record
 
 
 def test_episode_struct_matches_header():
@@ -25,30 +26,15 @@ def _pair(cfg, seed):
     return ref, dev
 
 
-def _blobs_equal(a, b, N):
-    return all(np.array_equal(a.download_state(i).blob, b.download_state(i).blob) for i in range(N))
-
-
-# mode 9: its one bot is the Aggressive type, which eats the random-walking agent in about one 37-step episode in ten (the
-# Hungry-Shy bot of mode 8 never does in the oracle over 64 seeds), so the run sees deaths as well as step-limit truncations
-CASES = {
-    "mode9_deaths_and_limit": dict(mode_number=9, num_bots=1, arena_size=200, num_pellets=300, num_viruses=0),
-    "configs1_two_agents": dict(num_agents=2),
-    "int16": dict(obs_dtype=OBS_I16, num_bots=4, arena_size=300, num_pellets=300, num_viruses=4),
-    "two_frames": dict(num_frames=2, num_bots=4, arena_size=300, num_pellets=300, num_viruses=4),
-    "strict_reference": dict(strict_reference=1, ticks_per_step=1, num_bots=4, arena_size=300, num_pellets=300, num_viruses=4),
-    "ram_obs1": dict(ram_obs=1, num_bots=4, arena_size=300, num_pellets=300, num_viruses=4),
-    "ram_obs2": dict(ram_obs=2, num_bots=4, arena_size=300, num_pellets=300, num_viruses=4),
-    # one step draws at most 2 * (150 + 2 + 4) = 312: a 1024-entry ring wraps within a few episodes
-    "mt19937_ring_wraps": dict(rng_mode=RNG_MT19937, cap_replay=1024, num_bots=3, arena_size=60, num_pellets=150, num_viruses=2),
-}
+AUTORESET_CASES = ["mode9_deaths_and_limit", "configs1_two_agents", "int16", "two_frames", "strict_reference", "ram_obs1", "ram_obs2",
+                   "mt19937_ring_wraps"]
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", list(CASES))
+@pytest.mark.parametrize("name", AUTORESET_CASES)
 def test_step_autoreset_equals_host_composition(name):
     import torch
-    kw = CASES[name]
+    kw = CASES[name][0]
     N, steps, max_steps = (16 if name == "configs1_two_agents" else 32), 200, 37
     cfg = make_cfg(n_instances=N, **kw)
     ref, dev = _pair(cfg, 1234)
@@ -88,8 +74,9 @@ def test_step_autoreset_equals_host_composition(name):
         dev.step_autoreset()
         torch.cuda.synchronize()
         img = torch.from_numpy(np.repeat(mask, A)).cuda()
-        assert torch.equal(dev.obs_tensor(), ref.obs_tensor()), t
-        assert torch.equal(dev.rewards_tensor(), ref.rewards_tensor()), t
+        r, d = device_record(ref), device_record(dev)
+        for k in r:  # state blobs, obs, rewards, dones and ram records
+            assert np.array_equal(r[k], d[k]), (t, k)
         assert np.array_equal(ep["done"].cpu().numpy(), done.reshape(-1).astype(np.uint8)), t
         assert np.array_equal(ep["reset_mask"].cpu().numpy(), mask.astype(np.uint8)), t
         if mask.any():
@@ -104,9 +91,6 @@ def test_step_autoreset_equals_host_composition(name):
             acc[agents] = 0.0
             host_steps[mask] = 0
         assert np.array_equal(ep["steps"].cpu().numpy(), host_steps), t
-        if cfg.ram_obs:
-            assert torch.equal(dev.ram_tensor(), ref.ram_tensor()), t
-        assert _blobs_equal(ref, dev, N), t
     assert truncations > 0
     if name == "mode9_deaths_and_limit":
         assert deaths > 0, "no agent died: the run did not cover natural episode ends"
@@ -148,16 +132,15 @@ def test_device_mask_reset(kw):
     bs[0].reset(mask)
     bs[1].reset_device(torch.from_numpy(mask).cuda().bool())
     bs[2].reset()
-    torch.cuda.synchronize()
-    assert torch.equal(bs[0].obs_tensor(), bs[1].obs_tensor())
-    assert _blobs_equal(bs[0], bs[1], N)
+    r0, r1 = device_record(bs[0]), device_record(bs[1])
+    for k in r0:
+        assert np.array_equal(r0[k], r1[k]), k
     img = torch.from_numpy(np.repeat(mask.astype(bool), bs[1].A)).cuda()
     m = torch.from_numpy(mask.astype(bool)).cuda()
     o1, o2 = bs[1].obs_tensor(), bs[2].obs_tensor()
     assert torch.equal(o1[img], o2[img]) and torch.equal(o1[~img], obs_before[~img])
     if cfg.ram_obs:
         r1 = bs[1].ram_tensor()
-        assert torch.equal(r1, bs[0].ram_tensor())
         assert int(r1[m].abs().sum()) == 0 and torch.equal(r1[~m], ram_before[~m])
     for i in range(N):
         if mask[i]:
@@ -188,15 +171,13 @@ def test_step_autoreset_does_not_wait_for_the_device():
     for _ in range(4):  # every kernel on the path is loaded before the timed calls (and some instances reset)
         env.step_autoreset(dxdy, act, stream=s.cuda_stream)
         env.reset(mask, stream=s.cuda_stream)
-    torch.cuda.synchronize()
-    with torch.cuda.stream(s):
-        torch.cuda._sleep(200_000_000)  # ~0.1 s at the B200's clock
-    for _ in range(3):
-        env.step_autoreset(dxdy, act, stream=s.cuda_stream)
-    env.reset(mask, stream=s.cuda_stream)
-    busy = not s.query()
-    s.synchronize()
-    assert busy, "a call waited for the device"
+
+    def calls():
+        for _ in range(3):
+            env.step_autoreset(dxdy, act, stream=s.cuda_stream)
+        env.reset(mask, stream=s.cuda_stream)
+
+    assert_no_host_wait(calls, s)
     steps = env.episode()["steps"].cpu().numpy()
     assert steps.max() <= 3 and (steps[::3] == 0).all()
     env.close()
@@ -206,13 +187,7 @@ def test_step_autoreset_does_not_wait_for_the_device():
     venv.reset()
     for _ in range(4):
         venv.step(dxdy, act)
-    torch.cuda.synchronize()
-    torch.cuda._sleep(200_000_000)
-    for _ in range(3):
-        venv.step(dxdy, act)
-    busy = not torch.cuda.current_stream().query()
-    torch.cuda.synchronize()
-    assert busy, "BatchedAgarioEnv.step waited for the device"
+    assert_no_host_wait(lambda: [venv.step(dxdy, act) for _ in range(3)], torch.cuda.current_stream())
     venv.close()
 
 

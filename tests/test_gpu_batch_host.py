@@ -45,9 +45,9 @@ def test_batches_on_two_devices_of_one_process():
     assert all(np.array_equal(a, b) for a, b in zip(s0, s1))
 
 
-# kernels per step of the configurations of test_gpu_autoreset.py: k_step + k_order, + k_ram with ram_obs; two frames:
-# four one-tick k_step launches, k_obs for each of the last two ticks and the closing k_step; strict_reference: k_obs
-# renders the frame (ticks_per_step = 1)
+# kernels per step of configurations of gpu_parity_lib.CASES: k_step + k_order, + k_ram with ram_obs; two frames: four
+# one-tick k_step launches, k_obs for each of the last two ticks and the closing k_step; strict_reference: k_obs renders the
+# frame (ticks_per_step = 1)
 LAUNCHES = {"mode9_deaths_and_limit": 2, "configs1_two_agents": 2, "int16": 2, "two_frames": 7, "strict_reference": 2,
             "ram_obs1": 3, "ram_obs2": 3, "mt19937_ring_wraps": 2}
 
@@ -55,9 +55,9 @@ LAUNCHES = {"mode9_deaths_and_limit": 2, "configs1_two_agents": 2, "int16": 2, "
 @pytest.mark.parametrize("name", list(LAUNCHES))
 def test_launches_per_step(name):
     from agarcl_b200.batch import Batch
-    from test_gpu_autoreset import CASES
+    from gpu_parity_lib import CASES
     N = 8
-    b = Batch(make_cfg(n_instances=N, **CASES[name]))
+    b = Batch(make_cfg(n_instances=N, **CASES[name][0]))
     b.seed(3)
     b.reset()
     b.set_actions(np.zeros((N * b.A, 2), np.float32), np.zeros(N * b.A, np.int32))

@@ -10,64 +10,13 @@ import sys
 import numpy as np
 import pytest
 
-from _helpers import ROOT, Oracle, oracle_layout, oracle_lib, random_actions
-from agarcl_b200 import OBS_I16, RNG_MT19937, RNG_REPLAY, make_cfg
-from agarcl_b200._abi import BOT_BAD_TYPE, BOT_DEAD, BOT_DECIDED, BOT_NO_PELLET, BOT_SKIPPED, compare_states, task_bits
-from test_bot_actions_oracle import oracle_bot_batch, oracle_bot_decide
+from _helpers import ROOT, Oracle, oracle_bot_batch, oracle_bot_decide, oracle_layout, oracle_lib, random_actions
+from agarcl_b200 import RNG_REPLAY, make_cfg
+from agarcl_b200._abi import BOT_BAD_TYPE, BOT_DEAD, BOT_DECIDED, BOT_NO_PELLET, BOT_SKIPPED, compare_states
+from gpu_parity_lib import SMALL, aged_batch, device_record, i32, step_random
 
-_BASE = dict(num_agents=1, num_bots=25, num_viruses=25, num_pellets=1000, arena_size=1000)
-_SMALL = dict(num_bots=4, arena_size=300, num_pellets=300, num_viruses=4)
-# name: (make_cfg keywords, p_feed, p_split, boost)
-CASES = {
-    "c1": (dict(num_viruses=0, num_bots=0), 1 / 3, 1 / 3, None),
-    "c2": (dict(), 1 / 3, 1 / 3, None),
-    "c3": (dict(num_bots=8, num_viruses=10), 0.0, 0.0, None),
-    "c4_four_agents": (dict(num_agents=4, num_bots=8, cap_foods=2048), 0.3, 0.3, 1000),
-    "c5": (dict(arena_size=2000, num_pellets=4000, num_viruses=50, cap_viruses=128), 1 / 3, 1 / 3, None),
-    "mode1": (dict(mode_number=1, num_bots=0), 1 / 3, 1 / 3, None),
-    "mode7": (dict(mode_number=7), 1 / 3, 1 / 3, None),
-    "mode8": (dict(mode_number=8), 1 / 3, 1 / 3, None),
-    "mode9": (dict(mode_number=9), 1 / 3, 1 / 3, None),
-    "mode10": (dict(mode_number=10), 1 / 3, 1 / 3, None),
-    "mixed_tasks": (dict(mode_number=1, task_modes=task_bits([1, 7, 8, 10]), num_bots=0, arena_size=400, num_pellets=400), 1 / 3,
-                    1 / 3, None),
-    "int16": (dict(obs_dtype=OBS_I16, **_SMALL), 1 / 3, 1 / 3, None),
-    "ram_obs2": (dict(ram_obs=2, **_SMALL), 1 / 3, 1 / 3, None),
-    "mt19937": (dict(rng_mode=RNG_MT19937, **_SMALL), 1 / 3, 1 / 3, None),
-    "strict_reference": (dict(strict_reference=1, num_agents=2, **_SMALL), 1 / 3, 1 / 3, None),
-}
-
-
-def _i32(x):
-    import torch
-    return torch.as_tensor(np.asarray(x, np.int32), device="cuda")
-
-
-def _batch(name, N=4, seed=5):
-    from agarcl_b200.batch import Batch
-    import torch
-    kw, p_feed, p_split, boost = CASES[name]
-    b = Batch(make_cfg(n_instances=N, **dict(_BASE, **kw)))
-    b.seed(seed)
-    if b.cfg.task_modes:
-        b.set_tasks(_i32([1, 7, 8, 10][:N] + [1] * max(0, N - 4)))
-    b.reset()
-    if b.cfg.strict_reference:
-        b.reset()  # a second unmasked reset: the player order of the reference's second episode
-    if boost:
-        for i in range(N):
-            sv = b.download_state(i)
-            for a in range(b.A):
-                sv.cells[a][0]["mass"] = boost
-            b.upload_state(i, sv)
-    torch.cuda.synchronize()
-    return b, np.random.default_rng(seed), p_feed, p_split
-
-
-def _step(b, rng, p_feed, p_split, k):
-    for _ in range(k):
-        b.set_actions(*random_actions(rng, b.N * b.A, p_feed, p_split))
-        b.step()
+CASES = ["c1", "c2", "c3", "c4_four_agents", "c5", "mode1", "mode7", "mode8", "mode9", "mode10", "mixed_tasks", "int16", "ram_obs2",
+         "mt19937", "strict_reference"]
 
 
 SENT_F, SENT_I, SENT_U8 = np.float32(-12345.5), -777, 0xEE
@@ -85,7 +34,7 @@ def _check(b, types):
     status = torch.full((NA,), SENT_U8, dtype=torch.uint8, device="cuda")
     torch.cuda.synchronize()
     blobs = np.stack([b.download_state(i).blob for i in range(b.N)])
-    out = b.bot_actions(_i32(types), out=(dxdy, act, status), target=target)
+    out = b.bot_actions(i32(types), out=(dxdy, act, status), target=target)
     assert out[0] is dxdy and out[1] is act and out[2] is status
     torch.cuda.synchronize()
     after = np.stack([b.download_state(i).blob for i in range(b.N)])
@@ -116,13 +65,13 @@ def _all_types(b, rng):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", list(CASES))
+@pytest.mark.parametrize("name", CASES)
 def test_bot_actions_match_oracle(name):
     """every agent and type at ages 0, 1 and 250"""
-    b, rng, p_feed, p_split = _batch(name)
+    b, rng, p_feed, p_split = aged_batch(name, second_reset=True)
     seen = set()
     for more in (0, 1, 249):
-        _step(b, rng, p_feed, p_split, more)
+        step_random(b, rng, p_feed, p_split, more)
         seen |= set(_all_types(b, rng).tolist())
     assert BOT_DECIDED in seen and BOT_SKIPPED in seen and BOT_BAD_TYPE in seen
     if name == "c4_four_agents":  # the agents did split
@@ -133,8 +82,8 @@ def test_bot_actions_match_oracle(name):
 @pytest.mark.gpu
 def test_aged_c2_multi_cell_and_popped_players():
     """c2 at 2000 steps: bots with many cells, players popped by viruses and eaten"""
-    b, rng, pf, ps = _batch("c2", N=2, seed=11)
-    _step(b, rng, pf, ps, 2000)
+    b, rng, pf, ps = aged_batch("c2", N=2, seed=11)
+    step_random(b, rng, pf, ps, 2000)
     st = _all_types(b, rng)
     assert BOT_DECIDED in st
     L = b.layout
@@ -203,36 +152,29 @@ def test_crafted_states():
     b.close()
 
 
-def _everything(b):
-    import torch
-    torch.cuda.synchronize()
-    return {"blobs": np.stack([b.download_state(i).blob for i in range(b.N)]), "obs": b.obs_tensor().cpu().numpy(),
-            "rewards": b.rewards_tensor().cpu().numpy(), "dones": b.dones_tensor().cpu().numpy()}
-
-
 @pytest.mark.gpu
 def test_state_untouched_against_a_twin():
     """the batch that computes bot actions every step stays identical to a twin that never does, over 50 steps"""
     from agarcl_b200.batch import Batch
-    cfg = make_cfg(n_instances=6, **dict(_BASE, num_agents=2, **_SMALL))
+    cfg = make_cfg(n_instances=6, num_agents=2, **SMALL)
     twins = [Batch(cfg), Batch(cfg)]
     for b in twins:
         b.seed(8)
         b.reset()
     rng = np.random.default_rng(0)
-    types = _i32(rng.choice([-1, 0, 1, 2, 3, 9], cfg.n_instances * 2))
+    types = i32(rng.choice([-1, 0, 1, 2, 3, 9], cfg.n_instances * 2))
     for t in range(50):
         dxdy, act = random_actions(rng, cfg.n_instances * 2)
-        before = _everything(twins[0])
+        before = device_record(twins[0])
         for ty in (types, 0, 1, 2, 3):
             twins[0].bot_actions(ty)
-        after = _everything(twins[0])
+        after = device_record(twins[0])
         for k in before:
             assert np.array_equal(before[k], after[k]), f"step {t}: bot_actions changed {k}"
         for b in twins:
             b.set_actions(dxdy, act)
             b.step()
-        a, c = _everything(twins[0]), _everything(twins[1])
+        a, c = device_record(twins[0]), device_record(twins[1])
         for k in a:
             assert np.array_equal(a[k], c[k]), f"step {t}: {k} differs from the twin"
 
@@ -247,7 +189,7 @@ def test_closed_loop_against_the_oracle():
     oracle_lib().oracle_set_trig_mode(1)
     seeds = [21, 22]
     n, A = len(seeds), 4
-    cfg = make_cfg(n_instances=n, rng_mode=RNG_REPLAY, cap_replay=1 << 16, **dict(_BASE, num_agents=A, **_SMALL))
+    cfg = make_cfg(n_instances=n, rng_mode=RNG_REPLAY, cap_replay=1 << 16, num_agents=A, **SMALL)
     b = Batch(cfg)
     L = b.layout
     Lo = oracle_layout(cfg)
@@ -263,7 +205,7 @@ def test_closed_loop_against_the_oracle():
     for o in oras:
         o.reset()
     types = np.array([0, 1, 2, 3, 3, -1, 1, 2], np.int32)
-    types_t = _i32(types)
+    types_t = i32(types)
     dxdy_t = torch.zeros((n * A, 2), dtype=torch.float32, device="cuda")
     act_t = torch.zeros(n * A, dtype=torch.int32, device="cuda")
     status_t = torch.zeros(n * A, dtype=torch.uint8, device="cuda")
@@ -307,9 +249,9 @@ def test_graph_capture_of_bot_actions_and_step_autoreset():
     eager run of a twin batch, step for step"""
     import torch
     from agarcl_b200.batch import Batch
-    cfg = make_cfg(n_instances=8, **dict(_BASE, num_agents=2, **_SMALL))
+    cfg = make_cfg(n_instances=8, num_agents=2, **SMALL)
     twins = [Batch(cfg), Batch(cfg)]
-    types = _i32(np.random.default_rng(1).choice([-1, 0, 1, 2, 3], 16))
+    types = i32(np.random.default_rng(1).choice([-1, 0, 1, 2, 3], 16))
     bufs = []
     for b in twins:
         b.seed(3)
@@ -335,14 +277,11 @@ def test_graph_capture_of_bot_actions_and_step_autoreset():
         twins[0].bot_actions(types, out=bufs[0])
         twins[0].step_autoreset()
         g.replay()
-        a, c = _everything(twins[0]), _everything(twins[1])
+        a, c = device_record(twins[0]), device_record(twins[1])
         for k in a:
             assert np.array_equal(a[k], c[k]), f"replay {t}: {k}"
         for x, y in zip(bufs[0], bufs[1]):
             assert torch.equal(x, y), f"replay {t}: outputs"
-        ea, ec = twins[0].episode(), twins[1].episode()
-        for k in ea:
-            assert torch.equal(ea[k], ec[k]), f"replay {t}: episode {k}"
 
 
 @pytest.mark.gpu
@@ -352,9 +291,9 @@ def test_refusals_enqueue_nothing():
     from agarcl_b200.batch import Batch
     L = _lib.lib()
     vp = C.c_void_p
-    cfg = make_cfg(n_instances=2, **dict(_BASE, num_agents=2, **_SMALL))
+    cfg = make_cfg(n_instances=2, num_agents=2, **SMALL)
     fresh = Batch(cfg)
-    types = _i32([0, 1, 2, 3])
+    types = i32([0, 1, 2, 3])
     dxdy = torch.full((5, 2), 7.0, dtype=torch.float32, device="cuda")
     target = torch.full((5, 2), 7.0, dtype=torch.float32, device="cuda")
     act = torch.full((4,), 7, dtype=torch.int32, device="cuda")
@@ -395,7 +334,7 @@ def test_refusals_enqueue_nothing():
     with pytest.raises(_lib.AgarclError, match="int32"):
         b.bot_actions(torch.zeros(4, dtype=torch.int64, device="cuda"))
     with pytest.raises(_lib.AgarclError, match="4 entries"):
-        b.bot_actions(_i32([0, 1, 2]))
+        b.bot_actions(i32([0, 1, 2]))
     with pytest.raises(_lib.AgarclError, match="act"):
         b.bot_actions(0, out=(dxdy[:4], act[:3], status))
     assert untouched()
@@ -419,13 +358,13 @@ def test_python_layers():
         dxdy, act, status = env.bot_actions(BOT_HUNGRY)
         assert dxdy.shape == (8, 2) and dxdy.dtype == torch.float32 and act.dtype == torch.int32 and status.dtype == torch.uint8
         obs, rew, done, trunc, info = env.step(dxdy, act)
-    ref = b.bot_actions(_i32([BOT_HUNGRY] * 8))
+    ref = b.bot_actions(i32([BOT_HUNGRY] * 8))
     got = env.bot_actions(BOT_HUNGRY)
     for x, y in zip(ref, got):
         assert torch.equal(x, y)
     buf = (torch.zeros((8, 2), device="cuda"), torch.zeros(8, dtype=torch.int32, device="cuda"),
            torch.zeros(8, dtype=torch.uint8, device="cuda"))
-    out = env.bot_actions(_i32([BOT_AGGRESSIVE, -1] * 4), out=buf)
+    out = env.bot_actions(i32([BOT_AGGRESSIVE, -1] * 4), out=buf)
     assert all(x is y for x, y in zip(out, buf))
     assert (buf[2][1::2] == BOT_SKIPPED).all() and (buf[0][1::2] == 0).all() and (buf[2][0::2] != BOT_SKIPPED).all()
     torch.cuda.synchronize()

@@ -6,63 +6,18 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from agarcl_b200 import OBS_I16, RNG_MT19937, make_cfg
-from agarcl_b200._abi import task_bits
-from test_draw_oracle import AGENT, ARENA, RGB, oracle_draw
+from _helpers import AGENT, ARENA, RGB, oracle_draw
+from agarcl_b200 import make_cfg
+from gpu_parity_lib import aged_batch, device_record, i32, step_random
 
-_BASE = dict(num_agents=1, num_bots=25, num_viruses=25, num_pellets=1000, arena_size=1000)
-# name: (make_cfg keywords, p_feed, p_split, boost)
-CASES = {
-    "c1": (dict(num_viruses=0, num_bots=0), 1 / 3, 1 / 3, None),
-    "c2": (dict(), 1 / 3, 1 / 3, None),
-    "c3": (dict(num_bots=8, num_viruses=10), 0.0, 0.0, None),
-    "c4_split_merge": (dict(num_agents=4, num_bots=8, cap_foods=2048), 0.3, 0.3, 1000),
-    "c5": (dict(arena_size=2000, num_pellets=4000, num_viruses=50, cap_viruses=128), 1 / 3, 1 / 3, None),
-    "mode1_squared_pellets": (dict(mode_number=1, num_bots=0), 1 / 3, 1 / 3, None),
-    "mode8_one_bot": (dict(mode_number=8), 1 / 3, 1 / 3, None),
-    "mixed_tasks": (dict(mode_number=1, task_modes=task_bits([1, 7, 8]), num_bots=0, arena_size=400, num_pellets=400), 1 / 3, 1 / 3, None),
-    "int16": (dict(obs_dtype=OBS_I16, num_bots=4, arena_size=300, num_pellets=300, num_viruses=4), 1 / 3, 1 / 3, None),
-    "ram_obs2": (dict(ram_obs=2, num_bots=4, arena_size=300, num_pellets=300, num_viruses=4), 1 / 3, 1 / 3, None),
-    "strict_reference": (dict(strict_reference=1, num_bots=4, arena_size=300, num_pellets=300, num_viruses=4), 1 / 3, 1 / 3, None),
-    "mt19937": (dict(rng_mode=RNG_MT19937, num_bots=4, arena_size=300, num_pellets=300, num_viruses=4), 1 / 3, 1 / 3, None),
-}
-
-
-def _i32(x):
-    import torch
-    return torch.as_tensor(np.asarray(x, np.int32), device="cuda")
-
-
-def _batch(name, N=4, seed=5):
-    from agarcl_b200.batch import Batch
-    import torch
-    kw, p_feed, p_split, boost = CASES[name]
-    b = Batch(make_cfg(n_instances=N, **dict(_BASE, **kw)))
-    b.seed(seed)
-    if b.cfg.task_modes:
-        b.set_tasks(_i32([1, 7, 8, 7][:N] + [1] * max(0, N - 4)))
-    b.reset()
-    if boost:
-        for i in range(N):
-            sv = b.download_state(i)
-            for a in range(b.A):
-                sv.cells[a][0]["mass"] = boost
-            b.upload_state(i, sv)
-    torch.cuda.synchronize()
-    return b, np.random.default_rng(seed), p_feed, p_split
-
-
-def _step(b, rng, p_feed, p_split, k):
-    from _helpers import random_actions
-    for _ in range(k):
-        b.set_actions(*random_actions(rng, b.N * b.A, p_feed, p_split))
-        b.step()
+CASES = ["c1", "c2", "c3", "c4_four_agents", "c5", "mode1", "mode8", "mixed_tasks", "int16", "ram_obs2", "strict_reference",
+         "mt19937"]
 
 
 def _check(b, view, size, src=None):
     """device pictures of src (None: every source) against oracle_draw on the downloaded blobs"""
     import torch
-    pics = b.draw(None if src is None else _i32(src), size, "agent" if view == AGENT else "arena")
+    pics = b.draw(None if src is None else i32(src), size, "agent" if view == AGENT else "arena")
     torch.cuda.synchronize()
     pics = pics.cpu().numpy()
     n_src = b.N * (b.A if view == AGENT else 1)
@@ -83,21 +38,21 @@ def _check(b, view, size, src=None):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", list(CASES))
+@pytest.mark.parametrize("name", CASES)
 def test_pictures_match_oracle(name):
     """both views at 16 and 128 for every source at ages 0, 1 and 250; 512 and 2048 on a few pictures of the aged state"""
-    b, rng, p_feed, p_split = _batch(name)
+    b, rng, p_feed, p_split = aged_batch(name)
     for age, more in ((0, 0), (1, 1), (250, 249)):
-        _step(b, rng, p_feed, p_split, more)
+        step_random(b, rng, p_feed, p_split, more)
         for view in (ARENA, AGENT):
             for size in (16, 128):
                 _check(b, view, size)
     _check(b, ARENA, 512, [0, 3])
     _check(b, AGENT, 512, [b.N * b.A - 1])
-    if name in ("c2", "c4_split_merge"):
+    if name in ("c2", "c4_four_agents"):
         _check(b, ARENA, 2048, [1])
         _check(b, AGENT, 2048, [0])
-    if name == "c4_split_merge":  # the agents did split
+    if name == "c4_four_agents":  # the agents did split
         assert max(int(b.download_state(i).players["n_cells"][:b.A].max()) for i in range(b.N)) > 1
     b.close()
 
@@ -141,13 +96,13 @@ def test_crafted_maximal_state():
 def test_source_indexing():
     """d_src NULL draws every source in order; duplicates repeat a picture; out-of-range entries give zeros"""
     import torch
-    b, rng, pf, ps = _batch("c4_split_merge", N=3)
-    _step(b, rng, pf, ps, 20)
+    b, rng, pf, ps = aged_batch("c4_four_agents", N=3)
+    step_random(b, rng, pf, ps, 20)
     for view, n_src in (("arena", b.N), ("agent", b.N * b.A)):
         every = b.draw(None, 64, view)
         assert every.shape == (n_src, 64, 64, 3)
         src = [2, 2, -1, n_src, 0, n_src - 1, -(1 << 31), (1 << 31) - 1]
-        some = b.draw(_i32(src), 64, view)
+        some = b.draw(i32(src), 64, view)
         torch.cuda.synchronize()
         every, some = every.cpu().numpy(), some.cpu().numpy()
         for k, s in enumerate(src):
@@ -159,24 +114,13 @@ def test_source_indexing():
     _check(b, AGENT, 64, [5, -1, 12, 11])
 
 
-def _everything(b):
-    import torch
-    torch.cuda.synchronize()
-    r = {"blobs": np.stack([b.download_state(i).blob for i in range(b.N)]), "obs": b.obs_tensor().cpu().numpy(),
-         "rewards": b.rewards_tensor().cpu().numpy(), "dones": b.dones_tensor().cpu().numpy(), "ram": b.ram_tensor().cpu().numpy()}
-    r.update({k: v.cpu().numpy() for k, v in b.episode().items()})
-    r["final_obs"] = b.final_obs().cpu().numpy()
-    r["mirror"] = b.mirror().copy()
-    return r
-
-
 @pytest.mark.gpu
 def test_drawing_changes_nothing():
-    """state blobs, observation, rewards, dones, ram records, episode buffers and the host mirror are bitwise the same after
-    drawing, and the following steps equal those of a twin batch that never drew"""
+    """state blobs, observation, rewards, dones, ram records, episode buffers, final observations and ram records and the host
+    mirror are bitwise the same after drawing, and the following steps equal those of a twin batch that never drew"""
     import torch
     from agarcl_b200.batch import Batch
-    cfg = make_cfg(n_instances=8, ram_obs=1, **dict(_BASE, num_bots=6, arena_size=300, num_pellets=300, num_viruses=4))
+    cfg = make_cfg(n_instances=8, ram_obs=1, num_bots=6, arena_size=300, num_pellets=300, num_viruses=4)
     twins = [Batch(cfg), Batch(cfg)]
     for b in twins:
         b.seed(42)
@@ -192,15 +136,15 @@ def test_drawing_changes_nothing():
             b.step_autoreset()
             b.sync_mirror()
         if t % 10 == 3:
-            before = _everything(twins[0])
+            before = device_record(twins[0])
             for view in ("arena", "agent"):
                 for size in (16, 144, 512):
                     twins[0].draw(None, size, view)
-            twins[0].draw(_i32([0, -5, 99]), 32, "arena")
-            after = _everything(twins[0])
+            twins[0].draw(i32([0, -5, 99]), 32, "arena")
+            after = device_record(twins[0])
             for k in before:
                 assert np.array_equal(before[k], after[k]), f"step {t}: draw changed {k}"
-        a, c = _everything(twins[0]), _everything(twins[1])
+        a, c = device_record(twins[0]), device_record(twins[1])
         for k in a:
             assert np.array_equal(a[k], c[k]), f"step {t}: {k} differs from the twin that never drew"
     torch.cuda.synchronize()
@@ -211,9 +155,9 @@ def test_no_host_wait_graph_capture_and_interleaved_steps():
     """after one warm-up the call is captured in a CUDA graph (capture fails on any synchronising call) and the replay gives
     the same bytes; interleaved with step_autoreset on one stream, every step gets its own picture"""
     import torch
-    b, rng, pf, ps = _batch("c2", N=4)
-    _step(b, rng, pf, ps, 30)
-    src = _i32([3, 1, 0])
+    b, rng, pf, ps = aged_batch("c2", N=4)
+    step_random(b, rng, pf, ps, 30)
+    src = i32([3, 1, 0])
     s = torch.cuda.Stream()
     out = torch.zeros((3, 128, 128, 3), dtype=torch.uint8, device="cuda")
     torch.cuda.synchronize()
@@ -253,7 +197,7 @@ def test_refusals_leave_the_output_untouched():
     from agarcl_b200.batch import Batch
     L = _lib.lib()
     vp = C.c_void_p
-    cfg = make_cfg(n_instances=2, **dict(_BASE, num_bots=2, arena_size=200, num_pellets=100, num_viruses=2))
+    cfg = make_cfg(n_instances=2, num_bots=2, arena_size=200, num_pellets=100, num_viruses=2)
     fresh = Batch(cfg)
     out = torch.full((2, 64, 64, 3), 0xAB, dtype=torch.uint8, device="cuda")
 
@@ -312,10 +256,10 @@ def test_python_layers():
     assert torch.equal(pics, b.draw(None, 256, "arena"))
     ids = torch.tensor([2, 0], dtype=torch.int64, device="cuda")
     agents = env.render(ids, size=96, view="agent")
-    assert torch.equal(agents, b.draw(_i32([4, 5, 0, 1]), 96, "agent"))
+    assert torch.equal(agents, b.draw(i32([4, 5, 0, 1]), 96, "agent"))
     buf = torch.empty((2, 64, 64, 3), dtype=torch.uint8, device="cuda")
     assert env.render(ids, size=64, out=buf).data_ptr() == buf.data_ptr()
-    assert torch.equal(buf, b.draw(_i32([2, 0]), 64))
+    assert torch.equal(buf, b.draw(i32([2, 0]), 64))
     env.close()
 
     e = AgarioEnv(render_mode="rgb_array", render_size=128)

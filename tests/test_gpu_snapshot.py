@@ -9,40 +9,26 @@ import numpy as np
 import pytest
 
 from agarcl_b200 import OBS_I16, RNG_MT19937, RNG_PHILOX, RNG_REPLAY, make_cfg
-from test_gpu_autoreset import CASES
+from gpu_parity_lib import CASES, SMALL, assert_no_host_wait, device_record, i32
 
-RT_CASES = {k: v for k, v in CASES.items() if k not in ("strict_reference", "mt19937_ring_wraps")}
-SMALL = dict(num_bots=4, arena_size=300, num_pellets=300, num_viruses=4)
-
-
-def _i32(x):
-    import torch
-    return torch.as_tensor(np.asarray(x, np.int32), device="cuda")
+RT_CASES = ["mode9_deaths_and_limit", "configs1_two_agents", "int16", "two_frames", "ram_obs1", "ram_obs2"]
 
 
 def _blobs(b):
     return np.stack([b.download_state(i).blob for i in range(b.N)])
 
 
-def _record(b, episode=False):
-    """everything an instance carries after a step, on the host (episode: and the buffers of the episode bookkeeping)"""
-    import torch
-    torch.cuda.synchronize()
-    r = {"blobs": _blobs(b), "rewards": b.rewards_tensor().cpu().numpy(), "dones": b.dones_tensor().cpu().numpy()}
-    if b.cfg.ram_obs != 2:
-        r["obs"] = b.obs_tensor().cpu().numpy()
-    if b.cfg.ram_obs:
-        r["ram"] = b.ram_tensor().cpu().numpy()
-    if episode:
-        e = b.episode()
-        r.update({k: v.cpu().numpy() for k, v in e.items()})
-        mask = r["reset_mask"].astype(bool)
-        r["episode_return"] = r["episode_return"].reshape(b.N, b.A)[mask]
-        r["episode_length"] = r["episode_length"][mask]
-        if b.cfg.ram_obs != 2:
-            r["final_obs"] = b.final_obs().cpu().numpy().reshape(b.N, -1)[mask]
-        if b.cfg.ram_obs:
-            r["final_ram"] = b.final_ram().cpu().numpy()[mask]
+def _record(b):
+    """device_record with the episode results of the instances the last step reset only (the others hold an earlier
+    episode's, which a restore does not bring back)"""
+    r = device_record(b)
+    mask = r["reset_mask"].astype(bool)
+    r["episode_return"] = r["episode_return"].reshape(b.N, b.A)[mask]
+    r["episode_length"] = r["episode_length"][mask]
+    if "final_obs" in r:
+        r["final_obs"] = r["final_obs"].reshape(b.N, -1)[mask]
+    if "final_ram" in r:
+        r["final_ram"] = r["final_ram"][mask]
     return r
 
 
@@ -62,12 +48,12 @@ def _actions(rng, n):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", list(RT_CASES))
+@pytest.mark.parametrize("name", RT_CASES)
 def test_round_trip(name):
     """step T, save all, step K recording everything, restore all, step the same K actions: bit-identical at every step"""
     from agarcl_b200.batch import Batch
     N, T, K = 16, 20, 40
-    cfg = make_cfg(n_instances=N, **RT_CASES[name])
+    cfg = make_cfg(n_instances=N, **CASES[name][0])
     b = Batch(cfg)
     b.seed(99)
     b.reset()
@@ -78,25 +64,25 @@ def test_round_trip(name):
         b.set_actions(*acts[t])
         b.step_autoreset()
     pool = b.snapshot_pool(N)
-    idx = _i32(np.arange(N))
+    idx = i32(np.arange(N))
     b.save_states(pool, idx)
-    at_save = _record(b, episode=True)
+    at_save = _record(b)
     first, resets = [], 0
     for t in range(T, T + K):
         b.set_actions(*acts[t])
         b.step_autoreset()
-        first.append(_record(b, episode=True))
+        first.append(_record(b))
         resets += int(first[-1]["reset_mask"].sum())
     assert resets > 0, "no episode ended inside the window"
     res = b.restore_states(pool, idx)
-    after = _record(b, episode=True)
+    after = _record(b)
     assert after is not None and (res.cpu().numpy() == 1).all()
     _assert_equal(at_save, after, "after restore", keys=[k for k in ("blobs", "obs", "ram", "steps") if k in after])
     assert not after["rewards"].any() and not after["dones"].any()  # zeroed, like after a reset
     for t in range(T, T + K):
         b.set_actions(*acts[t])
         b.step_autoreset()
-        _assert_equal(first[t - T], _record(b, episode=True), f"{name} step {t}")
+        _assert_equal(first[t - T], _record(b), f"{name} step {t}")
     b.close()
 
 
@@ -123,11 +109,11 @@ def test_fork_against_oracle():
         b.set_actions(*_actions(rng, N * A))
         b.step()
     pool = b.snapshot_pool(2)
-    b.save_states(pool, _i32([j]), _i32([1]))
+    b.save_states(pool, i32([j]), i32([1]))
     torch.cuda.synchronize()
     src_blob = b.download_state(j).blob.copy()
     src_obs = b.obs_tensor()[j * A:(j + 1) * A].clone()
-    res = b.restore_states(pool, _i32([1, -1, 1, 1]))
+    res = b.restore_states(pool, i32([1, -1, 1, 1]))
     torch.cuda.synchronize()
     assert res.tolist() == [1, 0, 1, 1]
     obs = b.obs_tensor()
@@ -186,13 +172,13 @@ def test_partial_restore_leaves_the_others_untouched(kw):
             x.set_actions(*acts)
             x.step_autoreset()
         if t == 10:
-            a.save_states(pool, _i32(np.arange(N)))
+            a.save_states(pool, i32(np.arange(N)))
     slot_of = np.full(N, -1, np.int32)
     slot_of[[0, 5, 6, 17]] = [3, 5, 5, 20]
-    res = a.restore_states(pool, _i32(slot_of)).cpu().numpy()
+    res = a.restore_states(pool, i32(slot_of)).cpu().numpy()
     assert np.array_equal(res, np.where(slot_of >= 0, 1, 0))
     keep = slot_of < 0
-    ra, rb = _record(a, episode=True), _record(b, episode=True)
+    ra, rb = _record(a), _record(b)
     _assert_equal(ra, rb, "at the restore", keys=[k for k in ("blobs", "obs", "ram", "rewards", "dones", "steps") if k in ra], rows=keep)
     # the restored instances hold the slots' blobs (slot layout: the blob at byte 64)
     S = a.layout.stride
@@ -205,7 +191,7 @@ def test_partial_restore_leaves_the_others_untouched(kw):
         for x in (a, b):
             x.set_actions(*acts)
             x.step_autoreset()
-        ra, rb = _record(a, episode=True), _record(b, episode=True)
+        ra, rb = _record(a), _record(b)
         _assert_equal(ra, rb, f"step {t} after the restore", keys=[k for k in ("blobs", "obs", "ram", "rewards", "dones", "steps") if k in ra],
                       rows=keep)
     a.close()
@@ -233,7 +219,7 @@ def test_rejections_and_acceptance():
         o.seed(1)
         o.reset()
         op = o.snapshot_pool(1)
-        o.save_states(op, _i32([1]))
+        o.save_states(op, i32([1]))
         torch.cuda.synchronize()
         w = min(sb, o.slot_bytes)
         pool[k, :w] = op[0, :w]
@@ -241,15 +227,15 @@ def test_rejections_and_acceptance():
             assert o.slot_bytes == sb  # only the fingerprint tells them apart
         o.close()
     assert grid_kw["grid_size"] != cfg.grid_size
-    b.save_states(pool, _i32([0, N + 3]), _i32([3, 4]))  # slot 4: a source out of range
+    b.save_states(pool, i32([0, N + 3]), i32([3, 4]))  # slot 4: a source out of range
     snapshot = pool.clone()
-    b.save_states(pool, _i32([2]), _i32([99]))  # a slot out of range is skipped
+    b.save_states(pool, i32([2]), i32([99]))  # a slot out of range is skipped
     torch.cuda.synchronize()
     assert torch.equal(pool, snapshot)
     assert int(pool[4, :4].view(torch.int32).item()) == 0  # magic 0
     before, obs0, ram0 = _blobs(b), b.obs_tensor().clone(), b.ram_tensor().clone()
     slot_of = np.array([0, 1, 2, 6, 4, -1, 3, -7], np.int32)
-    res = b.restore_states(pool, _i32(slot_of)).cpu().numpy()
+    res = b.restore_states(pool, i32(slot_of)).cpu().numpy()
     assert res.tolist() == [2, 2, 2, 2, 2, 0, 1, 0]
     after = _blobs(b)
     untouched = res != 1
@@ -263,7 +249,7 @@ def test_rejections_and_acceptance():
     c = Batch(make_cfg(n_instances=5, instance_base=100, ram_obs=1, **SMALL))
     c.seed(8)
     c.reset()
-    res = c.restore_states(pool, _i32([3, -1, -1, 0, 3])).cpu().numpy()
+    res = c.restore_states(pool, i32([3, -1, -1, 0, 3])).cpu().numpy()
     assert res.tolist() == [1, 0, 0, 2, 1]
     cb = _blobs(c)
     assert np.array_equal(cb[0], before[0]) and np.array_equal(cb[4], before[0])
@@ -280,7 +266,7 @@ def test_refusals_before_anything_is_enqueued():
     N = 4
     b = Batch(make_cfg(n_instances=N, **SMALL))
     pool = b.snapshot_pool(N)
-    idx = _i32(np.arange(N))
+    idx = i32(np.arange(N))
     with pytest.raises(AgarclError, match="before reset"):
         b.restore_states(pool, idx)
     with pytest.raises(AgarclError, match="before reset"):
@@ -309,7 +295,7 @@ def test_refusals_before_anything_is_enqueued():
     with pytest.raises(AgarclError, match="int32"):
         b.restore_states(pool, idx.long())
     with pytest.raises(AgarclError, match="4 entries"):
-        b.restore_states(pool, _i32(np.arange(N + 1)))
+        b.restore_states(pool, i32(np.arange(N + 1)))
     with pytest.raises(AgarclError, match=str(sb)):
         b.restore_states(pool[:, :sb - 128].contiguous(), idx)
     # the C ABI itself: host memory, pool_slots < 1, n < 0, null index arrays
@@ -353,19 +339,17 @@ def test_save_and_restore_do_not_wait_for_the_device():
     env.seed(1)
     env.reset()
     pool = env.snapshot_pool(N)
-    idx = _i32(np.arange(N))
+    idx = i32(np.arange(N))
     s = torch.cuda.Stream()
     for _ in range(2):  # every kernel on the path is loaded before the timed calls
         env.save_states(pool, idx, stream=s.cuda_stream)
         env.restore_states(pool, idx, stream=s.cuda_stream)
-    torch.cuda.synchronize()
-    with torch.cuda.stream(s):
-        torch.cuda._sleep(200_000_000)  # ~0.1 s at the B200's clock
-    env.save_states(pool, idx, stream=s.cuda_stream)
-    env.restore_states(pool, idx, stream=s.cuda_stream)
-    busy = not s.query()
-    s.synchronize()
-    assert busy, "a call waited for the device"
+
+    def calls():
+        env.save_states(pool, idx, stream=s.cuda_stream)
+        env.restore_states(pool, idx, stream=s.cuda_stream)
+
+    assert_no_host_wait(calls, s)
     env.close()
 
 
@@ -389,7 +373,7 @@ def test_pool_survives_torch_save_and_load():
     cfg = make_cfg(n_instances=N, num_frames=2, ram_obs=1, **SMALL)
     b = _stepped(cfg, 8)
     pool = b.snapshot_pool(N)
-    b.save_states(pool, _i32(np.arange(N)))
+    b.save_states(pool, i32(np.arange(N)))
     buf = io.BytesIO()
     torch.save(pool.cpu(), buf)
     buf.seek(0)
@@ -397,7 +381,7 @@ def test_pool_survives_torch_save_and_load():
     c = Batch(cfg)
     c.seed(77)
     c.reset()
-    res = c.restore_states(loaded, _i32(np.arange(N)[::-1].copy()))
+    res = c.restore_states(loaded, i32(np.arange(N)[::-1].copy()))
     assert (res.cpu().numpy() == 1).all()
     assert np.array_equal(_blobs(c), _blobs(b)[::-1])
     A = b.A
@@ -416,7 +400,7 @@ def test_pool_moved_to_another_device():
     N = 4
     b = _stepped(make_cfg(n_instances=N, **SMALL), 6)
     pool = b.snapshot_pool(N)
-    b.save_states(pool, _i32(np.arange(N)))
+    b.save_states(pool, i32(np.arange(N)))
     c = Batch(make_cfg(n_instances=N, device=1, **SMALL))
     c.seed(1)
     c.reset()
@@ -441,8 +425,8 @@ def test_mirror_after_restore():
     for t in range(12):
         b.step_mirror(*_actions(rng, N))
         if t == 4:
-            b.save_states(pool, _i32(np.arange(N)))
-    b.restore_states(pool, _i32([0, -1, 2, 2, -1, 5, 6, 0]))
+            b.save_states(pool, i32(np.arange(N)))
+    b.restore_states(pool, i32([0, -1, 2, 2, -1, 5, 6, 0]))
     m = b.sync_mirror()
     assert np.array_equal(m, b.obs_tensor().cpu().numpy())
     for _ in range(3):
@@ -468,11 +452,11 @@ def test_vector_env_restore():
         obs, _, _, _, info = env.step(*zeros())
     assert bool((info["steps"] == s).all())
     pool = env.snapshot_pool(N)
-    env.save_states(pool, _i32(np.arange(N)))
+    env.save_states(pool, i32(np.arange(N)))
     saved = obs.clone()
     for _ in range(5):
         env.step(*zeros())
-    obs = env.restore_states(pool, _i32(np.arange(N)))
+    obs = env.restore_states(pool, i32(np.arange(N)))
     assert torch.equal(obs, saved)
     assert (env.restore_result().cpu().numpy() == 1).all()
     assert bool((env._env.episode()["steps"] == s).all())
@@ -485,9 +469,9 @@ def test_vector_env_restore():
     env.close()
 
 
-LAUNCH_CASES = {"configs1": (dict(), ["k_obs", "k_snapshot"]), "int16": (RT_CASES["int16"], ["k_obs", "k_snapshot"]),
-                "two_frames": (RT_CASES["two_frames"], ["k_snapshot"]), "ram_obs1": (RT_CASES["ram_obs1"], ["k_obs", "k_snapshot"]),
-                "ram_obs2": (RT_CASES["ram_obs2"], ["k_snapshot"])}
+LAUNCH_CASES = {"configs1": (dict(), ["k_obs", "k_snapshot"]), "int16": (CASES["int16"][0], ["k_obs", "k_snapshot"]),
+                "two_frames": (CASES["two_frames"][0], ["k_snapshot"]), "ram_obs1": (CASES["ram_obs1"][0], ["k_obs", "k_snapshot"]),
+                "ram_obs2": (CASES["ram_obs2"][0], ["k_snapshot"])}
 
 
 @pytest.mark.gpu
@@ -500,7 +484,7 @@ def test_launches_of_a_restore(name):
     N = 8
     b = _stepped(make_cfg(n_instances=N, **kw), 2)
     pool = b.snapshot_pool(N)
-    idx = _i32(np.arange(N))
+    idx = i32(np.arange(N))
     torch.cuda.synchronize()
 
     def kernels(fn):

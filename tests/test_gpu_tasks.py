@@ -6,16 +6,12 @@ import pytest
 
 from agarcl_b200 import RNG_MT19937, RNG_REPLAY, make_cfg
 from agarcl_b200._abi import StateView, compare_states, task_bits
+from gpu_parity_lib import assert_no_host_wait, i32
 
 MODES = list(range(1, 11))
 # the ten AgarCL mini-games (bench/tasks_configs): arena 350, 500 pellets, no viruses, one bot in modes 7..10
 MINI = dict(arena_size=350, num_pellets=500, num_viruses=0, num_bots=0, grid_size=64)
 SEEDS_BASE, BASE = 500, 300
-
-
-def _i32(x):
-    import torch
-    return torch.as_tensor(np.asarray(x, np.int32), device="cuda")
 
 
 def mode_of(i):
@@ -52,7 +48,7 @@ def make_mixed(N, modes=None, limits=None, **kw):
     from agarcl_b200.batch import Batch
     b = Batch(make_cfg(n_instances=N, mode_number=1, task_modes=task_bits(MODES), instance_base=BASE, **dict(MINI, **kw)))
     b.seed(np.arange(N, dtype=np.uint64) + SEEDS_BASE)
-    res = b.set_tasks(_i32(modes if modes is not None else [mode_of(i) for i in range(N)]), _i32(limits) if limits is not None else None)
+    res = b.set_tasks(i32(modes if modes is not None else [mode_of(i) for i in range(N)]), i32(limits) if limits is not None else None)
     assert (res.cpu().numpy() == 1).all()
     return b
 
@@ -206,7 +202,7 @@ def test_a_new_task_starts_at_the_next_reset():
         b.reset()
     switch = {0: 8, 3: 2, 7: 5}  # instance: new mode
     new = [switch.get(i, -1) for i in range(N)]
-    res = a.set_tasks(_i32(new), _i32([25 if i in switch else -1 for i in range(N)]))
+    res = a.set_tasks(i32(new), i32([25 if i in switch else -1 for i in range(N)]))
     assert res.cpu().numpy().tolist() == [1] * N  # (a limit of -1 is a value too: every entry was set)
     t = a.tasks()
     assert t["mode"].cpu().numpy().tolist() == [mode_of(i) for i in range(N)]
@@ -253,13 +249,13 @@ def test_vector_env_tasks_and_episode_lengths():
     env.seed(3)
     modes = [(1, 2, 4, 6)[i % 4] for i in range(N)]
     lim = [(30, 45, 0, -1)[i % 4] if i < 8 else 20 for i in range(N)]
-    assert (env.set_tasks(_i32(modes), _i32(lim)).cpu().numpy() == 1).all()
+    assert (env.set_tasks(i32(modes), i32(lim)).cpu().numpy() == 1).all()
     env.reset()
     g = torch.Generator(device="cuda").manual_seed(0)
     seen_len = {i: set() for i in range(N)}
     for t in range(100):
         if t == 50:  # instances 8.. switch to mode 2 at their next truncation
-            assert (env.set_tasks(_i32([-1] * 8 + [2] * (N - 8))).cpu().numpy() == [0] * 8 + [1] * (N - 8)).all()
+            assert (env.set_tasks(i32([-1] * 8 + [2] * (N - 8))).cpu().numpy() == [0] * 8 + [1] * (N - 8)).all()
         _, _, done, _, info = env.step((torch.rand((N, 2), device="cuda", generator=g) * 2 - 1), torch.zeros(N, dtype=torch.int32, device="cuda"))
         m = info["reset_mask"].cpu().numpy()
         L = info["episode_length"].cpu().numpy()
@@ -284,7 +280,7 @@ def test_rejections_and_refusals():
     b = make_mixed(N, modes=[1] * N)
     b.reset()
     before = {k: v.clone() for k, v in b.tasks().items()}
-    res = b.set_tasks(_i32([11, 0, -1, 3, -1, -2]), _i32([10, 10, -2, -1, -1, 5]))
+    res = b.set_tasks(i32([11, 0, -1, 3, -1, -2]), i32([10, 10, -2, -1, -1, 5]))
     torch.cuda.synchronize()
     # mode 11 / mode 0 (not in the set) / limit -2 / fine / limit only / mode -2
     assert res.cpu().numpy().tolist() == [2, 2, 2, 1, 1, 2]
@@ -292,13 +288,13 @@ def test_rejections_and_refusals():
     assert t["next_mode"].cpu().numpy().tolist() == [1, 1, 1, 3, 1, 1]
     assert t["next_max_steps"].cpu().numpy().tolist() == [-1, -1, -1, -1, -1, -1]
     assert torch.equal(t["mode"], before["mode"]) and torch.equal(t["max_steps"], before["max_steps"])
-    assert b.set_tasks(_i32([-1] * N)).cpu().numpy().tolist() == [0] * N
+    assert b.set_tasks(i32([-1] * N)).cpu().numpy().tolist() == [0] * N
     with pytest.raises(AgarclError, match="mode"):
-        b.set_tasks(_i32([1] * (N - 1)))
+        b.set_tasks(i32([1] * (N - 1)))
     b.close()
     plain = Batch(make_cfg(n_instances=2, mode_number=1, **MINI))
     with pytest.raises(AgarclError, match="without task_modes"):
-        plain.set_tasks(_i32([1, 1]))
+        plain.set_tasks(i32([1, 1]))
     with pytest.raises(AgarclError, match="without task_modes"):
         plain.tasks()
     plain.close()
@@ -319,19 +315,17 @@ def test_set_tasks_and_step_autoreset_do_not_wait_for_the_device():
     b = make_mixed(N)
     b.reset()
     b.set_autoreset(50)
-    modes = _i32([mode_of(i + 1) for i in range(N)])
+    modes = i32([mode_of(i + 1) for i in range(N)])
     s = torch.cuda.Stream()
     for _ in range(2):  # every kernel on the path is loaded before the timed calls
         b.set_tasks(modes, stream=s.cuda_stream)
         b.step_autoreset(stream=s.cuda_stream)
-    torch.cuda.synchronize()
-    with torch.cuda.stream(s):
-        torch.cuda._sleep(200_000_000)  # ~0.1 s at the B200's clock
-    b.set_tasks(modes, stream=s.cuda_stream)
-    b.step_autoreset(stream=s.cuda_stream)
-    busy = not s.query()
-    s.synchronize()
-    assert busy, "a call waited for the device"
+
+    def calls():
+        b.set_tasks(modes, stream=s.cuda_stream)
+        b.step_autoreset(stream=s.cuda_stream)
+
+    assert_no_host_wait(calls, s)
     b.close()
 
 
@@ -354,8 +348,8 @@ def test_snapshots_carry_the_task(tmp_path):
             b.set_actions(*acts)
             b.step()
     pool = src.snapshot_pool(1)
-    src.save_states(pool, _i32([j]))
-    res = dst.restore_states(pool, _i32([0 if i == j else -1 for i in range(N)]))
+    src.save_states(pool, i32([j]))
+    res = dst.restore_states(pool, i32([0 if i == j else -1 for i in range(N)]))
     torch.cuda.synchronize()
     assert res.cpu().numpy().tolist() == [1 if i == j else 0 for i in range(N)]
     t = dst.tasks()
@@ -378,9 +372,9 @@ def test_snapshots_carry_the_task(tmp_path):
         b.reset()
     for a, b in ((mixed78, plain7), (plain7, mixed78)):
         p = a.snapshot_pool(1)
-        a.save_states(p, _i32([0]))
-        assert b.restore_states(p, _i32([0, -1])).cpu().numpy().tolist() == [2, 0]
-        assert a.restore_states(p, _i32([-1, 0])).cpu().numpy().tolist() == [0, 1]
+        a.save_states(p, i32([0]))
+        assert b.restore_states(p, i32([0, -1])).cpu().numpy().tolist() == [2, 0]
+        assert a.restore_states(p, i32([-1, 0])).cpu().numpy().tolist() == [0, 1]
     # JSON: the instance's current mode travels as mode_number and comes back as the loading instance's current task
     path = tmp_path / "mode8.json"
     src.save_env_state(j, path)

@@ -15,31 +15,19 @@ bench/tasks_configs (arena 350, 500 pellets, one bot) at 4096 instances; both ep
 import argparse
 import json
 import os
-import statistics
-import subprocess
 import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
+from exp_common import gpu_info, stats  # noqa: E402
+
 WORKLOADS = {
     "configs1": dict(n_instances=4096),
     "mode8": dict(n_instances=4096, mode_number=8, num_bots=1, arena_size=350, num_pellets=500, num_viruses=0),
 }
 MAX_STEPS = 500
-
-
-def gpu_info():
-    import torch
-    info = {"gpu": torch.cuda.get_device_name(0)}
-    try:
-        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"],
-                           capture_output=True, text=True, timeout=30).stdout.strip()
-        info["power_limit"], info["max_sm_clock"] = [x.strip() for x in q.split(",")]
-    except Exception as e:  # the timing stands without it; say so
-        info["power_limit"] = f"not read: {e}"
-    return info
 
 
 class Arm:
@@ -78,10 +66,6 @@ class Arm:
                 self.steps[mask] = 0
                 if count:
                     self.resets += int(mask.sum())
-
-
-def _stats(xs):
-    return {"median": statistics.median(xs), "min": min(xs), "max": max(xs)}
 
 
 def _timed(arms, acts, first, repeats, steps):
@@ -139,8 +123,8 @@ def main():
             diff = [(x - y) * 1e3 for x, y in zip(d, dev_ms["step"])]
             print(json.dumps({"workload": wl, "window": "no_resets", "arm": arm.name, "instances": N, "steps": [args.warmup, quiet_end],
                               "instances_reset": arm.resets if arm.name == "host_composition" else None,
-                              "event_ms_per_step": _stats(d), "host_ms_per_step": _stats(h),
-                              "event_us_over_step_same_repeat": _stats(diff), **info}), flush=True)
+                              "event_ms_per_step": stats(d), "host_ms_per_step": stats(h),
+                              "event_us_over_step_same_repeat": stats(diff), **info}), flush=True)
         # 2. a window that contains the step on which every instance reaches number_steps (both resetting arms; bare `step`
         #    would go on with older games from there, so it is left out)
         arms[1].resets = 0
@@ -154,7 +138,7 @@ def main():
         for arm in res:
             print(json.dumps({"workload": wl, "window": "limit_reached", "arm": arm.name, "instances": N,
                               "steps": [MAX_STEPS - 20, MAX_STEPS + 60], "instances_reset": res[0].resets,
-                              "event_ms_per_step": _stats(dev_ms[arm.name]), "host_ms_per_step": _stats(host_ms[arm.name]),
+                              "event_ms_per_step": stats(dev_ms[arm.name]), "host_ms_per_step": stats(host_ms[arm.name]),
                               "outputs_equal_to_host_composition": same, **info}), flush=True)
         if args.profile:
             from torch.profiler import ProfilerActivity, profile

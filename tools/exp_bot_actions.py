@@ -12,14 +12,13 @@ Each repeat times `--calls` back-to-back calls of every arm with device events, 
 repeat.  One JSON line per arm: ms per call (median / min / max over the repeats), with the GPU's name and power limit read in
 the same run."""
 import argparse
-import json
 import os
-import statistics
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tools"))
+
+from exp_common import aged_configs1, gpu_info, stats, time_arms, write_lines  # noqa: E402
 
 
 def main():
@@ -33,25 +32,9 @@ def main():
     import torch
     if not torch.cuda.is_available():
         sys.exit("exp_bot_actions.py measures on a GPU; none is visible")
-    from exp_snapshot import gpu_info
-    from agarcl_b200 import BOT_TYPES, make_cfg
-    from agarcl_b200.batch import Batch
+    from agarcl_b200 import BOT_TYPES
     N = a.instances
-    b = Batch(make_cfg(n_instances=N))
-    b.seed(2024)
-    b.reset()
-    g = torch.Generator(device="cuda").manual_seed(1)
-    dxdy = torch.empty((N, 2), device="cuda")
-    act = torch.zeros(N, dtype=torch.int32, device="cuda")
-
-    def step():
-        dxdy.uniform_(-1, 1, generator=g)
-        act.random_(0, 3, generator=g)
-        b.set_actions_device(dxdy.data_ptr(), act.data_ptr())
-        b.step()
-
-    for _ in range(a.age):
-        step()
+    b, step, _ = aged_configs1(N, a.age)
     NA = N * b.A
     out = (torch.empty((NA, 2), device="cuda"), torch.empty(NA, dtype=torch.int32, device="cuda"),
            torch.empty(NA, dtype=torch.uint8, device="cuda"))
@@ -67,37 +50,18 @@ def main():
                 b.bot_actions(t, out=out)
         arms[name + "_graph"] = graph.replay
     arms["step"] = step
-    ev = lambda: torch.cuda.Event(enable_timing=True)  # noqa: E731
-    times = {k: [] for k in arms}
-    for f in arms.values():  # warm-up of every arm
-        f()
-    torch.cuda.synchronize()
-    for _ in range(a.repeats):
-        for name, f in arms.items():
-            reps = 1 if name.endswith("_graph") else a.calls
-            e0, e1 = ev(), ev()
-            e0.record()
-            for _ in range(reps):
-                f()
-            e1.record()
-            e1.synchronize()
-            times[name].append(e0.elapsed_time(e1) / a.calls)
-    status = torch.bincount(out[2].long(), minlength=5).tolist()  # (of the last arm's type)
+    times = time_arms(arms, a.calls, a.repeats, graphs=[k for k in arms if k.endswith("_graph")])
+    status = torch.bincount(out[2].long(), minlength=5).tolist()  # (of the type called last)
     info = gpu_info()
     lines = []
     for name, ts in times.items():
-        rec = {"arm": name, "instances": N, "agents": NA, "age": a.age, "ms_median": statistics.median(ts), "ms_min": min(ts),
-               "ms_max": max(ts)}
+        rec = {"arm": name, "instances": N, "agents": NA, "age": a.age, **stats(ts, "ms_")}
         if name != "step":
             rec["players_per_instance"] = b.layout.P
         rec.update(info)
-        lines.append(json.dumps(rec))
-        print(lines[-1], flush=True)
-    lines.append(json.dumps({"last_status_counts": status}))
-    print(lines[-1])
-    if a.out:
-        with open(a.out, "w") as f:
-            f.write("\n".join(lines) + "\n")
+        lines.append(rec)
+    lines.append({"last_status_counts": status})
+    write_lines(lines, a.out)
 
 
 if __name__ == "__main__":

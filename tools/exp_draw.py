@@ -12,14 +12,13 @@ Each repeat times `--calls` back-to-back calls of every arm with device events; 
 line per arm: ms per call (median / min / max over the repeats), bytes written and GB/s, with the GPU's name and power limit
 read in the same run."""
 import argparse
-import json
 import os
-import statistics
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tools"))
+
+from exp_common import aged_configs1, gpu_info, stats, time_arms, write_lines  # noqa: E402
 
 
 def main():
@@ -33,25 +32,8 @@ def main():
     import torch
     if not torch.cuda.is_available():
         sys.exit("exp_draw.py measures on a GPU; none is visible")
-    from exp_snapshot import gpu_info
-    from agarcl_b200 import make_cfg
-    from agarcl_b200.batch import Batch
     N = a.instances
-    b = Batch(make_cfg(n_instances=N))
-    b.seed(2024)
-    b.reset()
-    g = torch.Generator(device="cuda").manual_seed(1)
-    dxdy = torch.empty((N, 2), device="cuda")
-    act = torch.zeros(N, dtype=torch.int32, device="cuda")
-
-    def step():
-        dxdy.uniform_(-1, 1, generator=g)
-        act.random_(0, 3, generator=g)
-        b.set_actions_device(dxdy.data_ptr(), act.data_ptr())
-        b.step()
-
-    for _ in range(a.age):
-        step()
+    b, step, _ = aged_configs1(N, a.age)
     src16 = torch.arange(0, N, max(1, N // 16), dtype=torch.int32, device="cuda")[:16].contiguous()
     bufs = {"arena16_512": torch.empty((src16.numel(), 512, 512, 3), dtype=torch.uint8, device="cuda"),
             "arena16_1024": torch.empty((src16.numel(), 1024, 1024, 3), dtype=torch.uint8, device="cuda"),
@@ -60,42 +42,19 @@ def main():
             "arena16_1024": lambda: b.draw(src16, 1024, "arena", out=bufs["arena16_1024"]),
             "agents_128": lambda: b.draw(None, 128, "agent", out=bufs["agents_128"])}
     # (stepping changes the games pictured: the step is timed after the drawing arms)
-    times = {k: [] for k in list(arms) + ["step"]}
-    for f in arms.values():
-        f()
-    torch.cuda.synchronize()
-    ev = lambda: torch.cuda.Event(enable_timing=True)  # noqa: E731
-    for _ in range(a.repeats):
-        for name, f in arms.items():
-            e0, e1 = ev(), ev()
-            e0.record()
-            for _ in range(a.calls):
-                f()
-            e1.record()
-            e1.synchronize()
-            times[name].append(e0.elapsed_time(e1) / a.calls)
-    for _ in range(a.repeats):
-        e0, e1 = ev(), ev()
-        e0.record()
-        for _ in range(a.calls):
-            step()
-        e1.record()
-        e1.synchronize()
-        times["step"].append(e0.elapsed_time(e1) / a.calls)
+    times = time_arms(arms, a.calls, a.repeats)
+    times.update(time_arms({"step": step}, a.calls, a.repeats))
     info = gpu_info()
     lines = []
     for name, ts in times.items():
-        rec = {"arm": name, "instances": N, "age": a.age, "ms_median": statistics.median(ts), "ms_min": min(ts), "ms_max": max(ts)}
+        rec = {"arm": name, "instances": N, "age": a.age, **stats(ts, "ms_")}
         if name in bufs:
             nbytes = bufs[name].numel()
             rec.update(pictures=int(bufs[name].shape[0]), size=int(bufs[name].shape[1]), bytes_written=nbytes,
                        write_GBps=nbytes / (rec["ms_median"] * 1e-3) / 1e9)
         rec.update(info)
-        lines.append(json.dumps(rec))
-        print(lines[-1], flush=True)
-    if a.out:
-        with open(a.out, "w") as f:
-            f.write("\n".join(lines) + "\n")
+        lines.append(rec)
+    write_lines(lines, a.out)
 
 
 if __name__ == "__main__":

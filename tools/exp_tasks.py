@@ -13,16 +13,13 @@ Every batch is aged by --age random-walk steps first (an early step is cheaper t
 between repeats.  One JSON line per arm: ms per env-step (median / min / max over the repeats) and env-steps/s, plus the GPU's
 name and power limit read in the same run."""
 import argparse
-import json
 import os
-import statistics
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tools"))
 
-from exp_snapshot import gpu_info  # noqa: E402
+from exp_common import RandomWalk, gpu_info, stats, time_arms, write_lines  # noqa: E402
 from run_tasks_configs import TASKS  # noqa: E402
 
 MODES = list(range(1, 11))
@@ -45,9 +42,7 @@ def main():
     N = a.instances
     common = dict(ticks_per_step=4, num_frames=1, arena_size=350, num_pellets=500, num_viruses=0, num_bots=0, pellet_regen=True,
                   grid_size=128, reward_type=1, c_death=0)
-    g = torch.Generator(device="cuda").manual_seed(1)
-    dxdy = torch.empty((N, 2), device="cuda")
-    act = torch.zeros(N, dtype=torch.int32, device="cuda")
+    walk = RandomWalk(N)
 
     def make(n, mode, base, tasks=False):
         b = Batch(make_cfg(n_instances=n, mode_number=mode, instance_base=base, task_modes=task_bits(MODES) if tasks else 0, **common))
@@ -63,7 +58,7 @@ def main():
     def step(batches):  # one env-step of every batch of the arm, the actions of instance j from slot j of the shared tensors
         off = 0
         for b in batches:
-            b.set_actions_device(dxdy[off:].data_ptr(), act[off:].data_ptr())
+            b.set_actions_device(walk.dxdy[off:].data_ptr(), walk.act[off:].data_ptr())
             b.step_autoreset()
             off += b.N
 
@@ -73,37 +68,21 @@ def main():
     for k in MODES:
         arms[f"big_{k}"] = [make(N, k, 0)]
     for _ in range(a.age):
-        dxdy.uniform_(-1, 1, generator=g)
-        act.random_(0, 3, generator=g)
+        walk.next()
         for bs in arms.values():
             step(bs)
-    torch.cuda.synchronize()
-    names = list(arms)
-    ms = {n: [] for n in names}
-    for r in range(a.repeats):
-        order = names[r % len(names):] + names[:r % len(names)]
-        for n in order:
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            for _ in range(a.calls):
-                step(arms[n])
-            e1.record()
-            e1.synchronize()
-            ms[n].append(e0.elapsed_time(e1) / a.calls)
+    ms = time_arms({n: (lambda bs=bs: step(bs)) for n, bs in arms.items()}, a.calls, a.repeats)
     info = gpu_info()
     flags = {n: sorted(set().union(*[set(b.flags()[1]) for b in bs])) for n, bs in arms.items()}
     lines = []
-    for n in names:
-        med = statistics.median(ms[n])
+    for n, t in ms.items():
+        s = stats(t)
         envs = sum(b.N for b in arms[n])
-        lines.append(dict(arm=n, instances=envs, ms_per_env_step=med, ms_min=min(ms[n]), ms_max=max(ms[n]),
-                          env_steps_per_s=envs / med * 1e3, age=a.age, calls=a.calls, repeats=a.repeats, state_flags=flags[n], **info))
+        lines.append(dict(arm=n, instances=envs, ms_per_env_step=s["median"], ms_min=s["min"], ms_max=s["max"],
+                          env_steps_per_s=envs / s["median"] * 1e3, age=a.age, calls=a.calls, repeats=a.repeats, state_flags=flags[n],
+                          **info))
     lines.append(dict(arm="summary", mixed_over_ten_small=lines[0]["ms_per_env_step"] / lines[1]["ms_per_env_step"], **info))
-    text = "\n".join(json.dumps(x) for x in lines)
-    print(text)
-    if a.out:
-        with open(a.out, "w") as f:
-            f.write(text + "\n")
+    write_lines(lines, a.out)
 
 
 if __name__ == "__main__":
