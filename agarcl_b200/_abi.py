@@ -44,6 +44,16 @@ class Cfg(C.Structure):
         "obs_dtype", "strict_reference", "rng_mode",
         "cap_viruses", "cap_foods", "cap_replay", "device", "instance_base", "ram_obs", "task_modes")] + [("reserved", C.c_int32 * 1)]
 
+    # the header's last field, pixel_obs, took the place of `reserved[1]`; the ctypes field keeps that name, so code that names
+    # it keeps working, and pixel_obs reads and writes it
+    @property
+    def pixel_obs(self):
+        return self.reserved[0]
+
+    @pixel_obs.setter
+    def pixel_obs(self, v):
+        self.reserved[0] = v
+
 
 class Layout(C.Structure):
     """struct agarcl_layout"""
@@ -78,9 +88,10 @@ def make_cfg(n_instances=1, num_agents=1, ticks_per_step=4, arena_size=1000, pel
              num_pellets=1000, num_viruses=25, num_bots=25, reward_type=1, c_death=0, mode_number=0,
              num_frames=1, grid_size=128, observe_cells=True, observe_others=True, observe_viruses=True,
              observe_pellets=True, obs_dtype=OBS_I32, strict_reference=False, rng_mode=RNG_PHILOX,
-             cap_viruses=0, cap_foods=0, cap_replay=0, device=0, instance_base=0, ram_obs=False, task_modes=0):
+             cap_viruses=0, cap_foods=0, cap_replay=0, device=0, instance_base=0, ram_obs=False, task_modes=0, pixel_obs=0):
     """task_modes: 0, or the bit mask of the modes a mixed-task batch may run (include/agarcl_b200.h); task_bits() makes one
-    from a list of modes"""
+    from a list of modes.  pixel_obs: 0, or the size S of the pixel observation (one RGB picture [S, S, 3] per agent after every
+    step and reset instead of the grid frame)"""
     c = Cfg()
     for k, v in list(locals().items()):
         if k in ("c",):

@@ -61,6 +61,7 @@ def lib():
         L.agarcl_batch_set_tasks.argtypes = [_vp, _vp, _vp, C.POINTER(_vp), _vp]
         L.agarcl_batch_tasks.argtypes = [_vp, _vp]
         L.agarcl_batch_draw.argtypes = [_vp, C.c_int32, C.c_int32, _vp, C.c_int32, _vp, _vp]
+        L.agarcl_batch_pixels.argtypes = [_vp, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(C.c_int64 * 4)]
         L.agarcl_batch_bot_actions.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp]
         L.agarcl_batch_mirror.argtypes = [_vp, C.POINTER(_vp), C.POINTER(C.c_int64 * 4), C.POINTER(C.c_int32)]
         L.agarcl_batch_sync_mirror.argtypes = [_vp, _vp]

@@ -417,6 +417,26 @@ class Batch:
                                                 n, _vp(out.data_ptr()), _vp(stream)))
         return out
 
+    # ---- the pixel observation (include/agarcl_b200.h, cfg.pixel_obs)
+    def _pixels(self, final):
+        import torch
+        p, f, shape = _vp(), _vp(), (C.c_int64 * 4)()
+        _lib.check(_lib.lib().agarcl_batch_pixels(self._h, C.byref(p), C.byref(f), C.byref(shape)))
+        ptr = f.value if final else p.value
+        if not ptr:
+            raise _lib.AgarclError("no final pictures: set_autoreset(keep_final_obs=True) with cfg.pixel_obs")
+        return torch.as_tensor(_CudaView(ptr, tuple(shape), "|u1", self), device=f"cuda:{self.cfg.device}")
+
+    def pixels(self):
+        """zero-copy device view uint8 [N*A, S, S, 3] of every agent's picture (cfg.pixel_obs = S), rewritten by every step, reset
+        and restore: the picture agarcl_batch_draw's agent view draws, with the players the step respawned still dead"""
+        return self._pixels(False)
+
+    def final_pixels(self):
+        """zero-copy device view uint8 [N*A, S, S, 3] of the pictures the reset instances of the last step_autoreset ended their
+        episode on (set_autoreset(keep_final_obs=True))"""
+        return self._pixels(True)
+
     # ---- built-in bot policies for agents (include/agarcl_b200.h, agarcl_batch_bot_actions)
     def bot_actions(self, types, out=None, target=None):
         """what a built-in bot would do for every agent on the current state, computed on the device on torch's current stream

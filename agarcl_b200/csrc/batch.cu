@@ -114,6 +114,9 @@ struct agarcl_batch {
   DevBuf<double> d_ret, d_final_ret;
   DevBuf<void> d_final_obs;          // [N*A, frames*C, G, G], only with keep_final_obs and a grid observation
   DevBuf<float> d_final_ram;         // [N, P, AGARCL_RAM_RECORD], only with keep_final_obs and cfg.ram_obs
+  // pixel observation (cfg.pixel_obs = S): every agent's picture [N*A, S, S, 3] after every step and reset, and the finishing ones
+  DevBuf<uint8_t> d_pixels, d_final_pixels;  // (d_final_pixels only with keep_final_obs)
+  size_t pixel_bytes = 0;
   // snapshot pools (agarcl_batch_save_states / _restore_states): the slot layout, the configuration's fingerprint, the
   // library-owned result of the last restore and the mask of the instances it restored
   ag::SnapLayout snap;
@@ -224,6 +227,9 @@ static void fill_sim_params(const agarcl_batch* b, ag::SimParams& P) {
   P.inst_first = 0;
 }
 
+// Whether the batch renders a grid frame: not under the structured observation only (agario-ram-v0), not with pixels
+static bool renders_grid(const agarcl_batch* b) { return b->cfg.ram_obs != 2 && !b->cfg.pixel_obs; }
+
 // Whether the engine-tick kernel writes the whole observation frame itself (SimParams::obs_finish): 0 no (k_obs renders
 // it), 1 int32, 2 int16.  Needs the fused clear, rows of whole 16-byte vectors, one row of channel 0 = one bulk store from
 // the ones tile, and the row of y masks in the collision scratch.
@@ -254,7 +260,7 @@ static bool fuse_obs_clear(const agarcl_batch* b, ag::SimParams& P, int frame) {
 // it finishes the observation itself, and an image's record (count, base, image, row and column masks, reward, done) is
 // one store of a warp's 32 lanes.
 static bool kernel_writes_lists(const agarcl_batch* b) {
-  return b->frames == 1 && !b->cfg.strict_reference && b->cfg.ram_obs != 2 && obs_finish_kind(b) != 0 &&
+  return b->frames == 1 && !b->cfg.strict_reference && renders_grid(b) && obs_finish_kind(b) != 0 &&
          6 + 2 * ((b->G + 31) / 32) <= 32;
 }
 
@@ -417,6 +423,7 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
   b->fingerprint = config_fingerprint(*cfg, L);
   CK(ag::setup_step(b->knobs.warps, b->step_launch));
   if (cfg->ram_obs) CK(ag::setup_ram(L, b->step_launch.smem_optin));
+  CK(ag::setup_draw_views());
   b->obs_elems = (size_t)b->N * b->A * b->frames * b->C * b->G * b->G;
   b->obs_bytes = b->obs_elems * (cfg->obs_dtype == AGARCL_OBS_I16 ? 2 : 4);
   // spatial hash resolution: about 3 pellets per hash cell, 4..64 cells per side
@@ -436,6 +443,7 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
       (rc = alloc(b->d_snap_result, (size_t)b->N, 0)) || (rc = alloc(b->d_snap_restored, (size_t)b->N, 0)) ||
       (L.cap_replay > 0 && (rc = alloc(b->d_replay, (size_t)b->N * L.cap_replay * sizeof(float), 0))) ||
       (cfg->ram_obs && (rc = alloc(b->d_ram, (size_t)b->N * L.P * AGARCL_RAM_RECORD * sizeof(float), 0))) ||
+      (cfg->pixel_obs && (rc = alloc(b->d_pixels, b->pixel_bytes = NA * cfg->pixel_obs * cfg->pixel_obs * 3, 0))) ||
       (rc = alloc(b->d_lut_radius, lut_bytes)) || (rc = alloc(b->d_lut_speed, lut_bytes)) || (rc = alloc(b->d_lut_split, lut_bytes)))
     return rc;
   { const uint32_t init[2] = {1u, 0u}; CK(cudaMemcpy(b->d_sched, init, sizeof(init), cudaMemcpyHostToDevice)); }
@@ -554,6 +562,41 @@ static int render_ram(agarcl_batch* b, cudaStream_t s, int pre_respawn) {
   return AGARCL_OK;
 }
 
+static ag::DrawParams draw_params(const agarcl_batch* b, int view, int size, const int32_t* d_src, int n, uint8_t* d_out) {
+  ag::DrawParams P;
+  P.L = b->L;
+  P.radius = b->T.radius;
+  P.state = b->d_state;
+  P.out = d_out;
+  P.src = d_src;
+  P.n = n;
+  P.S = size;
+  P.view = view;
+  P.N = b->N;
+  P.W = (float)b->cfg.arena_size;
+  P.pre_respawn = 0;
+  P.mask = nullptr;
+  return P;
+}
+
+// The pixel observation of the instances with d_mask != 0 (nullptr: all); pre_respawn 1 shows the step's moment, as k_obs does
+static int render_pixels(agarcl_batch* b, cudaStream_t s, int pre_respawn, const uint8_t* d_mask) {
+  ag::DrawParams P = draw_params(b, AGARCL_DRAW_AGENT, b->cfg.pixel_obs, nullptr, b->N * b->A, b->d_pixels);
+  P.pre_respawn = pre_respawn;
+  P.mask = d_mask;
+  CK(ag::launch_draw_views(P, s));
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_pixels(agarcl_batch* b, uint8_t** d_pixels, uint8_t** d_final_pixels, int64_t shape[4]) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (!b->cfg.pixel_obs) return agarcl_set_error(AGARCL_ERR_STATE, "batch was created without cfg.pixel_obs");
+  if (d_pixels) *d_pixels = b->d_pixels;
+  if (d_final_pixels) *d_final_pixels = b->keep_final ? b->d_final_pixels.get() : nullptr;
+  if (shape) { shape[0] = (int64_t)b->N * b->A; shape[1] = shape[2] = b->cfg.pixel_obs; shape[3] = 3; }
+  return AGARCL_OK;
+}
+
 extern "C" int agarcl_batch_ram(agarcl_batch* b, float** dev_ptr, int64_t shape[3]) {
   if (!b || !dev_ptr) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
   if (!b->d_ram) return agarcl_set_error(AGARCL_ERR_STATE, "batch was created without cfg.ram_obs");
@@ -648,7 +691,8 @@ static int reset_impl(agarcl_batch* b, const uint8_t* dm, cudaStream_t s, bool c
   if (b->d_ram)  // GoBiggerEnvironment::reset ends with observation.clear() (GoBiggerEnvironment.hpp:698-702)
     CK(clear(b->d_ram, (size_t)b->N * b->L.P * AGARCL_RAM_RECORD * sizeof(float)));
   // the reference ends reset() with _partial_observation (BaseEnvironment.hpp:202-203)
-  if (b->cfg.ram_obs == 2) return AGARCL_OK;  // no grid observation in this mode
+  if (b->cfg.pixel_obs) return render_pixels(b, s, 0, dm);
+  if (!renders_grid(b)) return AGARCL_OK;  // no grid observation in this mode
   if (b->cfg.strict_reference) {
     CK(clear(b->d_obs, b->obs_bytes));
     int frame = 0 - (b->cfg.ticks_per_step - b->frames);
@@ -707,10 +751,10 @@ static int step_impl(agarcl_batch* b, cudaStream_t s, bool want_lists, bool* lis
     CK(ag::launch_step(P, b->step_launch, s)); launches++;
     int frame = 0 - (tps - b->frames);
     if (frame >= 0) { int rc = render_frame(b, frame, s, 1); if (rc) return rc; launches++; }
-  } else if (b->cfg.ram_obs == 2 || b->frames == 1) {
-    // one k_step runs every tick of the step; a grid frame (none with the structured observation only, agario-ram-v0) is
-    // finished by k_step itself or by k_obs behind it
-    const bool grid = b->cfg.ram_obs != 2;
+  } else if (!renders_grid(b) || b->frames == 1) {
+    // one k_step runs every tick of the step; a grid frame (none with the structured observation only, agario-ram-v0, or with
+    // pixels) is finished by k_step itself or by k_obs behind it
+    const bool grid = renders_grid(b);
     P.n_ticks = tps; P.do_begin = 1; P.do_end = 1;
     const int fused = grid && fuse_obs_clear(b, P, 0) ? 1 : 0;
     if (want_lists && target && kernel_writes_lists(b)) {
@@ -744,6 +788,10 @@ static int step_impl(agarcl_batch* b, cudaStream_t s, bool want_lists, bool* lis
     int rc = render_ram(b, s, 1); if (rc) return rc; launches++;
     if (b->timing && b->cfg.ram_obs == 2) CK(cudaEventRecord(next_event(b), s));  // (k_ram is this mode's observation kernel)
   }
+  if (b->cfg.pixel_obs) {
+    int rc = render_pixels(b, s, 1, nullptr); if (rc) return rc; launches++;
+    if (b->timing) CK(cudaEventRecord(next_event(b), s));
+  }
   b->launches_last_step = launches;
   return refill_replay(b, s);
 }
@@ -765,7 +813,8 @@ extern "C" int agarcl_batch_set_autoreset(agarcl_batch* b, int32_t max_steps, in
       (rc = alloc(b->d_ret, NA * sizeof(double), 0)) || (rc = alloc(b->d_final_ret, NA * sizeof(double), 0)))
     return rc;
   if (keep_final_obs) {
-    if (b->cfg.ram_obs != 2 && (rc = alloc(b->d_final_obs, b->obs_bytes, 0))) return rc;
+    if (renders_grid(b) && (rc = alloc(b->d_final_obs, b->obs_bytes, 0))) return rc;
+    if (b->cfg.pixel_obs && (rc = alloc(b->d_final_pixels, b->pixel_bytes, 0))) return rc;
     if (b->d_ram && (rc = alloc(b->d_final_ram, (size_t)b->N * b->L.P * AGARCL_RAM_RECORD * sizeof(float), 0))) return rc;
   }
   // every instance starts counting here
@@ -789,6 +838,8 @@ extern "C" int agarcl_batch_step_autoreset(agarcl_batch* b, void* stream) {
   if (!b->autoreset_reset) return AGARCL_OK;
   if (b->keep_final) {  // the observation the finished episode ended on, before the reset overwrites it
     if (b->d_final_obs) CK(ag::launch_masked_bytes(b->d_final_obs, b->d_obs, b->obs_bytes / (size_t)b->N, b->d_reset_mask, b->N, s));
+    if (b->d_final_pixels)
+      CK(ag::launch_masked_bytes(b->d_final_pixels, b->d_pixels, b->pixel_bytes / (size_t)b->N, b->d_reset_mask, b->N, s));
     if (b->d_final_ram)
       CK(ag::launch_masked_bytes(b->d_final_ram, b->d_ram, (size_t)b->L.P * AGARCL_RAM_RECORD * sizeof(float), b->d_reset_mask, b->N, s));
   }
@@ -875,9 +926,16 @@ extern "C" int agarcl_batch_dones(agarcl_batch* b, uint8_t** dev_ptr) {
   return AGARCL_OK;
 }
 
+// The host paths of the grid observation: refused for a pixel batch, which renders no grid frame
+static int refuse_pixels(const agarcl_batch* b, const char* what) {
+  if (b->cfg.pixel_obs) return agarcl_set_error(AGARCL_ERR_STATE, "%s serves the grid observation: a pixel batch (cfg.pixel_obs) has none", what);
+  return AGARCL_OK;
+}
+
 extern "C" int agarcl_batch_step_host(agarcl_batch* b, const float* dxdy, const int32_t* act, void* obs_out,
                                       double* rewards_out, uint8_t* dones_out) {
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (int rc = refuse_pixels(b, "agarcl_batch_step_host")) return rc;
   int rc = agarcl_batch_set_actions(b, dxdy, act, 0, nullptr);
   if (rc) return rc;
   rc = agarcl_batch_step(b, nullptr);
@@ -900,6 +958,7 @@ static int ensure_mirror(agarcl_batch* b) {
 
 extern "C" int agarcl_batch_sync_mirror(agarcl_batch* b, void* stream) {
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (int rc = refuse_pixels(b, "agarcl_batch_sync_mirror")) return rc;
   int rc = ensure_mirror(b);
   if (rc) return rc;
   CK(cudaSetDevice(b->cfg.device));
@@ -924,6 +983,7 @@ extern "C" int agarcl_batch_mirror(agarcl_batch* b, void** host_ptr, int64_t sha
 extern "C" int agarcl_batch_step_mirror(agarcl_batch* b, const float* dxdy, const int32_t* act, double* rewards_out,
                                         uint8_t* dones_out) {
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (int rc = refuse_pixels(b, "agarcl_batch_step_mirror")) return rc;
   int rc = ensure_mirror(b);
   if (rc) return rc;
   if (!dxdy || !act) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
@@ -951,6 +1011,7 @@ extern "C" int agarcl_batch_step_mirror(agarcl_batch* b, const float* dxdy, cons
 extern "C" int agarcl_batch_step_lists(agarcl_batch* b, const float* dxdy, const int32_t* act, double* rewards_out, uint8_t* dones_out,
                                        agarcl_obs_lists* out) {
   if (!b || !dxdy || !act || !out) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
+  if (int rc = refuse_pixels(b, "agarcl_batch_step_lists")) return rc;
   if (b->frames != 1 || b->cfg.strict_reference || b->cfg.ram_obs == 2)
     return agarcl_set_error(AGARCL_ERR_STATE, "observation lists need the single fused step kernel (one frame, strict_reference = 0, a grid observation)");
   if (!kernel_writes_lists(b))  // (refused before anything is enqueued: the games do not move)
@@ -1152,7 +1213,8 @@ extern "C" int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, in
   P.slot_of = d_slot_of;
   CK(ag::launch_snapshot_restore(P, s));
   // a one-frame grid observation is re-rendered, as the step that produced the state showed it (respawned players still dead)
-  if (b->cfg.ram_obs != 2 && b->frames == 1 && (rc = render_frame(b, 0, s, 1, 0, b->d_snap_restored))) return rc;
+  if (renders_grid(b) && b->frames == 1 && (rc = render_frame(b, 0, s, 1, 0, b->d_snap_restored))) return rc;
+  if (b->cfg.pixel_obs && (rc = render_pixels(b, s, 1, b->d_snap_restored))) return rc;
   if (d_result) *d_result = b->d_snap_result;
   return AGARCL_OK;
 }
@@ -1179,18 +1241,9 @@ extern "C" int agarcl_batch_draw(agarcl_batch* b, int32_t view, int32_t size, co
   if (a.type != cudaMemoryTypeDevice || a.device != b->cfg.device)
     return agarcl_set_error(AGARCL_ERR_INVALID, "the output must be device memory of device %d", b->cfg.device);
   if (n == 0) return AGARCL_OK;
-  ag::DrawParams P;
-  P.L = b->L;
-  P.radius = b->T.radius;
-  P.state = b->d_state;
-  P.out = d_out;
-  P.src = d_src;
-  P.n = n;
-  P.S = size;
-  P.view = view;
-  P.N = b->N;
-  P.W = (float)b->cfg.arena_size;
-  CK(ag::launch_draw(P, (cudaStream_t)stream));
+  const ag::DrawParams P = draw_params(b, view, size, d_src, n, d_out);
+  if (view == AGARCL_DRAW_AGENT) CK(ag::launch_draw_views(P, (cudaStream_t)stream));
+  else CK(ag::launch_draw(P, (cudaStream_t)stream));
   return AGARCL_OK;
 }
 

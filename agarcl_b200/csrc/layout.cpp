@@ -49,6 +49,14 @@ extern "C" int agarcl_make_layout(const agarcl_cfg* c, agarcl_layout* L) {
   if (c->mode_number < 0 || c->mode_number > 10) return agarcl_set_error(AGARCL_ERR_INVALID, "Invalid mode number");
   if (c->grid_size < 1 || c->grid_size > 1024) return agarcl_set_error(AGARCL_ERR_INVALID, "grid_size out of range");
   if (c->num_frames < 1) return agarcl_set_error(AGARCL_ERR_INVALID, "num_frames must be >= 1");
+  if (c->pixel_obs) {  // the pixel observation (include/agarcl_b200.h, agarcl_cfg.pixel_obs)
+    if (c->pixel_obs < 16 || c->pixel_obs > 2048 || c->pixel_obs % 16)
+      return agarcl_set_error(AGARCL_ERR_INVALID, "pixel_obs %d must be 0 or a multiple of 16 in [16, 2048]", c->pixel_obs);
+    if (c->num_frames != 1)
+      return agarcl_set_error(AGARCL_ERR_INVALID, "pixel_obs needs num_frames = 1: frame stacking of pictures is the caller's");
+    if (c->strict_reference) return agarcl_set_error(AGARCL_ERR_INVALID, "pixel_obs is refused under strict_reference");
+    if (c->ram_obs == 2) return agarcl_set_error(AGARCL_ERR_INVALID, "pixel_obs is refused with ram_obs = 2 (one observation or the other)");
+  }
 
   const int mode = c->mode_number;
   const int task_modes = c->task_modes;

@@ -254,7 +254,8 @@ struct SnapParams {
 cudaError_t launch_snapshot_save(const SnapParams& P, int n, cudaStream_t stream);
 cudaError_t launch_snapshot_restore(const SnapParams& P, cudaStream_t stream);
 
-// Pictures of game states (draw_kernel.cu, k_draw): the spec of include/agarcl_b200.h, agarcl_batch_draw
+// Pictures of game states (draw_kernel.cu): the spec of include/agarcl_b200.h, agarcl_batch_draw.  k_draw draws arena views,
+// k_draw_views agent views and the pixel observation (cfg.pixel_obs)
 struct DrawParams {
   agarcl_layout L;
   const float* radius;     // Luts::radius
@@ -263,8 +264,13 @@ struct DrawParams {
   const int32_t* src;      // [n] or nullptr (picture k shows source k)
   int32_t n, S, view, N;
   float W;
+  int32_t pre_respawn;     // k_draw_views: 1 draws players respawned at the end of the last step as still dead (the observation)
+  const uint8_t* mask;     // k_draw_views: [N] or nullptr: only the pictures of instances with mask != 0 are written
 };
 cudaError_t launch_draw(const DrawParams& P, cudaStream_t stream);
+// On the current device: opts k_draw_views in to the dynamic shared memory of its largest picture
+cudaError_t setup_draw_views();
+cudaError_t launch_draw_views(const DrawParams& P, cudaStream_t stream);
 
 // Built-in bot policies for agents (bot_kernel.cu, k_bot_actions): the spec of include/agarcl_b200.h, agarcl_batch_bot_actions
 struct BotParams {

@@ -23,12 +23,12 @@ from .batch import Batch
 class _Base:
     def __init__(self, n_instances, num_agents, ticks_per_step, arena_size, pellet_regen, num_pellets, num_viruses,
                  num_bots, reward_type, c_death, mode_number, rng_mode, strict_reference, device, obs_dtype, instance_base=0,
-                 ram_obs=False, task_modes=0):
+                 ram_obs=False, task_modes=0, pixel_obs=0):
         self._ctor = dict(n_instances=n_instances, num_agents=num_agents, ticks_per_step=ticks_per_step,
                           arena_size=arena_size, pellet_regen=pellet_regen, num_pellets=num_pellets, num_viruses=num_viruses,
                           num_bots=num_bots, reward_type=reward_type, c_death=c_death, mode_number=mode_number,
                           rng_mode=rng_mode, strict_reference=strict_reference, device=device, obs_dtype=obs_dtype,
-                          instance_base=instance_base, ram_obs=ram_obs, task_modes=task_modes)
+                          instance_base=instance_base, ram_obs=ram_obs, task_modes=task_modes, pixel_obs=pixel_obs)
         self._obs_cfg = dict(num_frames=1, grid_size=128, observe_cells=True, observe_others=True, observe_viruses=True,
                              observe_pellets=True)
         self._seeds = None
@@ -87,9 +87,9 @@ class GridEnvironment(_Base):
     num_viruses, num_bots, reward_type, c_death, mode_number) — bindings.cpp:102."""
 
     def __init__(self, num_agents, ticks_per_step, arena_size, pellet_regen, num_pellets, num_viruses, num_bots,
-                 reward_type=0, c_death=0, mode_number=0, *, rng_mode=RNG_MT19937, strict_reference=False, device=0):
+                 reward_type=0, c_death=0, mode_number=0, *, rng_mode=RNG_MT19937, strict_reference=False, device=0, pixel_obs=0):
         super().__init__(1, num_agents, ticks_per_step, arena_size, pellet_regen, num_pellets, num_viruses, num_bots,
-                         reward_type, c_death, mode_number, rng_mode, strict_reference, device, OBS_I32)
+                         reward_type, c_death, mode_number, rng_mode, strict_reference, device, OBS_I32, pixel_obs=pixel_obs)
         self.num_agents = num_agents
         self._order_agents = None
 
@@ -317,14 +317,15 @@ class BatchedGridEnvironment(_Base):
     """N lockstep GridEnvironments on one GPU.  step() takes arrays/tensors and returns device tensors:
     obs [N*A, C*frames, G, G], rewards f64 [N*A], dones u8 [N*A].  With ram_obs=True the structured
     observation records [N, P, RAM_RECORD] are produced too (ram()).  tasks=(1, 2, ...) makes a mixed-task batch: every
-    instance plays its own mode of that set, mode_number first, and changes it at its next reset (set_tasks)."""
+    instance plays its own mode of that set, mode_number first, and changes it at its next reset (set_tasks).  pixel_obs=S: the
+    observation is every agent's RGB picture uint8 [N*A, S, S, 3] (Batch.pixels) instead of the grid frame."""
 
     def __init__(self, n_instances, num_agents=1, ticks_per_step=4, arena_size=1000, pellet_regen=True, num_pellets=1000,
                  num_viruses=25, num_bots=25, reward_type=1, c_death=0, mode_number=0, *, rng_mode=RNG_PHILOX,
-                 strict_reference=False, device=0, obs_dtype=OBS_I32, instance_base=0, ram_obs=False, tasks=None):
+                 strict_reference=False, device=0, obs_dtype=OBS_I32, instance_base=0, ram_obs=False, tasks=None, pixel_obs=0):
         super().__init__(n_instances, num_agents, ticks_per_step, arena_size, pellet_regen, num_pellets, num_viruses,
                          num_bots, reward_type, c_death, mode_number, rng_mode, strict_reference, device, obs_dtype,
-                         instance_base, ram_obs, task_bits(tasks) if tasks else 0)
+                         instance_base, ram_obs, task_bits(tasks) if tasks else 0, pixel_obs)
         self.n_instances = n_instances
         self.num_agents = num_agents
 
@@ -342,7 +343,10 @@ class BatchedGridEnvironment(_Base):
             b.reset_device(mask, stream)
         else:
             b.reset(mask, stream)
-        return b.obs_tensor()
+        return self._obs(b)
+
+    def _obs(self, b):
+        return b.pixels() if self._ctor["pixel_obs"] else b.obs_tensor()
 
     def _set_actions(self, b, dxdy, act, stream):
         if hasattr(dxdy, "data_ptr"):
@@ -367,7 +371,7 @@ class BatchedGridEnvironment(_Base):
         b = self._ensure()
         self._set_actions(b, dxdy, act, stream)
         b.step(stream)
-        return b.obs_tensor(), b.rewards_tensor(), b.dones_tensor()
+        return self._obs(b), b.rewards_tensor(), b.dones_tensor()
 
     def set_autoreset(self, max_steps=0, final_obs=False, reset=True):
         """enables step_autoreset: max_steps > 0 ends an episode after that many steps (0: continuing), final_obs keeps the
@@ -381,7 +385,7 @@ class BatchedGridEnvironment(_Base):
         b = self._ensure()
         self._set_actions(b, dxdy, act, stream)
         b.step_autoreset(stream)
-        return b.obs_tensor(), b.rewards_tensor(), b.episode()["done"]
+        return self._obs(b), b.rewards_tensor(), b.episode()["done"]
 
     def episode(self):
         return self._ensure().episode()

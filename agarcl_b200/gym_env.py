@@ -81,8 +81,8 @@ _OBS_KEYS = ("num_frames", "grid_size", "observe_cells", "observe_others", "obse
 class AgarioEnv(_EnvBase):
     metadata = {"render_modes": ["human", "rgb_array"], "render_fps": 60}
 
-    def __init__(self, obs_type="grid", render_mode=None, render_size=512, render_view="arena", **kwargs):
-        if obs_type not in ("ram", "screen", "grid", "gobigger"):
+    def __init__(self, obs_type="grid", render_mode=None, render_size=512, render_view="arena", pixel_size=128, **kwargs):
+        if obs_type not in ("ram", "screen", "grid", "gobigger", "pixels"):
             raise ValueError(obs_type)
         if render_view not in ("arena", "agent"):
             raise ValueError(f"render_view must be 'arena' or 'agent', got {render_view!r}")
@@ -108,6 +108,10 @@ class AgarioEnv(_EnvBase):
             self._env.configure_observation({k: kwargs[k] for k in _OBS_KEYS if k in kwargs})
             c, w, h = self._env.observation_shape()
             self.observation_space = spaces.Box(-1, np.iinfo(np.int32).max, (w, h, c), dtype=np.int32)
+        elif obs_type == "pixels":  # every agent's RGB picture, drawn on the device (include/agarcl_b200.h, cfg.pixel_obs)
+            S = int(pixel_size)
+            self._env = GridEnvironment(*pos, pixel_obs=S, **extra)
+            self.observation_space = spaces.Box(0, 255, (S, S, 3), dtype=np.uint8)
         else:
             self._env = GoBiggerEnvironment(kwargs.get("map_width", 512), kwargs.get("map_height", 512),
                                             kwargs.get("frame_limit", 1000), *pos, **extra)
@@ -167,6 +171,9 @@ class AgarioEnv(_EnvBase):
 
     # ---- helpers
     def _make_observations(self):
+        if self.obs_type == "pixels":
+            pics = self._env._ensure().pixels().cpu().numpy()
+            return [pics[a] for a in range(self.num_agents)]
         if self.obs_type == "grid":
             return [np.transpose(s, [1, 2, 0]) for s in self._env.get_state()]  # NCHW -> HWC view (AgarioEnv.py:192-194)
         if self.obs_type == "ram":
@@ -202,18 +209,22 @@ class BatchedAgarioEnv:
       reset_mask      bool [N]   instances reset by this step
       episode_return  f64 [N*A]  return of the episode an instance just finished (read where reset_mask is set)
       episode_length  i64 [N]    its length in steps (likewise)
-      final_obs       the observation that episode ended on (grid: [N*A, C*frames, G, G]; ram: [N, A, RAM_RECORD]); only
-                      with final_obs=True, which allocates as much device memory again as the observation
+      final_obs       the observation that episode ended on (grid: [N*A, C*frames, G, G]; ram: [N, A, RAM_RECORD]; pixels: [N*A,
+                      S, S, 3]); only with final_obs=True, which allocates as much device memory again as the observation
     obs, dones and every info tensor are views of library-owned buffers that the next step() overwrites: copy what must
     outlive it.  With auto_reset=False nothing is reset: the step limit is folded into dones, steps keeps counting, and
     info has "steps" only.
 
     tasks=[1, 2, ...]: a mixed-task batch, every environment plays its own mini-game (mode) of that set -- `mode` (default:
     the first of the list) to begin with -- and set_tasks() chooses what each one plays from its next reset on, with its own
-    step limit.  info["task"] (i32 [N]) is then every environment's current mode: after an auto-reset, the new episode's."""
+    step limit.  info["task"] (i32 [N]) is then every environment's current mode: after an auto-reset, the new episode's.
 
-    def __init__(self, n_envs, obs_type="grid", auto_reset=True, final_obs=False, tasks=None, **kwargs):
-        if obs_type not in ("grid", "ram"):
+    obs_type="pixels": the observation is every agent's RGB picture uint8 [N*A, pixel_size, pixel_size, 3] (HWC), drawn on the
+    device after every step from the same moment as the grid observation (include/agarcl_b200.h, cfg.pixel_obs); no grid frame
+    is rendered.  Frame stacking is the caller's: info["reset_mask"] says which stacks to clear."""
+
+    def __init__(self, n_envs, obs_type="grid", auto_reset=True, final_obs=False, tasks=None, pixel_size=128, **kwargs):
+        if obs_type not in ("grid", "ram", "pixels"):
             raise ValueError(obs_type)
         if tasks and "mode" not in kwargs:
             kwargs = dict(kwargs, mode=int(list(tasks)[0]))
@@ -230,7 +241,8 @@ class BatchedAgarioEnv:
         extra = {k: kwargs[k] for k in ("device", "rng_mode", "obs_dtype", "instance_base") if k in kwargs}
         self._env = BatchedGridEnvironment(n_envs, a["num_agents"], a["ticks_per_step"], a["arena_size"], a["pellet_regen"],
                                            a["num_pellets"], a["num_viruses"], a["num_bots"], a["reward_type"], a["c_death"],
-                                           a["mode"], ram_obs=(2 if obs_type == "ram" else 0), tasks=self.tasks, **extra)
+                                           a["mode"], ram_obs=(2 if obs_type == "ram" else 0), tasks=self.tasks,
+                                           pixel_obs=(int(pixel_size) if obs_type == "pixels" else 0), **extra)
         self._env.configure_observation({k: kwargs[k] for k in _OBS_KEYS if k in kwargs})
         self._ep_batch = None
         self._ep = None
@@ -242,6 +254,8 @@ class BatchedAgarioEnv:
     def _obs(self):
         if self.obs_type == "grid":
             return self._env.batch.obs_tensor()
+        if self.obs_type == "pixels":
+            return self._env.batch.pixels()
         ram = self._env.ram()
         return ram[:, :self.num_agents, :]
 
@@ -251,7 +265,8 @@ class BatchedAgarioEnv:
             b.set_autoreset(self.number_of_steps if self.env_type == 0 else 0, self.final_obs, self.auto_reset)
             self._ep_batch = b
             self._ep = b.episode()
-            self._final = (b.final_obs() if self.obs_type == "grid" else b.final_ram()[:, :self.num_agents, :]) if self.final_obs else None
+            final = {"grid": b.final_obs, "pixels": b.final_pixels}.get(self.obs_type, lambda: b.final_ram()[:, :self.num_agents, :])
+            self._final = final() if self.final_obs else None
             self._task = b.tasks()["mode"] if self.tasks else None
         self._env.reset()  # (restarts every instance's step counter and return)
         return self._obs(), {}

@@ -101,7 +101,10 @@ typedef struct agarcl_cfg {
                                (agario-ram-v0: the grid frame is not rendered, agarcl_batch_obs stays zero) */
   int32_t task_modes;       /* 0: every instance plays mode_number.  Otherwise a MIXED-TASK batch: bit m set = mode m may run in it
                                (see "mixed-task batches" below); mode_number's bit must be set, it is every instance's first task */
-  int32_t reserved[1];
+  int32_t pixel_obs;        /* 0: off.  S, a multiple of 16 in [16, 2048]: the PIXEL OBSERVATION -- every step and reset produce one
+                               RGB picture per agent (agarcl_batch_pixels) instead of the grid frame, which is not rendered
+                               (agarcl_batch_obs stays zero, as under ram_obs = 2).  Needs num_frames = 1 (frame stacking is the
+                               caller's: info reset_mask says which stacks to clear), strict_reference = 0 and ram_obs != 2 */
 } agarcl_cfg;
 
 /* ------------------------------------------------------------- state records */
@@ -342,7 +345,7 @@ int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, int64_t pool_
  * A picture is uint8 [S][S][3], RGB, row-major (HWC): row r is world y, column c world x, row 0 the smallest y.  S is a multiple of
  * 16 in [16, 2048].  It is drawn from the state blob as it is at the call: players respawned at the end of the last step are drawn
  * at their new cells.  It is not a training observation and claims no likeness to the reference's OpenGL frames; this spec is
- * what it means, and tests/draw_oracle.c (oracle_draw) restates it.
+ * what it means, and tests/draw_oracle.c (oracle_draw) restates it.  The training observation is cfg.pixel_obs below.
  * Views (every operation one rounded fp32 operation, no FMA, C order of evaluation):
  *   AGARCL_DRAW_ARENA  the arena [0, W)^2, W = (float)arena_size: pixel centre x = ((float)c + 0.5f) * W / (float)S, y the same
  *                      with r; pixel width px = W / (float)S.
@@ -370,6 +373,24 @@ int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, int64_t pool_
  *                      of 16 in [16, 2048], n < 0, a NULL or misaligned d_out or one that is not device memory of cfg.device. */
 #define AGARCL_DRAW_ARENA 0
 #define AGARCL_DRAW_AGENT 1
+
+/* ---------------------------------------------------- the pixel observation (cfg.pixel_obs = S): pictures for training
+ * A batch created with pixel_obs = S renders, after every step, reset and restore, the picture of every agent uint8
+ * [N*A, S, S, 3] (image instance * A + agent) in library-owned device memory, in place of the grid frame.  Picture j is what
+ * agarcl_batch_draw(AGARCL_DRAW_AGENT, S) would draw, with one difference: players respawned at the end of the step that
+ * produced the state are drawn as still dead (no cells), and an agent that was respawned is therefore a dead agent whose
+ * every pixel is AGARCL_DRAW_RGB_OUT.  The picture shows the same moment as the grid observation the step would have
+ * produced.  Equivalently: oracle_draw(AGARCL_DRAW_AGENT, S) on the instance's blob after setting n_cells = 0 for the players
+ * in hdr.respawned_lo / respawned_hi (a reset clears that mask; a restore keeps the saved one).
+ *   reset          the pictures of the instances it resets (masked: only those); the others are not touched
+ *   restore        the pictures of the restored instances; snapshot slots hold no pictures (they are re-rendered, never
+ *                  stored), so slot bytes and fingerprints are those of the same configuration without pixel_obs, and a pool
+ *                  moves between a pixel batch and a grid batch of the same game both ways
+ *   step_autoreset with keep_final_obs, the pictures of the instances it resets are first copied to final_pixels, as final_obs
+ * agarcl_batch_pixels: device pointers of the pictures and of the final pictures (NULL unless keep_final_obs) and their shape
+ * {N*A, S, S, 3}; AGARCL_ERR_STATE on a batch without pixel_obs.  The host paths of the grid observation
+ * (agarcl_batch_step_host, _step_mirror, _step_lists, _sync_mirror) refuse a pixel batch with AGARCL_ERR_STATE. */
+int agarcl_batch_pixels(agarcl_batch* b, uint8_t** d_pixels, uint8_t** d_final_pixels, int64_t shape[4]);
 #define AGARCL_DRAW_RGB_OUT 0x2B2B33u
 #define AGARCL_DRAW_RGB_BACKGROUND 0xF4F6F8u
 #define AGARCL_DRAW_RGB_PELLET 0x8CCB5Eu
