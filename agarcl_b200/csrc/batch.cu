@@ -733,10 +733,9 @@ extern "C" int agarcl_batch_set_actions(agarcl_batch* b, const float* dxdy, cons
   return AGARCL_OK;
 }
 
-// One env-step of every instance.  `want_lists`: the caller is agarcl_batch_step_mirror; when the step is the single
-// fused kernel, it also leaves the host mirror's transfer lists (*lists_made = true) and the k_pack pass is not needed.
-static int step_impl(agarcl_batch* b, cudaStream_t s, bool want_lists, bool* lists_made, ag::HostMirror* target = nullptr) {
-  if (!target) target = b->mirror;
+// One env-step of every instance.  `lists_to`: when the step is the single fused kernel, it also leaves the transfer lists of
+// that HostMirror in host memory (*lists_made = true); nullptr: no lists.
+static int step_impl(agarcl_batch* b, cudaStream_t s, ag::HostMirror* lists_to, bool* lists_made) {
   if (lists_made) *lists_made = false;
   if (!b->was_reset) return agarcl_set_error(AGARCL_ERR_STATE, "step() before reset()");
   CK(cudaSetDevice(b->cfg.device));
@@ -757,8 +756,8 @@ static int step_impl(agarcl_batch* b, cudaStream_t s, bool want_lists, bool* lis
     const bool grid = renders_grid(b);
     P.n_ticks = tps; P.do_begin = 1; P.do_end = 1;
     const int fused = grid && fuse_obs_clear(b, P, 0) ? 1 : 0;
-    if (want_lists && target && kernel_writes_lists(b)) {
-      P.pk = ag::mirror_pack_out(target);
+    if (lists_to && kernel_writes_lists(b)) {
+      P.pk = ag::mirror_pack_out(lists_to);
       *lists_made = true;
     }
     const bool sorted = P.tick_barrier && b->knobs.sort_schedule;
@@ -798,7 +797,7 @@ static int step_impl(agarcl_batch* b, cudaStream_t s, bool want_lists, bool* lis
 
 extern "C" int agarcl_batch_step(agarcl_batch* b, void* stream) {
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
-  return step_impl(b, (cudaStream_t)stream, false, nullptr);
+  return step_impl(b, (cudaStream_t)stream, nullptr, nullptr);
 }
 
 extern "C" int agarcl_batch_set_autoreset(agarcl_batch* b, int32_t max_steps, int32_t keep_final_obs, int32_t reset) {
@@ -832,7 +831,7 @@ extern "C" int agarcl_batch_step_autoreset(agarcl_batch* b, void* stream) {
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
   if (!b->autoreset) return agarcl_set_error(AGARCL_ERR_STATE, "agarcl_batch_step_autoreset before agarcl_batch_set_autoreset");
   cudaStream_t s = (cudaStream_t)stream;
-  int rc = step_impl(b, s, false, nullptr);
+  int rc = step_impl(b, s, nullptr, nullptr);
   if (rc) return rc;
   CK(ag::launch_episode(episode_params(b), s));
   if (!b->autoreset_reset) return AGARCL_OK;
@@ -948,12 +947,13 @@ extern "C" int agarcl_batch_step_host(agarcl_batch* b, const float* dxdy, const 
   return AGARCL_OK;
 }
 
-// ---- host-resident observation mirror (mirror.cu)
-static int ensure_mirror(agarcl_batch* b) {
-  if (b->mirror) return AGARCL_OK;
+// ---- host-resident observation mirror (mirror.cu): b->mirror, or its lists-only twin b->lists, created on first use
+static int ensure_mirror(agarcl_batch* b, bool lists_only = false) {
+  ag::HostMirror*& m = lists_only ? b->lists : b->mirror;
+  if (m) return AGARCL_OK;
   CK(cudaSetDevice(b->cfg.device));
-  b->mirror = ag::mirror_create(b->N * b->A, b->A, b->frames * b->C, b->C, b->G, b->cfg.obs_dtype);
-  return b->mirror ? AGARCL_OK : AGARCL_ERR_NOMEM;
+  m = ag::mirror_create(b->N * b->A, b->A, b->frames * b->C, b->C, b->G, b->cfg.obs_dtype, lists_only);
+  return m ? AGARCL_OK : AGARCL_ERR_NOMEM;
 }
 
 extern "C" int agarcl_batch_sync_mirror(agarcl_batch* b, void* stream) {
@@ -980,18 +980,28 @@ extern "C" int agarcl_batch_mirror(agarcl_batch* b, void** host_ptr, int64_t sha
   return AGARCL_OK;
 }
 
+// One step of agarcl_batch_step_mirror (lists_only = false) or agarcl_batch_step_lists: the kernel reads the actions straight
+// from the host-mapped staging of b->mirror or b->lists (no H2D copy in front of the launch) and, when the step is the single
+// fused kernel, writes that HostMirror's lists (*lists_made).  A step that cannot write them is refused for the lists-only
+// twin, before anything is enqueued: the games do not move.
+static int staged_step(agarcl_batch* b, bool lists_only, const float* dxdy, const int32_t* act, bool* lists_made) {
+  if (!b || !dxdy || !act) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
+  if (int rc = refuse_pixels(b, lists_only ? "agarcl_batch_step_lists" : "agarcl_batch_step_mirror")) return rc;
+  if (lists_only && (b->frames != 1 || b->cfg.strict_reference || b->cfg.ram_obs == 2))
+    return agarcl_set_error(AGARCL_ERR_STATE, "observation lists need the single fused step kernel (one frame, strict_reference = 0, a grid observation)");
+  if (lists_only && !kernel_writes_lists(b))
+    return agarcl_set_error(AGARCL_ERR_STATE, "this observation configuration is not finished by the step kernel: no lists");
+  if (int rc = ensure_mirror(b, lists_only)) return rc;
+  ag::HostMirror* m = lists_only ? b->lists : b->mirror;
+  ag::mirror_stage_actions(m, dxdy, act, &b->cur_dxdy, &b->cur_act);
+  return step_impl(b, nullptr, m, lists_made);
+}
+
 extern "C" int agarcl_batch_step_mirror(agarcl_batch* b, const float* dxdy, const int32_t* act, double* rewards_out,
                                         uint8_t* dones_out) {
-  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
-  if (int rc = refuse_pixels(b, "agarcl_batch_step_mirror")) return rc;
-  int rc = ensure_mirror(b);
-  if (rc) return rc;
-  if (!dxdy || !act) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
-  // the kernel reads the actions straight from host-mapped staging: no H2D copy in front of the launch
   const auto t0 = std::chrono::steady_clock::now();
-  ag::mirror_stage_actions(b->mirror, dxdy, act, &b->cur_dxdy, &b->cur_act);
   bool lists_made = false;
-  rc = step_impl(b, nullptr, true, &lists_made);
+  int rc = staged_step(b, false, dxdy, act, &lists_made);
   if (rc) return rc;
   b->mirror_launch_us = (uint64_t)(std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count() * 1e6);
   if (lists_made) {  // k_step lists what it scatters (and reward / done) into pinned host memory while it runs
@@ -1010,22 +1020,11 @@ extern "C" int agarcl_batch_step_mirror(agarcl_batch* b, const float* dxdy, cons
 
 extern "C" int agarcl_batch_step_lists(agarcl_batch* b, const float* dxdy, const int32_t* act, double* rewards_out, uint8_t* dones_out,
                                        agarcl_obs_lists* out) {
-  if (!b || !dxdy || !act || !out) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
-  if (int rc = refuse_pixels(b, "agarcl_batch_step_lists")) return rc;
-  if (b->frames != 1 || b->cfg.strict_reference || b->cfg.ram_obs == 2)
-    return agarcl_set_error(AGARCL_ERR_STATE, "observation lists need the single fused step kernel (one frame, strict_reference = 0, a grid observation)");
-  if (!kernel_writes_lists(b))  // (refused before anything is enqueued: the games do not move)
-    return agarcl_set_error(AGARCL_ERR_STATE, "this observation configuration is not finished by the step kernel: no lists");
-  CK(cudaSetDevice(b->cfg.device));
-  if (!b->lists) {
-    b->lists = ag::mirror_create(b->N * b->A, b->A, b->frames * b->C, b->C, b->G, b->cfg.obs_dtype, true);
-    if (!b->lists) return AGARCL_ERR_NOMEM;
-  }
-  ag::mirror_stage_actions(b->lists, dxdy, act, &b->cur_dxdy, &b->cur_act);
+  if (!out) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
   bool lists_made = false;
-  int rc = step_impl(b, nullptr, true, &lists_made, b->lists);
+  int rc = staged_step(b, true, dxdy, act, &lists_made);
   if (rc) return rc;
-  if (!lists_made) {  // (kernel_writes_lists said it would)
+  if (!lists_made) {  // (staged_step refuses a step that would not write them)
     CK(cudaStreamSynchronize(nullptr));
     return agarcl_set_error(AGARCL_ERR_STATE, "the step kernel did not write the observation lists");
   }

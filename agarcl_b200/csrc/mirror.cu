@@ -191,6 +191,14 @@ __global__ void __launch_bounds__(kPackThreads) k_pack(const PackParams P) {
 }
 
 // ------------------------------------------------------------------------------------------------ host pool
+static inline void cpu_relax() {
+#if defined(__x86_64__) || defined(__i386__)
+  __builtin_ia32_pause();
+#else
+  std::this_thread::yield();
+#endif
+}
+
 // Every worker (and, from join() on, the caller) runs the same job, which pulls work from atomic counters.
 // Workers sleep on a condition variable between jobs; the END of a job is awaited by spinning on an atomic
 // (a futex wake-up of the caller would add tens of microseconds to every step).
@@ -219,13 +227,7 @@ class Pool {
   }
   void join() {  // the caller works too, then waits for the workers
     (*job_)();
-    while (pending_.load(std::memory_order_acquire) != 0) {
-#if defined(__x86_64__) || defined(__i386__)
-      __builtin_ia32_pause();
-#else
-      std::this_thread::yield();
-#endif
-    }
+    while (pending_.load(std::memory_order_acquire) != 0) cpu_relax();
     job_ = nullptr;
   }
   void run(const std::function<void()>& job) {
@@ -258,14 +260,6 @@ class Pool {
   bool stop_ = false;
 };
 
-static inline void cpu_relax() {
-#if defined(__x86_64__) || defined(__i386__)
-  __builtin_ia32_pause();
-#else
-  std::this_thread::yield();
-#endif
-}
-
 struct HostMirror {
   int n_img = 0, CH = 0, C = 0, G = 0, frames = 0, MW = 0, dtype = 0;
   size_t esz = 4, img_elems = 0, img_bytes = 0;
@@ -293,6 +287,11 @@ struct HostMirror {
   bool lists_only = false;        // no dense mirror: the lists themselves are the product (agarcl_batch_step_lists)
   MirrorStats stats{};
   uint32_t* blk(int w, int chunk) const { return h_chunks[w] + (size_t)chunk * pk.chunk_words; }
+  // the record of list slot `slot` in staging buffer `w`, and the entries it counts
+  const uint32_t* rec(int w, uint32_t slot) const { return blk(w, (int)(slot / pk.ipc)) + pk_off_rec(pk) + (size_t)(slot % pk.ipc) * pk.rec_words; }
+  const uint2* entries(int w, uint32_t slot) const {
+    return reinterpret_cast<const uint2*>(blk(w, (int)(slot / pk.ipc)) + pk_off_entries(pk)) + rec(w, slot)[1];
+  }
 };
 
 static inline bool bit(const uint32_t* m, int i) { return (m[i >> 5] >> (i & 31)) & 1u; }
@@ -322,126 +321,148 @@ static void apply_mask_delta(T* p, const uint32_t* om, const uint32_t* nm, int G
   }
 }
 
+// Replays one image's lists over its dense frames `p`, which hold the previous step's masks and no entries: the mask delta of
+// every frame from `om` (the previous masks; nullptr: nothing out of bounds), then the entries.  The library's one replay of
+// the list format: it must stay bit-identical to batch.py ObsLists.decode.  Forced inline: the mirror's host threads spend
+// their time in this loop.
+static const uint32_t kZeroMasks[2 * 128] = {};  // (G <= 4096, mirror_create)
+template <typename T>
+static __forceinline__ void replay_image(const HostMirror* m, T* p, const uint32_t* om, const uint32_t* nm, const uint2* ne, uint32_t n) {
+  const size_t mw2 = 2 * (size_t)m->MW, plane = (size_t)m->G * m->G;
+  for (int f = 0; f < m->frames; f++) {
+    const uint32_t* o = om ? om + f * mw2 : kZeroMasks;
+    if (std::memcmp(o, nm + f * mw2, mw2 * 4) != 0) apply_mask_delta<T>(p + (size_t)f * m->C * plane, o, nm + f * mw2, m->G, m->MW);
+  }
+  // (operands are masses / counts >= 0; the 16-bit dtype saturates exactly like the device's updates, sim_kernel.cu FinOps<int16_t>)
+  constexpr int32_t kTop = sizeof(T) == 2 ? 32767 : 2147483647;
+  for (uint32_t e = 0; e < n; e++) {
+    T& x = p[ne[e].x & kPkOffMask];
+    const int32_t v32 = (int32_t)ne[e].y;
+    const T v = (T)(v32 > kTop ? kTop : v32);
+    switch (ne[e].x >> 29) {
+      case kPkSet: x = v; break;
+      case kPkAdd: { const int64_t t = (int64_t)x + v32; x = (T)(t > kTop ? kTop : t); break; }
+      case kPkMinNz: x = (x != 0 && x < v) ? x : v; break;
+      default: x = x > v ? x : v; break;
+    }
+  }
+}
+
 // The elements an image's two lists touch are scattered over its 512 KB: ask for their cache lines (for writing)
 // one slot ahead, so that the misses of the next image overlap the read-modify-writes of this one.
 template <typename T>
 static void prefetch_slot(const HostMirror* m, int slot) {
   const int cur = m->cur, prev = cur ^ 1;
-  const PackOut& k = m->pk;
-  const uint32_t* cb = m->blk(cur, slot / (int)k.ipc);
-  const uint32_t* crec = cb + pk_off_rec(k) + (size_t)(slot % (int)k.ipc) * k.rec_words;
+  const uint32_t* crec = m->rec(cur, (uint32_t)slot);
   const uint32_t img = crec[2];
   if (img >= (uint32_t)m->n_img) return;
   const T* p = reinterpret_cast<const T*>(m->h_obs) + (size_t)img * m->img_elems;
   if (crec[0] != kPackDense) {
-    const uint2* e = reinterpret_cast<const uint2*>(cb + pk_off_entries(k)) + crec[1];
+    const uint2* e = m->entries(cur, (uint32_t)slot);
     for (uint32_t i = 0; i < crec[0]; i++) __builtin_prefetch(p + (e[i].x & kPkOffMask), 1, 1);
   }
   const uint32_t ps = m->slot_of[prev][img];
-  const uint32_t* pb = m->blk(prev, (int)(ps / k.ipc));
-  const uint32_t* prec = pb + pk_off_rec(k) + (size_t)(ps % k.ipc) * k.rec_words;
+  const uint32_t* prec = m->rec(prev, ps);
   if (prec[0] != kPackDense) {
-    const uint2* e = reinterpret_cast<const uint2*>(pb + pk_off_entries(k)) + prec[1];
+    const uint2* e = m->entries(prev, ps);
     for (uint32_t i = 0; i < prec[0]; i++) __builtin_prefetch(p + (e[i].x & kPkOffMask), 1, 1);
   }
 }
 
 // Slots [lo, hi) of the current lists: every slot names its image; the image's previous lists are found through slot_of.
 template <typename T>
-static void expand_range(HostMirror* m, int lo, int hi, const uint32_t* zero_masks) {
+static void expand_range(HostMirror* m, int lo, int hi) {
   const int cur = m->cur, prev = cur ^ 1;
-  const PackOut& k = m->pk;
-  const size_t mw2 = 2 * (size_t)m->MW, plane = (size_t)m->G * m->G;
   static const int ahead = [] { const char* e = std::getenv("AGARCL_MIRROR_PREFETCH"); return e ? std::atoi(e) : 1; }();
   for (int a = 0; a < ahead && lo + a < hi; a++) prefetch_slot<T>(m, lo + a);
   for (int slot = lo; slot < hi; slot++) {
     if (slot + ahead < hi) prefetch_slot<T>(m, slot + ahead);
-    const uint32_t* cb = m->blk(cur, slot / (int)k.ipc);
-    const uint32_t* crec = cb + pk_off_rec(k) + (size_t)(slot % (int)k.ipc) * k.rec_words;
+    const uint32_t* crec = m->rec(cur, (uint32_t)slot);
     const uint32_t img = crec[2];
     if (img >= (uint32_t)m->n_img) continue;  // (cannot happen with lists the kernels wrote)
-    const uint32_t ps = m->slot_of[prev][img];
-    m->slot_of[cur][img] = (uint32_t)slot;
-    const uint32_t* pb = m->blk(prev, (int)(ps / k.ipc));
-    const uint32_t* prec = pb + pk_off_rec(k) + (size_t)(ps % k.ipc) * k.rec_words;
     const uint32_t cnt = crec[0];
     if (cnt == kPackDense) continue;  // the dense copy of this image is made by the calling thread
+    const uint32_t ps = m->slot_of[prev][img];
+    const uint32_t* prec = m->rec(prev, ps);
     T* p = reinterpret_cast<T*>(m->h_obs) + (size_t)img * m->img_elems;
     const uint32_t pcnt = prec[0];
-    const uint32_t* om = prec + 3;
-    const uint32_t* nm = crec + 3;
     if (pcnt == kPackDense) {
       std::memset(p, 0, m->img_bytes);
-      om = nullptr;
     } else {
-      const uint2* pe = reinterpret_cast<const uint2*>(pb + pk_off_entries(k)) + prec[1];
+      const uint2* pe = m->entries(prev, ps);
       for (uint32_t e = 0; e < pcnt; e++) p[pe[e].x & kPkOffMask] = 0;
     }
-    for (int f = 0; f < m->frames; f++) {
-      const uint32_t* o = om ? om + f * mw2 : zero_masks;
-      if (std::memcmp(o, nm + f * mw2, mw2 * 4) != 0) apply_mask_delta<T>(p + (size_t)f * m->C * plane, o, nm + f * mw2, m->G, m->MW);
-    }
-    const uint2* ne = reinterpret_cast<const uint2*>(cb + pk_off_entries(k)) + crec[1];
-    // (operands are masses / counts >= 0; the 16-bit dtype saturates exactly like the device's updates, sim_kernel.cu FinOps<int16_t>)
-    constexpr int32_t kTop = sizeof(T) == 2 ? 32767 : 2147483647;
-    for (uint32_t e = 0; e < cnt; e++) {
-      T& x = p[ne[e].x & kPkOffMask];
-      const int32_t v32 = (int32_t)ne[e].y;
-      const T v = (T)(v32 > kTop ? kTop : v32);
-      switch (ne[e].x >> 29) {
-        case kPkSet: x = v; break;
-        case kPkAdd: { const int64_t t = (int64_t)x + v32; x = (T)(t > kTop ? kTop : t); break; }
-        case kPkMinNz: x = (x != 0 && x < v) ? x : v; break;
-        default: x = x > v ? x : v; break;
+    replay_image<T>(m, p, pcnt == kPackDense ? nullptr : prec + 3, crec + 3, m->entries(cur, (uint32_t)slot), cnt);
+  }
+}
+
+// The records of chunk `c` of this step's lists: checks the image each names and points slot_of at its slot, adds the chunk's
+// entries to *entries and its dense images to *dense, and copies the step's reward and done flag out of the records (k_step
+// writes them there; rewards_out / dones_out may be null).
+static int read_records(HostMirror* m, int c, uint64_t* entries, std::vector<int>* dense, double* rewards_out, uint8_t* dones_out) {
+  const PackOut& k = m->pk;
+  const int lo = c * (int)k.ipc, hi = lo + (int)k.ipc < m->n_img ? lo + (int)k.ipc : m->n_img;
+  for (int i = lo; i < hi; i++) {
+    const uint32_t* rec = m->rec(m->cur, (uint32_t)i);
+    const uint32_t img = rec[2];
+    if (img >= (uint32_t)m->n_img) return agarcl_set_error(AGARCL_ERR_STATE, "list slot %d names image %u of %d", i, img, m->n_img);
+    m->slot_of[m->cur][img] = (uint32_t)i;
+    if (rec[0] == kPackDense) dense->push_back((int)img);
+    else *entries += rec[0];
+    if (rewards_out) std::memcpy(rewards_out + img, rec + k.rec_words - 3, sizeof(double));
+    if (dones_out) dones_out[img] = (uint8_t)rec[k.rec_words - 1];
+  }
+  return AGARCL_OK;
+}
+
+// What k_step writes over PCIe for one step's lists: every record, every chunk flag and the entries.
+static uint64_t lists_d2h_bytes(const HostMirror* m, uint64_t entries) {
+  return (uint64_t)m->n_img * m->pk.rec_words * 4 + (uint64_t)m->n_chunks * 4 + entries * 8;
+}
+
+// Waits for the kernel launched on `s` with mirror_pack_out() to flag every chunk of this step in host-mapped memory, and calls
+// on_chunk(c) for each as its flag arrives (in any order); an error on_chunk returns ends the wait.  Between polls the thread
+// runs idle(), which returns whether it did a piece of other work (counted as 64 spins, a pause as one).  Every `query_spins`
+// spins the stream is queried, so that a failed launch cannot hang the caller.
+template <typename OnChunk, typename Idle>
+static int wait_chunks(HostMirror* m, cudaStream_t s, uint32_t query_spins, OnChunk&& on_chunk, Idle&& idle) {
+  const int K = m->n_chunks;
+  std::vector<uint8_t> seen((size_t)K, 0);
+  int left = K;
+  bool finished = false;  // the stream is complete: a chunk not flagged at the next poll never will be
+  for (uint32_t spins = 0; left > 0;) {
+    bool any = false;
+    for (int c = 0; c < K; c++)
+      if (!seen[(size_t)c] && m->h_flags[c] == m->seq) {
+        seen[(size_t)c] = 1; left--; any = true;
+        if (const int rc = on_chunk(c)) return rc;
       }
+    if (any) continue;
+    if (finished) return agarcl_set_error(AGARCL_ERR_STATE, "step kernel finished without completing every list chunk");
+    if (idle()) spins += 64u;
+    else { cpu_relax(); spins += 1u; }
+    if (spins >= query_spins) {
+      spins = 0u;
+      const cudaError_t q = cudaStreamQuery(s);
+      if (q == cudaSuccess) finished = true;
+      else if (q != cudaErrorNotReady) return agarcl_set_error(AGARCL_ERR_CUDA, "cudaStreamQuery failed: %s", cudaGetErrorString(q));
     }
   }
+  return AGARCL_OK;
 }
 
 // ---- the lists as the observation (agarcl_batch_step_lists): wait for every chunk flag of the launch that was handed
 // mirror_pack_out(); nothing is expanded.  rewards / dones come from the records.
 int mirror_collect_lists(HostMirror* m, cudaStream_t s, double* rewards_out, uint8_t* dones_out) {
   m->cur ^= 1;
-  const int cur = m->cur, K = m->n_chunks;
-  const PackOut& k = m->pk;
-  std::vector<uint8_t> seen((size_t)K, 0);
-  int left = K;
-  uint32_t spins = 0;
-  uint64_t entries = 0, dense = 0;
-  while (left > 0) {
-    bool any = false;
-    for (int c = 0; c < K; c++)
-      if (!seen[(size_t)c] && m->h_flags[c] == m->seq) {
-        seen[(size_t)c] = 1; left--; any = true;
-        const uint32_t* hb = m->blk(cur, c);
-        const int lo = c * (int)k.ipc, hi = lo + (int)k.ipc < m->n_img ? lo + (int)k.ipc : m->n_img;
-        for (int i = lo; i < hi; i++) {
-          const uint32_t* rec = hb + pk_off_rec(k) + (size_t)(i - lo) * k.rec_words;
-          const uint32_t img = rec[2];
-          if (img >= (uint32_t)m->n_img) return agarcl_set_error(AGARCL_ERR_STATE, "list slot %d names image %u of %d", i, img, m->n_img);
-          m->slot_of[cur][img] = (uint32_t)i;
-          if (rec[0] == kPackDense) dense++; else entries += rec[0];
-          if (rewards_out) std::memcpy(rewards_out + img, rec + k.rec_words - 3, sizeof(double));
-          if (dones_out) dones_out[img] = (uint8_t)rec[k.rec_words - 1];
-        }
-      }
-    if (any || left == 0) continue;
-    cpu_relax();
-    if (++spins >= 4096u) {
-      spins = 0u;
-      const cudaError_t q = cudaStreamQuery(s);
-      if (q == cudaSuccess) {
-        bool all = true;
-        for (int c = 0; c < K; c++) all = all && (seen[(size_t)c] || m->h_flags[c] == m->seq);
-        if (!all) return agarcl_set_error(AGARCL_ERR_STATE, "step kernel finished without completing every list chunk");
-      } else if (q != cudaErrorNotReady) {
-        return agarcl_set_error(AGARCL_ERR_CUDA, "cudaStreamQuery failed: %s", cudaGetErrorString(q));
-      }
-    }
-  }
+  uint64_t entries = 0;
+  std::vector<int> dense;
+  const int rc = wait_chunks(m, s, 4096u, [&](int c) { return read_records(m, c, &entries, &dense, rewards_out, dones_out); },
+                             [] { return false; });
+  if (rc) return rc;
   m->stats.entries = entries;
-  m->stats.dense_images = dense;
-  m->stats.d2h_bytes = (uint64_t)m->n_img * k.rec_words * 4 + entries * 8 + (uint64_t)K * 4;
+  m->stats.dense_images = dense.size();
+  m->stats.d2h_bytes = lists_d2h_bytes(m, entries);
   return AGARCL_OK;
 }
 
@@ -459,28 +480,11 @@ void mirror_lists_view(const HostMirror* m, agarcl_obs_lists* out) {
 // not fit its slot (the caller takes it from the device tensor), 0 otherwise.
 template <typename T>
 static int lists_expand_t(const HostMirror* m, int img, T* p) {
-  const PackOut& k = m->pk;
   const uint32_t slot = m->slot_of[m->cur][(size_t)img];
-  const uint32_t* cb = m->h_chunks[m->cur] + (size_t)(slot / k.ipc) * k.chunk_words;
-  const uint32_t* rec = cb + pk_off_rec(k) + (size_t)(slot % k.ipc) * k.rec_words;
+  const uint32_t* rec = m->rec(m->cur, slot);
   if (rec[0] == kPackDense) return 1;
   std::memset(p, 0, m->img_bytes);
-  std::vector<uint32_t> zero_masks(2 * (size_t)m->MW, 0u);
-  const size_t plane = (size_t)m->G * m->G, mw2 = 2 * (size_t)m->MW;
-  for (int f = 0; f < m->frames; f++) apply_mask_delta<T>(p + (size_t)f * m->C * plane, zero_masks.data(), rec + 3 + f * mw2, m->G, m->MW);
-  const uint2* ne = reinterpret_cast<const uint2*>(cb + pk_off_entries(k)) + rec[1];
-  constexpr int32_t kTop = sizeof(T) == 2 ? 32767 : 2147483647;
-  for (uint32_t e = 0; e < rec[0]; e++) {
-    T& x = p[ne[e].x & kPkOffMask];
-    const int32_t v32 = (int32_t)ne[e].y;
-    const T v = (T)(v32 > kTop ? kTop : v32);
-    switch (ne[e].x >> 29) {
-      case kPkSet: x = v; break;
-      case kPkAdd: { const int64_t t = (int64_t)x + v32; x = (T)(t > kTop ? kTop : t); break; }
-      case kPkMinNz: x = (x != 0 && x < v) ? x : v; break;
-      default: x = x > v ? x : v; break;
-    }
-  }
+  replay_image<T>(m, p, nullptr, rec + 3, m->entries(m->cur, slot), rec[0]);
   return 0;
 }
 int mirror_lists_expand(const HostMirror* m, int img, void* dense_out) {
@@ -654,7 +658,6 @@ static int collect(HostMirror* m, const void* d_obs, cudaStream_t s, bool flagge
   m->cur ^= 1;
   const int cur = m->cur, K = m->n_chunks;
   const PackOut& k = m->pk;
-  std::vector<uint32_t> zero_masks(2 * (size_t)m->MW, 0u);
   // Chunks become ready in ANY order (under the cost-sorted schedule the first positions are the most expensive
   // instances and finish late): the calling thread appends them to `ready`, the workers take tasks (a chunk's slots in
   // pieces of `grab`) in that order.
@@ -672,8 +675,8 @@ static int collect(HostMirror* m, const void* d_obs, cudaStream_t s, bool flagge
     const int base = c * (int)k.ipc, end = base + (int)k.ipc < m->n_img ? base + (int)k.ipc : m->n_img;
     const int lo = base + (i % tpc) * grab, hi = lo + grab < end ? lo + grab : end;
     if (lo < hi) {
-      if (m->dtype == AGARCL_OBS_I16) expand_range<int16_t>(m, lo, hi, zero_masks.data());
-      else expand_range<int32_t>(m, lo, hi, zero_masks.data());
+      if (m->dtype == AGARCL_OBS_I16) expand_range<int16_t>(m, lo, hi);
+      else expand_range<int32_t>(m, lo, hi);
     }
     return 1;
   };
@@ -698,56 +701,21 @@ static int collect(HostMirror* m, const void* d_obs, cudaStream_t s, bool flagge
     rc = agarcl_set_error(AGARCL_ERR_CUDA, "%s failed: %s", what, cudaGetErrorString(e));
   };
   // one chunk has arrived in host memory: its records (dense fallbacks, rewards, dones), then hand it to the workers
-  auto publish = [&](int c) {
-    const uint32_t* hb = m->blk(cur, c);
-    const int lo = c * (int)k.ipc, hi = lo + (int)k.ipc < m->n_img ? lo + (int)k.ipc : m->n_img;
-    for (int i = lo; i < hi; i++) {
-      const uint32_t* rec = hb + pk_off_rec(k) + (size_t)(i - lo) * k.rec_words;
-      const uint32_t img = rec[2];
-      if (img >= (uint32_t)m->n_img) { rc = agarcl_set_error(AGARCL_ERR_STATE, "mirror slot %d names image %u of %d", i, img, m->n_img); return; }
-      if (rec[0] == kPackDense) dense_imgs.push_back((int)img);
-      else entries += rec[0];
-      if (flagged) {  // reward and done flag of the step came with the record
-        if (rewards_out) std::memcpy(rewards_out + img, rec + k.rec_words - 3, sizeof(double));
-        if (dones_out) dones_out[img] = (uint8_t)rec[k.rec_words - 1];
-      }
-    }
-    if (flagged) d2h += (size_t)(hi - lo) * k.rec_words * 4 + 4;  // what the kernel wrote over PCIe: records + flag (entries below)
+  auto publish = [&](int c) -> int {
+    if (const int r = read_records(m, c, &entries, &dense_imgs, rewards_out, dones_out)) return r;
     const int r = n_ready.load(std::memory_order_relaxed);
     ready[(size_t)r] = c;
     n_ready.store(r + 1, std::memory_order_release);
     if (trace) std::fprintf(stderr, "chunk %d ready at %.0f us, workers at task %d of %d\n", c,
                             std::chrono::duration<double>(clk::now() - t0).count() * 1e6, next.load(), K * tpc);
+    return AGARCL_OK;
   };
   if (flagged) {
-    // the kernel flags finished chunks in host-mapped memory; keep an eye on the stream so that a failed launch cannot hang us
-    std::vector<uint8_t> seen((size_t)K, 0);
-    int left = K;
-    uint32_t spins = 0;
+    // the kernel flags finished chunks in host-mapped memory; the calling thread patches too while it waits for the next flag
     const auto w0 = clk::now();
-    while (left > 0 && rc == AGARCL_OK) {
-      bool any = false;
-      for (int c = 0; c < K && rc == AGARCL_OK; c++)
-        if (!seen[(size_t)c] && m->h_flags[c] == m->seq) {
-          seen[(size_t)c] = 1; left--; any = true;
-          publish(c);
-        }
-      if (any || left == 0) continue;
-      if (try_one() == 1) spins += 64u;  // the calling thread patches too while it waits for the next flag
-      else { cpu_relax(); spins += 1u; }
-      if (spins >= 1024u) {
-        spins = 0u;
-        const cudaError_t q = cudaStreamQuery(s);
-        if (q == cudaSuccess) {
-          bool all = true;
-          for (int c = 0; c < K; c++) all = all && (seen[(size_t)c] || m->h_flags[c] == m->seq);
-          if (!all) rc = agarcl_set_error(AGARCL_ERR_STATE, "step kernel finished without completing every mirror chunk");
-        } else if (q != cudaErrorNotReady) {
-          fail(q, "cudaStreamQuery");
-        }
-      }
-    }
+    rc = wait_chunks(m, s, 1024u, publish, [&] { return try_one() == 1; });
     wait_s = std::chrono::duration<double>(clk::now() - w0).count();
+    d2h = lists_d2h_bytes(m, entries);
   } else {
     for (int c = 0; c < K && rc == AGARCL_OK; c++) {  // k_pack left compact blocks in device memory: one copy each (a second one if the guess was short)
       const auto w0 = clk::now();
@@ -768,10 +736,9 @@ static int collect(HostMirror* m, const void* d_obs, cudaStream_t s, bool flagge
       }
       m->guess[c] = total + total / 8 + 1024;
       wait_s += std::chrono::duration<double>(clk::now() - w0).count();
-      publish(c);
+      rc = publish(c);
     }
   }
-  if (flagged) d2h += entries * 8;
   // images that do not fit the scheme: dense copies into the pinned mirror (the workers skip them); in the fused
   // path the frames are only known to be complete in device memory once the kernel has ended
   if (rc == AGARCL_OK && !dense_imgs.empty()) {
