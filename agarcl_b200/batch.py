@@ -389,6 +389,32 @@ class Batch:
                                                           C.byref(r), _vp(stream)))
         return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
 
+    def set_start_states(self, pool, start_slot=None, stream=0):
+        """start-state table: from now on every reset of instance i (reset, reset_device and the auto-reset of step_autoreset)
+        with start_slot[i] >= 0 begins the new episode in the game of pool slot start_slot[i], on the instance's own draw stream,
+        instead of spawning a fresh one (include/agarcl_b200.h, agarcl_batch_set_start_states).  start_slot: int32 CUDA tensor
+        of N entries (-1: spawn), copied on `stream`.  The batch holds on to the pool while it is set; slots saved into it later
+        are read as they are when a reset runs.  pool None: every reset spawns again."""
+        import torch
+        if pool is None:
+            _lib.check(_lib.lib().agarcl_batch_set_start_states(self._h, None, 0, None, _vp(stream)))
+            self._start_pool = None
+            return
+        n_slots = self._check_pool(pool)
+        self._check_device_tensor(start_slot, torch.int32, "start_slot", self.N)
+        _lib.check(_lib.lib().agarcl_batch_set_start_states(self._h, _vp(pool.data_ptr()), n_slots, _vp(start_slot.data_ptr()),
+                                                            _vp(stream)))
+        self._start_pool = pool
+
+    def start_result(self):
+        """view of the library-owned result u8 [N] of the latest reset with a start-state table: 0 not reset or spawned (slot
+        -1), 1 started from its slot, 2 slot rejected (out of range, not saved from this configuration, or a mode outside the
+        set) and spawned instead"""
+        import torch
+        r = _vp()
+        _lib.check(_lib.lib().agarcl_batch_start_result(self._h, C.byref(r)))
+        return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
+
     # ---- pictures of game states (include/agarcl_b200.h, agarcl_batch_draw)
     def draw(self, src=None, size=256, view="arena", out=None, stream=0):
         """RGB pictures uint8 [n, size, size, 3] of the current states, drawn on the device (enqueued on `stream`, no host

@@ -122,6 +122,12 @@ struct agarcl_batch {
   ag::SnapLayout snap;
   uint64_t fingerprint = 0;
   DevBuf<uint8_t> d_snap_result, d_snap_restored;
+  // start states of resets (agarcl_batch_set_start_states): the pool (nullptr: every reset spawns), a start slot per instance,
+  // the result of the latest reset with a table and the mask of the instances that reset spawns
+  const void* start_pool = nullptr;
+  int64_t start_pool_slots = 0;
+  DevBuf<int32_t> d_start_slot;
+  DevBuf<uint8_t> d_start_result, d_spawn;
   // mixed-task batch (cfg.task_modes != 0, include/agarcl_b200.h): current and pending task per instance, result of the last set_tasks
   DevBuf<int32_t> d_task_mode, d_task_max_steps, d_next_mode, d_next_max_steps;
   DevBuf<uint8_t> d_task_result;
@@ -441,6 +447,8 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
       (rc = alloc(b->d_perm, (size_t)b->N * sizeof(uint32_t))) || (rc = alloc(b->d_sched, 2 * sizeof(uint32_t))) ||
       (rc = alloc(b->d_fresh, (size_t)b->N, 1)) || (rc = alloc(b->d_flagbuf, 33 * sizeof(uint32_t))) ||
       (rc = alloc(b->d_snap_result, (size_t)b->N, 0)) || (rc = alloc(b->d_snap_restored, (size_t)b->N, 0)) ||
+      (rc = alloc(b->d_start_slot, (size_t)b->N * sizeof(int32_t))) || (rc = alloc(b->d_start_result, (size_t)b->N, 0)) ||
+      (rc = alloc(b->d_spawn, (size_t)b->N)) ||
       (L.cap_replay > 0 && (rc = alloc(b->d_replay, (size_t)b->N * L.cap_replay * sizeof(float), 0))) ||
       (cfg->ram_obs && (rc = alloc(b->d_ram, (size_t)b->N * L.P * AGARCL_RAM_RECORD * sizeof(float), 0))) ||
       (cfg->pixel_obs && (rc = alloc(b->d_pixels, b->pixel_bytes = NA * cfg->pixel_obs * cfg->pixel_obs * 3, 0))) ||
@@ -639,16 +647,31 @@ static ag::EpisodeParams episode_params(const agarcl_batch* b) {
   return E;
 }
 
+static ag::SnapParams snapshot_params(const agarcl_batch* b, const void* pool, int64_t pool_slots);
+
 // The masked reset: instances with d_mask[i] != 0 (device memory; nullptr = all).  Everything is enqueued on `s`; the
 // host neither reads the mask nor waits, except for refill_replay's draw cursor read-back under AGARCL_RNG_MT19937.
 // clear_episode: restart the episode counters of the reset instances (agarcl_batch_step_autoreset has done so already).
+// With start states, k_snapshot first loads the slots of the instances that have one and k_reset spawns the others; every
+// launch behind it treats both alike (mask dm).
 static int reset_impl(agarcl_batch* b, const uint8_t* dm, cudaStream_t s, bool clear_episode) {
   CK(cudaSetDevice(b->cfg.device));
+  const uint8_t* spawn = dm;
+  if (b->start_pool) {
+    ag::SnapParams S = snapshot_params(b, b->start_pool, b->start_pool_slots);
+    S.slot_of = b->d_start_slot;
+    S.result = b->d_start_result;
+    S.mask = dm;
+    S.spawn = b->d_spawn;
+    S.next_max_steps = b->d_next_max_steps;
+    CK(ag::launch_snapshot_start(S, s));
+    spawn = b->d_spawn;
+  }
   ag::ResetParams P;
   P.L = b->L;
   P.T = b->T;
   P.state = b->d_state;
-  P.mask = dm;
+  P.mask = spawn;
   P.seeds = b->d_seeds;
   P.replay = b->d_replay;
   P.fresh = b->d_fresh;
@@ -1137,12 +1160,13 @@ extern "C" int agarcl_batch_upload_state(agarcl_batch* b, int32_t instance, cons
 }
 
 // ---- snapshot pools (include/agarcl_b200.h): refusals are decided here, before anything is enqueued
-static int snapshot_check(agarcl_batch* b, const void* pool, int64_t pool_slots) {
+// need_reset: refused before the first reset (save and restore read or write a game; start states only name a pool)
+static int snapshot_check(agarcl_batch* b, const void* pool, int64_t pool_slots, bool need_reset = true) {
   if (b->cfg.strict_reference)
     return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot pools are refused under strict_reference: the player order belongs to the batch");
   if (b->cfg.rng_mode == AGARCL_RNG_MT19937)
     return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot pools are refused under AGARCL_RNG_MT19937: its generators live on the host");
-  if (!b->was_reset) return agarcl_set_error(AGARCL_ERR_STATE, "save / restore of states before reset()");
+  if (need_reset && !b->was_reset) return agarcl_set_error(AGARCL_ERR_STATE, "save / restore of states before reset()");
   if (!pool) return agarcl_set_error(AGARCL_ERR_INVALID, "null pool");
   if ((uintptr_t)pool & 15u) return agarcl_set_error(AGARCL_ERR_INVALID, "the pool must be 16-byte aligned");
   if (pool_slots < 1) return agarcl_set_error(AGARCL_ERR_INVALID, "pool_slots must be >= 1");
@@ -1184,6 +1208,29 @@ static ag::SnapParams snapshot_params(const agarcl_batch* b, const void* pool, i
   P.A = b->A;
   P.instance_base = b->cfg.instance_base;
   return P;
+}
+
+extern "C" int agarcl_batch_set_start_states(agarcl_batch* b, const void* pool, int64_t pool_slots, const int32_t* d_start_slot,
+                                             void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (!pool) {  // every reset spawns again
+    b->start_pool = nullptr;
+    b->start_pool_slots = 0;
+    return AGARCL_OK;
+  }
+  if (!d_start_slot) return agarcl_set_error(AGARCL_ERR_INVALID, "null start slot array");
+  int rc = snapshot_check(b, pool, pool_slots, false);
+  if (rc) return rc;
+  CK(cudaMemcpyAsync(b->d_start_slot, d_start_slot, (size_t)b->N * sizeof(int32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  b->start_pool = pool;
+  b->start_pool_slots = pool_slots;
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_start_result(agarcl_batch* b, uint8_t** d_result) {
+  if (!b || !d_result) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
+  *d_result = b->d_start_result;
+  return AGARCL_OK;
 }
 
 extern "C" int agarcl_batch_save_states(agarcl_batch* b, void* pool, int64_t pool_slots, const int32_t* d_src, const int32_t* d_slot,

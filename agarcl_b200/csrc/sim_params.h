@@ -223,7 +223,7 @@ struct SnapLayout {
   uint64_t ep_bytes, ram_bytes, obs_bytes;      // segment sizes; ram_bytes / obs_bytes 0 when the segment is not stored
   uint64_t slot_bytes;                          // a multiple of 128
 };
-constexpr int kSnapThreads = 512;  // threads of k_snapshot, one CTA per saved entry / restored instance
+constexpr int kSnapThreads = 512;  // threads of k_snapshot and k_start_states, one CTA per saved entry / restored or reset instance
 struct SnapParams {
   uint8_t* pool;             // pool_slots slots of slot_bytes
   int64_t pool_slots;
@@ -250,9 +250,15 @@ struct SnapParams {
   int32_t* task_max_steps;   // [N]
   int32_t task_modes;        // cfg.task_modes: a restored slot's mode must be in it
   int32_t N, A, instance_base;
+  // start states (agarcl_batch_set_start_states, k_start_states): in front of k_reset, instance i in `mask` (nullptr: all) <-
+  // slot slot_of[i] where >= 0, with the instance's draw stream; result is the start result, not the restore's
+  const uint8_t* mask;       // [N] the reset mask, or nullptr
+  uint8_t* spawn;            // [N] out: the mask k_reset spawns (reset and not started from a slot)
+  const int32_t* next_max_steps;  // [N] mixed-task batch: the pending step limit, which becomes the current one
 };
 cudaError_t launch_snapshot_save(const SnapParams& P, int n, cudaStream_t stream);
 cudaError_t launch_snapshot_restore(const SnapParams& P, cudaStream_t stream);
+cudaError_t launch_snapshot_start(const SnapParams& P, cudaStream_t stream);
 
 // Pictures of game states (draw_kernel.cu): the spec of include/agarcl_b200.h, agarcl_batch_draw.  k_draw draws arena views,
 // k_draw_views agent views and the pixel observation (cfg.pixel_obs)

@@ -1,5 +1,6 @@
 // snapshot_kernel.cu — batched save / restore of game states into a caller-owned pool of slots
-// (agarcl_batch_save_states / agarcl_batch_restore_states; slot layout: include/agarcl_b200.h, agarcl_snapshot_hdr).
+// (agarcl_batch_save_states / agarcl_batch_restore_states; slot layout: include/agarcl_b200.h, agarcl_snapshot_hdr), and the
+// start states of resets (agarcl_batch_set_start_states, k_start_states).
 // A slot is the instance's state blob plus what the blob does not hold: the episode record of the vector environment,
 // the ram records (a player with nothing in view keeps its previous one) and, with several frames, the observation
 // history.  One CTA per entry; nothing is read back by the host.
@@ -19,6 +20,60 @@ __device__ __forceinline__ void copy_segment(uint8_t* __restrict__ d, const uint
     return;
   }
   for (size_t k = threadIdx.x; k < n; k += blockDim.x) d[k] = s[k];
+}
+
+// Whether slot `slot` (at sl) holds a state this batch may load: in range, saved from this configuration, a mode of the set
+// (the restore below makes the same checks)
+__device__ __forceinline__ bool slot_valid(const SnapParams& P, int32_t slot, const uint8_t* sl) {
+  bool valid = slot < P.pool_slots;
+  if (valid) {
+    const agarcl_snapshot_hdr* h = reinterpret_cast<const agarcl_snapshot_hdr*>(sl);
+    valid = h->magic == AGARCL_SNAPSHOT_MAGIC && h->version == AGARCL_SNAPSHOT_VERSION && h->fingerprint == P.fingerprint &&
+            h->slot_bytes == P.S.slot_bytes;
+    if (valid && P.task_mode) valid = h->task_mode >= 0 && h->task_mode <= 10 && ((P.task_modes >> h->task_mode) & 1);
+  }
+  return valid;
+}
+
+// The start states of a reset (agarcl_batch_set_start_states), launched in front of k_reset: the game of the slot in place of a
+// spawn, on the instance's own draw stream, which goes on where the spawn would have drawn first.  Everything else about the
+// reset (episode counters, ram records, observation) is done by the launches behind k_reset with the reset mask, as for a
+// spawned instance.  A kernel of its own beside k_snapshot's two directions, whose code stays as it was.
+__global__ void __launch_bounds__(kSnapThreads) k_start_states(const __grid_constant__ SnapParams P) {
+  const int i = blockIdx.x, t = threadIdx.x, A = P.A;
+  const uint8_t reset = P.mask ? P.mask[i] : (uint8_t)1;
+  const int32_t slot = reset ? P.slot_of[i] : -1;
+  if (slot < 0) {  // not reset, or spawned
+    if (t == 0) { P.spawn[i] = reset; P.result[i] = 0; }
+    return;
+  }
+  const uint8_t* sl = P.pool + (uint64_t)slot * P.S.slot_bytes;
+  if (!slot_valid(P, slot, sl)) {  // rejected: spawned, as without a start state
+    if (t == 0) { P.spawn[i] = 1; P.result[i] = 2; }
+    return;
+  }
+  uint8_t* blob = P.state + (size_t)i * P.stride;
+  __shared__ uint32_t cursor;  // (in shared memory: nothing stays live in registers across the copy)
+  if (t == 0) cursor = P.fresh[i] ? 0u : reinterpret_cast<const agarcl_inst_hdr*>(blob + P.off_hdr)->rng_cursor;  // where k_reset would draw first
+  __syncthreads();  // the cursor is read before the blob is overwritten
+  copy_segment(blob, sl + P.S.off_blob, P.stride);
+  for (int a = t; a < A; a += blockDim.x) P.dones[(size_t)i * A + a] = 0;
+  __syncthreads();  // the slot's header is in place before it is patched
+  if (t == 0) {
+    agarcl_inst_hdr* hdr = reinterpret_cast<agarcl_inst_hdr*>(P.state + (size_t)i * P.stride + P.off_hdr);
+    const uint64_t seed = P.seeds[i];
+    hdr->seed_lo = (uint32_t)seed;
+    hdr->seed_hi = (uint32_t)(seed >> 32);
+    hdr->rng_cursor = cursor;
+    hdr->respawned_lo = 0; hdr->respawned_hi = 0;
+    if (P.task_mode) {  // the game's mode becomes the current one; the step limit belongs to the episode: the pending one
+      P.task_mode[i] = reinterpret_cast<const agarcl_snapshot_hdr*>(sl)->task_mode;
+      P.task_max_steps[i] = P.next_max_steps[i];
+    }
+    P.fresh[i] = 0;
+    P.spawn[i] = 0;
+    P.result[i] = 1;
+  }
 }
 
 template <bool kSave>
@@ -64,7 +119,7 @@ __global__ void __launch_bounds__(kSnapThreads) k_snapshot(const __grid_constant
     return;
   }
   const uint8_t* sl = P.pool + (uint64_t)slot * P.S.slot_bytes;
-  bool valid = slot < P.pool_slots;
+  bool valid = slot < P.pool_slots;  // (slot_valid, written out: this code predates it and keeps its SASS)
   if (valid) {
     const agarcl_snapshot_hdr* h = reinterpret_cast<const agarcl_snapshot_hdr*>(sl);
     valid = h->magic == AGARCL_SNAPSHOT_MAGIC && h->version == AGARCL_SNAPSHOT_VERSION && h->fingerprint == P.fingerprint &&
@@ -111,6 +166,11 @@ cudaError_t launch_snapshot_save(const SnapParams& P, int n, cudaStream_t stream
 
 cudaError_t launch_snapshot_restore(const SnapParams& P, cudaStream_t stream) {
   k_snapshot<false><<<P.N, kSnapThreads, 0, stream>>>(P);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_snapshot_start(const SnapParams& P, cudaStream_t stream) {
+  k_start_states<<<P.N, kSnapThreads, 0, stream>>>(P);
   return cudaGetLastError();
 }
 

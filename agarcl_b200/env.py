@@ -402,6 +402,11 @@ class BatchedGridEnvironment(_Base):
         """instance i <- pool slot slot_of[i] where >= 0; returns the result u8 [N] (Batch.restore_states)"""
         return self._ensure().restore_states(pool, slot_of, stream)
 
+    def set_start_states(self, pool, start_slot=None, stream=0):
+        """every reset of instance i with start_slot[i] >= 0 begins in pool slot start_slot[i] (Batch.set_start_states); pool
+        None: every reset spawns"""
+        self._ensure().set_start_states(pool, start_slot, stream)
+
     def set_tasks(self, mode, max_steps=None, stream=0):
         """the task each instance's next reset plays; returns the result u8 [N] (Batch.set_tasks)"""
         return self._ensure().set_tasks(mode, max_steps, stream)

@@ -247,6 +247,7 @@ class BatchedAgarioEnv:
         self._ep_batch = None
         self._ep = None
         self._task = None
+        self._start = None
 
     def seed(self, seed):
         self._env.seed(seed)
@@ -285,6 +286,8 @@ class BatchedAgarioEnv:
                 info["final_obs"] = self._final
         if self._task is not None:
             info["task"] = self._task
+        if self._start is not None:
+            info["start_result"] = self._start
         return self._obs(), rew.float(), done, torch.zeros_like(done), info
 
     def set_tasks(self, modes, number_steps=None):
@@ -311,6 +314,22 @@ class BatchedAgarioEnv:
         assert self._ep is not None, "Cannot call restore_states() before calling reset()"
         self._restore_result = self._env.restore_states(pool, slot_of)
         return self._obs()
+
+    def set_start_states(self, pool, slot_of=None):
+        """start states: from now on every reset of environment i with slot_of[i] >= 0 -- the auto-resets of step() and reset()
+        -- begins the new episode in the game of pool slot slot_of[i] instead of a fresh spawn (int32 CUDA tensor of n_envs
+        entries, -1: spawn; copied in stream order).  The new episode counts from 0 and continues the environment's own
+        draw stream, so episodes started from one slot differ where the game draws.  info["start_result"] (u8 [n_envs]) then
+        says how the last reset began: 0 not reset or spawned, 1 from its slot, 2 slot rejected and spawned.  pool None: every
+        reset spawns again.  A Go-Explore loop, for example:
+
+            archive = env.snapshot_pool(1024)
+            env.save_states(archive, cells_to_keep, archive_slots)            # whenever new cells are found
+            env.set_start_states(archive, chosen_slot_per_env)                # e.g. sampled by visit count, on the device
+            obs, rew, done, trunc, info = env.step(dxdy, act)                 # finished episodes return into their cells
+        """
+        self._env.set_start_states(pool, slot_of)
+        self._start = self._env.batch.start_result() if pool is not None else None
 
     def restore_result(self):
         """u8 [n_envs] of the last restore_states: 0 not requested, 1 restored, 2 rejected"""

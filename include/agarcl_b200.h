@@ -340,6 +340,36 @@ int agarcl_batch_save_states(agarcl_batch* b, void* pool, int64_t pool_slots, co
 /* instance i <- pool slot d_slot_of[i] where >= 0; *d_result = the library-owned u8 [N] result above; enqueued on stream */
 int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, int64_t pool_slots, const int32_t* d_slot_of,
                                 uint8_t** d_result, void* stream);
+/* Start states: episodes that begin in saved games (a Go-Explore return, start-state curricula, evaluation on fixed start
+ * positions, continual runs that begin mid-game).  A batch may hold a START-STATE TABLE: a pool and a start slot per instance.
+ * EVERY reset (agarcl_batch_reset, _reset_device, the reset inside _step_autoreset) of an instance whose start slot is >= 0 is a
+ * reset whose spawn is replaced by the slot's game:
+ *   game          the instance's blob becomes the slot's blob (tick, cells, timers, flags, done_sticky, player records)
+ *   draw stream   it goes on where a spawn would have drawn first: hdr.seed = the instance's seed, hdr.rng_cursor = 0 when the
+ *                 stream is fresh (seeded since its last reset), else the instance's cursor before the reset; the stream is then
+ *                 no longer fresh.  Successive episodes from one slot, and instances started from one slot, differ where the game
+ *                 draws; a slot's own stream is never reused.  hdr.respawned_lo / respawned_hi are cleared, as by a reset.
+ *   around it     exactly what a reset does: dones zeroed (rewards are not: step_autoreset returns the finished step's), episode
+ *                 counters restarted, ram records cleared, a grid observation cleared and rendered (pre_respawn 0) or the
+ *                 pictures drawn; with keep_final_obs the final observation is copied before the reset, as always.
+ *   ignored       the slot's episode record, ram records, observation history and source.
+ *   mixed tasks   the slot's task_mode becomes the current mode (the game belongs to it); the current step limit is the PENDING
+ *                 one (next_max_steps: the limit belongs to the episode); the pending mode is left as it is.
+ * A slot is checked as agarcl_batch_restore_states checks it (range, magic, version, fingerprint, slot bytes, a mode of the set);
+ * an instance whose slot fails is spawned exactly as without a table, and reported.  Instances with start slot -1 (any negative
+ * value), and every reset of a batch without a table, are untouched: game, stream, observation and counters bit for bit those of
+ * a spawn.  A reset with a table is one more launch (k_start_states, one CTA per instance) in front of k_reset.
+ *   agarcl_batch_set_start_states  pool NULL: no table (every reset spawns).  d_start_slot: device int32 [N], copied on `stream`
+ *                                  into a library-owned array (the caller may reuse its buffer).  The pool pointer is kept: it
+ *                                  must stay allocated while it is set, and slots saved into it later are read as they are when
+ *                                  a reset runs (stream order).  May be called before the first reset.  Refused with an error,
+ *                                  the table left as it was: strict_reference, AGARCL_RNG_MT19937, a misaligned pool or one that
+ *                                  is not device memory of cfg.device, pool_slots < 1, a NULL d_start_slot with a pool.
+ *   agarcl_batch_start_result      the library-owned u8 [N] result of the latest reset with a table: 0 not reset or spawned with
+ *                                  slot -1, 1 started from its slot, 2 slot rejected -> spawned fresh.  The restore result is
+ *                                  not touched by resets. */
+int agarcl_batch_set_start_states(agarcl_batch* b, const void* pool, int64_t pool_slots, const int32_t* d_start_slot, void* stream);
+int agarcl_batch_start_result(agarcl_batch* b, uint8_t** d_result);
 
 /* ---------------------------------------------------- pictures of game states, for people (render() and videos)
  * A picture is uint8 [S][S][3], RGB, row-major (HWC): row r is world y, column c world x, row 0 the smallest y.  S is a multiple of
