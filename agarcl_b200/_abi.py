@@ -63,6 +63,17 @@ class Layout(C.Structure):
                [("order", C.c_int32 * MAX_PLAYERS), ("bot_type", C.c_int32 * MAX_PLAYERS)]
 
 
+class ArchiveCfg(C.Structure):
+    """struct agarcl_archive_cfg"""
+    _fields_ = [(n, C.c_int32) for n in ("cells_per_side", "agent", "select", "pad")] + [("seed", C.c_uint64)]
+
+
+class Archive(C.Structure):
+    """struct agarcl_archive"""
+    _fields_ = [(n, C.c_void_p) for n in ("cell_of", "base_score", "base_length", "key_entry", "visits", "entry_key", "entry_score",
+                                          "entry_length", "entry_chosen", "counters")] + [("keys", C.c_int64), ("entries", C.c_int64)]
+
+
 CELL_DT = np.dtype([("x", "<f4"), ("y", "<f4"), ("vx", "<f4"), ("vy", "<f4"), ("svx", "<f4"), ("svy", "<f4"),
                     ("mass", "<u4"), ("id", "<u4"), ("recomb_tick", "<u4"), ("pad", "<u4", (3,))])
 VIRUS_DT = np.dtype([("x", "<f4"), ("y", "<f4"), ("mass", "<u4"), ("hits", "<i4"), ("vx", "<f4"), ("vy", "<f4"),

@@ -3,7 +3,7 @@ missing or a call fails: there is no CPU path in this package."""
 import ctypes as C
 import os
 
-from ._abi import Cfg, Layout
+from ._abi import Archive, ArchiveCfg, Cfg, Layout
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libagarcl_b200.so")
@@ -17,7 +17,7 @@ SYMBOLS = [
     "agarcl_batch_obs", "agarcl_batch_rewards", "agarcl_batch_dones", "agarcl_batch_step_host",
     "agarcl_batch_reset_device", "agarcl_batch_set_autoreset", "agarcl_batch_step_autoreset", "agarcl_batch_episode",
     "agarcl_snapshot_slot_bytes", "agarcl_batch_save_states", "agarcl_batch_restore_states",
-    "agarcl_batch_set_start_states", "agarcl_batch_start_result",
+    "agarcl_batch_set_start_states", "agarcl_batch_start_result", "agarcl_batch_set_archive", "agarcl_batch_archive",
     "agarcl_batch_set_tasks", "agarcl_batch_tasks", "agarcl_batch_draw", "agarcl_batch_bot_actions",
     "agarcl_batch_mirror", "agarcl_batch_sync_mirror", "agarcl_batch_step_mirror", "agarcl_batch_mirror_stats", "agarcl_batch_mirror_timing", "agarcl_batch_step_lists", "agarcl_batch_lists_expand",
     "agarcl_batch_download_state", "agarcl_batch_upload_state", "agarcl_batch_save_env_state", "agarcl_batch_load_env_state",
@@ -61,6 +61,8 @@ def lib():
         L.agarcl_batch_restore_states.argtypes = [_vp, _vp, C.c_int64, _vp, C.POINTER(_vp), _vp]
         L.agarcl_batch_set_start_states.argtypes = [_vp, _vp, C.c_int64, _vp, _vp]
         L.agarcl_batch_start_result.argtypes = [_vp, C.POINTER(_vp)]
+        L.agarcl_batch_set_archive.argtypes = [_vp, _vp, C.c_int64, C.POINTER(ArchiveCfg)]
+        L.agarcl_batch_archive.argtypes = [_vp, C.POINTER(Archive)]
         L.agarcl_batch_set_tasks.argtypes = [_vp, _vp, _vp, C.POINTER(_vp), _vp]
         L.agarcl_batch_tasks.argtypes = [_vp, _vp]
         L.agarcl_batch_draw.argtypes = [_vp, C.c_int32, C.c_int32, _vp, C.c_int32, _vp, _vp]

@@ -415,6 +415,44 @@ class Batch:
         _lib.check(_lib.lib().agarcl_batch_start_result(self._h, C.byref(r)))
         return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
 
+    # ---- Go-Explore cell archive (include/agarcl_b200.h, agarcl_batch_set_archive)
+    def set_archive(self, pool, cells_per_side=None, agent=0, select=True, seed=0):
+        """attaches a cleared archive whose entry e is pool slot e: every step_autoreset then files each game under its cell
+        (agent `agent`'s position on a cells_per_side^2 grid x log2 of its mass), keeps the best game of every cell in the pool
+        and, with select, starts every reset in a cell drawn with weight 1 / (1 + isqrt(times chosen)).  Needs set_autoreset
+        first; synchronises the device.  The batch holds on to the pool while attached.  pool None detaches the archive."""
+        from ._abi import ArchiveCfg
+        if pool is None:
+            _lib.check(_lib.lib().agarcl_batch_set_archive(self._h, None, 0, None))
+            if getattr(self, "_archive_select", False):
+                self._start_pool = None
+            self._archive_pool, self._archive_select = None, False
+            return
+        n_slots = self._check_pool(pool)
+        if cells_per_side is None:
+            raise _lib.AgarclError("cells_per_side is needed to attach an archive")
+        cfg = ArchiveCfg(cells_per_side=int(cells_per_side), agent=int(agent), select=int(bool(select)), pad=0,
+                         seed=int(seed) & 0xFFFFFFFFFFFFFFFF)
+        _lib.check(_lib.lib().agarcl_batch_set_archive(self._h, _vp(pool.data_ptr()), n_slots, C.byref(cfg)))
+        if select or getattr(self, "_archive_select", False):  # (an archive that selected gave the table back)
+            self._start_pool = pool if select else None
+        self._archive_pool = pool
+        self._archive_select = bool(select)
+
+    def archive(self):
+        """zero-copy device views of the archive: per instance cell_of (i32, -1 none), base_score (f64), base_length (i64); per
+        key [32 n^2] key_entry (i32, -1 none) and visits (u32); per entry [K] entry_key, entry_score, entry_length, entry_chosen
+        (u32); counters (u64 [3]: used, dropped, improved)"""
+        import torch
+        from ._abi import Archive
+        a = Archive()
+        _lib.check(_lib.lib().agarcl_batch_archive(self._h, C.byref(a)))
+        N, n_keys, K, dev = self.N, int(a.keys), int(a.entries), f"cuda:{self.cfg.device}"
+        spec = {"cell_of": (N, "<i4"), "base_score": (N, "<f8"), "base_length": (N, "<i8"), "key_entry": (n_keys, "<i4"),
+                "visits": (n_keys, "<u4"), "entry_key": (K, "<i4"), "entry_score": (K, "<f8"), "entry_length": (K, "<i8"),
+                "entry_chosen": (K, "<u4"), "counters": (3, "<u8")}
+        return {k: torch.as_tensor(_CudaView(getattr(a, k), (n,), t, self), device=dev) for k, (n, t) in spec.items()}
+
     # ---- pictures of game states (include/agarcl_b200.h, agarcl_batch_draw)
     def draw(self, src=None, size=256, view="arena", out=None, stream=0):
         """RGB pictures uint8 [n, size, size, 3] of the current states, drawn on the device (enqueued on `stream`, no host

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libagarcl_b200.so")
-SOURCES = ["sim_kernel.cu", "obs_kernel.cu", "ram_kernel.cu", "reset_kernel.cu", "episode_kernel.cu", "snapshot_kernel.cu", "draw_kernel.cu", "bot_kernel.cu", "batch.cu", "mirror.cu", "layout.cpp", "host_util.cpp", "snapshot.cpp"]
+SOURCES = ["sim_kernel.cu", "obs_kernel.cu", "ram_kernel.cu", "reset_kernel.cu", "episode_kernel.cu", "snapshot_kernel.cu", "archive_kernel.cu", "draw_kernel.cu", "bot_kernel.cu", "batch.cu", "mirror.cu", "layout.cpp", "host_util.cpp", "snapshot.cpp"]
 HEADERS = ["device_math.cuh", "block_copy.cuh", "mode_rules.h", "sim_params.h", "sim_shared.cuh", "host_util.h", "mirror.h", os.path.join("..", "..", "include", "agarcl_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-fmad=false",  # the reference host build has no FMA contraction (SURVEY Appendix A)

@@ -38,6 +38,19 @@ class DevBuf {
   T* p_ = nullptr;
 };
 
+// The Go-Explore cell archive of a batch (agarcl_batch_set_archive): its settings and device arrays (ArchiveParams)
+struct Archive {
+  const void* pool = nullptr;
+  int64_t K = 0;
+  agarcl_archive_cfg cfg;
+  int64_t keys = 0;  // 32 n^2
+  DevBuf<int32_t> cell_of, cand_key, save_slot, src, key_entry, entry_key;
+  DevBuf<double> base_score, cand_s, entry_score;
+  DevBuf<int64_t> base_length, cand_l, entry_length;
+  DevBuf<uint32_t> draws, visits, entry_chosen;
+  DevBuf<uint64_t> best_s, best_li, prefix, counters;
+};
+
 // The A/B knobs of the step (names, defaults and effects: DESIGN.md section 8), read from the environment when a batch is created
 struct Knobs {
   int fuse_clear = 2, sort_schedule = 1, auto_schedule = 1, tick_barrier = 6, dyn_stripes = 1, zero_chunks = 0;
@@ -128,6 +141,7 @@ struct agarcl_batch {
   int64_t start_pool_slots = 0;
   DevBuf<int32_t> d_start_slot;
   DevBuf<uint8_t> d_start_result, d_spawn;
+  std::unique_ptr<Archive> archive;  // Go-Explore cell archive (agarcl_batch_set_archive), nullptr: none
   // mixed-task batch (cfg.task_modes != 0, include/agarcl_b200.h): current and pending task per instance, result of the last set_tasks
   DevBuf<int32_t> d_task_mode, d_task_max_steps, d_next_mode, d_next_max_steps;
   DevBuf<uint8_t> d_task_result;
@@ -649,6 +663,30 @@ static ag::EpisodeParams episode_params(const agarcl_batch* b) {
 
 static ag::SnapParams snapshot_params(const agarcl_batch* b, const void* pool, int64_t pool_slots);
 
+static ag::ArchiveParams archive_params(const agarcl_batch* b, const uint8_t* mask) {
+  const Archive& a = *b->archive;
+  ag::ArchiveParams P;
+  P.L = b->L;
+  P.state = b->d_state;
+  P.dones = b->d_dones;
+  P.rewards = b->d_rewards;
+  P.ret = b->d_ret;
+  P.steps = b->d_steps;
+  P.N = b->N; P.A = b->A; P.agent = a.cfg.agent; P.n = a.cfg.cells_per_side; P.K = (int32_t)a.K;
+  P.instance_base = b->cfg.instance_base;
+  P.W = (float)b->cfg.arena_size;
+  P.seed = a.cfg.seed;
+  P.cell_of = a.cell_of; P.base_score = a.base_score; P.base_length = a.base_length;
+  P.cand_key = a.cand_key; P.cand_s = a.cand_s; P.cand_l = a.cand_l; P.save_slot = a.save_slot; P.draws = a.draws;
+  P.key_entry = a.key_entry; P.visits = a.visits; P.best_s = a.best_s; P.best_li = a.best_li;
+  P.entry_key = a.entry_key; P.entry_score = a.entry_score; P.entry_length = a.entry_length; P.entry_chosen = a.entry_chosen;
+  P.prefix = a.prefix; P.counters = a.counters;
+  P.mask = mask;
+  P.start_slot = b->d_start_slot;
+  P.start_result = (b->start_pool && b->start_pool == a.pool) ? b->d_start_result.get() : nullptr;
+  return P;
+}
+
 // The masked reset: instances with d_mask[i] != 0 (device memory; nullptr = all).  Everything is enqueued on `s`; the
 // host neither reads the mask nor waits, except for refill_replay's draw cursor read-back under AGARCL_RNG_MT19937.
 // clear_episode: restart the episode counters of the reset instances (agarcl_batch_step_autoreset has done so already).
@@ -657,6 +695,7 @@ static ag::SnapParams snapshot_params(const agarcl_batch* b, const void* pool, i
 static int reset_impl(agarcl_batch* b, const uint8_t* dm, cudaStream_t s, bool clear_episode) {
   CK(cudaSetDevice(b->cfg.device));
   const uint8_t* spawn = dm;
+  if (b->archive && b->archive->cfg.select) CK(ag::launch_archive_select(archive_params(b, dm), s));  // (the archive owns the table)
   if (b->start_pool) {
     ag::SnapParams S = snapshot_params(b, b->start_pool, b->start_pool_slots);
     S.slot_of = b->d_start_slot;
@@ -667,6 +706,7 @@ static int reset_impl(agarcl_batch* b, const uint8_t* dm, cudaStream_t s, bool c
     CK(ag::launch_snapshot_start(S, s));
     spawn = b->d_spawn;
   }
+  if (b->archive) CK(ag::launch_archive_base(archive_params(b, dm), s));
   ag::ResetParams P;
   P.L = b->L;
   P.T = b->T;
@@ -827,6 +867,7 @@ extern "C" int agarcl_batch_set_autoreset(agarcl_batch* b, int32_t max_steps, in
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
   if (max_steps < 0) return agarcl_set_error(AGARCL_ERR_INVALID, "max_steps must be >= 0 (0: no step limit)");
   if (keep_final_obs && !reset) return agarcl_set_error(AGARCL_ERR_INVALID, "keep_final_obs needs reset: nothing is overwritten without one");
+  if (!reset && b->archive) return agarcl_set_error(AGARCL_ERR_STATE, "an attached archive needs reset: detach it first");
   CK(cudaSetDevice(b->cfg.device));
   const size_t NA = (size_t)b->N * b->A;
   int rc;
@@ -856,6 +897,14 @@ extern "C" int agarcl_batch_step_autoreset(agarcl_batch* b, void* stream) {
   cudaStream_t s = (cudaStream_t)stream;
   int rc = step_impl(b, s, nullptr, nullptr);
   if (rc) return rc;
+  if (b->archive) {  // the archive sees the step's games and counters before the bookkeeping and the reset
+    const Archive& a = *b->archive;
+    CK(ag::launch_archive_update(archive_params(b, nullptr), s));
+    ag::SnapParams S = snapshot_params(b, a.pool, a.K);
+    S.src = a.src;
+    S.slot = a.save_slot;
+    CK(ag::launch_snapshot_save(S, b->N, s));
+  }
   CK(ag::launch_episode(episode_params(b), s));
   if (!b->autoreset_reset) return AGARCL_OK;
   if (b->keep_final) {  // the observation the finished episode ended on, before the reset overwrites it
@@ -1213,6 +1262,8 @@ static ag::SnapParams snapshot_params(const agarcl_batch* b, const void* pool, i
 extern "C" int agarcl_batch_set_start_states(agarcl_batch* b, const void* pool, int64_t pool_slots, const int32_t* d_start_slot,
                                              void* stream) {
   if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (b->archive && b->archive->cfg.select)
+    return agarcl_set_error(AGARCL_ERR_STATE, "the attached archive (select = 1) owns the start-state table");
   if (!pool) {  // every reset spawns again
     b->start_pool = nullptr;
     b->start_pool_slots = 0;
@@ -1230,6 +1281,64 @@ extern "C" int agarcl_batch_set_start_states(agarcl_batch* b, const void* pool, 
 extern "C" int agarcl_batch_start_result(agarcl_batch* b, uint8_t** d_result) {
   if (!b || !d_result) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
   *d_result = b->d_start_result;
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_set_archive(agarcl_batch* b, void* pool, int64_t pool_slots, const agarcl_archive_cfg* cfg) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (!pool) {  // detach; an archive that selected gives the start-state table back (no table)
+    if (b->archive && b->archive->cfg.select) { b->start_pool = nullptr; b->start_pool_slots = 0; }
+    b->archive.reset();
+    return AGARCL_OK;
+  }
+  if (!cfg) return agarcl_set_error(AGARCL_ERR_INVALID, "null archive configuration");
+  if (b->cfg.task_modes)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "archives are refused in mixed-task batches: a reset would need one selection per pending mode");
+  int rc = snapshot_check(b, pool, pool_slots, false);
+  if (rc) return rc;
+  if (!b->autoreset || !b->autoreset_reset)
+    return agarcl_set_error(AGARCL_ERR_STATE, "an archive needs agarcl_batch_set_autoreset with reset = 1 first");
+  if (cfg->cells_per_side < 1 || cfg->cells_per_side > 256) return agarcl_set_error(AGARCL_ERR_INVALID, "cells_per_side must be in [1, 256]");
+  if (cfg->agent < 0 || cfg->agent >= b->A) return agarcl_set_error(AGARCL_ERR_INVALID, "agent %d out of [0, %d)", cfg->agent, b->A);
+  if (cfg->select != 0 && cfg->select != 1) return agarcl_set_error(AGARCL_ERR_INVALID, "select must be 0 or 1");
+  if (pool_slots > ag::kArchiveMaxSlots)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "an archive holds at most %lld entries", (long long)ag::kArchiveMaxSlots);
+  std::unique_ptr<Archive> a(new (std::nothrow) Archive());
+  if (!a) return agarcl_set_error(AGARCL_ERR_NOMEM, "out of host memory");
+  a->pool = pool;
+  a->K = pool_slots;
+  a->cfg = *cfg;
+  a->keys = 32ll * cfg->cells_per_side * cfg->cells_per_side;
+  const size_t N = (size_t)b->N, K = (size_t)pool_slots, keys = (size_t)a->keys;
+  if ((rc = alloc(a->cell_of, N * 4, 0xFF)) || (rc = alloc(a->cand_key, N * 4, 0xFF)) || (rc = alloc(a->save_slot, N * 4, 0xFF)) ||
+      (rc = alloc(a->src, N * 4)) || (rc = alloc(a->base_score, N * 8, 0)) || (rc = alloc(a->base_length, N * 8, 0)) ||
+      (rc = alloc(a->cand_s, N * 8, 0)) || (rc = alloc(a->cand_l, N * 8, 0)) || (rc = alloc(a->draws, N * 4, 0)) ||
+      (rc = alloc(a->key_entry, keys * 4, 0xFF)) || (rc = alloc(a->visits, keys * 4, 0)) || (rc = alloc(a->best_s, keys * 8, 0)) ||
+      (rc = alloc(a->best_li, keys * 8, 0xFF)) || (rc = alloc(a->entry_key, K * 4, 0xFF)) || (rc = alloc(a->entry_score, K * 8, 0)) ||
+      (rc = alloc(a->entry_length, K * 8, 0)) || (rc = alloc(a->entry_chosen, K * 4, 0)) || (rc = alloc(a->prefix, K * 8, 0)) ||
+      (rc = alloc(a->counters, 3 * 8, 0)))
+    return rc;
+  std::vector<int32_t> iota(N);
+  for (size_t i = 0; i < N; i++) iota[i] = (int32_t)i;
+  CK(cudaMemcpy(a->src, iota.data(), N * 4, cudaMemcpyHostToDevice));
+  if (cfg->select) CK(cudaMemset(b->d_start_slot, 0xFF, N * 4));
+  CK(cudaDeviceSynchronize());
+  if (b->archive && b->archive->cfg.select && !cfg->select) { b->start_pool = nullptr; b->start_pool_slots = 0; }
+  if (cfg->select) { b->start_pool = pool; b->start_pool_slots = pool_slots; }
+  b->archive = std::move(a);
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_archive(agarcl_batch* b, agarcl_archive* out) {
+  if (!b || !out) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
+  if (!b->archive) return agarcl_set_error(AGARCL_ERR_STATE, "no archive attached (agarcl_batch_set_archive)");
+  Archive& a = *b->archive;
+  out->cell_of = a.cell_of; out->base_score = a.base_score; out->base_length = a.base_length;
+  out->key_entry = a.key_entry; out->visits = a.visits;
+  out->entry_key = a.entry_key; out->entry_score = a.entry_score; out->entry_length = a.entry_length; out->entry_chosen = a.entry_chosen;
+  out->counters = a.counters;
+  out->keys = a.keys;
+  out->entries = a.K;
   return AGARCL_OK;
 }
 
@@ -1258,6 +1367,11 @@ extern "C" int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, in
   ag::SnapParams P = snapshot_params(b, pool, pool_slots);
   P.slot_of = d_slot_of;
   CK(ag::launch_snapshot_restore(P, s));
+  if (b->archive) {  // a restored game is no trajectory of the archive's: its base restarts at (0, 0)
+    ag::ArchiveParams A = archive_params(b, b->d_snap_restored);
+    A.start_result = nullptr;
+    CK(ag::launch_archive_base(A, s));
+  }
   // a one-frame grid observation is re-rendered, as the step that produced the state showed it (respawned players still dead)
   if (renders_grid(b) && b->frames == 1 && (rc = render_frame(b, 0, s, 1, 0, b->d_snap_restored))) return rc;
   if (b->cfg.pixel_obs && (rc = render_pixels(b, s, 1, b->d_snap_restored))) return rc;

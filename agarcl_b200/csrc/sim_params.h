@@ -260,6 +260,49 @@ cudaError_t launch_snapshot_save(const SnapParams& P, int n, cudaStream_t stream
 cudaError_t launch_snapshot_restore(const SnapParams& P, cudaStream_t stream);
 cudaError_t launch_snapshot_start(const SnapParams& P, cudaStream_t stream);
 
+// Go-Explore cell archive (archive_kernel.cu): the spec of include/agarcl_b200.h, agarcl_batch_set_archive
+constexpr int kArchiveThreads = 1024;         // threads of the one-CTA kernels k_archive_commit and k_archive_select
+constexpr int64_t kArchiveMaxSlots = 65536;   // entries of an archive at most: k_archive_select scans their weights in one CTA
+struct ArchiveParams {
+  agarcl_layout L;
+  const uint8_t* state;      // N blobs, L.stride apart
+  const uint8_t* dones;      // [N*A] of the step, before the step limit is folded in
+  const double* rewards;     // [N*A]
+  const double* ret;         // [N*A] episode return before this step (episode bookkeeping)
+  const int64_t* steps;      // [N] episode steps before this step
+  int32_t N, A, agent, n, K, instance_base;
+  float W;
+  uint64_t seed;
+  // per instance
+  int32_t* cell_of;          // key of the instance's cell, -1: none
+  double* base_score;        // trajectory base of the running episode
+  int64_t* base_length;
+  int32_t* cand_key;         // this step: the key of a candidate, -1 otherwise
+  double* cand_s;            // this step: a candidate's trajectory score and length
+  int64_t* cand_l;
+  int32_t* save_slot;        // this step: the slot instance i is saved into, -1 none (k_snapshot<true>'s slot list)
+  uint32_t* draws;           // selection draws made so far
+  // per key [32 n^2]
+  int32_t* key_entry;
+  uint32_t* visits;
+  uint64_t* best_s;          // winner scratch, neutral 0: max of ordered_bits(score)
+  uint64_t* best_li;         // winner scratch, neutral ~0: min of (min(length, 2^32 - 1) << 32 | instance)
+  // per entry [K]
+  int32_t* entry_key;
+  double* entry_score;
+  int64_t* entry_length;
+  uint32_t* entry_chosen;
+  uint64_t* prefix;          // k_archive_select scratch: inclusive prefix sums of the weights
+  uint64_t* counters;        // [3] used, dropped, improved
+  // resets
+  const uint8_t* mask;       // [N] the instances reset (or restored), nullptr: all
+  int32_t* start_slot;       // [N] the batch's start-state table
+  const uint8_t* start_result;  // k_archive_base: the start result when the table is the archive's pool, else nullptr
+};
+cudaError_t launch_archive_update(const ArchiveParams& P, cudaStream_t stream);  // k_archive_cells + k_archive_commit
+cudaError_t launch_archive_select(const ArchiveParams& P, cudaStream_t stream);
+cudaError_t launch_archive_base(const ArchiveParams& P, cudaStream_t stream);
+
 // Pictures of game states (draw_kernel.cu): the spec of include/agarcl_b200.h, agarcl_batch_draw.  k_draw draws arena views,
 // k_draw_views agent views and the pixel observation (cfg.pixel_obs)
 struct DrawParams {

@@ -407,6 +407,14 @@ class BatchedGridEnvironment(_Base):
         None: every reset spawns"""
         self._ensure().set_start_states(pool, start_slot, stream)
 
+    def set_archive(self, pool, cells_per_side=None, agent=0, select=True, seed=0):
+        """attaches a Go-Explore cell archive whose entries are the slots of `pool` (Batch.set_archive); pool None detaches it"""
+        self._ensure().set_archive(pool, cells_per_side, agent, select, seed)
+
+    def archive(self):
+        """device views of the archive (Batch.archive)"""
+        return self._ensure().archive()
+
     def set_tasks(self, mode, max_steps=None, stream=0):
         """the task each instance's next reset plays; returns the result u8 [N] (Batch.set_tasks)"""
         return self._ensure().set_tasks(mode, max_steps, stream)

@@ -248,6 +248,8 @@ class BatchedAgarioEnv:
         self._ep = None
         self._task = None
         self._start = None
+        self._cell = None
+        self._archive_select = False
 
     def seed(self, seed):
         self._env.seed(seed)
@@ -288,6 +290,8 @@ class BatchedAgarioEnv:
             info["task"] = self._task
         if self._start is not None:
             info["start_result"] = self._start
+        if self._cell is not None:
+            info["cell"] = self._cell
         return self._obs(), rew.float(), done, torch.zeros_like(done), info
 
     def set_tasks(self, modes, number_steps=None):
@@ -321,15 +325,45 @@ class BatchedAgarioEnv:
         entries, -1: spawn; copied in stream order).  The new episode counts from 0 and continues the environment's own
         draw stream, so episodes started from one slot differ where the game draws.  info["start_result"] (u8 [n_envs]) then
         says how the last reset began: 0 not reset or spawned, 1 from its slot, 2 slot rejected and spawned.  pool None: every
-        reset spawns again.  A Go-Explore loop, for example:
+        reset spawns again.  A Go-Explore loop keeps its archive on the device with set_archive, which chooses the slots itself:
 
-            archive = env.snapshot_pool(1024)
-            env.save_states(archive, cells_to_keep, archive_slots)            # whenever new cells are found
-            env.set_start_states(archive, chosen_slot_per_env)                # e.g. sampled by visit count, on the device
-            obs, rew, done, trunc, info = env.step(dxdy, act)                 # finished episodes return into their cells
+            env.reset()
+            env.set_archive(1024, cells_per_side=16)                          # 1024 cells, each with its best game
+            for _ in range(steps):
+                obs, rew, done, trunc, info = env.step(dxdy, act)             # finished episodes return into chosen cells
+                bonus = env.archive()["visits"][info["cell"].clamp(min=0)]    # e.g. a count-based exploration bonus
         """
         self._env.set_start_states(pool, slot_of)
         self._start = self._env.batch.start_result() if pool is not None else None
+
+    def set_archive(self, slots, cells_per_side=None, agent=0, select=True, seed=0):
+        """attaches a Go-Explore cell archive of `slots` entries, in a pool of its own (snapshot_pool): every step() files each
+        game under its cell -- agent `agent`'s position on a cells_per_side^2 grid and log2 of its mass -- and keeps the best
+        game of every cell (highest trajectory score: the score of the cell the episode started from plus the episode's return,
+        then the shortest trajectory).  With select, every reset -- the auto-resets of step() and reset() -- returns to a cell
+        drawn with weight 1 / (1 + isqrt(times chosen)); info["start_result"] says which began in one.  info["cell"] (i32
+        [n_envs], -1: no cell) is every environment's cell after the step.  Nothing is read back by the host.  slots None
+        detaches it.  Call after reset(); archive() has the tables."""
+        assert self._ep is not None, "Cannot call set_archive() before calling reset()"
+        if slots is None:
+            self._env.set_archive(None)
+            self._cell = None
+            if self._archive_select:
+                self._start = None
+            self._archive_select = False
+            return
+        self._env.set_archive(self._env.snapshot_pool(slots), cells_per_side, agent, select, seed)
+        self._cell = self._env.archive()["cell_of"]
+        if select:
+            self._start = self._env.batch.start_result()
+        elif self._archive_select:
+            self._start = None
+        self._archive_select = bool(select)
+
+    def archive(self):
+        """device views of the archive (Batch.archive): cell_of, base_score, base_length, key_entry, visits, entry_key,
+        entry_score, entry_length, entry_chosen, counters (used, dropped, improved)"""
+        return self._env.archive()
 
     def restore_result(self):
         """u8 [n_envs] of the last restore_states: 0 not requested, 1 restored, 2 rejected"""

@@ -371,6 +371,75 @@ int agarcl_batch_restore_states(agarcl_batch* b, const void* pool, int64_t pool_
 int agarcl_batch_set_start_states(agarcl_batch* b, const void* pool, int64_t pool_slots, const int32_t* d_start_slot, void* stream);
 int agarcl_batch_start_result(agarcl_batch* b, uint8_t** d_result);
 
+/* Go-Explore cell archive: every agarcl_batch_step_autoreset files each game under its CELL and keeps, per cell, the best game
+ * seen in a snapshot slot; with select = 1 every reset returns to a chosen cell.  A Go-Explore loop is then step_autoreset in a
+ * loop: the host never waits and writes no archive code.
+ *   agarcl_batch_set_archive  attaches an archive of K = pool_slots entries to the batch; entry e is slot e of `pool` (caller-
+ *                             owned, the slot format above, kept while attached).  Attaching clears the archive (nothing is read
+ *                             from the pool); it allocates and synchronises the device.  pool NULL detaches it.
+ *   agarcl_batch_archive      device pointers of the arrays below; nothing of the archive is ever read back by the host.
+ * CELL of instance i after a step, for agent a = cfg.agent: none (-1) if the agent has no cells.  Otherwise m = the u32 total
+ * mass of its cells and (cx, cy) its centroid exactly as the agent view of agarcl_batch_draw defines it (fp32, cell order);
+ * bx = clamp((int)(cx * (float)n / W), 0, n - 1), by the same with cy (each operation one rounded fp32 operation, no FMA, the
+ * conversion truncates); mb = 31 - clz(m); key = (mb * n + by) * n + bx in [0, 32 n^2).
+ * CANDIDATES: instance i is one when it has a cell and no agent of it is done by the game in this step (agarcl_batch_dones,
+ * before the step limit: an instance truncated by the limit is still a candidate).  Its trajectory score is s_i =
+ * base_score[i] + (return[a] + reward[a]) (f64: the agent's episode return including this step's reward), its trajectory
+ * length l_i = base_length[i] + (steps + 1) (i64).  Every candidate adds 1 to visits[key].
+ * UPDATE, once per step_autoreset, behind the step and in front of the episode bookkeeping (it sees the games before any reset):
+ *   winner     per key with candidates: the highest s, then the lowest l, then the lowest instance index
+ *   new key    gets the next entry if fewer than K are in use; the entries created in one step are numbered after those in
+ *              use, in ascending order of their winner's instance.  When the archive is full the discovery is counted in
+ *              `dropped` and nothing is stored (its visits still count)
+ *   known key  its entry is replaced when s > score, or s == score and l < length; each replacement counts in `improved`
+ *   stored     a new or replaced entry takes (key, s, l), and the winner's game is saved into slot e exactly as
+ *              agarcl_batch_save_states would save it at that moment (header, blob, ram records, observation history; the
+ *              episode record holds the counters before this step's bookkeeping, and start states ignore it)
+ *   cell_of[i] the key, or -1: what a count-based exploration bonus reads (visits[cell_of])
+ * SELECTION (select = 1): the archive owns the start-state table (agarcl_batch_set_start_states returns AGARCL_ERR_STATE), and at
+ * every reset (agarcl_batch_reset, _reset_device, the reset inside _step_autoreset) each reset instance i draws an entry:
+ *   weight     w_e = floor(2^20 / (1 + isqrt(chosen_e))) for the entries in use (Go-Explore's 1 / sqrt(C + 1) in integers), from
+ *              the counts before this reset; W = sum of w_e (u64)
+ *   draw       Philox4x32-10 (the spawn generator) with key = (seed low, seed high word) and counter = (c_i, 0x41524348,
+ *              instance_base + i, 0), c_i = the draws instance i made before; x = word 0 | word 1 << 32; the pick is the first e
+ *              in entry order whose inclusive prefix sum of weights exceeds x mod W.  After the picks of the reset every
+ *              chosen_e grows by the instances that picked it.  With an empty archive the instance spawns (no draw).
+ *   start      the instance starts from slot e as start states define it (agarcl_batch_start_result reports it)
+ * With select = 0 the start-state table stays the caller's (a caller may fill it from the read-out).
+ * TRAJECTORY BASE: a reset instance that starts from a slot of the archive's pool (result 1, the slot an entry in use) gets
+ * base = (score_e, length_e) as they are at that reset; any other reset instance -- spawned, rejected, started from another pool --
+ * and every instance agarcl_batch_restore_states restores gets (0, 0).  Every launch is stream-ordered; no host wait.
+ * Refused with an error before anything is enqueued, the archive left as it was: strict_reference, AGARCL_RNG_MT19937, a
+ * mixed-task batch (task_modes != 0: a reset would need one selection per pending mode; not supported), a call before
+ * agarcl_batch_set_autoreset or with its reset = 0 (agarcl_batch_set_autoreset(reset = 0) is refused while one is attached),
+ * cells_per_side outside [1, 256], agent outside [0, A), select not 0 or 1, a pool that is misaligned or not device memory of
+ * cfg.device, pool_slots < 1 or > 65536 (the selection scans the weights in one CTA).
+ * A batch without an archive launches nothing new.  With one, step_autoreset adds k_archive_cells, k_archive_commit and the save
+ * (k_snapshot, one CTA per instance: those of the non-winners exit at once), every reset k_archive_base, and with select = 1
+ * k_archive_select (one CTA; it exits at once when nothing resets) and k_start_states. */
+typedef struct agarcl_archive_cfg {
+  int32_t cells_per_side;  /* n, 1..256 */
+  int32_t agent;           /* whose cell it is, 0..A-1 */
+  int32_t select;          /* 1: the archive chooses the start slot of every reset; 0: the caller's start-state table */
+  int32_t pad;
+  uint64_t seed;           /* Philox key of the selection */
+} agarcl_archive_cfg;
+typedef struct agarcl_archive {
+  int32_t* cell_of;        /* [N] key of the instance's cell after the last step, -1: none */
+  double* base_score;      /* [N] trajectory base of the running episode */
+  int64_t* base_length;    /* [N] */
+  int32_t* key_entry;      /* [32 n^2] entry of a key, -1: none */
+  uint32_t* visits;        /* [32 n^2] candidates seen in the key */
+  int32_t* entry_key;      /* [K] key of entry e (entries [0, used) are in use) */
+  double* entry_score;     /* [K] best trajectory score of the cell */
+  int64_t* entry_length;   /* [K] its trajectory length */
+  uint32_t* entry_chosen;  /* [K] selections of the entry */
+  uint64_t* counters;      /* [3] used, dropped, improved */
+  int64_t keys, entries;   /* 32 n^2, K */
+} agarcl_archive;
+int agarcl_batch_set_archive(agarcl_batch* b, void* pool, int64_t pool_slots, const agarcl_archive_cfg* cfg);
+int agarcl_batch_archive(agarcl_batch* b, agarcl_archive* out);
+
 /* ---------------------------------------------------- pictures of game states, for people (render() and videos)
  * A picture is uint8 [S][S][3], RGB, row-major (HWC): row r is world y, column c world x, row 0 the smallest y.  S is a multiple of
  * 16 in [16, 2048].  It is drawn from the state blob as it is at the call: players respawned at the end of the last step are drawn
