@@ -42,17 +42,7 @@ class Cfg(C.Structure):
         "reward_type", "c_death", "mode_number",
         "num_frames", "grid_size", "observe_cells", "observe_others", "observe_viruses", "observe_pellets",
         "obs_dtype", "strict_reference", "rng_mode",
-        "cap_viruses", "cap_foods", "cap_replay", "device", "instance_base", "ram_obs", "task_modes")] + [("reserved", C.c_int32 * 1)]
-
-    # the header's last field, pixel_obs, took the place of `reserved[1]`; the ctypes field keeps that name, so code that names
-    # it keeps working, and pixel_obs reads and writes it
-    @property
-    def pixel_obs(self):
-        return self.reserved[0]
-
-    @pixel_obs.setter
-    def pixel_obs(self, v):
-        self.reserved[0] = v
+        "cap_viruses", "cap_foods", "cap_replay", "device", "instance_base", "ram_obs", "task_modes", "pixel_obs")]
 
 
 class Layout(C.Structure):

@@ -7,9 +7,10 @@ This is the host-side mirror of the batched hot path.  Device buffers are owned 
 import ctypes as C
 
 import numpy as np
+import torch
 
 from . import _lib
-from ._abi import OBS_I16, Layout, StateView
+from ._abi import DRAW_VIEWS, FLAG_NAMES, OBS_I16, RAM_RECORD, Archive, ArchiveCfg, Layout, StateView
 
 _vp = C.c_void_p
 
@@ -141,6 +142,14 @@ class Batch:
         except Exception:
             pass
 
+    @property
+    def _device(self):
+        return torch.device("cuda", self.cfg.device)
+
+    def _tensor(self, ptr, shape, typestr):
+        """zero-copy torch view of library-owned device memory (typestr: numpy's, "<f4"); it keeps the batch alive"""
+        return torch.as_tensor(_CudaView(ptr, shape, typestr, self), device=self._device)
+
     # ---- reference-shaped calls
     def seed(self, seeds):
         s = np.ascontiguousarray(np.broadcast_to(np.asarray(seeds, dtype=np.uint64), (self.N,)) if np.ndim(seeds) else
@@ -151,21 +160,15 @@ class Batch:
         m = None
         if mask is not None:
             m = np.ascontiguousarray(mask, dtype=np.uint8)
-            assert m.size == self.N
+            if m.size != self.N:
+                raise _lib.AgarclError(f"the reset mask must have {self.N} entries (one per instance), got {m.size}")
         _lib.check(_lib.lib().agarcl_batch_reset(self._h, m.ctypes.data_as(_vp) if m is not None else None, _vp(stream)))
         if m is None:  # strict_reference: the player order of the new episode (quirk Q3)
             _lib.check(_lib.lib().agarcl_batch_get_layout(self._h, C.byref(self.layout)))
 
     def reset_device(self, mask, stream=0):
         """masked reset with a CUDA uint8 / bool tensor of N entries: read by the device, the host does not wait"""
-        import torch
-        dev = torch.device("cuda", self.cfg.device)
-        if not (isinstance(mask, torch.Tensor) and mask.is_cuda and mask.device == dev):
-            raise _lib.AgarclError(f"the reset mask must be a tensor on {dev}")
-        if mask.dtype not in (torch.uint8, torch.bool):
-            raise _lib.AgarclError(f"the reset mask must be uint8 or bool, got {mask.dtype}")
-        if not mask.is_contiguous() or mask.numel() != self.N:
-            raise _lib.AgarclError(f"the reset mask must be contiguous with {self.N} entries (one per instance)")
+        self._check_device_tensor(mask, (torch.uint8, torch.bool), "the reset mask", self.N)
         _lib.check(_lib.lib().agarcl_batch_reset_device(self._h, _vp(mask.data_ptr()), _vp(stream)))
 
     def set_autoreset(self, max_steps=0, keep_final_obs=False, reset=True):
@@ -189,35 +192,35 @@ class Batch:
         """zero-copy device views of the episode buffers, overwritten by every step_autoreset: done (u8 [N*A]), reset_mask
         (u8 [N]), steps (i64 [N]), episode_return (f64 [N*A]) and episode_length (i64 [N]); the last two hold each instance's
         last finished episode, to be read where reset_mask is set"""
-        import torch
-        e, N, NA, dev = self._episode_struct(), self.N, self.N * self.A, f"cuda:{self.cfg.device}"
-        view = lambda p, n, t: torch.as_tensor(_CudaView(p, (n,), t, self), device=dev)  # noqa: E731
-        return {"done": view(e.done_out, NA, "|u1"), "reset_mask": view(e.reset_mask, N, "|u1"), "steps": view(e.steps, N, "<i8"),
-                "episode_return": view(e.final_return, NA, "<f8"), "episode_length": view(e.final_length, N, "<i8")}
+        e, N, NA = self._episode_struct(), self.N, self.N * self.A
+        return {"done": self._tensor(e.done_out, (NA,), "|u1"), "reset_mask": self._tensor(e.reset_mask, (N,), "|u1"),
+                "steps": self._tensor(e.steps, (N,), "<i8"), "episode_return": self._tensor(e.final_return, (NA,), "<f8"),
+                "episode_length": self._tensor(e.final_length, (N,), "<i8")}
 
     def final_obs(self):
         """observation images [N*A, frames*C, G, G] the reset instances of the last step_autoreset ended their episode on"""
-        import torch
         e = self._episode_struct()
         if not e.final_obs:
             raise _lib.AgarclError("no final observation images: set_autoreset(keep_final_obs=True) with a grid observation")
-        return torch.as_tensor(_CudaView(e.final_obs, self.obs_shape, "<i2" if self.obs_dtype == np.int16 else "<i4", self),
-                               device=f"cuda:{self.cfg.device}")
+        return self._tensor(e.final_obs, self.obs_shape, np.dtype(self.obs_dtype).str)
 
     def final_ram(self):
         """ram records [N, P, RAM_RECORD] float32 the reset instances of the last step_autoreset ended their episode on"""
-        import torch
-        from ._abi import RAM_RECORD
         e = self._episode_struct()
         if not e.final_ram:
             raise _lib.AgarclError("no final ram records: set_autoreset(keep_final_obs=True) with cfg.ram_obs")
-        return torch.as_tensor(_CudaView(e.final_ram, (self.N, self.layout.P, RAM_RECORD), "<f4", self),
-                               device=f"cuda:{self.cfg.device}")
+        return self._tensor(e.final_ram, (self.N, self.layout.P, RAM_RECORD), "<f4")
 
     def set_actions(self, dxdy, act, stream=0):
-        dxdy = np.ascontiguousarray(dxdy, dtype=np.float32)
-        act = np.ascontiguousarray(act, dtype=np.int32)
-        assert dxdy.size == self.N * self.A * 2 and act.size == self.N * self.A, "Number of actions does not match number of agents"
+        """the actions of the next step: dxdy [N*A, 2] float32 and act [N*A] int32, as host arrays (converted and copied) or as
+        CUDA tensors on the batch's device (read by the device in place, so they are not converted: another dtype is refused)"""
+        if isinstance(dxdy, torch.Tensor) or isinstance(act, torch.Tensor):
+            self._check_device_tensor(dxdy, torch.float32, "dxdy")
+            self._check_device_tensor(act, torch.int32, "act")
+            self._check_action_sizes(dxdy.numel(), act.numel())
+            self.set_actions_device(dxdy.data_ptr(), act.data_ptr(), stream)
+            return
+        dxdy, act = self._host_actions(dxdy, act)
         _lib.check(_lib.lib().agarcl_batch_set_actions(self._h, dxdy.ctypes.data_as(_vp), act.ctypes.data_as(_vp), 0, _vp(stream)))
 
     def set_actions_device(self, dxdy_ptr, act_ptr, stream=0):
@@ -234,17 +237,20 @@ class Batch:
 
     def ram_tensor(self):
         """structured observation records [N, P, RAM_RECORD] float32 on the device (cfg.ram_obs)"""
-        import torch
         p, shape = _vp(), (C.c_int64 * 3)()
         _lib.check(_lib.lib().agarcl_batch_ram(self._h, C.byref(p), C.byref(shape)))
-        return torch.as_tensor(_CudaView(p.value, tuple(shape), "<f4", self), device=f"cuda:{self.cfg.device}")
+        return self._tensor(p.value, tuple(shape), "<f4")
+
+    def _check_action_sizes(self, n_dxdy, n_act):
+        """the C ABI reads N*A (dx, dy) float32 pairs and N*A int32 actions"""
+        if n_dxdy != self.N * self.A * 2 or n_act != self.N * self.A:
+            raise _lib.AgarclError(f"Number of actions does not match number of agents ({self.N * self.A})")
 
     def _host_actions(self, dxdy, act):
         """the C ABI reads raw float32 / int32 buffers: coerce (and check the sizes of) whatever the caller hands in"""
         dxdy = np.ascontiguousarray(dxdy, dtype=np.float32)
         act = np.ascontiguousarray(act, dtype=np.int32)
-        if dxdy.size != self.N * self.A * 2 or act.size != self.N * self.A:
-            raise _lib.AgarclError("Number of actions does not match number of agents")
+        self._check_action_sizes(dxdy.size, act.size)
         return dxdy, act
 
     @staticmethod
@@ -325,7 +331,6 @@ class Batch:
 
     def flags(self, stream=0):
         """(OR of hdr.flags over all instances, {flag name: instances with it set}); reduced on the device"""
-        from ._abi import FLAG_NAMES
         o, counts = C.c_uint32(), (C.c_uint32 * 32)()
         _lib.check(_lib.lib().agarcl_batch_flags(self._h, _vp(stream), C.byref(o), C.byref(counts)))
         return int(o.value), {FLAG_NAMES.get(1 << i, f"bit{i}"): int(counts[i]) for i in range(32) if counts[i]}
@@ -340,25 +345,23 @@ class Batch:
 
     def snapshot_pool(self, slots):
         """a zeroed pool of `slots` slots: torch.uint8 [slots, slot_bytes] on the batch's device"""
-        import torch
         if int(slots) < 1:
             raise _lib.AgarclError("a pool needs at least one slot")
-        return torch.zeros((int(slots), self.slot_bytes), dtype=torch.uint8, device=f"cuda:{self.cfg.device}")
+        return torch.zeros((int(slots), self.slot_bytes), dtype=torch.uint8, device=self._device)
 
     def _check_device_tensor(self, t, dtype, what, numel=None):
-        import torch
-        dev = torch.device("cuda", self.cfg.device)
-        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.device == dev):
-            raise _lib.AgarclError(f"{what} must be a tensor on {dev}")
-        if t.dtype != dtype:
-            raise _lib.AgarclError(f"{what} must be {dtype}, got {t.dtype}")
+        """refuses what the library could not read as `what`: dtype is a torch dtype or a tuple of those allowed"""
+        dtypes = dtype if isinstance(dtype, tuple) else (dtype,)
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.device == self._device):
+            raise _lib.AgarclError(f"{what} must be a tensor on {self._device}")
+        if t.dtype not in dtypes:
+            raise _lib.AgarclError(f"{what} must be {' or '.join(str(d).removeprefix('torch.') for d in dtypes)}, got {t.dtype}")
         if not t.is_contiguous():
-            raise _lib.AgarclError(f"{what} must be contiguous")
+            raise _lib.AgarclError(f"{what} must be contiguous" + (f" with {numel} entries" if numel is not None else ""))
         if numel is not None and t.numel() != numel:
             raise _lib.AgarclError(f"{what} must have {numel} entries, got {t.numel()}")
 
     def _check_pool(self, pool):
-        import torch
         self._check_device_tensor(pool, torch.uint8, "the pool")
         if pool.dim() != 2 or pool.shape[1] != self.slot_bytes or pool.shape[0] < 1:
             raise _lib.AgarclError(f"the pool must be [slots >= 1, {self.slot_bytes}] (slot bytes of this configuration), "
@@ -368,7 +371,6 @@ class Batch:
     def save_states(self, pool, src, slots=None, stream=0):
         """pool slot slots[k] (None: slot k) <- instance src[k], for every k; int32 CUDA tensors; enqueued on `stream`, no host
         wait.  A slot index out of range is skipped; a source out of range leaves a slot that restores reject."""
-        import torch
         n_slots = self._check_pool(pool)
         self._check_device_tensor(src, torch.int32, "src")
         n = src.numel()
@@ -381,13 +383,12 @@ class Batch:
         """instance i <- pool slot slot_of[i] wherever slot_of[i] >= 0 (int32 CUDA tensor of N entries); enqueued on `stream`,
         no host wait.  Returns a view of the library-owned result u8 [N] (0 not requested, 1 restored, 2 rejected: the slot
         index is out of range or the slot was not saved from this configuration), which the next restore overwrites."""
-        import torch
         n_slots = self._check_pool(pool)
         self._check_device_tensor(slot_of, torch.int32, "slot_of", self.N)
         r = _vp()
         _lib.check(_lib.lib().agarcl_batch_restore_states(self._h, _vp(pool.data_ptr()), n_slots, _vp(slot_of.data_ptr()),
                                                           C.byref(r), _vp(stream)))
-        return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
+        return self._tensor(r.value, (self.N,), "|u1")
 
     def set_start_states(self, pool, start_slot=None, stream=0):
         """start-state table: from now on every reset of instance i (reset, reset_device and the auto-reset of step_autoreset)
@@ -395,7 +396,6 @@ class Batch:
         instead of spawning a fresh one (include/agarcl_b200.h, agarcl_batch_set_start_states).  start_slot: int32 CUDA tensor
         of N entries (-1: spawn), copied on `stream`.  The batch holds on to the pool while it is set; slots saved into it later
         are read as they are when a reset runs.  pool None: every reset spawns again."""
-        import torch
         if pool is None:
             _lib.check(_lib.lib().agarcl_batch_set_start_states(self._h, None, 0, None, _vp(stream)))
             self._start_pool = None
@@ -410,10 +410,9 @@ class Batch:
         """view of the library-owned result u8 [N] of the latest reset with a start-state table: 0 not reset or spawned (slot
         -1), 1 started from its slot, 2 slot rejected (out of range, not saved from this configuration, or a mode outside the
         set) and spawned instead"""
-        import torch
         r = _vp()
         _lib.check(_lib.lib().agarcl_batch_start_result(self._h, C.byref(r)))
-        return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
+        return self._tensor(r.value, (self.N,), "|u1")
 
     # ---- Go-Explore cell archive (include/agarcl_b200.h, agarcl_batch_set_archive)
     def set_archive(self, pool, cells_per_side=None, agent=0, select=True, seed=0):
@@ -421,7 +420,6 @@ class Batch:
         (agent `agent`'s position on a cells_per_side^2 grid x log2 of its mass), keeps the best game of every cell in the pool
         and, with select, starts every reset in a cell drawn with weight 1 / (1 + isqrt(times chosen)).  Needs set_autoreset
         first; synchronises the device.  The batch holds on to the pool while attached.  pool None detaches the archive."""
-        from ._abi import ArchiveCfg
         if pool is None:
             _lib.check(_lib.lib().agarcl_batch_set_archive(self._h, None, 0, None))
             if getattr(self, "_archive_select", False):
@@ -443,15 +441,13 @@ class Batch:
         """zero-copy device views of the archive: per instance cell_of (i32, -1 none), base_score (f64), base_length (i64); per
         key [32 n^2] key_entry (i32, -1 none) and visits (u32); per entry [K] entry_key, entry_score, entry_length, entry_chosen
         (u32); counters (u64 [3]: used, dropped, improved)"""
-        import torch
-        from ._abi import Archive
         a = Archive()
         _lib.check(_lib.lib().agarcl_batch_archive(self._h, C.byref(a)))
-        N, n_keys, K, dev = self.N, int(a.keys), int(a.entries), f"cuda:{self.cfg.device}"
+        N, n_keys, K = self.N, int(a.keys), int(a.entries)
         spec = {"cell_of": (N, "<i4"), "base_score": (N, "<f8"), "base_length": (N, "<i8"), "key_entry": (n_keys, "<i4"),
                 "visits": (n_keys, "<u4"), "entry_key": (K, "<i4"), "entry_score": (K, "<f8"), "entry_length": (K, "<i8"),
                 "entry_chosen": (K, "<u4"), "counters": (3, "<u8")}
-        return {k: torch.as_tensor(_CudaView(getattr(a, k), (n,), t, self), device=dev) for k, (n, t) in spec.items()}
+        return {k: self._tensor(getattr(a, k), (n,), t) for k, (n, t) in spec.items()}
 
     # ---- pictures of game states (include/agarcl_b200.h, agarcl_batch_draw)
     def draw(self, src=None, size=256, view="arena", out=None, stream=0):
@@ -459,8 +455,6 @@ class Batch:
         wait).  view "arena": the whole arena of instance src[k]; "agent": the observation window of image src[k] = instance * A
         + agent.  src: int32 CUDA tensor, or None for every instance (N pictures) or every agent (N * A).  A source out of range
         gives an all-zero picture.  out: a preallocated contiguous uint8 CUDA tensor [n, size, size, 3] to draw into."""
-        import torch
-        from ._abi import DRAW_VIEWS
         if view not in DRAW_VIEWS:
             raise _lib.AgarclError(f"unknown view {view!r}: 'arena' or 'agent'")
         if src is None:
@@ -470,7 +464,7 @@ class Batch:
             n = src.numel()
         size = int(size)
         if out is None:
-            out = torch.empty((n, size, size, 3), dtype=torch.uint8, device=f"cuda:{self.cfg.device}")
+            out = torch.empty((n, size, size, 3), dtype=torch.uint8, device=self._device)
         else:
             self._check_device_tensor(out, torch.uint8, "out")
             if tuple(out.shape) != (n, size, size, 3):
@@ -483,13 +477,12 @@ class Batch:
 
     # ---- the pixel observation (include/agarcl_b200.h, cfg.pixel_obs)
     def _pixels(self, final):
-        import torch
         p, f, shape = _vp(), _vp(), (C.c_int64 * 4)()
         _lib.check(_lib.lib().agarcl_batch_pixels(self._h, C.byref(p), C.byref(f), C.byref(shape)))
         ptr = f.value if final else p.value
         if not ptr:
             raise _lib.AgarclError("no final pictures: set_autoreset(keep_final_obs=True) with cfg.pixel_obs")
-        return torch.as_tensor(_CudaView(ptr, tuple(shape), "|u1", self), device=f"cuda:{self.cfg.device}")
+        return self._tensor(ptr, tuple(shape), "|u1")
 
     def pixels(self):
         """zero-copy device view uint8 [N*A, S, S, 3] of every agent's picture (cfg.pixel_obs = S), rewritten by every step, reset
@@ -510,8 +503,7 @@ class Batch:
         not clamped.  status: 0 skipped, 1 decided, 2 no pellet to go for (dxdy 0), 3 the agent is dead (dxdy 0), 4 not a bot
         type.  out: preallocated (dxdy, act, status) tensors to write into (new ones start at zero).  target: an f32 CUDA tensor
         [N*A, 2] that also receives the targets in world coordinates."""
-        import torch
-        NA, dev = self.N * self.A, torch.device("cuda", self.cfg.device)
+        NA, dev = self.N * self.A, self._device
         if isinstance(types, torch.Tensor):
             self._check_device_tensor(types, torch.int32, "types", NA)
         else:
@@ -540,23 +532,20 @@ class Batch:
         max_steps (int32 CUDA tensor of N entries or None: every pending limit kept; -1 the set_autoreset limit, 0 none).
         Checked on the device, enqueued on `stream`, no host wait.  Returns a view of the library-owned result u8 [N] (0 nothing
         set, 1 set, 2 rejected: mode not in task_modes or limit < -1), which the next call overwrites."""
-        import torch
         self._check_device_tensor(mode, torch.int32, "mode", self.N)
         if max_steps is not None:
             self._check_device_tensor(max_steps, torch.int32, "max_steps", self.N)
         r = _vp()
         _lib.check(_lib.lib().agarcl_batch_set_tasks(self._h, _vp(mode.data_ptr()), _vp(max_steps.data_ptr()) if max_steps is not None else None,
                                                      C.byref(r), _vp(stream)))
-        return torch.as_tensor(_CudaView(r.value, (self.N,), "|u1", self), device=f"cuda:{self.cfg.device}")
+        return self._tensor(r.value, (self.N,), "|u1")
 
     def tasks(self):
         """zero-copy int32 device views [N] of the task state: mode and max_steps of the current episode, next_mode and
         next_max_steps of the next"""
-        import torch
         t = _TasksStruct()
         _lib.check(_lib.lib().agarcl_batch_tasks(self._h, C.byref(t)))
-        return {k: torch.as_tensor(_CudaView(getattr(t, k), (self.N,), "<i4", self), device=f"cuda:{self.cfg.device}")
-                for k in ("mode", "max_steps", "next_mode", "next_max_steps")}
+        return {k: self._tensor(getattr(t, k), (self.N,), "<i4") for k in ("mode", "max_steps", "next_mode", "next_max_steps")}
 
     # ---- parity / snapshot transport
     def download_state(self, i):
@@ -565,6 +554,8 @@ class Batch:
         return sv
 
     def upload_state(self, i, sv):
+        if sv.blob.size != self.layout.stride:
+            raise _lib.AgarclError(f"the state must be {self.layout.stride} bytes (one instance of this batch), got {sv.blob.size}")
         _lib.check(_lib.lib().agarcl_batch_upload_state(self._h, i, sv.ptr))
 
     def save_env_state(self, i, path):
@@ -588,13 +579,10 @@ class Batch:
         return _CudaView(self._done_ptr, (self.N * self.A,), "|u1", self)
 
     def obs_tensor(self):
-        import torch
-        return torch.as_tensor(self.obs_view(), device=f"cuda:{self.cfg.device}")
+        return self._tensor(self._obs_ptr, self.obs_shape, np.dtype(self.obs_dtype).str)
 
     def rewards_tensor(self):
-        import torch
-        return torch.as_tensor(self.rewards_view(), device=f"cuda:{self.cfg.device}")
+        return self._tensor(self._rew_ptr, (self.N * self.A,), "<f8")
 
     def dones_tensor(self):
-        import torch
-        return torch.as_tensor(self.dones_view(), device=f"cuda:{self.cfg.device}")
+        return self._tensor(self._done_ptr, (self.N * self.A,), "|u1")

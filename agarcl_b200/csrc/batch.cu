@@ -1136,13 +1136,23 @@ extern "C" int agarcl_batch_mirror_timing(const agarcl_batch* b, uint64_t out[4]
   return AGARCL_OK;
 }
 
-extern "C" int agarcl_batch_save_env_state(agarcl_batch* b, int32_t instance, const char* path) {
-  if (!b || !path) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
+// Copies the L.stride bytes of one instance's game between the device and `host` (kind: cudaMemcpyDeviceToHost or
+// cudaMemcpyHostToDevice) once the device has finished everything enqueued.
+static int copy_instance(agarcl_batch* b, int32_t instance, void* host, cudaMemcpyKind kind) {
   if (instance < 0 || instance >= b->N) return agarcl_set_error(AGARCL_ERR_INVALID, "instance out of range");
   CK(cudaSetDevice(b->cfg.device));
   CK(cudaDeviceSynchronize());
+  uint8_t* dev = b->d_state + (size_t)instance * b->L.stride;
+  if (kind == cudaMemcpyHostToDevice) CK(cudaMemcpy(dev, host, b->L.stride, kind));
+  else CK(cudaMemcpy(host, dev, b->L.stride, kind));
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_save_env_state(agarcl_batch* b, int32_t instance, const char* path) {
+  if (!b || !path) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
   std::vector<uint8_t> blob(b->L.stride);
-  CK(cudaMemcpy(blob.data(), b->d_state + (size_t)instance * b->L.stride, b->L.stride, cudaMemcpyDeviceToHost));
+  int rc = copy_instance(b, instance, blob.data(), cudaMemcpyDeviceToHost);
+  if (rc) return rc;
   if (!b->cfg.task_modes) return agarcl_snapshot_write(&b->cfg, &b->L, blob.data(), path);
   // mixed-task batch: the instance as a batch of its current mode sees it (its players, its mode_number)
   agarcl_cfg c = b->cfg;
@@ -1154,22 +1164,20 @@ extern "C" int agarcl_batch_save_env_state(agarcl_batch* b, int32_t instance, co
 
 extern "C" int agarcl_batch_load_env_state(agarcl_batch* b, int32_t instance, const char* path, int lossless) {
   if (!b || !path) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
-  if (instance < 0 || instance >= b->N) return agarcl_set_error(AGARCL_ERR_INVALID, "instance out of range");
-  if (!b->was_reset) return agarcl_set_error(AGARCL_ERR_STATE, "load_env_state() before reset()");
-  CK(cudaSetDevice(b->cfg.device));
-  CK(cudaDeviceSynchronize());
   std::vector<uint8_t> blob(b->L.stride);
-  CK(cudaMemcpy(blob.data(), b->d_state + (size_t)instance * b->L.stride, b->L.stride, cudaMemcpyDeviceToHost));
+  int rc = copy_instance(b, instance, blob.data(), cudaMemcpyDeviceToHost);
+  if (rc) return rc;
+  if (!b->was_reset) return agarcl_set_error(AGARCL_ERR_STATE, "load_env_state() before reset()");
   agarcl_cfg c = b->cfg;
   agarcl_layout L = b->L;
   if (b->cfg.task_modes) {  // mixed-task batch: any mode of the set, which becomes the instance's current task
-    int rc = snapshot_file_mode(path, &c.mode_number);
+    rc = snapshot_file_mode(path, &c.mode_number);
     if (rc) return rc;
     if (c.mode_number < 0 || c.mode_number > 10 || !((b->cfg.task_modes >> c.mode_number) & 1))
       return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot mode_number %d is not in the batch's task_modes 0x%x", c.mode_number, b->cfg.task_modes);
     task_layout(&b->cfg, &b->L, c.mode_number, &L);
   }
-  int rc = agarcl_snapshot_read(&c, &L, blob.data(), path, lossless);
+  rc = agarcl_snapshot_read(&c, &L, blob.data(), path, lossless);
   if (rc) return rc;
   if (b->cfg.task_modes) {
     agarcl_player* pls = reinterpret_cast<agarcl_player*>(blob.data() + b->L.off_players);
@@ -1186,25 +1194,31 @@ extern "C" int agarcl_batch_load_env_state(agarcl_batch* b, int32_t instance, co
     rc = mt_restart(b, instance, hdr->seed_lo, hdr->rng_cursor);
     if (rc) return rc;
   }
-  CK(cudaMemcpy(b->d_state + (size_t)instance * b->L.stride, blob.data(), b->L.stride, cudaMemcpyHostToDevice));
-  return AGARCL_OK;
+  return copy_instance(b, instance, blob.data(), cudaMemcpyHostToDevice);
 }
 
 extern "C" int agarcl_batch_download_state(agarcl_batch* b, int32_t instance, void* blob) {
   if (!b || !blob) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
-  if (instance < 0 || instance >= b->N) return agarcl_set_error(AGARCL_ERR_INVALID, "instance out of range");
-  CK(cudaSetDevice(b->cfg.device));
-  CK(cudaDeviceSynchronize());
-  CK(cudaMemcpy(blob, b->d_state + (size_t)instance * b->L.stride, b->L.stride, cudaMemcpyDeviceToHost));
-  return AGARCL_OK;
+  return copy_instance(b, instance, blob, cudaMemcpyDeviceToHost);
 }
 extern "C" int agarcl_batch_upload_state(agarcl_batch* b, int32_t instance, const void* blob) {
   if (!b || !blob) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
-  if (instance < 0 || instance >= b->N) return agarcl_set_error(AGARCL_ERR_INVALID, "instance out of range");
-  CK(cudaSetDevice(b->cfg.device));
-  CK(cudaDeviceSynchronize());
-  CK(cudaMemcpy(b->d_state + (size_t)instance * b->L.stride, blob, b->L.stride, cudaMemcpyHostToDevice));
+  const int rc = copy_instance(b, instance, const_cast<void*>(blob), cudaMemcpyHostToDevice);
+  if (rc) return rc;
   b->was_reset = true;
+  return AGARCL_OK;
+}
+
+// Refuses a caller's array that is not device memory of the batch's device; `what` names it in the message ("the pool").
+static int check_device_array(const agarcl_batch* b, const void* p, const char* what) {
+  cudaPointerAttributes a;
+  const cudaError_t e = cudaPointerGetAttributes(&a, p);  // (does not synchronise)
+  if (e != cudaSuccess) {
+    cudaGetLastError();  // (clears the error, which would otherwise be reported by the next CUDA call)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "%s is not device memory: %s", what, cudaGetErrorString(e));
+  }
+  if (a.type != cudaMemoryTypeDevice || a.device != b->cfg.device)
+    return agarcl_set_error(AGARCL_ERR_INVALID, "%s must be device memory of device %d", what, b->cfg.device);
   return AGARCL_OK;
 }
 
@@ -1220,15 +1234,7 @@ static int snapshot_check(agarcl_batch* b, const void* pool, int64_t pool_slots,
   if ((uintptr_t)pool & 15u) return agarcl_set_error(AGARCL_ERR_INVALID, "the pool must be 16-byte aligned");
   if (pool_slots < 1) return agarcl_set_error(AGARCL_ERR_INVALID, "pool_slots must be >= 1");
   CK(cudaSetDevice(b->cfg.device));
-  cudaPointerAttributes a;
-  const cudaError_t e = cudaPointerGetAttributes(&a, pool);  // (does not synchronise)
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    return agarcl_set_error(AGARCL_ERR_INVALID, "the pool is not device memory: %s", cudaGetErrorString(e));
-  }
-  if (a.type != cudaMemoryTypeDevice || a.device != b->cfg.device)
-    return agarcl_set_error(AGARCL_ERR_INVALID, "the pool must be device memory of device %d", b->cfg.device);
-  return AGARCL_OK;
+  return check_device_array(b, pool, "the pool");
 }
 
 static ag::SnapParams snapshot_params(const agarcl_batch* b, const void* pool, int64_t pool_slots) {
@@ -1392,15 +1398,8 @@ extern "C" int agarcl_batch_draw(agarcl_batch* b, int32_t view, int32_t size, co
   if (!d_out) return agarcl_set_error(AGARCL_ERR_INVALID, "null output");
   if ((uintptr_t)d_out & 15u) return agarcl_set_error(AGARCL_ERR_INVALID, "the output must be 16-byte aligned");
   CK(cudaSetDevice(b->cfg.device));
-  cudaPointerAttributes a;
-  const cudaError_t e = cudaPointerGetAttributes(&a, d_out);  // (does not synchronise)
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    return agarcl_set_error(AGARCL_ERR_INVALID, "the output is not device memory: %s", cudaGetErrorString(e));
-  }
-  if (a.type != cudaMemoryTypeDevice || a.device != b->cfg.device)
-    return agarcl_set_error(AGARCL_ERR_INVALID, "the output must be device memory of device %d", b->cfg.device);
-  if (n == 0) return AGARCL_OK;
+  const int rc = check_device_array(b, d_out, "the output");
+  if (rc || n == 0) return rc;
   const ag::DrawParams P = draw_params(b, view, size, d_src, n, d_out);
   if (view == AGARCL_DRAW_AGENT) CK(ag::launch_draw_views(P, (cudaStream_t)stream));
   else CK(ag::launch_draw(P, (cudaStream_t)stream));
@@ -1416,18 +1415,11 @@ extern "C" int agarcl_batch_bot_actions(agarcl_batch* b, const int32_t* d_type, 
   if (((uintptr_t)d_dxdy | (uintptr_t)d_target) & 7u)
     return agarcl_set_error(AGARCL_ERR_INVALID, "dxdy and target must be 8-byte aligned");
   CK(cudaSetDevice(b->cfg.device));
-  const std::pair<const void*, const char*> arrays[] = {{d_type, "type"}, {d_dxdy, "dxdy"}, {d_act, "act"}, {d_target, "target"},
-                                                        {d_status, "status"}};
+  const std::pair<const void*, const char*> arrays[] = {{d_type, "the type array"}, {d_dxdy, "the dxdy array"}, {d_act, "the act array"},
+                                                        {d_target, "the target array"}, {d_status, "the status array"}};
   for (const auto& p : arrays) {
-    if (!p.first) continue;
-    cudaPointerAttributes a;
-    const cudaError_t e = cudaPointerGetAttributes(&a, p.first);  // (does not synchronise)
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      return agarcl_set_error(AGARCL_ERR_INVALID, "the %s array is not device memory: %s", p.second, cudaGetErrorString(e));
-    }
-    if (a.type != cudaMemoryTypeDevice || a.device != b->cfg.device)
-      return agarcl_set_error(AGARCL_ERR_INVALID, "the %s array must be device memory of device %d", p.second, b->cfg.device);
+    const int rc = p.first ? check_device_array(b, p.first, p.second) : AGARCL_OK;
+    if (rc) return rc;
   }
   ag::BotParams P;
   P.L = b->L;

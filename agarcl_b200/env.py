@@ -348,28 +348,10 @@ class BatchedGridEnvironment(_Base):
     def _obs(self, b):
         return b.pixels() if self._ctor["pixel_obs"] else b.obs_tensor()
 
-    def _set_actions(self, b, dxdy, act, stream):
-        if hasattr(dxdy, "data_ptr"):
-            import torch
-            # the C ABI reads the raw device buffers as float32 / int32: anything else would be silently reinterpreted
-            na = self.n_instances * self.num_agents
-            dev = torch.device("cuda", self._ctor["device"])
-            if not (dxdy.is_cuda and act.is_cuda and dxdy.device == dev and act.device == dev):
-                raise RuntimeError(f"actions must live on {dev}")
-            if dxdy.dtype != torch.float32 or act.dtype != torch.int32:
-                raise RuntimeError(f"actions must be float32 (dx, dy) and int32 (action), got {dxdy.dtype} / {act.dtype}")
-            if not (dxdy.is_contiguous() and act.is_contiguous()):
-                raise RuntimeError("action tensors must be contiguous")
-            if dxdy.numel() != na * 2 or act.numel() != na:
-                raise RuntimeError(f"Number of actions does not match number of agents ({na})")
-            b.set_actions_device(dxdy.data_ptr(), act.data_ptr(), stream)
-        else:
-            b.set_actions(dxdy, act, stream)
-
     def step(self, dxdy, act, stream=0):
         """dxdy: [N*A, 2] float32, act: [N*A] int32 — numpy (copied) or CUDA torch tensors (zero-copy)"""
         b = self._ensure()
-        self._set_actions(b, dxdy, act, stream)
+        b.set_actions(dxdy, act, stream)
         b.step(stream)
         return self._obs(b), b.rewards_tensor(), b.dones_tensor()
 
@@ -383,7 +365,7 @@ class BatchedGridEnvironment(_Base):
         """step() followed, on the device, by the episode bookkeeping and the reset of every instance with a done agent;
         returns obs, rewards and the done flags with the step limit folded in (u8 [N*A]); episode() has the rest"""
         b = self._ensure()
-        self._set_actions(b, dxdy, act, stream)
+        b.set_actions(dxdy, act, stream)
         b.step_autoreset(stream)
         return self._obs(b), b.rewards_tensor(), b.episode()["done"]
 

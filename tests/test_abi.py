@@ -1,15 +1,18 @@
-"""CPU: the C-ABI library loads, exports every symbol include/agarcl_b200.h declares, derives the same
-layout as the oracle's independent restatement, and reports errors the way the reference does."""
+"""CPU: the C-ABI library loads, exports every symbol include/agarcl_b200.h declares and the ctypes binding binds exactly
+those, derives the same layout as the oracle's independent restatement, and reports errors the way the reference does."""
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
+import textwrap
 
 import numpy as np
 import pytest
 
 from _helpers import ROOT, oracle_layout, oracle_lib
 from agarcl_b200 import _lib, make_cfg
-from agarcl_b200._abi import Cfg, Layout
+from agarcl_b200._abi import Archive, ArchiveCfg, Cfg, Layout
 
 
 def header_symbols():
@@ -23,13 +26,16 @@ def test_library_exports_every_declared_symbol():
     assert len(syms) >= 20
     for s in syms:
         assert hasattr(lib, s), f"{s} declared in include/agarcl_b200.h but not exported"
-    assert set(_lib.SYMBOLS) <= set(syms)
+        assert getattr(lib, s).argtypes is not None, f"{s} is not bound"
+    assert set(_lib.SYMBOLS) == set(syms)
     assert b"sm_100a" in lib.agarcl_version()
 
 
 def test_struct_sizes_match_header():
     assert C.sizeof(Cfg) == 28 * 4
     assert C.sizeof(Layout) == (7 + 7 + 5 + 64 + 64) * 4
+    assert C.sizeof(ArchiveCfg) == 24
+    assert C.sizeof(Archive) == 10 * 8 + 16
 
 
 @pytest.mark.parametrize("kw", [dict(), dict(num_agents=4, num_bots=8), dict(num_bots=40, num_agents=3),
@@ -103,6 +109,32 @@ def test_take_actions_size_check_like_reference():
     assert env.observation_shape() == (8, 128, 128)
     env.configure_observation({"grid_size": 64, "observe_others": False, "num_frames": 2})
     assert env.observation_shape() == (12, 64, 64)
+
+
+def test_host_buffer_checks_hold_under_python_O():
+    """Batch refuses host arrays of the wrong size before the library reads them: the checks are no asserts, so `python -O`
+    keeps them.  (Batch.__new__: no library batch is needed, each call is refused before it would reach one.)"""
+    script = textwrap.dedent("""
+        import numpy as np
+        from agarcl_b200._abi import Layout, StateView
+        from agarcl_b200._lib import AgarclError
+        from agarcl_b200.batch import Batch
+        b = Batch.__new__(Batch)
+        b.N, b.A = 3, 2
+        b.layout = Layout(stride=256)
+        calls = {"short dxdy": lambda: b.set_actions(np.zeros((5, 2), np.float32), np.zeros(6, np.int32)),
+                 "short act": lambda: b.set_actions(np.zeros((6, 2), np.float32), np.zeros(5, np.int32)),
+                 "short reset mask": lambda: b.reset(np.ones(2, np.uint8)),
+                 "short state": lambda: b.upload_state(0, StateView(Layout(stride=128)))}
+        for what, call in calls.items():
+            try:
+                call()
+            except AgarclError:
+                continue
+            raise SystemExit(what + " was not refused")
+    """)
+    r = subprocess.run([sys.executable, "-O", "-c", script], cwd=ROOT, capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_compiled_agarcl_module_surface():

@@ -1,21 +1,10 @@
-"""The cell archive without a GPU: its entry points are in the library and bound, the ctypes structs have the header's sizes,
-and the archive kernels compile for sm_100a without stack or spills."""
-import ctypes as C
+"""The cell archive without a GPU: the archive kernels compile for sm_100a without stack or spills."""
 import os
 import re
 import subprocess
 import tempfile
 
 KERNELS = ("k_archive_cells", "k_archive_commit", "k_archive_select", "k_archive_base")
-
-
-def test_entry_points_are_bound():
-    from agarcl_b200 import _lib
-    from agarcl_b200._abi import Archive, ArchiveCfg
-    L = _lib.lib()
-    for name in ("agarcl_batch_set_archive", "agarcl_batch_archive"):
-        assert name in _lib.SYMBOLS and getattr(L, name).argtypes, name
-    assert C.sizeof(ArchiveCfg) == 24 and C.sizeof(Archive) == 10 * 8 + 16
 
 
 def test_archive_kernels_have_no_spills():

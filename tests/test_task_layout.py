@@ -109,9 +109,10 @@ def test_order_check_matches_the_batch_of_each_mode_alone():
             assert same
 
 
-def test_ctypes_cfg_keeps_its_size():
-    from agarcl_b200._abi import Cfg
-    assert C.sizeof(Cfg) == 28 * 4 and [f[0] for f in Cfg._fields_][-2:] == ["task_modes", "reserved"]
+def test_ctypes_cfg_names_the_header_fields():
+    from agarcl_b200._abi import Cfg, make_cfg
+    assert C.sizeof(Cfg) == 28 * 4 and [f[0] for f in Cfg._fields_][-2:] == ["task_modes", "pixel_obs"]
+    assert make_cfg(pixel_obs=32).pixel_obs == 32
 
 
 def test_kernels_touched_by_tasks_have_no_spills():
