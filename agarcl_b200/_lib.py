@@ -38,6 +38,8 @@ _PROTOTYPES = {
     "agarcl_batch_archive": [_vp, C.POINTER(Archive)],
     "agarcl_batch_set_tasks": [_vp, _vp, _vp, C.POINTER(_vp), _vp],
     "agarcl_batch_tasks": [_vp, _vp],
+    "agarcl_batch_set_task_sizes": [_vp, _vp, _vp, _vp, C.POINTER(_vp), _vp],
+    "agarcl_batch_task_sizes": [_vp, _vp],
     "agarcl_batch_draw": [_vp, C.c_int32, C.c_int32, _vp, C.c_int32, _vp, _vp],
     "agarcl_batch_pixels": [_vp, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(C.c_int64 * 4)],
     "agarcl_batch_bot_actions": [_vp, _vp, _vp, _vp, _vp, _vp, _vp],

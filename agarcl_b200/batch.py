@@ -39,6 +39,11 @@ class _TasksStruct(C.Structure):
     _fields_ = [(n, _vp) for n in ("mode", "max_steps", "next_mode", "next_max_steps")]
 
 
+class _TaskSizesStruct(C.Structure):
+    """struct agarcl_task_sizes"""
+    _fields_ = [(n, _vp) for n in ("bots", "pellets", "viruses", "next_bots", "next_pellets", "next_viruses")]
+
+
 class ObsLists:
     """numpy view of the lists of the last Batch.step_lists (layout: include/agarcl_b200.h, agarcl_obs_lists)"""
 
@@ -546,6 +551,28 @@ class Batch:
         t = _TasksStruct()
         _lib.check(_lib.lib().agarcl_batch_tasks(self._h, C.byref(t)))
         return {k: self._tensor(getattr(t, k), (self.N,), "<i4") for k in ("mode", "max_steps", "next_mode", "next_max_steps")}
+
+    def set_task_sizes(self, bots=None, pellets=None, viruses=None, stream=0):
+        """the game sizes each instance's NEXT reset plays: bots (mode 0), pellets and viruses, each an int32 CUDA tensor of N
+        entries or None (every pending value kept); an entry of -1 keeps that value.  cfg.num_bots / num_pellets / num_viruses
+        are the maxima.  Checked on the device, enqueued on `stream`, no host wait.  Returns a view of the library-owned result
+        u8 [N] (0 nothing set, 1 set, 2 rejected: a value outside [0, maximum] or a bot count the batch's player order does not
+        allow; a rejected instance keeps all its pending sizes), which the next call overwrites."""
+        ptrs = []
+        for name, t in (("bots", bots), ("pellets", pellets), ("viruses", viruses)):
+            if t is not None:
+                self._check_device_tensor(t, torch.int32, name, self.N)
+            ptrs.append(_vp(t.data_ptr()) if t is not None else None)
+        r = _vp()
+        _lib.check(_lib.lib().agarcl_batch_set_task_sizes(self._h, *ptrs, C.byref(r), _vp(stream)))
+        return self._tensor(r.value, (self.N,), "|u1")
+
+    def task_sizes(self):
+        """zero-copy int32 device views [N] of the game sizes: bots, pellets and viruses of the current episode, next_bots,
+        next_pellets and next_viruses of the next"""
+        t = _TaskSizesStruct()
+        _lib.check(_lib.lib().agarcl_batch_task_sizes(self._h, C.byref(t)))
+        return {k: self._tensor(getattr(t, k), (self.N,), "<i4") for k, _ in _TaskSizesStruct._fields_}
 
     # ---- parity / snapshot transport
     def download_state(self, i):

@@ -145,6 +145,10 @@ struct agarcl_batch {
   // mixed-task batch (cfg.task_modes != 0, include/agarcl_b200.h): current and pending task per instance, result of the last set_tasks
   DevBuf<int32_t> d_task_mode, d_task_max_steps, d_next_mode, d_next_max_steps;
   DevBuf<uint8_t> d_task_result;
+  // and its game sizes (agarcl_batch_set_task_sizes): current and pending bots, pellets, viruses, their limits, the last result
+  DevBuf<int32_t> d_bots, d_pellets, d_viruses, d_next_bots, d_next_pellets, d_next_viruses;
+  DevBuf<uint8_t> d_size_result;
+  ag::SizeLimits size_lim = {};
   ag::HostMirror* mirror = nullptr;  // host-resident observation mirror (mirror.cu), created on first use
   ag::HostMirror* lists = nullptr;   // the lists-only twin behind agarcl_batch_step_lists (no dense tensor, no worker threads)
   uint64_t mirror_launch_us = 0, mirror_call_us = 0;  // last agarcl_batch_step_mirror: staging + launch, whole call
@@ -201,6 +205,14 @@ static int alloc(DevBuf<T>& buf, size_t bytes, int fill = -1) {
   return AGARCL_OK;
 }
 
+// The six game-size arrays of a mixed-task batch (all nullptr otherwise)
+static agarcl_task_sizes task_sizes_of(const agarcl_batch* b) {
+  agarcl_task_sizes z;
+  z.bots = b->d_bots; z.pellets = b->d_pellets; z.viruses = b->d_viruses;
+  z.next_bots = b->d_next_bots; z.next_pellets = b->d_next_pellets; z.next_viruses = b->d_next_viruses;
+  return z;
+}
+
 static void fill_sim_params(const agarcl_batch* b, ag::SimParams& P) {
   P.L = b->L;
   P.T = b->T;
@@ -224,6 +236,7 @@ static void fill_sim_params(const agarcl_batch* b, ag::SimParams& P) {
   P.rng_mode = b->cfg.rng_mode;
   P.target_pellets = b->cfg.num_pellets;
   P.target_viruses = b->cfg.num_viruses;
+  P.task_bots = b->d_bots; P.task_pellets = b->d_pellets; P.task_viruses = b->d_viruses;
   P.HG = b->HG;
   P.W = (float)b->cfg.arena_size;
   P.hash_scale = (float)b->HG / (float)b->cfg.arena_size;
@@ -479,6 +492,15 @@ extern "C" int agarcl_batch_create(const agarcl_cfg* cfg, agarcl_batch** out) {
     CK(cudaMemcpy(b->d_next_mode, modes.data(), bytes, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(b->d_task_max_steps, limits.data(), bytes, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(b->d_next_max_steps, limits.data(), bytes, cudaMemcpyHostToDevice));
+    // game sizes: the configured counts are the maxima, which every instance plays until it is given others
+    b->size_lim = {cfg->num_bots, cfg->num_pellets, cfg->num_viruses, !(cfg->task_modes & 1), task_bot_counts(cfg, &L)};
+    DevBuf<int32_t>* bufs[6] = {&b->d_bots, &b->d_pellets, &b->d_viruses, &b->d_next_bots, &b->d_next_pellets, &b->d_next_viruses};
+    for (int k = 0; k < 6; k++) {
+      if ((rc = alloc(*bufs[k], bytes))) return rc;
+      const std::vector<int32_t> v((size_t)b->N, k % 3 == 0 ? cfg->num_bots : k % 3 == 1 ? cfg->num_pellets : cfg->num_viruses);
+      CK(cudaMemcpy(*bufs[k], v.data(), bytes, cudaMemcpyHostToDevice));
+    }
+    if ((rc = alloc(b->d_size_result, (size_t)b->N, 0))) return rc;
   }
   b->cur_dxdy = b->d_dxdy;
   b->cur_act = b->d_act;
@@ -721,11 +743,11 @@ static int reset_impl(agarcl_batch* b, const uint8_t* dm, cudaStream_t s, bool c
   P.rng_mode = b->cfg.rng_mode;
   P.num_pellets = b->cfg.num_pellets;
   P.num_viruses = b->cfg.num_viruses;
-  P.num_bots = b->cfg.num_bots;
   P.task_mode = b->d_task_mode;
   P.task_max_steps = b->d_task_max_steps;
   P.next_mode = b->d_next_mode;
   P.next_max_steps = b->d_next_max_steps;
+  P.sizes = task_sizes_of(b);
   P.W = (float)b->cfg.arena_size;
   if (b->cfg.strict_reference && !dm) {
     // BaseEnvironment::reset of every instance (BaseEnvironment.hpp:179-197): players.clear(), then add_player for the agents and
@@ -1154,11 +1176,14 @@ extern "C" int agarcl_batch_save_env_state(agarcl_batch* b, int32_t instance, co
   int rc = copy_instance(b, instance, blob.data(), cudaMemcpyDeviceToHost);
   if (rc) return rc;
   if (!b->cfg.task_modes) return agarcl_snapshot_write(&b->cfg, &b->L, blob.data(), path);
-  // mixed-task batch: the instance as a batch of its current mode sees it (its players, its mode_number)
+  // mixed-task batch: the instance as a batch of its current task sees it (its players, its mode_number and sizes)
   agarcl_cfg c = b->cfg;
   CK(cudaMemcpy(&c.mode_number, b->d_task_mode + instance, sizeof(int32_t), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(&c.num_bots, b->d_bots + instance, sizeof(int32_t), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(&c.num_pellets, b->d_pellets + instance, sizeof(int32_t), cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(&c.num_viruses, b->d_viruses + instance, sizeof(int32_t), cudaMemcpyDeviceToHost));
   agarcl_layout L;
-  task_layout(&b->cfg, &b->L, c.mode_number, &L);
+  task_layout(&b->cfg, &b->L, c.mode_number, c.num_bots, &L);
   return agarcl_snapshot_write(&c, &L, blob.data(), path);
 }
 
@@ -1170,12 +1195,16 @@ extern "C" int agarcl_batch_load_env_state(agarcl_batch* b, int32_t instance, co
   if (!b->was_reset) return agarcl_set_error(AGARCL_ERR_STATE, "load_env_state() before reset()");
   agarcl_cfg c = b->cfg;
   agarcl_layout L = b->L;
-  if (b->cfg.task_modes) {  // mixed-task batch: any mode of the set, which becomes the instance's current task
-    rc = snapshot_file_mode(path, &c.mode_number);
+  if (b->cfg.task_modes) {  // mixed-task batch: any mode of the set and sizes within the maxima, which become the instance's current task
+    rc = snapshot_file_task(path, &c);
     if (rc) return rc;
     if (c.mode_number < 0 || c.mode_number > 10 || !((b->cfg.task_modes >> c.mode_number) & 1))
       return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot mode_number %d is not in the batch's task_modes 0x%x", c.mode_number, b->cfg.task_modes);
-    task_layout(&b->cfg, &b->L, c.mode_number, &L);
+    if (c.mode_number != 0) c.num_bots = b->cfg.num_bots;  // (the bot count means something in mode 0 only: the file's is not checked)
+    if (!ag::sizes_allowed(b->size_lim, c.num_bots, c.num_pellets, c.num_viruses))
+      return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot sizes (num_bots %d, num_pellets %d, num_viruses %d) are not allowed in the batch",
+                              c.num_bots, c.num_pellets, c.num_viruses);
+    task_layout(&b->cfg, &b->L, c.mode_number, c.num_bots, &L);
   }
   rc = agarcl_snapshot_read(&c, &L, blob.data(), path, lossless);
   if (rc) return rc;
@@ -1186,6 +1215,9 @@ extern "C" int agarcl_batch_load_env_state(agarcl_batch* b, int32_t instance, co
       pls[p].bot_type = ag::mode_bot_type(c.mode_number, p, b->L.A);
     }
     CK(cudaMemcpy(b->d_task_mode + instance, &c.mode_number, sizeof(int32_t), cudaMemcpyHostToDevice));  // (its step limit stays)
+    CK(cudaMemcpy(b->d_bots + instance, &c.num_bots, sizeof(int32_t), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(b->d_pellets + instance, &c.num_pellets, sizeof(int32_t), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(b->d_viruses + instance, &c.num_viruses, sizeof(int32_t), cudaMemcpyHostToDevice));
   }
   const agarcl_inst_hdr* hdr = reinterpret_cast<const agarcl_inst_hdr*>(blob.data() + b->L.off_hdr);
   b->seeds[instance] = (uint64_t)hdr->seed_lo | ((uint64_t)hdr->seed_hi << 32);
@@ -1259,6 +1291,8 @@ static ag::SnapParams snapshot_params(const agarcl_batch* b, const void* pool, i
   P.task_mode = b->d_task_mode;
   P.task_max_steps = b->d_task_max_steps;
   P.task_modes = b->cfg.task_modes;
+  P.sizes = task_sizes_of(b);
+  P.lim = b->size_lim;
   P.N = b->N;
   P.A = b->A;
   P.instance_base = b->cfg.instance_base;
@@ -1460,5 +1494,28 @@ extern "C" int agarcl_batch_tasks(agarcl_batch* b, agarcl_tasks* out) {
   out->max_steps = b->d_task_max_steps;
   out->next_mode = b->d_next_mode;
   out->next_max_steps = b->d_next_max_steps;
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_set_task_sizes(agarcl_batch* b, const int32_t* d_bots, const int32_t* d_pellets, const int32_t* d_viruses,
+                                           uint8_t** d_result, void* stream) {
+  if (!b) return agarcl_set_error(AGARCL_ERR_INVALID, "null batch");
+  if (!b->cfg.task_modes) return agarcl_set_error(AGARCL_ERR_STATE, "the batch was created without task_modes");
+  CK(cudaSetDevice(b->cfg.device));
+  ag::SetTaskSizesParams P;
+  P.bots = d_bots; P.pellets = d_pellets; P.viruses = d_viruses;
+  P.next_bots = b->d_next_bots; P.next_pellets = b->d_next_pellets; P.next_viruses = b->d_next_viruses;
+  P.result = b->d_size_result;
+  P.lim = b->size_lim;
+  P.N = b->N;
+  CK(ag::launch_set_task_sizes(P, (cudaStream_t)stream));
+  if (d_result) *d_result = b->d_size_result;
+  return AGARCL_OK;
+}
+
+extern "C" int agarcl_batch_task_sizes(agarcl_batch* b, agarcl_task_sizes* out) {
+  if (!b || !out) return agarcl_set_error(AGARCL_ERR_INVALID, "null argument");
+  if (!b->cfg.task_modes) return agarcl_set_error(AGARCL_ERR_STATE, "the batch was created without task_modes");
+  *out = task_sizes_of(b);
   return AGARCL_OK;
 }

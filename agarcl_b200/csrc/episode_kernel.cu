@@ -63,6 +63,21 @@ __global__ void __launch_bounds__(256) k_set_tasks(const __grid_constant__ SetTa
   P.result[i] = (set_mode || set_limit) ? 1 : 0;
 }
 
+// One thread per instance: agarcl_batch_set_task_sizes.  The entries given (not -1, array not nullptr) replace the pending sizes
+// only when the resulting sizes are all valid; a rejected instance keeps all three.
+__global__ void __launch_bounds__(256) k_set_task_sizes(const __grid_constant__ SetTaskSizesParams P) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.N) return;
+  const int32_t b = P.bots ? P.bots[i] : -1, p = P.pellets ? P.pellets[i] : -1, v = P.viruses ? P.viruses[i] : -1;
+  if (b == -1 && p == -1 && v == -1) { P.result[i] = 0; return; }
+  const int32_t nb = b == -1 ? P.next_bots[i] : b, np = p == -1 ? P.next_pellets[i] : p, nv = v == -1 ? P.next_viruses[i] : v;
+  if (!sizes_allowed(P.lim, nb, np, nv)) { P.result[i] = 2; return; }
+  P.next_bots[i] = nb;
+  P.next_pellets[i] = np;
+  P.next_viruses[i] = nv;
+  P.result[i] = 1;
+}
+
 // One CTA per instance: bytes [i * per, (i + 1) * per) of dst get those of src (kCopy) or zeros, for the instances with
 // mask[i] != 0; the CTAs of the others exit at once.  dst and src are allocations of the same alignment, so the slices
 // of one instance share their alignment modulo 16 (block_copy).
@@ -81,6 +96,11 @@ cudaError_t launch_episode(const EpisodeParams& P, cudaStream_t stream) {
 
 cudaError_t launch_set_tasks(const SetTasksParams& P, cudaStream_t stream) {
   k_set_tasks<<<(P.N + 255) / 256, 256, 0, stream>>>(P);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_set_task_sizes(const SetTaskSizesParams& P, cudaStream_t stream) {
+  k_set_task_sizes<<<(P.N + 255) / 256, 256, 0, stream>>>(P);
   return cudaGetLastError();
 }
 

@@ -24,9 +24,27 @@ static void player_order(int P, int32_t* order) {
   for (auto& kv : m) order[k++] = kv.second;
 }
 
-void task_layout(const agarcl_cfg* c, const agarcl_layout* L, int mode, agarcl_layout* out) {
+// whether the order of L's players, restricted to players < Pm, is the order of a batch of Pm players alone
+static bool order_restricts(const agarcl_layout* L, int Pm) {
+  int alone[AGARCL_MAX_PLAYERS];
+  player_order(Pm, alone);
+  int k = 0;
+  for (int j = 0; j < L->P; j++)
+    if (L->order[j] < Pm && L->order[j] != alone[k++]) return false;
+  return true;
+}
+
+uint64_t task_bot_counts(const agarcl_cfg* c, const agarcl_layout* L) {
+  uint64_t bits = 0;
+  if (!(c->task_modes & 1)) return bits;
+  for (int b = 0; b <= c->num_bots; b++)  // (mode 0 in the set: P = A + num_bots <= 64, so b < 64)
+    if (order_restricts(L, L->A + b)) bits |= 1ull << b;
+  return bits;
+}
+
+void task_layout(const agarcl_cfg* c, const agarcl_layout* L, int mode, int bots, agarcl_layout* out) {
   *out = *L;
-  const ag::ModeRules R = ag::mode_rules(mode, c->num_bots);
+  const ag::ModeRules R = ag::mode_rules(mode, bots);
   out->P = L->A + R.bots;
   out->mass_decay = R.mass_decay;
   out->squared_pellets = R.squared_pellets;
@@ -92,12 +110,8 @@ extern "C" int agarcl_make_layout(const agarcl_cfg* c, agarcl_layout* L) {
     if (!((task_modes >> m) & 1)) continue;
     // an instance of mode m plays players 0 .. P_m - 1 in the batch's order: it must be the order of a batch of mode m alone
     const int Pm = L->A + ag::mode_rules(m, c->num_bots).bots;
-    int alone[AGARCL_MAX_PLAYERS];
-    player_order(Pm, alone);
-    int k = 0;
-    for (int j = 0; j < L->P; j++)
-      if (L->order[j] < Pm && L->order[j] != alone[k++])
-        return agarcl_set_error(AGARCL_ERR_INVALID, "task_modes: the player order of mode %d differs from the batch's (%d agents, %d players)", m,
+    if (!order_restricts(L, Pm))
+      return agarcl_set_error(AGARCL_ERR_INVALID, "task_modes: the player order of mode %d differs from the batch's (%d agents, %d players)", m,
                                 L->A, L->P);
   }
 

@@ -54,14 +54,20 @@ __global__ void __launch_bounds__(128) k_reset(const __grid_constant__ ResetPara
   // the rules this episode plays: mode_number's (the layout's flags), or in a mixed-task batch the instance's pending task,
   // which becomes its current one here
   int squared = P.L.squared_pellets, agent_mass = P.L.agent_mass, Pm = P.L.P, mode = 0;
+  int num_pellets = P.num_pellets, num_viruses = P.num_viruses;
   if (P.task_mode) {
     mode = P.next_mode[inst];
-    const int32_t ms = P.next_max_steps[inst];
-    const ModeRules R = mode_rules(mode, P.num_bots);
+    const int32_t ms = P.next_max_steps[inst], bots = P.sizes.next_bots[inst];
+    num_pellets = P.sizes.next_pellets[inst];
+    num_viruses = P.sizes.next_viruses[inst];
+    const ModeRules R = mode_rules(mode, bots);
     squared = R.squared_pellets;
     agent_mass = R.agent_mass;
     Pm = P.L.A + R.bots;
-    if (lane == 0) { P.task_mode[inst] = mode; P.task_max_steps[inst] = ms; }
+    if (lane == 0) {
+      P.task_mode[inst] = mode; P.task_max_steps[inst] = ms;
+      P.sizes.bots[inst] = bots; P.sizes.pellets[inst] = num_pellets; P.sizes.viruses[inst] = num_viruses;
+    }
   }
   // Engine::reset does not touch the RNG (Engine.hpp:98-117): a second episode goes on in the stream; only seed() restarts it
   uint32_t cursor = (P.fresh && !P.fresh[inst]) ? hdr->rng_cursor : 0u;
@@ -93,24 +99,24 @@ __global__ void __launch_bounds__(128) k_reset(const __grid_constant__ ResetPara
     }
   } else {
     float r = radius_of(P.T, AGARCL_PELLET_MASS);
-    for (int k = lane; k < P.num_pellets; k += 32) {
+    for (int k = lane; k < num_pellets; k += 32) {
       float x, y;
       rloc(c, cursor + 2u * (uint32_t)k, r, x, y);
       if (k < P.L.cap_pellets) pel[k] = make_float2(x, y);
     }
-    cursor += 2u * (uint32_t)P.num_pellets;
-    n_pellets = min(P.num_pellets, P.L.cap_pellets);
+    cursor += 2u * (uint32_t)num_pellets;
+    n_pellets = min(num_pellets, P.L.cap_pellets);
   }
   {
     float r = radius_of(P.T, AGARCL_VIRUS_INITIAL_MASS);
-    for (int k = lane; k < P.num_viruses; k += 32) {
+    for (int k = lane; k < num_viruses; k += 32) {
       float x, y;
       rloc(c, cursor + 2u * (uint32_t)k, r, x, y);
       float4* v = reinterpret_cast<float4*>(vir + k);
       v[0] = make_float4(x, y, __uint_as_float(AGARCL_VIRUS_INITIAL_MASS), __int_as_float(0));
       v[1] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    cursor += 2u * (uint32_t)P.num_viruses;
+    cursor += 2u * (uint32_t)num_viruses;
   }
   __syncwarp();
   // players: Player ctor defaults + respawn (Player.hpp:25-41; Engine.hpp:119-137)
@@ -153,7 +159,7 @@ __global__ void __launch_bounds__(128) k_reset(const __grid_constant__ ResetPara
     hdr->tick = 0;
     hdr->next_cell_id = 1u + (uint32_t)Pm;
     hdr->n_pellets = n_pellets;
-    hdr->n_viruses = min(P.num_viruses, P.L.cap_viruses);
+    hdr->n_viruses = min(num_viruses, P.L.cap_viruses);
     hdr->n_foods = 0;
     hdr->rng_cursor = cursor;
     hdr->flags = c.flags;

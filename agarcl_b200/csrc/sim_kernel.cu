@@ -2370,7 +2370,8 @@ __device__ void move_foods(Ctx& c) {
 
 // add_pellets / add_viruses for the regen tick (Engine.hpp:230-237)
 __device__ void regen(Ctx& c) {
-  int dp = c.P.target_pellets - c.n_pellets;
+  const int inst = c.cold().inst_local;  // (a mixed-task batch tops up to the instance's own sizes)
+  int dp = (c.P.task_pellets ? c.P.task_pellets[inst] : c.P.target_pellets) - c.n_pellets;
   if (dp > 0) {
     float r = radius_of(c.P.T, AGARCL_PELLET_MASS);
     const uint32_t cur = c.cold().cursor;
@@ -2385,7 +2386,7 @@ __device__ void regen(Ctx& c) {
     c.hash_valid = false;
     c.pel_dirty = true;
   }
-  int dv = c.P.target_viruses - c.n_viruses;
+  int dv = (c.P.task_viruses ? c.P.task_viruses[inst] : c.P.target_viruses) - c.n_viruses;
   if (dv > 0) {
     float r = radius_of(c.P.T, AGARCL_VIRUS_INITIAL_MASS);
     int room = c.P.L.cap_viruses - c.n_viruses;
@@ -2972,13 +2973,15 @@ __device__ __forceinline__ void step_instance(const SimParams& P, uint8_t* smem_
     else if (P.obs_finish == 2) obs_finish_warp<int16_t>(c);
     const int mode_now = c.cold().mode;
     if (mode_now == 0) {
-      // repsawn_all_players in map order: the r-th dead player takes draw pair r
+      // repsawn_all_players in map order: the r-th dead player takes draw pair r.  Players >= Pm are absent (a mixed-task batch's
+      // instance of fewer bots): not respawned, ranked or reported
+      const int Pm = P.task_bots ? A + P.task_bots[inst] : Pn;
       uint32_t rank_base = 0;
       uint32_t resp_lo = 0, resp_hi = 0;
       for (int base = 0; base < Pn; base += 32) {
         int k = base + lane;
         int p = k < Pn ? P.L.order[k] : 0;
-        bool dead = k < Pn && __float_as_int(c.sm.psum()[p].w) == 0;
+        bool dead = k < Pn && p < Pm && __float_as_int(c.sm.psum()[p].w) == 0;
         unsigned dm = __ballot_sync(AG_FULL, dead);
         if (dead) {
           uint32_t r = rank_base + (uint32_t)__popc(dm & lanemask_lt(lane));

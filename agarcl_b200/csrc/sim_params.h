@@ -95,6 +95,9 @@ struct SimParams {
                              // nullptr: every instance plays `mode` with the flags of L
   int32_t num_bots;          // cfg.num_bots (mode_rules, mixed-task batch)
   int32_t target_pellets, target_viruses;
+  // mixed-task batch: each instance's current game sizes (agarcl_batch_set_task_sizes), read from global memory at the regen tick
+  // (the regen targets) and at the mode-0 respawn (players >= A + bots are absent); nullptr: target_* and L.P for all
+  const int32_t *task_bots, *task_pellets, *task_viruses;
   int32_t HG;              // spatial hash is HG x HG over the arena
   float W;                 // arena width == height
   float hash_scale;        // HG / W
@@ -153,7 +156,8 @@ struct ResetParams {
   // and is spawned by the rules of that mode, with players P_m .. P-1 absent
   int32_t *task_mode, *task_max_steps;
   const int32_t *next_mode, *next_max_steps;
-  int32_t N, instance_base, rng_mode, num_pellets, num_viruses, num_bots;
+  agarcl_task_sizes sizes;   // the same for the game sizes: next_* become the current ones and are what the reset spawns
+  int32_t N, instance_base, rng_mode, num_pellets, num_viruses;
   float W;
 };
 cudaError_t launch_reset(const ResetParams& P, cudaStream_t stream);
@@ -214,6 +218,25 @@ struct SetTasksParams {
   int32_t N, task_modes;
 };
 cudaError_t launch_set_tasks(const SetTasksParams& P, cudaStream_t stream);
+// The maxima and allowed bot counts of a mixed-task batch's game sizes (agarcl_batch_set_task_sizes)
+struct SizeLimits {
+  int32_t bots, pellets, viruses;  // cfg.num_bots, num_pellets, num_viruses
+  int32_t bots_any;                // 1: mode 0 is not in task_modes, the bot count means nothing and every one of 0 .. bots is allowed
+  uint64_t bots_allowed;           // otherwise bit b: b bots pass the player-order check (layout.cpp, task_bot_counts; bots < 64)
+};
+__host__ __device__ inline bool sizes_allowed(const SizeLimits& M, int32_t bots, int32_t pellets, int32_t viruses) {
+  return bots >= 0 && bots <= M.bots && (M.bots_any || ((M.bots_allowed >> bots) & 1u)) && pellets >= 0 && pellets <= M.pellets &&
+         viruses >= 0 && viruses <= M.viruses;
+}
+// agarcl_batch_set_task_sizes: pending sizes of instance i <- the given entries (-1 or a nullptr array: kept) when all are valid
+struct SetTaskSizesParams {
+  const int32_t *bots, *pellets, *viruses;  // [N] or nullptr
+  int32_t *next_bots, *next_pellets, *next_viruses;
+  uint8_t* result;
+  SizeLimits lim;
+  int32_t N;
+};
+cudaError_t launch_set_task_sizes(const SetTaskSizesParams& P, cudaStream_t stream);
 // dst = src (nullptr: zeros) in the `per`-byte slices of the instances with mask != 0
 cudaError_t launch_masked_bytes(void* dst, const void* src, size_t per, const uint8_t* mask, int N, cudaStream_t stream);
 
@@ -249,6 +272,8 @@ struct SnapParams {
   int32_t* task_mode;        // [N] mixed-task batch: the current task, stored in the slot header and restored from it; else nullptr
   int32_t* task_max_steps;   // [N]
   int32_t task_modes;        // cfg.task_modes: a restored slot's mode must be in it
+  agarcl_task_sizes sizes;   // mixed-task batch: the slot's game sizes become the current ones (maxima without the marker)
+  SizeLimits lim;            //   and must be within these
   int32_t N, A, instance_base;
   // start states (agarcl_batch_set_start_states, k_start_states): in front of k_reset, instance i in `mask` (nullptr: all) <-
   // slot slot_of[i] where >= 0, with the instance's draw stream; result is the start result, not the restore's

@@ -137,12 +137,15 @@ int parse_file(const char* path, JV& root) {
 
 }  // namespace
 
-int snapshot_file_mode(const char* path, int* mode) {
+int snapshot_file_task(const char* path, agarcl_cfg* c) {
   JV root;
   int rc = parse_file(path, root);
   if (rc) return rc;
   if (!root.get("mode_number")) return agarcl_set_error(AGARCL_ERR_INVALID, "snapshot %s has no mode_number", path);
-  *mode = (int)root.n("mode_number");
+  c->mode_number = (int)root.n("mode_number");
+  c->num_bots = (int)root.n("num_bots", c->num_bots);
+  c->num_pellets = (int)root.n("num_pellets", c->num_pellets);
+  c->num_viruses = (int)root.n("num_viruses", c->num_viruses);
   return AGARCL_OK;
 }
 
@@ -164,6 +167,8 @@ extern "C" int agarcl_snapshot_write(const agarcl_cfg* c, const agarcl_layout* L
           c->arena_size, c->c_death, c->mode_number, c->num_agents, c->num_bots);
   fprintf(f, "    \"pellet_count\": %d,\n    \"pellet_regen\": %s,\n    \"reward_type\": %d,\n    \"ticks_per_step\": %d,\n",
           hdr->n_pellets, c->pellet_regen ? "true" : "false", c->reward_type, c->ticks_per_step);
+  if (c->task_modes)  // a mixed-task batch's instance: its game sizes (agarcl_batch_set_task_sizes)
+    fprintf(f, "    \"num_pellets\": %d,\n    \"num_viruses\": %d,\n", c->num_pellets, c->num_viruses);
   // "seed" is what the reference reads back (Engine.hpp:346, 32 bits); the upper half of a 64-bit Philox key travels as an extra key
   fprintf(f, "    \"seed\": %u,\n    \"seed_hi\": %u,\n    \"ticks\": %u,\n    \"rng_cursor\": %u,\n    \"next_cell_id\": %u,\n", hdr->seed_lo,
           hdr->seed_hi, hdr->tick, hdr->rng_cursor, hdr->next_cell_id);

@@ -22,7 +22,28 @@ __device__ __forceinline__ void copy_segment(uint8_t* __restrict__ d, const uint
   for (size_t k = threadIdx.x; k < n; k += blockDim.x) d[k] = s[k];
 }
 
-// Whether slot `slot` (at sl) holds a state this batch may load: in range, saved from this configuration, a mode of the set
+// The game sizes (bots, pellets, viruses) a slot of a mixed-task batch carries: its own with the marker, else the maxima (a slot
+// saved before sizes were stored)
+__device__ __forceinline__ int3 slot_sizes(const SnapParams& P, const agarcl_snapshot_hdr* h) {
+  return h->sizes_marker == AGARCL_SNAPSHOT_SIZES_MARKER ? make_int3(h->task_bots, h->task_pellets, h->task_viruses)
+                                                         : make_int3(P.lim.bots, P.lim.pellets, P.lim.viruses);
+}
+// A mixed-task slot's task is one this batch may play: a mode of the set, sizes within the maxima and an allowed bot count
+__device__ __forceinline__ bool slot_task_valid(const SnapParams& P, const agarcl_snapshot_hdr* h) {
+  const int3 z = slot_sizes(P, h);
+  return h->task_mode >= 0 && h->task_mode <= 10 && ((P.task_modes >> h->task_mode) & 1) && sizes_allowed(P.lim, z.x, z.y, z.z);
+}
+// The slot's task becomes instance i's current one (its step limit is the caller's: the slot's or the pending one)
+__device__ __forceinline__ void take_slot_task(const SnapParams& P, const agarcl_snapshot_hdr* h, int i, int32_t max_steps) {
+  const int3 z = slot_sizes(P, h);
+  P.task_mode[i] = h->task_mode;
+  P.task_max_steps[i] = max_steps;
+  P.sizes.bots[i] = z.x;
+  P.sizes.pellets[i] = z.y;
+  P.sizes.viruses[i] = z.z;
+}
+
+// Whether slot `slot` (at sl) holds a state this batch may load: in range, saved from this configuration, a task of the batch
 // (the restore below makes the same checks)
 __device__ __forceinline__ bool slot_valid(const SnapParams& P, int32_t slot, const uint8_t* sl) {
   bool valid = slot < P.pool_slots;
@@ -30,7 +51,7 @@ __device__ __forceinline__ bool slot_valid(const SnapParams& P, int32_t slot, co
     const agarcl_snapshot_hdr* h = reinterpret_cast<const agarcl_snapshot_hdr*>(sl);
     valid = h->magic == AGARCL_SNAPSHOT_MAGIC && h->version == AGARCL_SNAPSHOT_VERSION && h->fingerprint == P.fingerprint &&
             h->slot_bytes == P.S.slot_bytes;
-    if (valid && P.task_mode) valid = h->task_mode >= 0 && h->task_mode <= 10 && ((P.task_modes >> h->task_mode) & 1);
+    if (valid && P.task_mode) valid = slot_task_valid(P, h);
   }
   return valid;
 }
@@ -66,10 +87,8 @@ __global__ void __launch_bounds__(kSnapThreads) k_start_states(const __grid_cons
     hdr->seed_hi = (uint32_t)(seed >> 32);
     hdr->rng_cursor = cursor;
     hdr->respawned_lo = 0; hdr->respawned_hi = 0;
-    if (P.task_mode) {  // the game's mode becomes the current one; the step limit belongs to the episode: the pending one
-      P.task_mode[i] = reinterpret_cast<const agarcl_snapshot_hdr*>(sl)->task_mode;
-      P.task_max_steps[i] = P.next_max_steps[i];
-    }
+    if (P.task_mode)  // the game's mode and sizes become the current ones; the step limit belongs to the episode: the pending one
+      take_slot_task(P, reinterpret_cast<const agarcl_snapshot_hdr*>(sl), i, P.next_max_steps[i]);
     P.fresh[i] = 0;
     P.spawn[i] = 0;
     P.result[i] = 1;
@@ -100,15 +119,16 @@ __global__ void __launch_bounds__(kSnapThreads) k_snapshot(const __grid_constant
       if (P.S.obs_bytes) copy_segment(sl + P.S.off_obs, P.obs + (size_t)src * P.S.obs_bytes, P.S.obs_bytes);
     }
     __syncthreads();  // the header goes last; a source out of range leaves magic 0, which a restore rejects
-    if (t == 0) {  // agarcl_snapshot_hdr: magic, version, fingerprint, slot_bytes, source, task (mixed-task batch), zero padding
+    if (t == 0) {  // agarcl_snapshot_hdr: magic, version, fingerprint, slot_bytes, source, task and sizes (mixed-task batch), zero padding
       const uint4 z = make_uint4(0u, 0u, 0u, 0u);
       uint4* hv = reinterpret_cast<uint4*>(sl);
       const bool task = ok && P.task_mode;
       hv[0] = ok ? make_uint4(AGARCL_SNAPSHOT_MAGIC, AGARCL_SNAPSHOT_VERSION, (uint32_t)P.fingerprint, (uint32_t)(P.fingerprint >> 32)) : z;
       hv[1] = ok ? make_uint4((uint32_t)P.S.slot_bytes, (uint32_t)(P.S.slot_bytes >> 32), (uint32_t)(P.instance_base + src),
                               task ? (uint32_t)P.task_mode[src] : 0u) : z;
-      hv[2] = make_uint4(task ? (uint32_t)P.task_max_steps[src] : 0u, 0u, 0u, 0u);
-      hv[3] = z;
+      hv[2] = task ? make_uint4((uint32_t)P.task_max_steps[src], AGARCL_SNAPSHOT_SIZES_MARKER, (uint32_t)P.sizes.bots[src],
+                                (uint32_t)P.sizes.pellets[src]) : z;
+      hv[3] = make_uint4(task ? (uint32_t)P.sizes.viruses[src] : 0u, 0u, 0u, 0u);
     }
     return;
   }
@@ -124,7 +144,7 @@ __global__ void __launch_bounds__(kSnapThreads) k_snapshot(const __grid_constant
     const agarcl_snapshot_hdr* h = reinterpret_cast<const agarcl_snapshot_hdr*>(sl);
     valid = h->magic == AGARCL_SNAPSHOT_MAGIC && h->version == AGARCL_SNAPSHOT_VERSION && h->fingerprint == P.fingerprint &&
             h->slot_bytes == P.S.slot_bytes;
-    if (valid && P.task_mode) valid = h->task_mode >= 0 && h->task_mode <= 10 && ((P.task_modes >> h->task_mode) & 1);
+    if (valid && P.task_mode) valid = slot_task_valid(P, h);
   }
   if (!valid) {  // rejected: the instance is not touched
     if (t == 0) { P.result[i] = 2; P.restored[i] = 0; }
@@ -150,8 +170,7 @@ __global__ void __launch_bounds__(kSnapThreads) k_snapshot(const __grid_constant
     P.seeds[i] = (uint64_t)ih->seed_lo | ((uint64_t)ih->seed_hi << 32);
     if (P.task_mode) {  // the slot's task becomes the current one; the pending task is left alone
       const agarcl_snapshot_hdr* h = reinterpret_cast<const agarcl_snapshot_hdr*>(sl);
-      P.task_mode[i] = h->task_mode;
-      P.task_max_steps[i] = h->task_max_steps;
+      take_slot_task(P, h, i, h->task_max_steps);
     }
     P.fresh[i] = 0;
     P.result[i] = 1;

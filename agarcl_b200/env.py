@@ -405,6 +405,15 @@ class BatchedGridEnvironment(_Base):
         """device views of the current and pending task of every instance (Batch.tasks)"""
         return self._ensure().tasks()
 
+    def set_task_sizes(self, num_bots=None, num_pellets=None, num_viruses=None, stream=0):
+        """the game sizes each instance's next reset plays, at most the constructor's counts; returns the result u8 [N]
+        (Batch.set_task_sizes)"""
+        return self._ensure().set_task_sizes(num_bots, num_pellets, num_viruses, stream)
+
+    def task_sizes(self):
+        """device views of the current and pending game sizes of every instance (Batch.task_sizes)"""
+        return self._ensure().task_sizes()
+
     def bot_actions(self, types, out=None, target=None):
         """(dxdy, act, status) of a built-in bot policy for every agent, on the device (Batch.bot_actions); dxdy and act go
         straight into step()"""

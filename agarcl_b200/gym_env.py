@@ -302,6 +302,15 @@ class BatchedAgarioEnv:
             raise ValueError("set_tasks needs a mixed-task environment (tasks=[...])")
         return self._env.set_tasks(modes, number_steps)
 
+    def set_task_sizes(self, num_bots=None, num_pellets=None, num_viruses=None):
+        """the game sizes every environment plays from its next reset on, each an int32 CUDA tensor of n_envs entries or None
+        (pending values kept), -1 keeping an entry: num_bots (mode 0 only), num_pellets (not the squared-pellet modes 1, 2, 5)
+        and num_viruses.  The constructor's counts are the maxima.  Returns the per-environment result u8 [n_envs]: 0 nothing
+        set, 1 set, 2 rejected (a value above its maximum or below 0, or a bot count the player order does not allow)"""
+        if not self.tasks:
+            raise ValueError("set_task_sizes needs a mixed-task environment (tasks=[...])")
+        return self._env.set_task_sizes(num_bots, num_pellets, num_viruses)
+
     # ---- snapshot pools (Batch.save_states / restore_states): save and restore whole games, episode counters included
     def snapshot_pool(self, slots):
         return self._env.snapshot_pool(slots)

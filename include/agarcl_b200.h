@@ -276,6 +276,44 @@ typedef struct agarcl_tasks {
 } agarcl_tasks;
 int agarcl_batch_set_tasks(agarcl_batch* b, const int32_t* d_mode, const int32_t* d_max_steps, uint8_t** d_result, void* stream);
 int agarcl_batch_tasks(agarcl_batch* b, agarcl_tasks* out);
+/* Game sizes per instance (mixed-task batch): three more task values with the lifecycle of mode / max_steps.
+ *   bots      bot players of a mode-0 episode (modes 1..10 keep their own roster: none, or the one custom bot of 7..10)
+ *   pellets   pellets spawned at the reset and the target of pellet regen (ignored by the squared-pellet modes 1, 2 and 5)
+ *   viruses   viruses spawned at the reset and the target of virus regen (every mode)
+ * cfg.num_bots, num_pellets and num_viruses are the MAXIMA: the layout is sized from them (P, cap_pellets, cap_viruses) as without
+ * sizes, and current and pending sizes start at them, so a batch that never sets sizes plays exactly as before.  An instance with
+ * current (mode, bots, pellets, viruses) is bit-identical to the same instance (seed, global index, actions) of a batch created with
+ * mode_number = mode, num_bots = bots, num_pellets = pellets, num_viruses = viruses and the same cap_viruses.  A mode-0 instance
+ * plays A + bots players; players A + bots .. P-1 are absent (never spawned, respawned, drawn for or ticked).
+ * Allowed bot counts: 0 .. num_bots, every one of them when mode 0 is not in task_modes (the count then means nothing, and num_bots
+ * may exceed the players of the layout); when mode 0 is in task_modes only those whose A + bots players keep the player-order check
+ * above (the batch's order restricted to players < A + bots is the order of a batch of A + bots players alone).  Not every count
+ * passes, even for one agent: with 1 agent and 25 bots the counts 1 .. 12 fail (the unordered_map rehashes between 13 and 26
+ * players), and 0 and 13 .. 25 pass.
+ *   agarcl_batch_set_task_sizes  d_bots, d_pellets, d_viruses: device int32 [N] each, or NULL to keep every pending value; an entry
+ *                                of -1 keeps that value.  Checked on the device; *d_result (may be NULL) receives the library-owned
+ *                                u8 [N] result, overwritten by the next call: 0 nothing set, 1 set, 2 rejected (a value outside
+ *                                [0, maximum] or a bot count that is not allowed: none of that instance's pending sizes is touched).
+ *                                Stream-ordered, no host wait.  AGARCL_ERR_STATE on a batch without task_modes.
+ *   agarcl_batch_task_sizes      the six device pointers; AGARCL_ERR_STATE on a batch without task_modes.
+ * Every reset copies the pending sizes to the current ones together with the mode.  Snapshot slots of a mixed batch carry the
+ * source's current sizes (agarcl_snapshot_hdr.sizes_marker = AGARCL_SNAPSHOT_SIZES_MARKER, task_bots / task_pellets /
+ * task_viruses); a restore or a start-state reset makes them current, and rejects (result 2) a slot whose sizes exceed the
+ * destination's maxima or whose bot count the destination does not allow.  A slot without the marker restores with the maxima.
+ * agarcl_batch_save_env_state writes the instance's current num_bots / num_pellets / num_viruses; agarcl_batch_load_env_state
+ * accepts any within the maxima (and an allowed bot count) and makes them current; the num_bots of a file whose mode_number is not 0
+ * is not checked, and the instance's bot count becomes the maximum. */
+typedef struct agarcl_task_sizes {
+  int32_t* bots;          /* [N] */
+  int32_t* pellets;       /* [N] */
+  int32_t* viruses;       /* [N] */
+  int32_t* next_bots;     /* [N] */
+  int32_t* next_pellets;  /* [N] */
+  int32_t* next_viruses;  /* [N] */
+} agarcl_task_sizes;
+int agarcl_batch_set_task_sizes(agarcl_batch* b, const int32_t* d_bots, const int32_t* d_pellets, const int32_t* d_viruses,
+                                uint8_t** d_result, void* stream);
+int agarcl_batch_task_sizes(agarcl_batch* b, agarcl_task_sizes* out);
 
 /* ---------------------------------------------------- snapshot pools: save and restore game states on the device
  * The batched counterpart of agarcl_batch_save_env_state / load_env_state: chosen instances are copied into slots of a
@@ -330,8 +368,13 @@ typedef struct agarcl_snapshot_hdr { /* 64 B */
   int32_t source;          /* global index (instance_base + i) of the instance saved */
   int32_t task_mode;       /* mixed-task batch (cfg.task_modes != 0): the source's current mode; 0 otherwise */
   int32_t task_max_steps;  /* mixed-task batch: the source's current step limit (-1 default, 0 none); 0 otherwise */
-  uint32_t pad[7];
+  uint32_t sizes_marker;   /* mixed-task batch: AGARCL_SNAPSHOT_SIZES_MARKER when the three sizes below are stored; 0 otherwise */
+  int32_t task_bots;       /* mixed-task batch: the source's current game sizes (agarcl_batch_set_task_sizes); 0 otherwise */
+  int32_t task_pellets;
+  int32_t task_viruses;
+  uint32_t pad[3];
 } agarcl_snapshot_hdr;
+#define AGARCL_SNAPSHOT_SIZES_MARKER 0x5A534741u /* "AGSZ" */
 /* bytes of one snapshot slot of configuration c: a multiple of 128; no device needed */
 int agarcl_snapshot_slot_bytes(const agarcl_cfg* c, int64_t* out);
 /* pool slot d_slot[k] <- instance d_src[k], k < n (device int32 arrays; d_slot NULL = slots 0..n-1); enqueued on stream */
